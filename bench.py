@@ -1,9 +1,11 @@
 #!/usr/bin/env python
-"""bench.py - AO-ADMM outer iterations/s on B200 (metric of BASELINE.json), driver contract in the task prompt.
+"""bench.py - AO-ADMM outer iterations/s on B200 (metric of BASELINE.json).
 
   python bench.py --gpus N --steps K --warmup W            our engine (CUDA, C ABI of include/aoadmm.h)
   python bench.py --impl reference --gpus N --steps K ...  the reference's algorithm on the host cores
                                                            (NumPy/OpenBLAS oracle port: MATLAB cannot run offline)
+  --dump-outputs DIR   after the timed steps, write what the timed run returned as DIR/<name>.npy (float64), so that
+                       two builds can be compared output for output (the inputs are the same from run to run)
 
 A "step" is one outer AO-ADMM iteration (one sweep over all modes: 3 tensor MTTKRPs + 2 matrix products + every
 inner ADMM loop with all tolerances 0, i.e. MaxInnerIters=5 inner iterations per mode group) of the workload below.
@@ -51,6 +53,29 @@ FP64_NOMINAL_TFLOPS = 40.0     # NVIDIA's B200 FP64 / FP64-tensor figure (HGX B2
 # `value` is measured on the reference's own work per step: three independent MTTKRP passes (options.dimtree = 0).
 # The dimension-tree sweep (2 tensor passes per step, results equal to rounding) is reported beside it as `dimtree`.
 DIMTREE = int(os.environ.get('BENCH_DIMTREE', '0'))
+
+
+# --dump-outputs: what a caller of the timed run receives, the state G (cmtf_fun_AOADMM.m:1) and the per-iteration arrays
+# of `out`.  Left out: time_at_it (wall-clock stamps) and func_rel_missing (all NaN without a missing-data mask).
+DUMP_STATE_KEYS = ('fac', 'constraint_fac', 'constraint_dual_fac', 'coupling_fac', 'coupling_dual_fac')
+DUMP_OUT_KEYS = ('func_val_conv', 'func_coupl_conv', 'func_constr_conv', 'func_PAR2_coupl', 'innerIters')
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(path, G, out):
+    """G[key][m] -> <path>/<key>_<m>.npy, out[key] -> <path>/<key>.npy, all float64."""
+    arrays = {}
+    for key in DUMP_STATE_KEYS:
+        for m, a in enumerate(G.get(key) or []):
+            if a is not None:
+                arrays['%s_%d' % (key, m)] = np.asarray(a, dtype=np.float64)
+    for key in DUMP_OUT_KEYS:
+        arrays[key] = np.asarray(out[key], dtype=np.float64)
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, 'outputs of %d bytes exceed the %d-byte dump limit' % (total, DUMP_MAX_BYTES)
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + '.npy'), a)
 
 
 def zero_tol_options(iters):
@@ -208,7 +233,10 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-e2e', action='store_true')
     ap.add_argument('--no-c3-full', action='store_true', help='skip the extra 4096x4096x2048 run of the N >= 2 lines')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the outputs of the last timed step as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     wl = WORKLOADS[args.workload]
     rank = int(os.environ.get('RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
@@ -230,8 +258,10 @@ def main():
         # exactly `steps` timed steps after `warmup` untimed ones; a step of this arm is one outer iteration on the bounded
         # sample of the workload (cpu_baseline.sample), so ms_per_step is the measured time of such a step and `value`
         # is the whole-workload rate it extrapolates to (flop-proportional, factor in `sample_scale`)
-        steps = max(1, args.steps)
-        cb = cpu_baseline_run(wl, steps, args.warmup)
+        steps = args.steps
+        cb, (_, _, _, Go, oo) = cpu_baseline_run(wl, steps, args.warmup, keep=True)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, Go, oo)
         sm = wl['sample']
         scale = (wl['I'] * wl['J'] * wl['K']) / float(sm['I'] * sm['J'] * sm['K'])
         line = {'impl': 'reference', 'metric': 'ao_admm_outer_iters_per_s', 'value': cb['value'], 'unit': 'outer_iters/s',
@@ -318,6 +348,11 @@ def main():
     traj = np.array(warm_out[0]['func_val_conv'])   # objective of the first W iterations from G (device-resident data)
     call_ms = whole_ms[0]
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        G_out = solver.get_state()   # collective: every rank takes part, rank 0 writes
+        if rank == 0:
+            dump_outputs(args.dump_outputs, G_out, out)
+        del G_out
     if world == 1 and (clocks is None or not clocks.get('samples')):
         # the timed region was shorter than the nvidia-smi sampling period: sample the clocks over a repeat of the same
         # steps (not used for timing) so that the record still shows the clocks under this load
