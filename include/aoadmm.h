@@ -30,7 +30,9 @@ extern "C" {
 /* 1: first release; 2: Z.miss masks, device Znorm_const, engine options (dimtree, fuse_inner, graph,
  * mttkrp_precision), out.f_rel_missing; 3: aoadmm_nvecs, aoadmm_object_mttkrp (no struct changed since 2);
  * 4: aoadmm_create_multi / aoadmm_gpu_count / aoadmm_comm_release, communicators cached per process,
- *    aoadmm_out.non_finite_mode appended (a non-finite inner residual no longer aborts the run). */
+ *    aoadmm_out.non_finite_mode appended (a non-finite inner residual no longer aborts the run);
+ *    later additions that leave every v4 struct and entry point unchanged: aoadmm_sparse_object / aoadmm_create_sparse
+ *    (sparse CP objects). */
 #define AOADMM_ABI_VERSION 4
 
 typedef struct aoadmm_handle aoadmm_handle;
@@ -218,6 +220,27 @@ int aoadmm_gpu_count(const aoadmm_handle *h, int32_t *n_gpus);
 int aoadmm_comm_release(void);
 int aoadmm_destroy(aoadmm_handle *h);
 const char *aoadmm_last_error(const aoadmm_handle *h); /* h may be NULL: last creation error */
+
+/* One sparse CP object (Tensor Toolbox sptensor / MATLAB sparse): COO, 0-based. */
+typedef struct {
+  int64_t nnz;
+  const int64_t *subs;   /* nnz x order, column-major: subs[d*nnz + e] = index of nonzero e in mode position d */
+  const double *vals;    /* nnz values */
+} aoadmm_sparse_object;
+
+/* aoadmm_create with per-object sparse data: sparse[p] (n_objects entries) is NULL for a dense object, else the COO
+ * data of CP object p (problem->objects[p].data must then be NULL).  dist: NULL or world_size 1.
+ * Duplicate subscripts are summed (as the sptensor(subs,vals) constructor does); explicit zeros are kept.  The data is
+ * sorted once on the device (one copy per mode); results do not depend on the order of the nonzeros.  A sparse object
+ * always runs the FP64 sparse MTTKRP (options.mttkrp_precision and options.dimtree act on dense objects only);
+ * Znorm_const = NaN is the sum of the squared (merged) values.
+ * Checked before any device is touched: AOADMM_ERR_INVALID_ARG for nnz < 0, nnz > 0 with NULL subs / vals, a subscript
+ * out of range, data and sparse[p] both set, a sparse object with a mode of more than 2^31 - 1 rows;
+ * AOADMM_ERR_UNSUPPORTED for a sparse object with Z.miss, a sparse PARAFAC2 object, world_size > 1.
+ * aoadmm_generate_cp_data, aoadmm_get_object_data and aoadmm_nvecs on a mode of a sparse object return
+ * AOADMM_ERR_UNSUPPORTED; every other entry point works on such a handle. */
+int aoadmm_create_sparse(const aoadmm_problem *problem, const aoadmm_sparse_object *const *sparse,
+                         const aoadmm_dist *dist, aoadmm_handle **out);
 
 /* ---- state in / out (G is both input and output of cmtf_fun_AOADMM.m:1) ------------------- */
 int aoadmm_set_state(aoadmm_handle *h, int32_t field, int32_t index, int32_t slice,

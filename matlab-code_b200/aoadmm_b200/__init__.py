@@ -7,7 +7,8 @@ There is no CPU path: importing this package fails when the library is missing, 
 AoadmmError(NO_DEVICE) when no GPU is present.
 
 Struct conventions (dicts mirroring the MATLAB structs, 1-based labels where they are data):
-  Z : 'object', 'model', 'modes', 'size', 'coupling' {'lin_coupled_modes','coupling_type',
+  Z : 'object' (dense arrays; a CP object may also be a sparse `sptensor` or, 2-way, any SciPy sparse matrix), 'model',
+      'modes', 'size', 'coupling' {'lin_coupled_modes','coupling_type',
       'coupl_trafo_matrices'[,'coupl_trafo_matrices2']}, 'constrained_modes', 'constraints', 'weights',
       'loss_function', optional 'ridge'
   G : 'fac', 'constraint_fac', 'constraint_dual_fac', 'coupling_dual_fac' (per mode), 'coupling_fac' (per coupling)
@@ -20,7 +21,7 @@ import numpy as np
 from . import _capi
 from ._capi import AoadmmError, lib
 
-__all__ = ['cmtf_fun_AOADMM', 'cmtf_AOADMM', 'cmtf_nvecs', 'init_coupled_AOADMM_CMTF', 'Solver', 'AoadmmError', 'mttkrp',
+__all__ = ['cmtf_fun_AOADMM', 'cmtf_AOADMM', 'cmtf_nvecs', 'init_coupled_AOADMM_CMTF', 'Solver', 'AoadmmError', 'sptensor', 'mttkrp',
            'prox', 'chol_solve', 'gram',
            'shard_range', 'device_count', 'nccl_unique_id']
 
@@ -31,6 +32,43 @@ def _dp(a):
 
 def _f64(a):
     return np.asfortranarray(np.asarray(a, dtype=np.float64))
+
+
+class sptensor:
+    """A sparse tensor in coordinate form, the Tensor Toolbox sptensor(subs, vals, sz) with 0-based subscripts: `subs` is
+    nnz x N, `vals` nnz values, `shape` the N extents.  Duplicate subscripts are summed when the object is used."""
+
+    def __init__(self, subs, vals, shape):
+        self.shape = tuple(int(s) for s in shape)
+        self.subs = np.asarray(subs, dtype=np.int64).reshape(-1, len(self.shape))
+        self.vals = np.asarray(vals, dtype=np.float64).reshape(-1)
+        if self.subs.shape[0] != self.vals.size:
+            raise ValueError('sptensor: subs has %d rows but there are %d values' % (self.subs.shape[0], self.vals.size))
+
+    @property
+    def ndim(self):
+        return len(self.shape)
+
+    @property
+    def nnz(self):
+        return self.vals.size
+
+    def full(self):
+        """The dense array (column-major), duplicates summed."""
+        X = np.zeros(self.shape, order='F')
+        np.add.at(X, tuple(self.subs.T), self.vals)
+        return X
+
+
+def as_sparse(X):
+    """`X` as an sptensor when it is sparse (an sptensor, or anything with `tocoo()` such as a SciPy sparse matrix),
+    else None.  Duck typing keeps SciPy an optional dependency."""
+    if isinstance(X, sptensor):
+        return X
+    if hasattr(X, 'tocoo') and not isinstance(X, np.ndarray):
+        c = X.tocoo()
+        return sptensor(np.stack([np.asarray(c.row), np.asarray(c.col)], axis=1), c.data, c.shape)
+    return None
 
 
 def device_count():
@@ -106,6 +144,21 @@ class Solver:
             if Z['loss_function'][p] != 'Frobenius':
                 raise AoadmmError(2, "loss function %r is not supported (Frobenius only)" % (Z['loss_function'][p],))
         miss = Z.get('miss') or [None] * P
+        # sparse objects (aoadmm_create_sparse): the refused combinations raise here, before any device call
+        sparse = [as_sparse(Z['object'][p]) if model[p] == 'CP' else None for p in range(P)]
+        for p in range(P):
+            if model[p] != 'CP' and any(as_sparse(x) is not None for x in Z['object'][p]):
+                raise AoadmmError(2, 'object %d: PARAFAC2 objects with sparse slices are not supported' % (p + 1))
+            if sparse[p] is None:
+                continue
+            if n_gpus > 1 or world_size > 1:
+                raise AoadmmError(2, 'object %d is sparse: sparse objects run on one GPU' % (p + 1))
+            if miss[p] is not None:
+                raise AoadmmError(2, 'object %d is sparse: Z.miss needs a dense object' % (p + 1))
+            want = tuple(int(Z['size'][m - 1]) for m in modes[p])
+            if sparse[p].shape != want:
+                raise AoadmmError(1, 'object %d: sparse shape %s does not match Z.size %s' % (p + 1, sparse[p].shape, want))
+        sp_objs = (C.POINTER(_capi.SparseObject) * P)()
         ranks = self._infer_ranks(Z)
         rows = np.zeros(nb_modes, dtype=np.int64)
         nsl = np.zeros(nb_modes, dtype=np.int32)
@@ -131,7 +184,22 @@ class Solver:
             o.modes = marr.ctypes.data_as(_capi.c_int32_p)
             o.weight = float(Z['weights'][p])
             o.znorm_const = float(Znorm_const[p])
-            if model[p] == 'CP':
+            if model[p] == 'CP' and sparse[p] is not None:
+                full_last = int(Z['size'][modes[p][-1] - 1])
+                self.shards.append((0, full_last))
+                subs = np.asfortranarray(sparse[p].subs)    # column-major: subs[d*nnz + e]
+                vals = np.ascontiguousarray(sparse[p].vals)
+                so = _capi.SparseObject()
+                so.nnz = vals.size
+                so.subs = subs.ctypes.data_as(_capi.c_int64_p)
+                so.vals = _dp(vals)
+                self._keep += [subs, vals, so]
+                sp_objs[p] = C.pointer(so)
+                o.data = None
+                o.shard_offset, o.shard_extent = 0, full_last
+                o.slices, o.n_slices = None, 0
+                o.miss, o.miss_slices = None, None
+            elif model[p] == 'CP':
                 X = Z['object'][p]
                 full_last = int(Z['size'][modes[p][-1] - 1])
                 if shard is not None and shard[p] is not None:
@@ -263,7 +331,11 @@ class Solver:
         else:
             if devices is not None:
                 dist.device = int(list(devices)[0])
-            _capi.check(lib.aoadmm_create(C.byref(pb), C.byref(dist), C.byref(self._h)))
+            if any(sp is not None for sp in sparse):
+                self._keep.append(sp_objs)
+                _capi.check(lib.aoadmm_create_sparse(C.byref(pb), sp_objs, C.byref(dist), C.byref(self._h)))
+            else:
+                _capi.check(lib.aoadmm_create(C.byref(pb), C.byref(dist), C.byref(self._h)))
         self._keep_problem = pb
 
     # ------------------------------------------------------------------------------------------
@@ -554,7 +626,9 @@ def cmtf_AOADMM(Z, init, alg_options, init_options=None, **dist):
     zn = []
     miss = Z.get('miss') or [None] * P
     for p in range(P):                                                     # :124-156 (with Z.miss: observed entries only)
-        if Z['model'][p] == 'CP':
+        if Z['model'][p] == 'CP' and as_sparse(Z['object'][p]) is not None:
+            zn.append(float('nan'))                                        # computed on the device from the nonzeros
+        elif Z['model'][p] == 'CP':
             X = np.asarray(Z['object'][p])
             if miss[p] is not None:
                 X = X * (np.asarray(miss[p]) != 0)
@@ -612,9 +686,18 @@ def gram(F, device=0):
 
 
 # ---- initialisation front end (the caller side of the boundary, SURVEY 8f-4) -------------------
+def _refuse_sparse_nvecs(Z, mode_ids):
+    """nvecs (cmtf_nvecs.m:6,13 refuses sparse input too) needs a dense unfolding of the first object holding the mode."""
+    for n in mode_ids:
+        p = [q for q in range(len(Z['modes'])) if n in list(Z['modes'][q])][0]
+        if Z['model'][p] == 'CP' and as_sparse(Z['object'][p]) is not None:
+            raise AoadmmError(2, 'nvecs: mode %d belongs to sparse object %d (initialise it from a distribution)' % (n, p + 1))
+
+
 def cmtf_nvecs(Z, n, r, solver=None, **dist):
     """U = cmtf_nvecs(Z,n,r)  (cmtf_nvecs.m:33-58): r leading eigenvectors of X_(n) X_(n)', computed on the device from
     the tensor resident in `solver` (or in a temporary handle), so a large tensor never has to be unfolded on the host."""
+    _refuse_sparse_nvecs(Z, [n])
     if solver is not None:
         return solver.nvecs(n, r)
     P = len(Z['object'])
@@ -652,6 +735,8 @@ def init_coupled_AOADMM_CMTF(Z, init_options, rng=None, Delta=None, **dist):
         return int(sz[n - 1])
 
     solver = None
+    if use_nvecs:
+        _refuse_sparse_nvecs(Z, [n for p in range(P) for n in modes[p]])
     try:
         if use_nvecs:
             solver = Solver(dict(Z, rank=[len(l) for l in lambdas]), [float('nan')] * P, **dist)

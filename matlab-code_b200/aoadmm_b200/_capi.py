@@ -61,6 +61,10 @@ class Problem(C.Structure):
                 ('constrained_modes', c_int32_p), ('constraints', C.POINTER(Constraint)), ('ridge', c_double_p)]
 
 
+class SparseObject(C.Structure):
+    _fields_ = [('nnz', C.c_int64), ('subs', c_int64_p), ('vals', c_double_p)]
+
+
 class Dist(C.Structure):
     _fields_ = [('rank', C.c_int32), ('world_size', C.c_int32), ('device', C.c_int32),
                 ('nccl_unique_id', C.c_uint8 * 128)]
@@ -91,12 +95,14 @@ EXPORTS = ['aoadmm_abi_version', 'aoadmm_device_count', 'aoadmm_nccl_unique_id',
            'aoadmm_last_error', 'aoadmm_set_state', 'aoadmm_get_state', 'aoadmm_run', 'aoadmm_mttkrp', 'aoadmm_prox',
            'aoadmm_chol_solve', 'aoadmm_gram', 'aoadmm_generate_cp_data', 'aoadmm_time_mttkrp', 'aoadmm_launch_count',
            'aoadmm_phase_ms', 'aoadmm_last_run_ms', 'aoadmm_get_object_data', 'aoadmm_last_loop_ms', 'aoadmm_object_mttkrp', 'aoadmm_nvecs',
-           'aoadmm_create_multi', 'aoadmm_gpu_count', 'aoadmm_comm_release']
+           'aoadmm_create_multi', 'aoadmm_gpu_count', 'aoadmm_comm_release', 'aoadmm_create_sparse']
 
 lib.aoadmm_abi_version.restype = C.c_int
 lib.aoadmm_device_count.argtypes = [C.POINTER(C.c_int)]
 lib.aoadmm_nccl_unique_id.argtypes = [C.POINTER(C.c_uint8)]
 lib.aoadmm_create.argtypes = [C.POINTER(Problem), C.POINTER(Dist), C.POINTER(HandleP)]
+lib.aoadmm_create_sparse.argtypes = [C.POINTER(Problem), C.POINTER(C.POINTER(SparseObject)), C.POINTER(Dist),
+                                     C.POINTER(HandleP)]
 lib.aoadmm_create_multi.argtypes = [C.POINTER(Problem), C.c_int32, c_int32_p, C.POINTER(HandleP)]
 lib.aoadmm_gpu_count.argtypes = [HandleP, c_int32_p]
 lib.aoadmm_comm_release.argtypes = []

@@ -458,18 +458,20 @@ struct Engine::ObjTerms {
 // ---------------------------------------------------------------------------------------------------
 // construction
 // ---------------------------------------------------------------------------------------------------
-Engine::Engine(const aoadmm_problem* prob, const aoadmm_dist* dist, void* shared_comm) {
+Engine::Engine(const aoadmm_problem* prob, const aoadmm_dist* dist, void* shared_comm,
+               const aoadmm_sparse_object* const* sparse) {
   // A constructor that throws never runs the destructor: everything acquired so far (up to the whole tensor in HBM,
   // streams, events, pinned buffers) is released here before the error leaves.
   try {
-    construct(prob, dist, shared_comm);
+    construct(prob, dist, shared_comm, sparse);
   } catch (...) {
     release();
     throw;
   }
 }
 
-void Engine::construct(const aoadmm_problem* prob, const aoadmm_dist* dist, void* shared_comm) {
+void Engine::construct(const aoadmm_problem* prob, const aoadmm_dist* dist, void* shared_comm,
+                       const aoadmm_sparse_object* const* sparse) {
   if (prob == nullptr) throw CudaError(1, "problem is NULL");
   if (dist != nullptr) {
     rank_ = dist->rank;
@@ -557,6 +559,15 @@ void Engine::construct(const aoadmm_problem* prob, const aoadmm_dist* dist, void
       o.shard_extent = o.last_full;
     }
     o.dims.back() = o.shard_extent;
+    if (sparse != nullptr && sparse[p] != nullptr) {
+      // sparse CP object (aoadmm_create_sparse): one GPU, no mask; sorted device copies instead of a dense array
+      if (world_ > 1 || src.miss != nullptr || src.data != nullptr) throw CudaError(2, "sparse object: unsupported combination");
+      const aoadmm_sparse_object& so = *sparse[p];
+      std::vector<long long> dl(o.dims.begin(), o.dims.end());
+      o.sp = new SparseTensor();
+      sparse_build(*o.sp, o.order, dl.data(), R, so.nnz, reinterpret_cast<const long long*>(so.subs), so.vals, st_);
+      continue;
+    }
     o.ld0 = round_up(o.dims[0], 2);
     size_t slab = 1;
     for (int d = 1; d < o.order; ++d) slab *= (size_t)o.dims[d];
@@ -709,13 +720,14 @@ void Engine::construct(const aoadmm_problem* prob, const aoadmm_dist* dist, void
   for (auto& s : par2_) ws_bytes = std::max(ws_bytes, mttkrp_workspace_bytes(s.view, s.R));
   for (auto& o : objects_) {
     if (o.model == AOADMM_MODEL_PAR2) continue;
+    cp0 = std::max(cp0, (size_t)mode(o.modes[0]).rows * mode(o.modes[0]).R);
+    if (o.sp != nullptr) continue;   // sparse objects own their scratch (sparse_build)
     build_views(o);
     for (auto& v : o.views) {
       ws_bytes = std::max(ws_bytes, mttkrp_workspace_bytes(v.t, mode(o.modes[0]).R));
       if (v.f0_modes.size() >= 2) kr_doubles = std::max(kr_doubles, (size_t)v.f0_rows * mode(o.modes[0]).R);
       if (v.f1_modes.size() >= 2) kr_doubles = std::max(kr_doubles, (size_t)v.f1_rows * mode(o.modes[0]).R);
     }
-    cp0 = std::max(cp0, (size_t)mode(o.modes[0]).rows * mode(o.modes[0]).R);
   }
   mws_.ws_bytes = ws_bytes;
   AO_CUDA(cudaMalloc(&mws_.ws, ws_bytes));
@@ -737,6 +749,9 @@ void Engine::construct(const aoadmm_problem* prob, const aoadmm_dist* dist, void
       if (s.sharded) {   // sum of the ranks' slices (the communicator exists since the top of the constructor)
         allreduce(res, 1);
       }
+    } else if (o.sp != nullptr) {
+      launches_ += sparse_norm2(*o.sp, st_);
+      res = o.sp->norm_out;
     } else {
       size_t slab = 1;
       for (int d = 1; d < o.order; ++d) slab *= (size_t)o.dims[d];
@@ -831,6 +846,11 @@ void Engine::release() {
   }
   modes_.clear();
   for (auto& o : objects_) {
+    if (o.sp != nullptr) {
+      sparse_free(*o.sp);
+      delete o.sp;
+      o.sp = nullptr;
+    }
     dfree(o.data);
     dfree(o.dataT);
     dfree(o.Tbuf);
@@ -1060,7 +1080,25 @@ void Engine::allreduce(double* buf, size_t count) {
   AO_NCCL(nccl_->AllReduce(buf, buf, count, ncclDouble, ncclSum, static_cast<ncclComm_t>(comm_), st_));
 }
 
+// sparse objects: always FP64, no dimension tree (options.mttkrp_precision / dimtree apply to dense objects only)
+int Engine::sparse_mttkrp_of(ObjectState& o, int pos, double scale, double* out, int64_t ldout) {
+  const double* fac[8];
+  long long ld[8];
+  for (int d = 0; d < o.order; ++d) {
+    const ModeState& mm = mode(o.modes[d]);
+    fac[d] = mm.fac.p;
+    ld[d] = mm.rows;
+  }
+  return sparse_mttkrp(*o.sp, pos, fac, ld, scale, out, ldout, st_);
+}
+
 void Engine::compute_mttkrp(ObjectState& o, int pos, double scale, double* out, int64_t ldout) {
+  if (o.sp != nullptr) {
+    phase_begin(o.order >= 3 ? 0 : 1);
+    launches_ += sparse_mttkrp_of(o, pos, scale, out, ldout);
+    phase_end();
+    return;
+  }
   View3& v = o.views[pos];
   const int R = mode(o.modes[0]).R;
   const bool last_sharded = o.sharded && o.order >= 3 && pos == o.order - 1;
@@ -2201,7 +2239,7 @@ void Engine::run(const aoadmm_options* opt, aoadmm_out* out) {
     for (auto& o : objects_) {
       double e = 1.0;
       for (auto d : o.dims) e *= (double)d;
-      elems += e;
+      elems += o.sp != nullptr ? (double)o.sp->nnz : e;   // sparse objects: the work scales with nnz
     }
     graph_ok = (opt_.graph > 0) || elems <= 33554432.0;
   }
@@ -2312,6 +2350,7 @@ void Engine::generate_cp_data(int object, const double* const* factors, double n
   if (object < 1 || object > n_objects_) throw CudaError(1, "generate_cp_data: object out of range");
   ObjectState& o = objects_[object - 1];
   if (o.model != AOADMM_MODEL_CP) throw CudaError(1, "generate_cp_data: not a CP object");
+  if (o.sp != nullptr) throw CudaError(2, "generate_cp_data: object " + std::to_string(object) + " is sparse (dense objects only)");
   const int R = mode(o.modes[0]).R;
   GenArgs g{};
   g.order = o.order;
@@ -2364,6 +2403,7 @@ void Engine::object_slab(int object, int64_t* offset_elems, int64_t* n_elems) co
   if (object < 1 || object > n_objects_) throw CudaError(1, "object out of range");
   const ObjectState& o = objects_[object - 1];
   if (o.model != AOADMM_MODEL_CP) throw CudaError(1, "not a CP object");
+  if (o.sp != nullptr) throw CudaError(2, "get_object_data: object " + std::to_string(object) + " is sparse (dense objects only)");
   int64_t lead = 1;
   for (int d = 0; d + 1 < o.order; ++d) lead *= o.dims[d];
   *offset_elems = lead * o.shard_offset;
@@ -2375,6 +2415,7 @@ void Engine::object_to_host(int object, double* out, int64_t n_elements) {
   if (object < 1 || object > n_objects_) throw CudaError(1, "get_object_data: object out of range");
   ObjectState& o = objects_[object - 1];
   if (o.model != AOADMM_MODEL_CP) throw CudaError(1, "get_object_data: not a CP object");
+  if (o.sp != nullptr) throw CudaError(2, "get_object_data: object " + std::to_string(object) + " is sparse (dense objects only)");
   size_t slab = 1;
   for (int d = 1; d < o.order; ++d) slab *= (size_t)o.dims[d];
   if ((int64_t)((size_t)o.dims[0] * slab) != n_elements) throw CudaError(1, "get_object_data: size mismatch");
@@ -2399,6 +2440,8 @@ void Engine::nvecs_to_host(int mode_id, int slice, int r, double* out, int64_t r
   ObjectState& o = objects_[p];
   UnfoldSpec s;
   bool reduce_over_ranks = false, skip_local_gram = false;
+  if (o.sp != nullptr)
+    throw CudaError(2, "nvecs: mode " + std::to_string(mode_id) + " belongs to a sparse object (initialise it from a distribution)");
   if (o.model == AOADMM_MODEL_CP) {
     if (slice != 0) throw CudaError(1, "nvecs: slice given for a CP mode");
     if (o.sharded && pos == o.order - 1) {
@@ -2625,10 +2668,24 @@ float Engine::time_mttkrp(int object, int pos, int reps) {
   if (o.model != AOADMM_MODEL_CP) throw CudaError(1, "time_mttkrp: not a CP object");
   if (pos < 1 || pos > o.order) throw CudaError(1, "time_mttkrp: position out of range");
   ModeState& m = mode(o.modes[pos - 1]);
+  cudaEvent_t a, b;
+  if (o.sp != nullptr) {   // the whole sparse MTTKRP: factor transposes, unit pass, fix-up, output transpose
+    AO_CUDA(cudaEventCreate(&a));
+    AO_CUDA(cudaEventCreate(&b));
+    launches_ += sparse_mttkrp_of(o, pos - 1, 1.0, m.Alast.p, m.rows);  // warm-up
+    AO_CUDA(cudaEventRecord(a, st_));
+    for (int r = 0; r < reps; ++r) launches_ += sparse_mttkrp_of(o, pos - 1, 1.0, m.Alast.p, m.rows);
+    AO_CUDA(cudaEventRecord(b, st_));
+    AO_CUDA(cudaEventSynchronize(b));
+    float ms = 0.f;
+    AO_CUDA(cudaEventElapsedTime(&ms, a, b));
+    cudaEventDestroy(a);
+    cudaEventDestroy(b);
+    return ms / (float)std::max(reps, 1);
+  }
   View3& v = o.views[pos - 1];
   pack_operand(v, 0);
   pack_operand(v, 1);
-  cudaEvent_t a, b;
   AO_CUDA(cudaEventCreate(&a));
   AO_CUDA(cudaEventCreate(&b));
   const int R = m.R;

@@ -13,6 +13,7 @@
 #include "nvecs.cuh"
 #include "par2.cuh"
 #include "smallops.cuh"
+#include "sparse.cuh"
 
 namespace aoadmm {
 
@@ -168,13 +169,16 @@ struct ObjectState {
   double* em_fkT = nullptr;   // masked objects of order >= 3: transposed third factor for the pipelined EM kernel
   double* Tbuf = nullptr;     // dimension tree: T(j,k,r) = sum_i X(i,j,k) F1(i,r), emitted by the mode-2 MTTKRP
   uint64_t T_version = 0;     // version of the mode-1 factor T was computed from (0 = invalid)
+  SparseTensor* sp = nullptr; // sparse (COO) object: sorted device copies (sparse.cuh); data, views stay empty
 };
 
 class Engine {
  public:
   // shared_comm: communicator of this rank created by the caller (single-process device group), else nullptr and the
-  // communicator of dist->nccl_unique_id is taken from the process-wide cache
-  Engine(const aoadmm_problem* prob, const aoadmm_dist* dist, void* shared_comm = nullptr);
+  // communicator of dist->nccl_unique_id is taken from the process-wide cache.  sparse: nullptr, or n_objects entries
+  // (nullptr for a dense object) with the COO data of sparse CP objects (aoadmm_create_sparse, validated by the caller)
+  Engine(const aoadmm_problem* prob, const aoadmm_dist* dist, void* shared_comm = nullptr,
+         const aoadmm_sparse_object* const* sparse = nullptr);
   ~Engine();
   Engine(const Engine&) = delete;
   Engine& operator=(const Engine&) = delete;
@@ -209,7 +213,9 @@ class Engine {
 
  private:
   // setup
-  void construct(const aoadmm_problem* prob, const aoadmm_dist* dist, void* shared_comm);
+  void construct(const aoadmm_problem* prob, const aoadmm_dist* dist, void* shared_comm,
+                 const aoadmm_sparse_object* const* sparse);
+  int sparse_mttkrp_of(ObjectState& o, int pos, double scale, double* out, int64_t ldout);
   void release();
   void build_views(ObjectState& o);
   void refresh_transposed(ObjectState& o);

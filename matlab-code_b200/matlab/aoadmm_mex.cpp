@@ -11,6 +11,10 @@
 // Engine knobs read from options (all optional): b200_gpus (number of B200s this MATLAB session drives through
 // aoadmm_create_multi, default 1), b200_dimtree, b200_mttkrp_precision, b200_fuse_inner, b200_graph.
 //
+// Sparse CP objects arrive as struct('subs',S,'vals',V,'size',sz) (cmtf_fun_AOADMM.m unwrap_data: sptensor or a MATLAB
+// sparse matrix through find); the 1-based double subscripts become 0-based int64 and the handle is created with
+// aoadmm_create_sparse (one GPU, no Z.miss, CP only: anything else raises aoadmm:unsupported).
+//
 // Error handling: mexErrMsgIdAndTxt leaves mexFunction with a longjmp that runs no C++ destructor, so nothing in
 // here calls it directly - failures travel as a C++ exception (MexError) to the bottom of mexFunction, where every
 // local (mask byte vectors, the engine handle, property copies) has already been destroyed.
@@ -119,6 +123,34 @@ std::vector<uint8_t> mask_bytes(const mxArray* m, size_t expected, int p, Proper
   return out;
 }
 
+// a sparse object as cmtf_fun_AOADMM.m's unwrap_data hands it over: struct('subs',S,'vals',V,'size',sz) with S the
+// nnz x N matrix of 1-based subscripts (Tensor Toolbox sptensor .subs, or [i j] from find() for a MATLAB sparse matrix)
+bool is_coo_struct(const mxArray* a) {
+  return a != nullptr && mxIsStruct(a) && mxGetField(a, 0, "subs") != nullptr && mxGetField(a, 0, "vals") != nullptr;
+}
+
+// subs (1-based doubles, nnz x order) -> 0-based int64, column-major, with an integer and range check per entry
+void coo_subs(const mxArray* a, int p, int order, const std::vector<int64_t>& rows, std::vector<int64_t>& subs, int64_t* nnz) {
+  const mxArray* S = mxGetField(a, 0, "subs");
+  const mxArray* V = mxGetField(a, 0, "vals");
+  const std::string who = "Z.object{" + std::to_string(p + 1) + "} (sparse): ";
+  if (!mxIsDouble(S) || !mxIsDouble(V)) fail("aoadmm:invalidArg", who + "subs and vals must be double");
+  const size_t n = mxGetNumberOfElements(V);
+  if (n > 0 && (mxGetM(S) != n || (int)mxGetN(S) != order))
+    fail("aoadmm:invalidArg", who + "subs must be nnz x " + std::to_string(order) + " with one row per value");
+  const double* s = n > 0 ? mxGetPr(S) : nullptr;
+  subs.resize(n * (size_t)order);
+  for (int d = 0; d < order; ++d)
+    for (size_t e = 0; e < n; ++e) {
+      const double v = s[(size_t)d * n + e];
+      if (!(v >= 1.0 && v <= (double)rows[d]) || v != (double)(int64_t)v)
+        fail("aoadmm:invalidArg", who + "subscript " + std::to_string(v) + " in column " + std::to_string(d + 1) +
+                                      " is not an integer in 1.." + std::to_string(rows[d]));
+      subs[(size_t)d * n + e] = (int64_t)v - 1;
+    }
+  *nnz = (int64_t)n;
+}
+
 int constraint_kind(const std::string& n) {  // constraints_to_prox.m:13-91
   static const struct { const char* name; int kind; } table[] = {
       {"non-negativity", AOADMM_CON_NONNEG}, {"box", AOADMM_CON_BOX}, {"simplex column-wise", AOADMM_CON_SIMPLEX_COL},
@@ -180,6 +212,10 @@ void solve(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
   const int nb_modes = (int)mxGetNumberOfElements(size_c);
   const mxArray* miss = field(Z, "miss", false);
   std::vector<std::vector<uint8_t>> miss_cp(P);
+  std::vector<std::vector<int64_t>> sp_subs(P);
+  std::vector<aoadmm_sparse_object> sp_obj(P);
+  std::vector<const aoadmm_sparse_object*> sp_ptr(P, nullptr);
+  bool any_sparse = false;
   std::vector<std::vector<std::vector<uint8_t>>> miss_par2(P);
   std::vector<std::vector<const uint8_t*>> miss_par2_ptr(P);
   for (int p = 0; p < P; ++p)
@@ -231,9 +267,23 @@ void solve(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
     if (par2) {
       const int K = (int)mxGetNumberOfElements(obj);
       obj_slices[p].resize(K);
-      for (int k = 0; k < K; ++k) obj_slices[p][k] = mxGetPr(dense_data(mxGetCell(obj, k), pc));
+      for (int k = 0; k < K; ++k) {
+        if (is_coo_struct(mxGetCell(obj, k))) fail("aoadmm:unsupported", "PARAFAC2 objects with sparse slices are not supported");
+        obj_slices[p][k] = mxGetPr(dense_data(mxGetCell(obj, k), pc));
+      }
       o.slices = obj_slices[p].data();
       o.n_slices = K;
+    } else if (is_coo_struct(obj)) {   // sparse object -> aoadmm_create_sparse
+      std::vector<int64_t> rows(order);
+      for (int d = 0; d < order; ++d) rows[d] = mode_rows[obj_modes[p][d] - 1];
+      coo_subs(obj, p, order, rows, sp_subs[p], &sp_obj[p].nnz);
+      sp_obj[p].subs = sp_subs[p].data();
+      sp_obj[p].vals = sp_obj[p].nnz > 0 ? mxGetPr(mxGetField(obj, 0, "vals")) : nullptr;
+      sp_ptr[p] = &sp_obj[p];
+      any_sparse = true;
+      o.data = nullptr;
+      o.shard_offset = 0;
+      o.shard_extent = rows[order - 1];
     } else {
       const mxArray* dd = dense_data(obj, pc);
       size_t expect = 1;
@@ -244,6 +294,8 @@ void solve(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
       o.shard_extent = mode_rows[obj_modes[p][order - 1] - 1];
     }
     const mxArray* mp = (miss != nullptr && mxIsCell(miss) && p < (int)mxGetNumberOfElements(miss)) ? mxGetCell(miss, p) : nullptr;
+    if (mp != nullptr && !mxIsEmpty(mp) && sp_ptr[p] != nullptr)
+      fail("aoadmm:unsupported", "Z.miss{" + std::to_string(p + 1) + "} on a sparse object: missing data needs a dense object");
     if (mp != nullptr && !mxIsEmpty(mp)) {  // EM imputation of the entries with Z.miss == 0 (cmtf_fun_AOADMM.m:408-441)
       if (par2) {
         const int K = o.n_slices;
@@ -360,8 +412,12 @@ void solve(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
   // one MATLAB session drives options.b200_gpus devices (default 1): the library cuts the mode-3 slabs itself
   const int n_gpus = (int)opt_scalar(opt, "b200_gpus", 1.0);
   if (n_gpus < 1) fail("aoadmm:invalidArg", "options.b200_gpus must be >= 1");
+  if (any_sparse && n_gpus > 1) fail("aoadmm:unsupported", "sparse objects run on one GPU (options.b200_gpus must be 1)");
   HandleGuard guard;
-  check(n_gpus > 1 ? aoadmm_create_multi(&pb, n_gpus, nullptr, &guard.h) : aoadmm_create(&pb, nullptr, &guard.h), nullptr);
+  if (any_sparse)
+    check(aoadmm_create_sparse(&pb, sp_ptr.data(), nullptr, &guard.h), nullptr);
+  else
+    check(n_gpus > 1 ? aoadmm_create_multi(&pb, n_gpus, nullptr, &guard.h) : aoadmm_create(&pb, nullptr, &guard.h), nullptr);
   aoadmm_handle* h = guard.h;
 
   // ---- state in ------------------------------------------------------------------------------

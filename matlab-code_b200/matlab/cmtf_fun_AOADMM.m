@@ -46,7 +46,11 @@ function X = unwrap_data(X)
     if iscell(X)
         for k = 1:numel(X), X{k} = unwrap_data(X{k}); end
     elseif isa(X,'sptensor')
-        X = double(full(X));
+        % sparse objects stay sparse: the gateway hands them to aoadmm_create_sparse (1-based subscripts)
+        X = struct('subs',double(X.subs),'vals',double(X.vals),'size',X.size);
+    elseif issparse(X)
+        [i,j,v] = find(X);
+        X = struct('subs',[i j],'vals',full(v),'size',size(X));
     elseif isa(X,'tensor')
         X = X.data;
     end
