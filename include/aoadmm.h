@@ -32,7 +32,7 @@ extern "C" {
  * 4: aoadmm_create_multi / aoadmm_gpu_count / aoadmm_comm_release, communicators cached per process,
  *    aoadmm_out.non_finite_mode appended (a non-finite inner residual no longer aborts the run);
  *    later additions that leave every v4 struct and entry point unchanged: aoadmm_sparse_object / aoadmm_create_sparse
- *    (sparse CP objects). */
+ *    (sparse CP objects), aoadmm_create_sparse_masked (sparse Z.miss masks on sparse objects). */
 #define AOADMM_ABI_VERSION 4
 
 typedef struct aoadmm_handle aoadmm_handle;
@@ -241,6 +241,21 @@ typedef struct {
  * AOADMM_ERR_UNSUPPORTED; every other entry point works on such a handle. */
 int aoadmm_create_sparse(const aoadmm_problem *problem, const aoadmm_sparse_object *const *sparse,
                          const aoadmm_dist *dist, aoadmm_handle **out);
+
+/* aoadmm_create_sparse with sparse missing-data masks (Z.miss{p} given as an sptensor / MATLAB sparse matrix): masks is
+ * NULL (= aoadmm_create_sparse) or n_objects entries; masks[p] may only be set where sparse[p] is.  A mask entry is
+ * observed when its merged value (duplicates summed) is nonzero, and the observed entries must be exactly the stored
+ * entries of the object (explicit zeros included): unstored entries are unobserved, not zero.  The run then equals the
+ * dense EM path (cmtf_fun_AOADMM.m:408-441) on full(X) with the dense mask of that pattern: the unobserved entries start
+ * at 0, the masked objective and f_rel_missing / func_rel_missing and its stopping rule (:457-459) are the same, and
+ * nothing of size prod(size) is formed (memory grows by about 24 + 4*(order-1) bytes per nonzero plus a few
+ * factor-sized buffers).  A second aoadmm_run continues from the last imputation.  aoadmm_object_mttkrp and
+ * aoadmm_time_mttkrp act on the stored values, not on the imputed tensor.
+ * Checked before any device is touched: AOADMM_ERR_INVALID_ARG for a malformed mask (as for sparse[p]), a mask on a
+ * dense object, a mask together with a dense objects[p].miss.  After the device sort: AOADMM_ERR_UNSUPPORTED when the
+ * observed pattern differs from the stored one (the message names the object). */
+int aoadmm_create_sparse_masked(const aoadmm_problem *problem, const aoadmm_sparse_object *const *sparse,
+                                const aoadmm_sparse_object *const *masks, const aoadmm_dist *dist, aoadmm_handle **out);
 
 /* ---- state in / out (G is both input and output of cmtf_fun_AOADMM.m:1) ------------------- */
 int aoadmm_set_state(aoadmm_handle *h, int32_t field, int32_t index, int32_t slice,

@@ -10,7 +10,8 @@ Struct conventions (dicts mirroring the MATLAB structs, 1-based labels where the
   Z : 'object' (dense arrays; a CP object may also be a sparse `sptensor` or, 2-way, any SciPy sparse matrix), 'model',
       'modes', 'size', 'coupling' {'lin_coupled_modes','coupling_type',
       'coupl_trafo_matrices'[,'coupl_trafo_matrices2']}, 'constrained_modes', 'constraints', 'weights',
-      'loss_function', optional 'ridge'
+      'loss_function', optional 'ridge', optional 'miss' (Z.miss: dense 0/1 arrays; for a sparse object a sparse mask
+      whose nonzeros are exactly its stored entries, the unstored entries being unobserved)
   G : 'fac', 'constraint_fac', 'constraint_dual_fac', 'coupling_dual_fac' (per mode), 'coupling_fac' (per coupling)
   options : fields of example_script6...m:120-132
 """
@@ -146,6 +147,12 @@ class Solver:
         miss = Z.get('miss') or [None] * P
         # sparse objects (aoadmm_create_sparse): the refused combinations raise here, before any device call
         sparse = [as_sparse(Z['object'][p]) if model[p] == 'CP' else None for p in range(P)]
+        # sparse Z.miss masks (aoadmm_create_sparse_masked): only on sparse objects
+        smask = [as_sparse(miss[p]) if model[p] == 'CP' and miss[p] is not None else None for p in range(P)]
+        for p in range(P):
+            if smask[p] is not None and sparse[p] is None:
+                raise AoadmmError(1, 'Z.miss{%d} is sparse but Z.object{%d} is dense (a dense object takes a dense mask)'
+                                  % (p + 1, p + 1))
         for p in range(P):
             if model[p] != 'CP' and any(as_sparse(x) is not None for x in Z['object'][p]):
                 raise AoadmmError(2, 'object %d: PARAFAC2 objects with sparse slices are not supported' % (p + 1))
@@ -153,12 +160,17 @@ class Solver:
                 continue
             if n_gpus > 1 or world_size > 1:
                 raise AoadmmError(2, 'object %d is sparse: sparse objects run on one GPU' % (p + 1))
-            if miss[p] is not None:
-                raise AoadmmError(2, 'object %d is sparse: Z.miss needs a dense object' % (p + 1))
+            if miss[p] is not None and smask[p] is None:
+                raise AoadmmError(2, 'object %d is sparse: a dense Z.miss needs a dense object (a sparse object takes a '
+                                     'sparse mask of its stored entries)' % (p + 1))
             want = tuple(int(Z['size'][m - 1]) for m in modes[p])
             if sparse[p].shape != want:
                 raise AoadmmError(1, 'object %d: sparse shape %s does not match Z.size %s' % (p + 1, sparse[p].shape, want))
+            if smask[p] is not None and smask[p].shape != want:
+                raise AoadmmError(1, 'Z.miss{%d}: sparse mask shape %s does not match Z.object{%d} %s'
+                                  % (p + 1, smask[p].shape, p + 1, want))
         sp_objs = (C.POINTER(_capi.SparseObject) * P)()
+        sp_masks = (C.POINTER(_capi.SparseObject) * P)()
         ranks = self._infer_ranks(Z)
         rows = np.zeros(nb_modes, dtype=np.int64)
         nsl = np.zeros(nb_modes, dtype=np.int32)
@@ -195,6 +207,15 @@ class Solver:
                 so.vals = _dp(vals)
                 self._keep += [subs, vals, so]
                 sp_objs[p] = C.pointer(so)
+                if smask[p] is not None:
+                    msubs = np.asfortranarray(smask[p].subs)
+                    mvals = np.ascontiguousarray(smask[p].vals)
+                    mo = _capi.SparseObject()
+                    mo.nnz = mvals.size
+                    mo.subs = msubs.ctypes.data_as(_capi.c_int64_p)
+                    mo.vals = _dp(mvals)
+                    self._keep += [msubs, mvals, mo]
+                    sp_masks[p] = C.pointer(mo)
                 o.data = None
                 o.shard_offset, o.shard_extent = 0, full_last
                 o.slices, o.n_slices = None, 0
@@ -331,7 +352,11 @@ class Solver:
         else:
             if devices is not None:
                 dist.device = int(list(devices)[0])
-            if any(sp is not None for sp in sparse):
+            if any(m is not None for m in smask):
+                self._keep += [sp_objs, sp_masks]
+                _capi.check(lib.aoadmm_create_sparse_masked(C.byref(pb), sp_objs, sp_masks, C.byref(dist),
+                                                            C.byref(self._h)))
+            elif any(sp is not None for sp in sparse):
                 self._keep.append(sp_objs)
                 _capi.check(lib.aoadmm_create_sparse(C.byref(pb), sp_objs, C.byref(dist), C.byref(self._h)))
             else:

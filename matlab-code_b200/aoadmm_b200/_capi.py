@@ -95,7 +95,8 @@ EXPORTS = ['aoadmm_abi_version', 'aoadmm_device_count', 'aoadmm_nccl_unique_id',
            'aoadmm_last_error', 'aoadmm_set_state', 'aoadmm_get_state', 'aoadmm_run', 'aoadmm_mttkrp', 'aoadmm_prox',
            'aoadmm_chol_solve', 'aoadmm_gram', 'aoadmm_generate_cp_data', 'aoadmm_time_mttkrp', 'aoadmm_launch_count',
            'aoadmm_phase_ms', 'aoadmm_last_run_ms', 'aoadmm_get_object_data', 'aoadmm_last_loop_ms', 'aoadmm_object_mttkrp', 'aoadmm_nvecs',
-           'aoadmm_create_multi', 'aoadmm_gpu_count', 'aoadmm_comm_release', 'aoadmm_create_sparse']
+           'aoadmm_create_multi', 'aoadmm_gpu_count', 'aoadmm_comm_release', 'aoadmm_create_sparse',
+           'aoadmm_create_sparse_masked']
 
 lib.aoadmm_abi_version.restype = C.c_int
 lib.aoadmm_device_count.argtypes = [C.POINTER(C.c_int)]
@@ -103,6 +104,8 @@ lib.aoadmm_nccl_unique_id.argtypes = [C.POINTER(C.c_uint8)]
 lib.aoadmm_create.argtypes = [C.POINTER(Problem), C.POINTER(Dist), C.POINTER(HandleP)]
 lib.aoadmm_create_sparse.argtypes = [C.POINTER(Problem), C.POINTER(C.POINTER(SparseObject)), C.POINTER(Dist),
                                      C.POINTER(HandleP)]
+lib.aoadmm_create_sparse_masked.argtypes = [C.POINTER(Problem), C.POINTER(C.POINTER(SparseObject)),
+                                            C.POINTER(C.POINTER(SparseObject)), C.POINTER(Dist), C.POINTER(HandleP)]
 lib.aoadmm_create_multi.argtypes = [C.POINTER(Problem), C.c_int32, c_int32_p, C.POINTER(HandleP)]
 lib.aoadmm_gpu_count.argtypes = [HandleP, c_int32_p]
 lib.aoadmm_comm_release.argtypes = []

@@ -126,8 +126,32 @@ int aoadmm_create(const aoadmm_problem* problem, const aoadmm_dist* dist, aoadmm
   return AOADMM_OK;
 }
 
-int aoadmm_create_sparse(const aoadmm_problem* problem, const aoadmm_sparse_object* const* sparse, const aoadmm_dist* dist,
-                         aoadmm_handle** out) {
+namespace {
+
+// subscripts of one COO descriptor against the mode sizes of CP object `ob`
+void check_coo(const aoadmm_problem* problem, const aoadmm_object& ob, const aoadmm_sparse_object* so,
+               const std::string& who) {
+  using aoadmm::CudaError;
+  if (so->nnz < 0) throw CudaError(AOADMM_ERR_INVALID_ARG, who + "nnz is negative");
+  if (so->nnz > 0 && (so->subs == nullptr || so->vals == nullptr))
+    throw CudaError(AOADMM_ERR_INVALID_ARG, who + "subs / vals is NULL");
+  if (ob.order < 2 || ob.order > 8 || ob.modes == nullptr || problem->mode_rows == nullptr)
+    throw CudaError(AOADMM_ERR_INVALID_ARG, who + "order must be in 2..8 with its modes given");
+  for (int d = 0; d < ob.order; ++d) {
+    const int mid = ob.modes[d];
+    if (mid < 1 || mid > problem->nb_modes) throw CudaError(AOADMM_ERR_INVALID_ARG, who + "mode id out of range");
+    const int64_t rows = problem->mode_rows[mid - 1];
+    if (rows > 0x7fffffffLL) throw CudaError(AOADMM_ERR_INVALID_ARG, who + "a mode has more than 2^31 - 1 rows");
+    const int64_t* sd = so->subs + (size_t)d * (size_t)so->nnz;
+    for (int64_t e = 0; e < so->nnz; ++e)
+      if (sd[e] < 0 || sd[e] >= rows)
+        throw CudaError(AOADMM_ERR_INVALID_ARG, who + "subscript " + std::to_string(sd[e]) + " of nonzero " + std::to_string(e) +
+                                                    " is out of range for mode position " + std::to_string(d + 1));
+  }
+}
+
+int create_sparse(const aoadmm_problem* problem, const aoadmm_sparse_object* const* sparse,
+                  const aoadmm_sparse_object* const* masks, const aoadmm_dist* dist, aoadmm_handle** out) {
   if (!out) return AOADMM_ERR_INVALID_ARG;
   *out = nullptr;
   aoadmm_handle* h = nullptr;
@@ -135,7 +159,16 @@ int aoadmm_create_sparse(const aoadmm_problem* problem, const aoadmm_sparse_obje
     using aoadmm::CudaError;
     if (problem == nullptr) throw CudaError(AOADMM_ERR_INVALID_ARG, "problem is NULL");
     if (problem->n_objects > 0 && problem->objects == nullptr) throw CudaError(AOADMM_ERR_INVALID_ARG, "objects is NULL");
-    // every check on the sparse descriptors happens here, before a device is touched
+    // every check on the sparse descriptors and masks happens here, before a device is touched
+    for (int p = 0; masks != nullptr && p < problem->n_objects; ++p) {
+      if (masks[p] == nullptr) continue;
+      const std::string who = "sparse mask " + std::to_string(p + 1) + ": ";
+      if (sparse == nullptr || sparse[p] == nullptr)
+        throw CudaError(AOADMM_ERR_INVALID_ARG, who + "a sparse mask needs a sparse object (dense objects take Z.miss)");
+      if (problem->objects[p].miss != nullptr)
+        throw CudaError(AOADMM_ERR_INVALID_ARG, who + "both a dense Z.miss and a sparse mask are set");
+      if (problem->objects[p].model == AOADMM_MODEL_CP) check_coo(problem, problem->objects[p], masks[p], who);
+    }
     for (int p = 0; sparse != nullptr && p < problem->n_objects; ++p) {
       const aoadmm_sparse_object* so = sparse[p];
       if (so == nullptr) continue;
@@ -146,26 +179,11 @@ int aoadmm_create_sparse(const aoadmm_problem* problem, const aoadmm_sparse_obje
       if (ob.model != AOADMM_MODEL_CP) throw CudaError(AOADMM_ERR_UNSUPPORTED, who + "PARAFAC2 objects must be dense");
       if (ob.miss != nullptr) throw CudaError(AOADMM_ERR_UNSUPPORTED, who + "missing-data masks (Z.miss) need a dense object");
       if (ob.data != nullptr) throw CudaError(AOADMM_ERR_INVALID_ARG, who + "both dense data and sparse data are set");
-      if (so->nnz < 0) throw CudaError(AOADMM_ERR_INVALID_ARG, who + "nnz is negative");
-      if (so->nnz > 0 && (so->subs == nullptr || so->vals == nullptr))
-        throw CudaError(AOADMM_ERR_INVALID_ARG, who + "subs / vals is NULL");
-      if (ob.order < 2 || ob.order > 8 || ob.modes == nullptr || problem->mode_rows == nullptr)
-        throw CudaError(AOADMM_ERR_INVALID_ARG, who + "order must be in 2..8 with its modes given");
-      for (int d = 0; d < ob.order; ++d) {
-        const int mid = ob.modes[d];
-        if (mid < 1 || mid > problem->nb_modes) throw CudaError(AOADMM_ERR_INVALID_ARG, who + "mode id out of range");
-        const int64_t rows = problem->mode_rows[mid - 1];
-        if (rows > 0x7fffffffLL) throw CudaError(AOADMM_ERR_INVALID_ARG, who + "a mode has more than 2^31 - 1 rows");
-        const int64_t* sd = so->subs + (size_t)d * (size_t)so->nnz;
-        for (int64_t e = 0; e < so->nnz; ++e)
-          if (sd[e] < 0 || sd[e] >= rows)
-            throw CudaError(AOADMM_ERR_INVALID_ARG, who + "subscript " + std::to_string(sd[e]) + " of nonzero " + std::to_string(e) +
-                                                        " is out of range for mode position " + std::to_string(d + 1));
-      }
+      check_coo(problem, ob, so, who);
     }
     h = new aoadmm_handle();
     h->eng.push_back(nullptr);
-    h->eng[0] = new aoadmm::Engine(problem, dist, nullptr, sparse);
+    h->eng[0] = new aoadmm::Engine(problem, dist, nullptr, sparse, masks);
   });
   if (rc != AOADMM_OK) {
     delete h;
@@ -173,6 +191,18 @@ int aoadmm_create_sparse(const aoadmm_problem* problem, const aoadmm_sparse_obje
   }
   *out = h;
   return AOADMM_OK;
+}
+
+}  // namespace
+
+int aoadmm_create_sparse(const aoadmm_problem* problem, const aoadmm_sparse_object* const* sparse, const aoadmm_dist* dist,
+                         aoadmm_handle** out) {
+  return create_sparse(problem, sparse, nullptr, dist, out);
+}
+
+int aoadmm_create_sparse_masked(const aoadmm_problem* problem, const aoadmm_sparse_object* const* sparse,
+                                const aoadmm_sparse_object* const* masks, const aoadmm_dist* dist, aoadmm_handle** out) {
+  return create_sparse(problem, sparse, masks, dist, out);
 }
 
 int aoadmm_create_multi(const aoadmm_problem* problem, int32_t n_gpus, const int32_t* devices, aoadmm_handle** out) {

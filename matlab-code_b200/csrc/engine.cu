@@ -459,11 +459,11 @@ struct Engine::ObjTerms {
 // construction
 // ---------------------------------------------------------------------------------------------------
 Engine::Engine(const aoadmm_problem* prob, const aoadmm_dist* dist, void* shared_comm,
-               const aoadmm_sparse_object* const* sparse) {
+               const aoadmm_sparse_object* const* sparse, const aoadmm_sparse_object* const* masks) {
   // A constructor that throws never runs the destructor: everything acquired so far (up to the whole tensor in HBM,
   // streams, events, pinned buffers) is released here before the error leaves.
   try {
-    construct(prob, dist, shared_comm, sparse);
+    construct(prob, dist, shared_comm, sparse, masks);
   } catch (...) {
     release();
     throw;
@@ -471,7 +471,7 @@ Engine::Engine(const aoadmm_problem* prob, const aoadmm_dist* dist, void* shared
 }
 
 void Engine::construct(const aoadmm_problem* prob, const aoadmm_dist* dist, void* shared_comm,
-                       const aoadmm_sparse_object* const* sparse) {
+                       const aoadmm_sparse_object* const* sparse, const aoadmm_sparse_object* const* masks) {
   if (prob == nullptr) throw CudaError(1, "problem is NULL");
   if (dist != nullptr) {
     rank_ = dist->rank;
@@ -560,12 +560,21 @@ void Engine::construct(const aoadmm_problem* prob, const aoadmm_dist* dist, void
     }
     o.dims.back() = o.shard_extent;
     if (sparse != nullptr && sparse[p] != nullptr) {
-      // sparse CP object (aoadmm_create_sparse): one GPU, no mask; sorted device copies instead of a dense array
+      // sparse CP object (aoadmm_create_sparse): one GPU, no dense mask; sorted device copies instead of a dense array.
+      // A sparse mask (aoadmm_create_sparse_masked) must mark exactly the stored entries; EM state in o.sp.
       if (world_ > 1 || src.miss != nullptr || src.data != nullptr) throw CudaError(2, "sparse object: unsupported combination");
       const aoadmm_sparse_object& so = *sparse[p];
+      const aoadmm_sparse_object* mk = masks != nullptr ? masks[p] : nullptr;
       std::vector<long long> dl(o.dims.begin(), o.dims.end());
       o.sp = new SparseTensor();
-      sparse_build(*o.sp, o.order, dl.data(), R, so.nnz, reinterpret_cast<const long long*>(so.subs), so.vals, st_);
+      try {
+        sparse_build(*o.sp, o.order, dl.data(), R, so.nnz, reinterpret_cast<const long long*>(so.subs), so.vals, st_,
+                     mk != nullptr, mk ? mk->nnz : 0, mk ? reinterpret_cast<const long long*>(mk->subs) : nullptr,
+                     mk ? mk->vals : nullptr);
+      } catch (const CudaError& e) {
+        throw CudaError(e.code, "sparse object " + std::to_string(p + 1) + ": " + e.what());
+      }
+      if (mk != nullptr) has_missing_ = true;
       continue;
     }
     o.ld0 = round_up(o.dims[0], 2);
@@ -1081,7 +1090,7 @@ void Engine::allreduce(double* buf, size_t count) {
 }
 
 // sparse objects: always FP64, no dimension tree (options.mttkrp_precision / dimtree apply to dense objects only)
-int Engine::sparse_mttkrp_of(ObjectState& o, int pos, double scale, double* out, int64_t ldout) {
+int Engine::sparse_mttkrp_of(ObjectState& o, int pos, double scale, double* out, int64_t ldout, bool imputed) {
   const double* fac[8];
   long long ld[8];
   for (int d = 0; d < o.order; ++d) {
@@ -1089,13 +1098,13 @@ int Engine::sparse_mttkrp_of(ObjectState& o, int pos, double scale, double* out,
     fac[d] = mm.fac.p;
     ld[d] = mm.rows;
   }
-  return sparse_mttkrp(*o.sp, pos, fac, ld, scale, out, ldout, st_);
+  return sparse_mttkrp(*o.sp, pos, fac, ld, scale, out, ldout, st_, imputed);
 }
 
-void Engine::compute_mttkrp(ObjectState& o, int pos, double scale, double* out, int64_t ldout) {
+void Engine::compute_mttkrp(ObjectState& o, int pos, double scale, double* out, int64_t ldout, bool imputed) {
   if (o.sp != nullptr) {
     phase_begin(o.order >= 3 ? 0 : 1);
-    launches_ += sparse_mttkrp_of(o, pos, scale, out, ldout);
+    launches_ += sparse_mttkrp_of(o, pos, scale, out, ldout, imputed);
     phase_end();
     return;
   }
@@ -1173,6 +1182,8 @@ int Engine::tc_mttkrp(ObjectState& o, int pos, double scale, double* out, int64_
 
 void Engine::refresh_gram(ModeState& m) {
   launches_ += gram(m.fac.p, m.rows, m.rows, m.R, m.GtG.p, gram_ws_, st_, nullptr);
+  if (m.p >= 0 && sparse_masked(objects_[m.p]))   // B_pos' F_pos for the low-rank term of the imputed MTTKRP
+    launches_ += sparse_cross_gram(*objects_[m.p].sp, m.pos, m.fac.p, m.rows, st_);
 }
 
 void Engine::precompute_mode(ModeState& m, int n_rho_terms, bool do_chol) {
@@ -1188,7 +1199,7 @@ void Engine::precompute_mode(ModeState& m, int n_rho_terms, bool do_chol) {
   AO_CUDA(cudaStreamWaitEvent(st2_, ev_fork_, 0));
   launches_ += prep_system(a, st2_, nullptr);
   AO_CUDA(cudaEventRecord(ev_join_, st2_));
-  compute_mttkrp(o, m.pos, o.weight, m.A.p, m.rows);  // A{m} = w * mttkrp (:97, :108, :111)
+  compute_mttkrp(o, m.pos, o.weight, m.A.p, m.rows, true);  // A{m} = w * mttkrp (:97, :108, :111)
   AO_CUDA(cudaStreamWaitEvent(st_, ev_join_, 0));
   apply_bsum(m);
 }
@@ -1682,6 +1693,18 @@ void Engine::em_step(bool impute) {
       launches_ += em_pass(a, em_sums_ + 5 * p, st_);
       if (s.sharded) allreduce(em_sums_ + 5 * p, 5);
       if (impute) s.T_version = 0;
+    } else if (sparse_masked(o)) {
+      // model at the stored entries + telescoped norms of the unobserved part, nothing dense (sparse.cuh)
+      phase_begin(2);
+      const double* fac[8];
+      long long ld[8];
+      for (int d = 0; d < o.order; ++d) {
+        const ModeState& md = mode(o.modes[d]);
+        fac[d] = md.fac.p;
+        ld[d] = md.rows;
+      }
+      launches_ += sparse_em(*o.sp, fac, ld, impute, em_sums_ + 5 * p, st_);
+      phase_end();
     } else {
       if (o.mask == nullptr) continue;
       ModeState &m0 = mode(o.modes[0]), &m1 = mode(o.modes[1]);
@@ -1742,7 +1765,7 @@ void Engine::enqueue_objective(bool first) {
     for (int p = 0; p < n_objects_; ++p) {
       ObjectState& o = objects_[p];
       if (o.model == AOADMM_MODEL_PAR2) continue;  // explicit residual below (:1262-1264)
-      if (o.mask != nullptr) continue;             // masked objective from the EM sums (:1224-1226)
+      if (o.mask != nullptr || sparse_masked(o)) continue;   // masked objective from the EM sums (:1224-1226)
       ModeState& m0 = mode(o.modes[0]);
       double* M = cp0_tmp_;
       double* scr = cp0_tmp_ + (size_t)m0.rows * m0.R;  // C | B | L | invdiag | rho
@@ -1854,7 +1877,7 @@ void Engine::finish_objective(bool first, double f[4]) {
   for (int p = 0; p < n_objects_; ++p) {
     ObjectState& o = objects_[p];
     const bool masked = has_missing_ && ((o.model == AOADMM_MODEL_PAR2) ? par2_[mode(o.modes[0]).par2].mask != nullptr
-                                                                        : o.mask != nullptr);
+                                                                        : (o.mask != nullptr || sparse_masked(o)));
     if (masked) {
       const double* e = em_sums_host_ + 5 * p;
       f_obj[p] = (o.model == AOADMM_MODEL_PAR2) ? o.weight * e[4]                               // :1249-1252, :1267

@@ -176,9 +176,10 @@ class Engine {
  public:
   // shared_comm: communicator of this rank created by the caller (single-process device group), else nullptr and the
   // communicator of dist->nccl_unique_id is taken from the process-wide cache.  sparse: nullptr, or n_objects entries
-  // (nullptr for a dense object) with the COO data of sparse CP objects (aoadmm_create_sparse, validated by the caller)
+  // (nullptr for a dense object) with the COO data of sparse CP objects (aoadmm_create_sparse, validated by the caller);
+  // masks: nullptr, or n_objects entries with the sparse Z.miss masks of sparse objects (aoadmm_create_sparse_masked)
   Engine(const aoadmm_problem* prob, const aoadmm_dist* dist, void* shared_comm = nullptr,
-         const aoadmm_sparse_object* const* sparse = nullptr);
+         const aoadmm_sparse_object* const* sparse = nullptr, const aoadmm_sparse_object* const* masks = nullptr);
   ~Engine();
   Engine(const Engine&) = delete;
   Engine& operator=(const Engine&) = delete;
@@ -214,15 +215,17 @@ class Engine {
  private:
   // setup
   void construct(const aoadmm_problem* prob, const aoadmm_dist* dist, void* shared_comm,
-                 const aoadmm_sparse_object* const* sparse);
-  int sparse_mttkrp_of(ObjectState& o, int pos, double scale, double* out, int64_t ldout);
+                 const aoadmm_sparse_object* const* sparse, const aoadmm_sparse_object* const* masks);
+  // imputed: the MTTKRP of the EM-imputed tensor of a masked sparse object (the sweep); else of the stored values
+  int sparse_mttkrp_of(ObjectState& o, int pos, double scale, double* out, int64_t ldout, bool imputed = false);
+  static bool sparse_masked(const ObjectState& o) { return o.sp != nullptr && o.sp->masked; }
   void release();
   void build_views(ObjectState& o);
   void refresh_transposed(ObjectState& o);
   void build_objective_jobs();
   // sweep pieces
   void refresh_gram(ModeState& m);
-  void compute_mttkrp(ObjectState& o, int pos, double scale, double* out, int64_t ldout);
+  void compute_mttkrp(ObjectState& o, int pos, double scale, double* out, int64_t ldout, bool imputed = false);
   int tc_mttkrp(ObjectState& o, int pos, double scale, double* out, int64_t ldout, double* emit, int prec);
   void pack_operand(View3& v, int which);
   void precompute_mode(ModeState& m, int n_rho_terms, bool do_chol);

@@ -3,14 +3,17 @@
 #include <algorithm>
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
+#include <type_traits>
 #include <utility>
 
+#include "linalg.cuh"
 #include "sparse.cuh"
 
 namespace aoadmm {
 namespace {
 
 constexpr int kNormBlocks = 512;
+constexpr int kTeleBlocks = 64;         // CTAs of the telescoped-norm reduction at most (2 partial sums each)
 
 inline unsigned grid_for(long long n, int threads = 256) {
   return (unsigned)std::max<long long>(1, std::min<long long>(ceil_div(n, threads), 148LL * 32));
@@ -151,11 +154,14 @@ struct SpArgs {
   double* outT;
   double* head;
   double* tail;
+  const int* perm;      // PERM instantiation: vals is read through perm (copy position -> canonical index)
 };
 
 // One group of G lanes per unit; lane j of a group owns columns j, j+G, ... (CPL of them).  The row sums run in the
 // sorted nonzero order, so every value depends on the data and kSparseChunk only.
-template <int G, int CPL>
+// PERM (imputed MTTKRP of a masked object, positions >= 2): the value of nonzero e is vals[perm[e]]; the unmasked
+// instantiation (PERM = false) is the original kernel.
+template <int G, int CPL, bool PERM>
 __global__ void __launch_bounds__(256) sp_mttkrp_kernel(const SpArgs a) {
   const long long unit = ((long long)blockIdx.x * blockDim.x + threadIdx.x) / G;
   const int gl = threadIdx.x % G;
@@ -172,7 +178,7 @@ __global__ void __launch_bounds__(256) sp_mttkrp_kernel(const SpArgs a) {
     for (int q = 0; q < CPL; ++q) acc[q] = 0.0;
 #pragma unroll 2
     for (; e < stop; ++e) {
-      const double v = __ldg(a.vals + e);
+      const double v = PERM ? __ldg(a.vals + __ldg(a.perm + e)) : __ldg(a.vals + e);
       double p[CPL];
 #pragma unroll
       for (int q = 0; q < CPL; ++q) p[q] = v;
@@ -226,14 +232,219 @@ __global__ void __launch_bounds__(256) sp_fixup_kernel(const SpArgs a) {
   }
 }
 
-template <int G, int CPL>
+template <int G, int CPL, bool PERM>
 void launch_sp(const SpArgs& a, cudaStream_t st) {
   const long long threads = a.units * G;
   const unsigned blocks = (unsigned)ceil_div(threads, 256);
-  sp_mttkrp_kernel<G, CPL><<<blocks, 256, 0, st>>>(a);
+  sp_mttkrp_kernel<G, CPL, PERM><<<blocks, 256, 0, st>>>(a);
   AO_CHECK_LAUNCH();
   sp_fixup_kernel<G, CPL><<<blocks, 256, 0, st>>>(a);
   AO_CHECK_LAUNCH();
+}
+
+// lanes per nonzero (G) and columns per lane (CPL) for rank R: f(integral_constant<G>, integral_constant<CPL>)
+template <typename Fn>
+void rank_dispatch(int R, Fn&& f) {
+  using std::integral_constant;
+  if (R <= 1) f(integral_constant<int, 1>{}, integral_constant<int, 1>{});
+  else if (R <= 2) f(integral_constant<int, 2>{}, integral_constant<int, 1>{});
+  else if (R <= 4) f(integral_constant<int, 4>{}, integral_constant<int, 1>{});
+  else if (R <= 8) f(integral_constant<int, 8>{}, integral_constant<int, 1>{});
+  else if (R <= 16) f(integral_constant<int, 16>{}, integral_constant<int, 1>{});
+  else if (R <= 32) f(integral_constant<int, 32>{}, integral_constant<int, 1>{});
+  else if (R <= 64) f(integral_constant<int, 32>{}, integral_constant<int, 2>{});
+  else if (R <= 128) f(integral_constant<int, 32>{}, integral_constant<int, 4>{});
+  else f(integral_constant<int, 32>{}, integral_constant<int, 8>{});
+}
+
+// ---- EM imputation of masked sparse objects ----
+struct ModelArgs {
+  long long nnz;
+  int no, R, impute;
+  const int* row0;      // canonical order: position-1 subscripts
+  const int* idx;       // canonical order: (order-1) x nnz subscripts of positions 2..order
+  const double* vals;   // s
+  const double* F[8];   // row-major factors of every position
+  double* m;            // model at the last imputation (in), m' (out, impute)
+  double* r;            // s - m' (out, impute)
+  double* part;         // 4 per CTA
+};
+
+// m'(e) = sum_c prod_d F_d(i_d, c): a group of G lanes walks one unit of kSparseChunk consecutive nonzeros (columns
+// across lanes, a fixed xor tree across them; consecutive nonzeros share rows and index sectors, as in the MTTKRP).
+// Every group runs kSparseChunk steps so that each shuffle has the whole warp.  Per CTA, in a fixed order:
+// [0] sum s m', [1] sum m'^2, [2] sum (m' - m)^2, [3] sum m^2.
+template <int G, int CPL>
+__global__ void __launch_bounds__(256) sp_model_kernel(const ModelArgs a) {
+  __shared__ double scratch[32];
+  const int gl = threadIdx.x % G;
+  const long long e0 = (((long long)blockIdx.x * blockDim.x + threadIdx.x) / G) * kSparseChunk;
+  const int R = a.R;
+  double s0 = 0.0, s1 = 0.0, s2 = 0.0, s3 = 0.0;
+  for (int q0 = 0; q0 < kSparseChunk; ++q0) {
+    const long long e = e0 + q0;
+    const bool ok = e < a.nnz;
+    double t = 0.0;
+    if (ok) {
+      double p[CPL];
+      const double* f0 = a.F[0] + (long long)__ldg(a.row0 + e) * R;
+#pragma unroll
+      for (int q = 0; q < CPL; ++q) {
+        const int c = gl + G * q;
+        p[q] = c < R ? __ldg(f0 + c) : 0.0;
+      }
+      for (int m = 0; m < a.no; ++m) {
+        const double* f = a.F[m + 1] + (long long)__ldg(a.idx + m * a.nnz + e) * R;
+#pragma unroll
+        for (int q = 0; q < CPL; ++q) {
+          const int c = gl + G * q;
+          if (c < R) p[q] *= __ldg(f + c);
+        }
+      }
+#pragma unroll
+      for (int q = 0; q < CPL; ++q) t += p[q];
+    }
+#pragma unroll
+    for (int off = G / 2; off > 0; off >>= 1) t += __shfl_xor_sync(0xffffffffu, t, off);
+    if (ok && gl == 0) {
+      const double s = __ldg(a.vals + e), mo = a.m[e], d = t - mo;
+      s0 = fma(s, t, s0);
+      s1 = fma(t, t, s1);
+      s2 = fma(d, d, s2);
+      s3 = fma(mo, mo, s3);
+      if (a.impute) {
+        a.m[e] = t;
+        a.r[e] = s - t;
+      }
+    }
+  }
+  s0 = block_sum(s0, scratch);
+  s1 = block_sum(s1, scratch);
+  s2 = block_sum(s2, scratch);
+  s3 = block_sum(s3, scratch);
+  if (threadIdx.x == 0) {
+    double* o = a.part + 4 * (long long)blockIdx.x;
+    o[0] = s0;
+    o[1] = s1;
+    o[2] = s2;
+    o[3] = s3;
+  }
+}
+
+// CTAs of the model pass: one group of G lanes per unit of kSparseChunk nonzeros
+long long model_blocks(long long nnz, int R) {
+  long long b = 0;
+  rank_dispatch(R, [&](auto g, auto) { b = ceil_div(ceil_div(nnz, kSparseChunk) * decltype(g)::value, 256); });
+  return b;
+}
+
+// S = [F | B | F - B] (rows x 3R, ld = rows); impute: B = F afterwards
+__global__ void stack3_kernel(const double* __restrict__ F, long long ldf, double* __restrict__ B, long long rows, int R,
+                              double* __restrict__ S, int impute) {
+  const long long n = rows * R;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+    const long long r = i % rows, c = i / rows;
+    const double f = F[r + ldf * c], b = B[i];
+    S[i] = f;
+    S[i + n] = b;
+    S[i + 2 * n] = f - b;
+    if (impute) B[i] = f;
+  }
+}
+
+// With G_d = [F_d | B_d | D_d]' [F_d | B_d | D_d], D_d = F_d - B_d (3R x 3R, blocks 0 = F, 1 = B, 2 = D):
+//   ||[[F]] - [[B]]||^2 = sum_{k,l} <T_k, T_l>,  T_k = [[F_1..F_{k-1}, D_k, B_{k+1}..B_N]]  (telescoped difference)
+//   ||[[B]]||^2 = sum(Hadamard of the B'B blocks)
+// so that near convergence the difference is never formed from two nearly equal model norms.  Per CTA: [0], [1].
+__global__ void __launch_bounds__(256) tele_partials_kernel(const double* __restrict__ g3, int order, int R,
+                                                            double* __restrict__ part) {
+  __shared__ double scratch[32];
+  const int R3 = 3 * R, G9 = R3 * R3;   // (3 * 256)^2 * 8 < 2^31
+  double acc = 0.0, mm = 0.0;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < R * R; i += gridDim.x * blockDim.x) {
+    const int r = i % R, c = i / R;
+    double sk = 0.0;
+#pragma unroll 1
+    for (int k = 0; k < order; ++k)
+#pragma unroll 1
+      for (int l = 0; l < order; ++l) {
+        double p = 1.0;
+        const double* g = g3 + r + R3 * c;
+#pragma unroll 1
+        for (int d = 0; d < order; ++d, g += G9) {
+          const int tk = d < k ? 0 : (d == k ? 2 : 1), tl = d < l ? 0 : (d == l ? 2 : 1);
+          p *= __ldg(g + tk * R + R3 * tl * R);
+        }
+        sk += p;
+      }
+    acc += sk;
+    double q = 1.0;
+    for (int d = 0; d < order; ++d) q *= __ldg(g3 + d * G9 + (R + r) + R3 * (R + c));
+    mm += q;
+  }
+  acc = block_sum(acc, scratch);
+  mm = block_sum(mm, scratch);
+  if (threadIdx.x == 0) {
+    part[2 * blockIdx.x] = acc;
+    part[2 * blockIdx.x + 1] = mm;
+  }
+}
+
+// em_sums slots of the object: [0] ||M'-M||^2 - sum_W (m'-m)^2, [1] ||M||^2 - sum_W m^2 (both clamped at 0: they are
+// sums of squares over the unobserved entries, a negative value is rounding), [2] sum s m', [3] sum m'^2, [4] 0
+__global__ void em_final_kernel(const double* __restrict__ mpart, unsigned nm, const double* __restrict__ tpart, unsigned nt,
+                                double* __restrict__ sums) {
+  const double a0 = warp_sum_partials(mpart, nm, 4), a1 = warp_sum_partials(mpart + 1, nm, 4);
+  const double a2 = warp_sum_partials(mpart + 2, nm, 4), a3 = warp_sum_partials(mpart + 3, nm, 4);
+  const double t = warp_sum_partials(tpart, nt, 2), mm = warp_sum_partials(tpart + 1, nt, 2);
+  if (threadIdx.x == 0) {
+    const double num = t - a2, den = mm - a3;
+    sums[0] = num > 0.0 ? num : 0.0;
+    sums[1] = den > 0.0 ? den : 0.0;
+    sums[2] = a0;
+    sums[3] = a1;
+    sums[4] = 0.0;
+  }
+}
+
+// cg_d = leading R x R block of g3_d (= F_d' F_d = B_d' F_d right after B = F)
+__global__ void cg_from_g3_kernel(const double* __restrict__ g3, int order, int R, double* __restrict__ cg) {
+  const long long R3 = 3LL * R, RR = (long long)R * R, n = order * RR;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+    const long long d = i / RR, j = i % RR, r = j % R, c = j / R;
+    cg[i] = g3[d * R3 * R3 + r + R3 * c];
+  }
+}
+
+// H = Hadamard product of cg_k over k != n (ascending k)
+__global__ void hadamard_others_kernel(const double* __restrict__ cg, int order, int n, int R, double* __restrict__ H) {
+  const long long RR = (long long)R * R;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < RR; i += (long long)gridDim.x * blockDim.x) {
+    double h = 1.0;
+    for (int k = 0; k < order; ++k)
+      if (k != n) h *= cg[k * RR + i];
+    H[i] = h;
+  }
+}
+
+__global__ void nonzero_flags_kernel(const double* __restrict__ v, long long n, int* __restrict__ flags) {
+  for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x)
+    flags[e] = v[e] != 0.0;
+}
+
+// observed entries of the merged mask, in the same (full lexicographic) order
+__global__ void compact_kernel(const int* __restrict__ ms, const int* __restrict__ flags, const int* __restrict__ pos,
+                               long long n, int order, int* __restrict__ out, long long nout) {
+  for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x) {
+    if (!flags[e]) continue;
+    const long long t = pos[e] - 1;
+    for (int d = 0; d < order; ++d) out[d * nout + t] = ms[d * n + e];
+  }
+}
+
+__global__ void differ_kernel(const int* __restrict__ a, const int* __restrict__ b, long long n, int* __restrict__ bad) {
+  for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x)
+    if (a[e] != b[e]) atomicOr(bad, 1);
 }
 
 __global__ void __launch_bounds__(256) sq_partials_kernel(const double* __restrict__ v, long long n, double* __restrict__ part) {
@@ -270,13 +481,111 @@ struct Temps {
   }
 };
 
+// radix-sort scratch shared by the merge and the per-mode sorts of one COO set
+struct SortWs {
+  unsigned *k0 = nullptr, *k1 = nullptr;
+  int *p0 = nullptr, *p1 = nullptr;
+  void* tmp = nullptr;
+  size_t bytes = 0;
+};
+
+// uploads n > 0 COO entries, sorts them into full lexicographic order (mode 0 major) and sums duplicates (the Tensor
+// Toolbox sptensor(subs,vals) constructor sums them): ms (order x nm, column-major), mv (nm).  Returns nm.
+long long sort_merge(Temps& tmp, SortWs& w, int order, const long long* dims, long long n, const long long* subs,
+                     const double* vals, cudaStream_t st, int*& ms, double*& mv) {
+  std::vector<int> h((size_t)order * n);
+  for (size_t i = 0; i < h.size(); ++i) h[i] = (int)subs[i];
+  int* raw = tmp.get<int>((size_t)order * n);
+  double* rv = tmp.get<double>(n);
+  AO_CUDA(cudaMemcpyAsync(raw, h.data(), h.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+  AO_CUDA(cudaMemcpyAsync(rv, vals, (size_t)n * sizeof(double), cudaMemcpyHostToDevice, st));
+  AO_CUDA(cudaStreamSynchronize(st));
+  w.k0 = tmp.get<unsigned>(n);
+  w.k1 = tmp.get<unsigned>(n);
+  w.p0 = tmp.get<int>(n);
+  w.p1 = tmp.get<int>(n);
+  AO_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, w.bytes, w.k0, w.k1, w.p0, w.p1, (int)n, 0, 32, st));
+  size_t scan_bytes = 0;
+  AO_CUDA(cub::DeviceScan::InclusiveSum(nullptr, scan_bytes, (int*)w.k0, (int*)w.k1, (int)n, st));
+  w.bytes = std::max(w.bytes, scan_bytes);
+  w.tmp = tmp.get<char>(w.bytes);
+  // full lexicographic order (mode 0 major): stable LSD passes from the last mode to the first
+  iota_kernel<<<grid_for(n), 256, 0, st>>>(w.p0, n);
+  AO_CHECK_LAUNCH();
+  for (int d = order - 1; d >= 0; --d) {
+    gather_keys_kernel<<<grid_for(n), 256, 0, st>>>(raw + (size_t)d * n, w.p0, w.k0, n);
+    AO_CHECK_LAUNCH();
+    size_t b = w.bytes;
+    AO_CUDA(cub::DeviceRadixSort::SortPairs(w.tmp, b, w.k0, w.k1, w.p0, w.p1, (int)n, 0, key_bits(dims[d]), st));
+    std::swap(w.p0, w.p1);
+  }
+  int* ss = tmp.get<int>((size_t)order * n);
+  double* sv = tmp.get<double>(n);
+  gather_coo_kernel<<<grid_for(n), 256, 0, st>>>(raw, rv, w.p0, n, order, ss, sv);
+  AO_CHECK_LAUNCH();
+  int* flags = (int*)w.k0;
+  int* pos = (int*)w.k1;
+  head_flags_kernel<<<grid_for(n), 256, 0, st>>>(ss, order, n, flags);
+  AO_CHECK_LAUNCH();
+  size_t b = w.bytes;
+  AO_CUDA(cub::DeviceScan::InclusiveSum(w.tmp, b, flags, pos, (int)n, st));
+  int last = 0;
+  AO_CUDA(cudaMemcpyAsync(&last, pos + n - 1, sizeof(int), cudaMemcpyDeviceToHost, st));
+  AO_CUDA(cudaStreamSynchronize(st));
+  const long long nm = last;
+  ms = tmp.get<int>((size_t)order * nm);
+  mv = tmp.get<double>(nm);
+  merge_kernel<<<grid_for(n), 256, 0, st>>>(ss, sv, flags, pos, n, order, ms, mv, nm);
+  AO_CHECK_LAUNCH();
+  return nm;
+}
+
+// true when the observed entries of the mask (merged value != 0) are exactly the merged subscripts ms (order x nm)
+bool mask_matches(Temps& tmp, int order, const long long* dims, long long nm, const int* ms, long long mask_nnz,
+                  const long long* mask_subs, const double* mask_vals, cudaStream_t st) {
+  long long nobs = 0;
+  int* obs = nullptr;
+  if (mask_nnz > 0) {
+    SortWs w;
+    int* mms = nullptr;
+    double* mmv = nullptr;
+    const long long mm = sort_merge(tmp, w, order, dims, mask_nnz, mask_subs, mask_vals, st, mms, mmv);
+    int* flags = (int*)w.k0;
+    int* pos = (int*)w.k1;
+    nonzero_flags_kernel<<<grid_for(mm), 256, 0, st>>>(mmv, mm, flags);
+    AO_CHECK_LAUNCH();
+    size_t b = w.bytes;
+    AO_CUDA(cub::DeviceScan::InclusiveSum(w.tmp, b, flags, pos, (int)mm, st));
+    int last = 0;
+    AO_CUDA(cudaMemcpyAsync(&last, pos + mm - 1, sizeof(int), cudaMemcpyDeviceToHost, st));
+    AO_CUDA(cudaStreamSynchronize(st));
+    nobs = last;
+    obs = tmp.get<int>((size_t)order * nobs);
+    compact_kernel<<<grid_for(mm), 256, 0, st>>>(mms, flags, pos, mm, order, obs, nobs);
+    AO_CHECK_LAUNCH();
+  }
+  if (nobs != nm) return false;
+  if (nm == 0) return true;
+  int* bad = tmp.get<int>(1);
+  AO_CUDA(cudaMemsetAsync(bad, 0, sizeof(int), st));
+  differ_kernel<<<grid_for((long long)order * nm), 256, 0, st>>>(ms, obs, (long long)order * nm, bad);
+  AO_CHECK_LAUNCH();
+  int hb = 0;
+  AO_CUDA(cudaMemcpyAsync(&hb, bad, sizeof(int), cudaMemcpyDeviceToHost, st));
+  AO_CUDA(cudaStreamSynchronize(st));
+  return hb == 0;
+}
+
 }  // namespace
 
 void sparse_build(SparseTensor& s, int order, const long long* dims, int R, long long nnz, const long long* subs,
-                  const double* vals, cudaStream_t st) {
+                  const double* vals, cudaStream_t st, bool masked, long long mask_nnz, const long long* mask_subs,
+                  const double* mask_vals) {
   if (order < 2 || order > 8) throw CudaError(1, "sparse object: order must be in 2..8");
   if (nnz < 0) throw CudaError(1, "sparse object: negative nnz");
   if (nnz > 0x7fffffffLL - kSparseChunk) throw CudaError(2, "sparse object: more than 2^31 - 257 nonzeros");
+  if (masked && (mask_nnz < 0 || mask_nnz > 0x7fffffffLL - kSparseChunk))
+    throw CudaError(1, "sparse object: mask nnz out of range");
   s.order = order;
   s.R = R;
   for (int d = 0; d < order; ++d) {
@@ -284,61 +593,14 @@ void sparse_build(SparseTensor& s, int order, const long long* dims, int R, long
     s.dims[d] = dims[d];
   }
   Temps tmp;   // temporaries of the preprocessing: released on every exit path
-  const long long n = nnz;
   long long nm = 0;
   int* ms = nullptr;
   double* mv = nullptr;
-  unsigned *k0 = nullptr, *k1 = nullptr;
-  int *p0 = nullptr, *p1 = nullptr;
-  void* sort_tmp = nullptr;
-  size_t sort_bytes = 0;
-  if (n > 0) {
-    std::vector<int> h((size_t)order * n);
-    for (size_t i = 0; i < h.size(); ++i) h[i] = (int)subs[i];
-    int* raw = tmp.get<int>((size_t)order * n);
-    double* rv = tmp.get<double>(n);
-    AO_CUDA(cudaMemcpyAsync(raw, h.data(), h.size() * sizeof(int), cudaMemcpyHostToDevice, st));
-    AO_CUDA(cudaMemcpyAsync(rv, vals, (size_t)n * sizeof(double), cudaMemcpyHostToDevice, st));
-    AO_CUDA(cudaStreamSynchronize(st));
-    k0 = tmp.get<unsigned>(n);
-    k1 = tmp.get<unsigned>(n);
-    p0 = tmp.get<int>(n);
-    p1 = tmp.get<int>(n);
-    AO_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, k0, k1, p0, p1, (int)n, 0, 32, st));
-    size_t scan_bytes = 0;
-    AO_CUDA(cub::DeviceScan::InclusiveSum(nullptr, scan_bytes, (int*)k0, (int*)k1, (int)n, st));
-    sort_bytes = std::max(sort_bytes, scan_bytes);
-    sort_tmp = tmp.get<char>(sort_bytes);
-    // full lexicographic order (mode 0 major): stable LSD passes from the last mode to the first
-    iota_kernel<<<grid_for(n), 256, 0, st>>>(p0, n);
-    AO_CHECK_LAUNCH();
-    for (int d = order - 1; d >= 0; --d) {
-      gather_keys_kernel<<<grid_for(n), 256, 0, st>>>(raw + (size_t)d * n, p0, k0, n);
-      AO_CHECK_LAUNCH();
-      size_t b = sort_bytes;
-      AO_CUDA(cub::DeviceRadixSort::SortPairs(sort_tmp, b, k0, k1, p0, p1, (int)n, 0, key_bits(dims[d]), st));
-      std::swap(p0, p1);
-    }
-    int* ss = tmp.get<int>((size_t)order * n);
-    double* sv = tmp.get<double>(n);
-    gather_coo_kernel<<<grid_for(n), 256, 0, st>>>(raw, rv, p0, n, order, ss, sv);
-    AO_CHECK_LAUNCH();
-    // merge duplicates (the Tensor Toolbox sptensor(subs,vals) constructor sums them)
-    int* flags = (int*)k0;
-    int* pos = (int*)k1;
-    head_flags_kernel<<<grid_for(n), 256, 0, st>>>(ss, order, n, flags);
-    AO_CHECK_LAUNCH();
-    size_t b = sort_bytes;
-    AO_CUDA(cub::DeviceScan::InclusiveSum(sort_tmp, b, flags, pos, (int)n, st));
-    int last = 0;
-    AO_CUDA(cudaMemcpyAsync(&last, pos + n - 1, sizeof(int), cudaMemcpyDeviceToHost, st));
-    AO_CUDA(cudaStreamSynchronize(st));
-    nm = last;
-    ms = tmp.get<int>((size_t)order * nm);
-    mv = tmp.get<double>(nm);
-    merge_kernel<<<grid_for(n), 256, 0, st>>>(ss, sv, flags, pos, n, order, ms, mv, nm);
-    AO_CHECK_LAUNCH();
-  }
+  SortWs w;
+  if (nnz > 0) nm = sort_merge(tmp, w, order, dims, nnz, subs, vals, st, ms, mv);
+  if (masked && !mask_matches(tmp, order, dims, nm, ms, mask_nnz, mask_subs, mask_vals, st))
+    throw CudaError(2, "the observed entries of the sparse mask (Z.miss) differ from the stored entries of the object "
+                       "(a sparse mask must mark exactly the stored entries)");
   s.nnz = nm;
   const long long units = ceil_div(nm, kSparseChunk);
   long long max_rows = 1;
@@ -353,6 +615,7 @@ void sparse_build(SparseTensor& s, int order, const long long* dims, int R, long
     sm.tail_row = dalloc<int>(units);
     sm.vals = dalloc<double>(nm);
     sm.idx = dalloc<int>((size_t)(order - 1) * nm);
+    if (masked && m > 0) sm.perm = dalloc<int>(nm);
     if (nm == 0) {
       AO_CUDA(cudaMemsetAsync(sm.rowptr, 0, (rows + 1) * sizeof(long long), st));
       continue;
@@ -362,12 +625,13 @@ void sparse_build(SparseTensor& s, int order, const long long* dims, int R, long
     const unsigned* keys = (const unsigned*)(ms + (size_t)m * nm);
     const int* perm = nullptr;
     if (m > 0) {
-      iota_kernel<<<grid_for(nm), 256, 0, st>>>(p0, nm);
+      iota_kernel<<<grid_for(nm), 256, 0, st>>>(w.p0, nm);
       AO_CHECK_LAUNCH();
-      size_t b = sort_bytes;
-      AO_CUDA(cub::DeviceRadixSort::SortPairs(sort_tmp, b, keys, k1, p0, p1, (int)nm, 0, key_bits(rows), st));
-      keys = k1;
-      perm = p1;
+      size_t b = w.bytes;
+      AO_CUDA(cub::DeviceRadixSort::SortPairs(w.tmp, b, keys, w.k1, w.p0, w.p1, (int)nm, 0, key_bits(rows), st));
+      keys = w.k1;
+      perm = w.p1;
+      if (masked) AO_CUDA(cudaMemcpyAsync(sm.perm, perm, (size_t)nm * sizeof(int), cudaMemcpyDeviceToDevice, st));
     }
     mode_copy_kernel<<<grid_for(nm), 256, 0, st>>>(ms, mv, perm, nm, order, m, sm.vals, sm.idx);
     AO_CHECK_LAUNCH();
@@ -383,6 +647,33 @@ void sparse_build(SparseTensor& s, int order, const long long* dims, int R, long
   s.tail = dalloc<double>((size_t)units * R);
   s.norm_partials = dalloc<double>(kNormBlocks);
   s.norm_out = dalloc<double>(1);
+  if (masked) {
+    // EM state: m = 0, r = s, B = 0 ("the unobserved entries start at 0"), every buffer of sparse_em / the imputed MTTKRP
+    s.masked = true;
+    s.row0 = dalloc<int>(nm);
+    s.mvals = dalloc<double>(nm);
+    s.rvals = dalloc<double>(nm);
+    if (nm > 0) {
+      AO_CUDA(cudaMemcpyAsync(s.row0, ms, (size_t)nm * sizeof(int), cudaMemcpyDeviceToDevice, st));
+      AO_CUDA(cudaMemsetAsync(s.mvals, 0, (size_t)nm * sizeof(double), st));
+      AO_CUDA(cudaMemcpyAsync(s.rvals, s.modes[0].vals, (size_t)nm * sizeof(double), cudaMemcpyDeviceToDevice, st));
+    }
+    const long long RR = (long long)R * R, R3 = 3LL * R;
+    size_t ws = 1;
+    for (int d = 0; d < order; ++d) {
+      s.B[d] = dalloc<double>((size_t)dims[d] * R);
+      AO_CUDA(cudaMemsetAsync(s.B[d], 0, (size_t)dims[d] * R * sizeof(double), st));
+      ws = std::max<size_t>(ws, (size_t)dgemm_splitk_count(R, R, dims[d]) * RR);
+      ws = std::max<size_t>(ws, (size_t)dgemm_splitk_count(R3, R3, dims[d]) * R3 * R3);
+    }
+    s.cg = dalloc<double>((size_t)order * RR);
+    AO_CUDA(cudaMemsetAsync(s.cg, 0, (size_t)order * RR * sizeof(double), st));
+    s.H = dalloc<double>(RR);
+    s.stack = dalloc<double>((size_t)max_rows * R3);
+    s.g3 = dalloc<double>((size_t)order * R3 * R3);
+    s.gemm_ws = dalloc<double>(ws);
+    s.em_partials = dalloc<double>(2 * kTeleBlocks + 4 * (size_t)model_blocks(nm, R));
+  }
   AO_CUDA(cudaStreamSynchronize(st));
 }
 
@@ -398,6 +689,7 @@ void sparse_free(SparseTensor& s) {
     f(m.tail_row);
     f(m.vals);
     f(m.idx);
+    f(m.perm);
   }
   s.modes.clear();
   for (auto& p : s.factT) f(p);
@@ -406,6 +698,16 @@ void sparse_free(SparseTensor& s) {
   f(s.tail);
   f(s.norm_partials);
   f(s.norm_out);
+  f(s.row0);
+  f(s.mvals);
+  f(s.rvals);
+  for (auto& p : s.B) f(p);
+  f(s.cg);
+  f(s.H);
+  f(s.stack);
+  f(s.g3);
+  f(s.gemm_ws);
+  f(s.em_partials);
 }
 
 int sparse_norm2(const SparseTensor& s, cudaStream_t st) {
@@ -418,10 +720,11 @@ int sparse_norm2(const SparseTensor& s, cudaStream_t st) {
 }
 
 int sparse_mttkrp(SparseTensor& s, int n, const double* const* fac, const long long* ld, double scale, double* out,
-                  long long ldout, cudaStream_t st) {
+                  long long ldout, cudaStream_t st, bool imputed) {
   const long long rows = s.dims[n];
   const int R = s.R;
   const SparseMode& sm = s.modes[n];
+  const bool imp = imputed && s.masked;
   int launches = 0;
   AO_CUDA(cudaMemsetAsync(s.outT, 0, (size_t)std::max<long long>(rows, 1) * R * sizeof(double), st));
   SpArgs a{};
@@ -429,7 +732,8 @@ int sparse_mttkrp(SparseTensor& s, int n, const double* const* fac, const long l
   a.chunk_row = sm.chunk_row;
   a.head_row = sm.head_row;
   a.tail_row = sm.tail_row;
-  a.vals = sm.vals;
+  a.vals = imp ? s.rvals : sm.vals;   // imputed: the residual values, read through the copy -> canonical permutation
+  a.perm = imp ? sm.perm : nullptr;   // (position 1 is the canonical order itself: perm == nullptr)
   a.idx = sm.idx;
   a.nnz = s.nnz;
   a.units = ceil_div(s.nnz, kSparseChunk);
@@ -445,19 +749,82 @@ int sparse_mttkrp(SparseTensor& s, int n, const double* const* fac, const long l
       launches += transpose_scale(fac[d], s.dims[d], R, ld[d], s.factT[d], R, 1.0, st);
       a.F[q++] = s.factT[d];
     }
-    if (R <= 1) launch_sp<1, 1>(a, st);
-    else if (R <= 2) launch_sp<2, 1>(a, st);
-    else if (R <= 4) launch_sp<4, 1>(a, st);
-    else if (R <= 8) launch_sp<8, 1>(a, st);
-    else if (R <= 16) launch_sp<16, 1>(a, st);
-    else if (R <= 32) launch_sp<32, 1>(a, st);
-    else if (R <= 64) launch_sp<32, 2>(a, st);
-    else if (R <= 128) launch_sp<32, 4>(a, st);
-    else launch_sp<32, 8>(a, st);
+    rank_dispatch(R, [&](auto g, auto c) {
+      if (a.perm != nullptr) launch_sp<decltype(g)::value, decltype(c)::value, true>(a, st);
+      else launch_sp<decltype(g)::value, decltype(c)::value, false>(a, st);
+    });
     launches += 2;
   }
   // out(i, c) = scale * outT(c + R*i)
   launches += transpose_scale(s.outT, R, rows, R, out, ldout, scale, st);
+  if (imp && rows > 0) {
+    // low-rank term of the imputed tensor: out += scale * B_n * (Hadamard of B_k' F_k, k != n)
+    const long long RR = (long long)R * R;
+    hadamard_others_kernel<<<grid_for(RR), 256, 0, st>>>(s.cg, s.order, n, R, s.H);
+    AO_CHECK_LAUNCH();
+    launches += 1 + dgemm_small(0, 0, rows, R, R, scale, nullptr, s.B[n], rows, s.H, R, 1.0, out, ldout, st, nullptr);
+  }
+  return launches;
+}
+
+int sparse_cross_gram(SparseTensor& s, int n, const double* F, long long ld, cudaStream_t st) {
+  if (!s.masked || s.dims[n] == 0) return 0;
+  const int R = s.R;
+  return dgemm_small_splitk(1, 0, R, R, s.dims[n], 1.0, s.B[n], s.dims[n], F, ld, 0.0, s.cg + (size_t)n * R * R, R,
+                            s.gemm_ws, st, nullptr);
+}
+
+int sparse_em(SparseTensor& s, const double* const* fac, const long long* ld, bool impute, double* sums, cudaStream_t st) {
+  const int R = s.R;
+  int launches = 0;
+  // 1. model at the nonzeros (canonical order), four fixed-order sums; impute: m = m', r = s - m'
+  unsigned nbm = 0;
+  if (s.nnz > 0) {
+    ModelArgs a{};
+    a.nnz = s.nnz;
+    a.no = s.order - 1;
+    a.R = R;
+    a.impute = impute ? 1 : 0;
+    a.row0 = s.row0;
+    a.idx = s.modes[0].idx;
+    a.vals = s.modes[0].vals;
+    for (int d = 0; d < s.order; ++d) {
+      launches += transpose_scale(fac[d], s.dims[d], R, ld[d], s.factT[d], R, 1.0, st);
+      a.F[d] = s.factT[d];
+    }
+    a.m = s.mvals;
+    a.r = s.rvals;
+    a.part = s.em_partials + 2 * kTeleBlocks;
+    nbm = (unsigned)model_blocks(s.nnz, R);
+    rank_dispatch(R, [&](auto g, auto c) { sp_model_kernel<decltype(g)::value, decltype(c)::value><<<nbm, 256, 0, st>>>(a); });
+    AO_CHECK_LAUNCH();
+    ++launches;
+  }
+  // 2. Grams of [F_d | B_d | F_d - B_d] (impute: B_d = F_d afterwards), telescoped ||M' - M||^2 and ||M||^2
+  const long long R3 = 3LL * R;
+  for (int d = 0; d < s.order; ++d) {
+    const long long rows = s.dims[d];
+    double* g = s.g3 + (size_t)d * R3 * R3;
+    if (rows == 0) {
+      AO_CUDA(cudaMemsetAsync(g, 0, (size_t)R3 * R3 * sizeof(double), st));
+      continue;
+    }
+    stack3_kernel<<<grid_for(rows * R), 256, 0, st>>>(fac[d], ld[d], s.B[d], rows, R, s.stack, impute ? 1 : 0);
+    AO_CHECK_LAUNCH();
+    launches += 1 + dgemm_small_splitk(1, 0, R3, R3, rows, 1.0, s.stack, rows, s.stack, rows, 0.0, g, R3, s.gemm_ws, st, nullptr);
+  }
+  const unsigned nbt = (unsigned)std::min<long long>(ceil_div((long long)R * R, 256), kTeleBlocks);
+  double* tpart = s.em_partials;
+  tele_partials_kernel<<<nbt, 256, 0, st>>>(s.g3, s.order, R, tpart);
+  AO_CHECK_LAUNCH();
+  em_final_kernel<<<1, 32, 0, st>>>(s.em_partials + 2 * kTeleBlocks, nbm, tpart, nbt, sums);
+  AO_CHECK_LAUNCH();
+  launches += 2;
+  if (impute) {   // B = F: the cross-Grams B_d' F_d are the F_d' F_d blocks just computed
+    cg_from_g3_kernel<<<grid_for((long long)s.order * R * R), 256, 0, st>>>(s.g3, s.order, R, s.cg);
+    AO_CHECK_LAUNCH();
+    ++launches;
+  }
   return launches;
 }
 

@@ -28,6 +28,7 @@ struct SparseMode {
   int* tail_row = nullptr;          // per unit: its last row when that row goes on in a later unit, else -1
   double* vals = nullptr;           // nnz
   int* idx = nullptr;               // (order-1) x nnz: indices of the other modes in ascending position
+  int* perm = nullptr;              // masked objects, positions >= 1: canonical index of every nonzero of this copy
 };
 
 struct SparseTensor {
@@ -41,18 +42,44 @@ struct SparseTensor {
   double* tail = nullptr;           // units x R: partial sums of the tail rows
   double* norm_partials = nullptr;  // deterministic two-level reduction
   double* norm_out = nullptr;
+  // Z.miss on a sparse object (aoadmm_create_sparse_masked): EM imputation state, allocated for masked objects only.
+  // Canonical order = the order of the position-1 copy.
+  bool masked = false;
+  int* row0 = nullptr;              // nnz: position-1 subscript of every nonzero (canonical order)
+  double* mvals = nullptr;          // nnz: model [[B]] at the nonzeros (canonical order)
+  double* rvals = nullptr;          // nnz: residual s - m (canonical order); the imputed MTTKRP streams these
+  double* B[8] = {nullptr};         // dims[d] x R column-major: factors at the last imputation (all zero before it)
+  double* cg = nullptr;             // order x R x R: cross-Grams B_d' F_d with the current factors F_d
+  double* H = nullptr;              // R x R: Hadamard product of the cross-Grams of the other positions
+  double* stack = nullptr;          // max rows x 3R: [F_d | B_d | F_d - B_d]
+  double* g3 = nullptr;             // order x (3R)^2: Grams of the stacks
+  double* gemm_ws = nullptr;        // split-K partial tiles of the Gram products
+  double* em_partials = nullptr;    // per-CTA sums of the model pass (4 per CTA) and of the telescoped norms (2 per CTA)
 };
 
 // Uploads and preprocesses one COO object: subs is nnz x order column-major (0-based, validated by the caller), vals nnz
 // values.  Duplicates are summed.  Allocates every scratch buffer the MTTKRP needs.  Synchronous on `st`.
+// masked: the object has a sparse Z.miss mask (mask_nnz entries, same layout as subs / vals).  An entry is observed when its merged value
+// is nonzero; the observed set must equal the stored set of the object (else CudaError UNSUPPORTED).  Allocates the EM
+// state (sparse.cuh above) with m = 0, r = s, B = 0.
 void sparse_build(SparseTensor& s, int order, const long long* dims, int R, long long nnz, const long long* subs,
-                  const double* vals, cudaStream_t st);
+                  const double* vals, cudaStream_t st, bool masked = false, long long mask_nnz = 0,
+                  const long long* mask_subs = nullptr, const double* mask_vals = nullptr);
 void sparse_free(SparseTensor& s);
 // ||X||_F^2 = sum of the squared merged values (fixed-order reduction); the result lands in s.norm_out (device)
 int sparse_norm2(const SparseTensor& s, cudaStream_t st);
 // out (rows(n) x R, column-major, leading dimension ldout) = scale * MTTKRP of mode position n, from the column-major
 // factors fac[d] (leading dimension ld[d]) of all mode positions.  Returns the number of kernel launches.
+// imputed (masked objects): the MTTKRP of the imputed tensor S + (1-W).*[[B]] = (S - W.*[[B]]) + [[B]], i.e. the sparse
+// pass over r plus the low-rank term B_n * (Hadamard of cg_k, k != n); else the MTTKRP of the stored values.
 int sparse_mttkrp(SparseTensor& s, int n, const double* const* fac, const long long* ld, double scale, double* out,
-                  long long ldout, cudaStream_t st);
+                  long long ldout, cudaStream_t st, bool imputed = false);
+// masked objects: cg_n = B_n' * F (F: dims[n] x R, leading dimension ld), after every update of position n
+int sparse_cross_gram(SparseTensor& s, int n, const double* F, long long ld, cudaStream_t st);
+// masked objects: the EM step of cmtf_fun_AOADMM.m:408-441 without a dense tensor.  One pass over the nonzeros computes
+// m' = [[F]] there; sums[2] = sum s m', sums[3] = sum m'^2 (masked objective), sums[0] / sums[1] = the missing-entry
+// numerator / denominator of f_rel_missing from the telescoped ||[[F]] - [[B]]||^2 and ||[[B]]||^2, sums[4] = 0.
+// impute: afterwards m = m', r = s - m', B = F and the cross-Grams are refreshed.  Graph-capturable.
+int sparse_em(SparseTensor& s, const double* const* fac, const long long* ld, bool impute, double* sums, cudaStream_t st);
 
 }  // namespace aoadmm

@@ -13,7 +13,8 @@
 //
 // Sparse CP objects arrive as struct('subs',S,'vals',V,'size',sz) (cmtf_fun_AOADMM.m unwrap_data: sptensor or a MATLAB
 // sparse matrix through find); the 1-based double subscripts become 0-based int64 and the handle is created with
-// aoadmm_create_sparse (one GPU, no Z.miss, CP only: anything else raises aoadmm:unsupported).
+// aoadmm_create_sparse (one GPU, CP only: anything else raises aoadmm:unsupported).  Z.miss{p} of a sparse object must
+// be sparse too (the same struct); its nonzeros mark the observed entries (aoadmm_create_sparse_masked).
 //
 // Error handling: mexErrMsgIdAndTxt leaves mexFunction with a longjmp that runs no C++ destructor, so nothing in
 // here calls it directly - failures travel as a C++ exception (MexError) to the bottom of mexFunction, where every
@@ -215,7 +216,10 @@ void solve(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
   std::vector<std::vector<int64_t>> sp_subs(P);
   std::vector<aoadmm_sparse_object> sp_obj(P);
   std::vector<const aoadmm_sparse_object*> sp_ptr(P, nullptr);
-  bool any_sparse = false;
+  bool any_sparse = false, any_mask = false;
+  std::vector<std::vector<int64_t>> mk_subs(P);
+  std::vector<aoadmm_sparse_object> mk_obj(P);
+  std::vector<const aoadmm_sparse_object*> mk_ptr(P, nullptr);
   std::vector<std::vector<std::vector<uint8_t>>> miss_par2(P);
   std::vector<std::vector<const uint8_t*>> miss_par2_ptr(P);
   for (int p = 0; p < P; ++p)
@@ -294,8 +298,20 @@ void solve(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
       o.shard_extent = mode_rows[obj_modes[p][order - 1] - 1];
     }
     const mxArray* mp = (miss != nullptr && mxIsCell(miss) && p < (int)mxGetNumberOfElements(miss)) ? mxGetCell(miss, p) : nullptr;
+    if (mp != nullptr && is_coo_struct(mp)) {   // sparse mask (unwrap_data of an sptensor / sparse Z.miss{p})
+      if (sp_ptr[p] == nullptr)
+        fail("aoadmm:invalidArg", "Z.miss{" + std::to_string(p + 1) + "} is sparse but Z.object{" + std::to_string(p + 1) + "} is dense");
+      std::vector<int64_t> rows(order);
+      for (int d = 0; d < order; ++d) rows[d] = mode_rows[obj_modes[p][d] - 1];
+      coo_subs(mp, p, order, rows, mk_subs[p], &mk_obj[p].nnz);
+      mk_obj[p].subs = mk_subs[p].data();
+      mk_obj[p].vals = mk_obj[p].nnz > 0 ? mxGetPr(mxGetField(mp, 0, "vals")) : nullptr;
+      mk_ptr[p] = &mk_obj[p];
+      any_mask = true;
+      continue;
+    }
     if (mp != nullptr && !mxIsEmpty(mp) && sp_ptr[p] != nullptr)
-      fail("aoadmm:unsupported", "Z.miss{" + std::to_string(p + 1) + "} on a sparse object: missing data needs a dense object");
+      fail("aoadmm:unsupported", "Z.miss{" + std::to_string(p + 1) + "} on a sparse object: a sparse object needs a sparse mask");
     if (mp != nullptr && !mxIsEmpty(mp)) {  // EM imputation of the entries with Z.miss == 0 (cmtf_fun_AOADMM.m:408-441)
       if (par2) {
         const int K = o.n_slices;
@@ -414,7 +430,9 @@ void solve(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
   if (n_gpus < 1) fail("aoadmm:invalidArg", "options.b200_gpus must be >= 1");
   if (any_sparse && n_gpus > 1) fail("aoadmm:unsupported", "sparse objects run on one GPU (options.b200_gpus must be 1)");
   HandleGuard guard;
-  if (any_sparse)
+  if (any_mask)
+    check(aoadmm_create_sparse_masked(&pb, sp_ptr.data(), mk_ptr.data(), nullptr, &guard.h), nullptr);
+  else if (any_sparse)
     check(aoadmm_create_sparse(&pb, sp_ptr.data(), nullptr, &guard.h), nullptr);
   else
     check(n_gpus > 1 ? aoadmm_create_multi(&pb, n_gpus, nullptr, &guard.h) : aoadmm_create(&pb, nullptr, &guard.h), nullptr);

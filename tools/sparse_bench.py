@@ -9,13 +9,25 @@
                 sparse 2^20 x 2^16 matrix with ~2e7 nonzeros: a problem whose dense form (2^54 = 1.8e16 entries) cannot exist.
                 CPU baseline: NumPy COO MTTKRP on the host cores on a 1 % nonzero sample, extrapolated in proportion to nnz.
 
+  m1            131072 x 32768 rating matrix with ~2.5e7 observed entries (power-law rows and columns, rank 32 + noise)
+                and a sparse mask of exactly those entries, coupled in mode 2 to a dense 32768 x 1024 side matrix, R = 32,
+                nonneg: the sparse-mask engine against the dense EM engine on full(S) + the dense mask (34 GB + 4.3 GB
+                on the host and the device; that arm is skipped, with the reason, when the host cannot hold it), both
+                from the same state; outer it/s, the per-iteration phase split (torch.profiler kernel times), compare,
+                and the held-out RMSE on 1 % of the entries withheld from both.
+  m2            2^20 x 2^16 x 2^10 with 1e8 observed power-law entries and their mask, R = 32, nonneg (no dense form):
+                it/s, the phase split, the create time, and the overhead against the same object without the mask.
+                CPU baseline as in s2: NumPy imputed pass (model at the entries + residual MTTKRP per mode) on a 1 %
+                sample, extrapolated in proportion to nnz.
+
 Every line carries the card name and power limit (nvidia-smi, read in the same call), the create time (upload + sorts),
 the per-mode sparse MTTKRP time (CUDA events, aoadmm_time_mttkrp), outer iterations/s, and the algorithmic bytes per mode
 computed from the shapes: stream = nnz (8 + 4 (N-1)) + row pointers + output, gathered upper bound = nnz (N-1) 8 R, and
 the stream rate against the 6557 GB/s measured copy peak.  nnz is the number of nonzeros handed to the engine (before
 duplicates are merged).
 
-usage: python tools/sparse_bench.py [--workloads s1,s2] [--densities 0.001,0.01,0.1] [--s2-scale 1.0] [--iters 5]
+usage: python tools/sparse_bench.py [--workloads s1,s2,m1,m2] [--densities 0.001,0.01,0.1] [--s2-scale 1.0]
+                                    [--m-scale 1.0] [--iters 5]
 """
 import argparse
 import json
@@ -198,11 +210,204 @@ def s2(scale, iters, reps, seed=0, R=32):
                                              'cores': os.cpu_count(), 'ms_per_mode': cpu_ms}}
 
 
+# ---- m1 / m2: sparse objects with a sparse Z.miss mask ------------------------------------------------------------
+def mem_available_bytes():
+    try:
+        with open('/proc/meminfo') as f:
+            for line in f:
+                if line.startswith('MemAvailable:'):
+                    return int(line.split()[1]) * 1024
+    except OSError:
+        pass
+    return 0
+
+
+def phase_split(solver, G, iters, order):
+    """Per-iteration device time of the masked-sparse phases from one profiled run (graph off so that every kernel is
+    listed): the imputation pass, each mode's sparse MTTKRP (unit pass + fix-up), the low-rank terms, the EM norms
+    (stacked Grams + telescoped reduction) and everything else, in ms."""
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+    solver.set_state(G)
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        solver.run(options(iters, graph=-1))
+        torch.cuda.synchronize()
+    ev = sorted((e for e in prof.events() if e.device_type == torch.autograd.DeviceType.CUDA),
+                key=lambda e: e.time_range.start)
+    out = {'impute_pass': 0.0, 'lowrank': 0.0, 'em_norms': 0.0, 'factor_transposes': 0.0, 'other': 0.0}
+    for n in range(order):
+        out['mttkrp_mode%d' % (n + 1)] = 0.0
+    k_sp = k_fix = 0
+    follow = None      # category of the GEMM launched right after a hadamard / stack kernel
+    for e in ev:
+        nm, us = e.name, e.time_range.elapsed_us() / 1e3
+        if 'sp_model_kernel' in nm:
+            cat = 'impute_pass'
+        elif 'sp_mttkrp_kernel' in nm:
+            cat = 'mttkrp_mode%d' % (k_sp % order + 1)
+            k_sp += 1
+        elif 'sp_fixup_kernel' in nm:
+            cat = 'mttkrp_mode%d' % (k_fix % order + 1)
+            k_fix += 1
+        elif 'hadamard_others' in nm:
+            cat, follow = 'lowrank', 'lowrank'
+        elif 'stack3' in nm or 'tele_partials' in nm or 'em_final' in nm or 'cg_from_g3' in nm:
+            cat, follow = 'em_norms', 'em_norms'
+        elif 'dgemm' in nm and follow is not None:
+            cat = follow
+            if 'reduce' in nm or follow == 'lowrank':
+                follow = None
+        elif 'transpose_scale' in nm:
+            cat = 'factor_transposes'
+        else:
+            cat = 'other'
+            follow = None
+        out[cat] += us
+    return {k: v / iters for k, v in out.items()}
+
+
+def rating_data(rng, I, J, n_obs, n_test, R, noise=0.1):
+    """~n_obs + n_test distinct power-law (i, j) with values (A B')_ij (1 + noise N(0,1)), A, B ~ U(0,1)."""
+    want = n_obs + n_test
+    lin = np.empty(0, dtype=np.int64)
+    while lin.size < want:
+        m = int(1.3 * (want - lin.size)) + 1000
+        lin = np.unique(np.r_[lin, powerlaw(rng, m, I) * J + np.minimum((J * rng.rand(m) ** 2).astype(np.int64), J - 1)])
+    lin = lin[rng.permutation(lin.size)[:want]]
+    i, j = lin // J, lin % J
+    A, B = rng.rand(I, R), rng.rand(J, R)
+    vals = np.empty(want)
+    for a in range(0, want, 1 << 22):
+        sl = slice(a, a + (1 << 22))
+        v = np.einsum('er,er->e', A[i[sl]], B[j[sl]])
+        vals[sl] = v * (1.0 + noise * rng.randn(v.size))
+    return i, j, vals, B
+
+
+def m1(scale, iters, seed=0, R=32):
+    rng = np.random.RandomState(seed)
+    I, J, L = 131072, 32768, 1024
+    n_obs = int(2.5e7 * scale)
+    n_test = n_obs // 100
+    i, j, vals, B = rating_data(rng, I, J, n_obs, n_test, R)
+    nrm = np.linalg.norm(vals[:n_obs])
+    vals /= nrm                                                            # observed part at unit norm
+    subs = np.stack([i[:n_obs], j[:n_obs]], axis=1)
+    S = ab.sptensor(subs, vals[:n_obs], (I, J))
+    Wm = ab.sptensor(subs, np.ones(n_obs), (I, J))
+    Y = B @ rng.rand(L, R).T
+    Y = np.asfortranarray(Y * (1.0 + 0.1 * rng.randn(J, L)))
+    Y /= np.linalg.norm(Y)
+    zY = float(np.sum(Y * Y))
+    n = 4
+
+    def Zof(obj, miss):
+        return {'loss_function': ['Frobenius'] * 2, 'model': ['CP'] * 2, 'modes': [[1, 2], [3, 4]],
+                'size': [I, J, J, L],
+                'coupling': {'lin_coupled_modes': [0, 1, 1, 0], 'coupling_type': [0], 'coupl_trafo_matrices': [None] * n},
+                'constrained_modes': [1] * n, 'constraints': [('non-negativity',)] * n, 'weights': [0.5, 0.5],
+                'object': [obj, Y], 'miss': [miss, None], 'rank': [R, R]}
+
+    Zs = Zof(S, Wm)
+    G = init_state(Zs, R, seed + 1)
+    sp, t_sp = timed_create(Zs, [float('nan'), zY])
+    line = {'workload': 'm1', 'shape': [I, J], 'side_shape': [J, L], 'R': R, 'observed': n_obs, 'held_out': n_test,
+            'iters': iters, 'create_s': {'sparse_mask': t_sp}}
+    sp.set_state(G)
+    o_sp = sp.run(options(iters))
+    G_sp = sp.get_state()
+    dense_bytes = I * J * 9
+    avail = mem_available_bytes()
+    de = None
+    if avail < 2.5 * dense_bytes:
+        line['dense_arm'] = 'skipped: the host has %.1f GB available, the dense arm needs about %.1f GB' % (
+            avail / 1e9, 2.5 * dense_bytes / 1e9)
+    else:
+        Xd = np.zeros((I, J), order='F')
+        Xd[subs[:, 0], subs[:, 1]] = vals[:n_obs]
+        Md = np.zeros((I, J), dtype=np.uint8, order='F')
+        Md[subs[:, 0], subs[:, 1]] = 1
+        de, t_de = timed_create(Zof(Xd, Md), [float('nan'), zY])
+        del Xd, Md
+        line['create_s']['dense_em'] = t_de
+        de.set_state(G)
+        o_de = de.run(options(iters))
+        G_de = de.get_state()
+        line['compare'] = {
+            'factors_max_rel': max(float(np.linalg.norm(a - b) / np.linalg.norm(b)) for a, b in zip(G_sp['fac'], G_de['fac'])),
+            'objective_max_abs': float(np.max(np.abs(o_sp['func_val_conv'] - o_de['func_val_conv']))),
+            'f_rel_missing_max_abs': float(np.max(np.abs(o_sp['func_rel_missing'][1:] - o_de['func_rel_missing'][1:])))}
+    ips = {'sparse_mask': [], 'dense_em': []}
+    for _ in range(2):
+        ips['sparse_mask'].append(iters_per_s(sp, G, iters))
+        if de is not None:
+            ips['dense_em'].append(iters_per_s(de, G, iters))
+    line['outer_iters_per_s'] = {k: float(np.median(v)) for k, v in ips.items() if v}
+    line['phase_ms_per_iter'] = {'sparse_mask': phase_split(sp, G, iters, 2)}
+    pred = np.einsum('er,er->e', G_sp['fac'][0][i[n_obs:]], G_sp['fac'][1][j[n_obs:]])
+    line['held_out_rmse'] = float(np.sqrt(np.mean((pred - vals[n_obs:]) ** 2)))
+    line['held_out_rms_value'] = float(np.sqrt(np.mean(vals[n_obs:] ** 2)))
+    line['f_rel_missing_last'] = float(o_sp['f_rel_missing'])
+    sp.close()
+    if de is not None:
+        de.close()
+    return line
+
+
+def m2(scale, iters, seed=0, R=32):
+    rng = np.random.RandomState(seed)
+    shape = (1 << 20, 1 << 16, 1 << 10)
+    nnz = int(1e8 * scale)
+    subs = np.stack([powerlaw(rng, nnz, shape[0]), powerlaw(rng, nnz, shape[1]), powerlaw(rng, nnz, shape[2])], axis=1)
+    vals = rng.rand(nnz)
+    n = 3
+    Z = {'loss_function': ['Frobenius'], 'model': ['CP'], 'modes': [[1, 2, 3]], 'size': list(shape),
+         'coupling': {'lin_coupled_modes': [0] * n, 'coupling_type': [], 'coupl_trafo_matrices': [None] * n},
+         'constrained_modes': [1] * n, 'constraints': [('non-negativity',)] * n, 'weights': [1.0],
+         'object': [ab.sptensor(subs, vals, shape)], 'rank': [R]}
+    Zm = dict(Z, miss=[ab.sptensor(subs, np.ones(nnz), shape)])
+    G = init_state(Zm, R, seed + 1)
+    sp, t_sp = timed_create(Zm, [float('nan')])
+    un, t_un = timed_create(Z, [float('nan')])
+    ips = {'sparse_mask': [], 'no_mask': []}
+    for _ in range(2):
+        ips['sparse_mask'].append(iters_per_s(sp, G, iters))
+        ips['no_mask'].append(iters_per_s(un, G, iters))
+    med = {k: float(np.median(v)) for k, v in ips.items()}
+    phases = {'sparse_mask': phase_split(sp, G, iters, 3), 'no_mask': phase_split(un, G, iters, 3)}
+    sp.close()
+    un.close()
+    # CPU baseline: the imputed pass in NumPy on a 1 % sample, extrapolated in proportion to nnz
+    pick = rng.rand(nnz) < 0.01
+    ss, sv = subs[pick], vals[pick]
+    U = [np.random.RandomState(k).rand(s, R) for k, s in enumerate(shape)]
+    t0 = time.perf_counter()
+    m = np.ones((ss.shape[0], R))
+    for d in range(3):
+        m *= U[d][ss[:, d]]
+    r = sv - m.sum(axis=1)
+    for k in range(3):
+        contrib = r[:, None] * np.ones((1, R))
+        for d in range(3):
+            if d != k:
+                contrib *= U[d][ss[:, d]]
+        out = np.zeros((shape[k], R))
+        np.add.at(out, ss[:, k], contrib)
+    cpu_ms = (time.perf_counter() - t0) * 1e3 * nnz / max(int(pick.sum()), 1)
+    return {'workload': 'm2', 'shape': list(shape), 'R': R, 'nnz': nnz, 'iters': iters,
+            'create_s': {'sparse_mask': t_sp, 'no_mask': t_un}, 'outer_iters_per_s': med,
+            'mask_overhead': med['no_mask'] / med['sparse_mask'] - 1.0, 'phase_ms_per_iter': phases,
+            'cpu_baseline': {'kind': 'numpy imputed pass (model at the entries + residual MTTKRP of every mode) on the '
+                                     'host cores, 1 % nonzero sample, extrapolated in proportion to nnz',
+                             'cores': os.cpu_count(), 'ms_per_iteration': cpu_ms}}
+
+
 def main():
     ap = argparse.ArgumentParser(description=__doc__.split('\n')[0])
     ap.add_argument('--workloads', default='s1,s2')
     ap.add_argument('--densities', default='0.001,0.01,0.1')
     ap.add_argument('--s2-scale', type=float, default=1.0, help='fraction of the s2 nonzero counts (1.0 = 2e8 / 2e7)')
+    ap.add_argument('--m-scale', type=float, default=1.0, help='fraction of the m1 / m2 observed-entry counts')
     ap.add_argument('--iters', type=int, default=5)
     ap.add_argument('--reps', type=int, default=5)
     a = ap.parse_args()
@@ -215,6 +420,10 @@ def main():
             print(json.dumps(dict(s1(d, a.iters, a.reps), card=c)), flush=True)
     if 's2' in wl:
         print(json.dumps(dict(s2(a.s2_scale, a.iters, a.reps), card=c)), flush=True)
+    if 'm1' in wl:
+        print(json.dumps(dict(m1(a.m_scale, a.iters), card=c)), flush=True)
+    if 'm2' in wl:
+        print(json.dumps(dict(m2(a.m_scale, a.iters), card=c)), flush=True)
 
 
 if __name__ == '__main__':
