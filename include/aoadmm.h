@@ -32,7 +32,8 @@ extern "C" {
  * 4: aoadmm_create_multi / aoadmm_gpu_count / aoadmm_comm_release, communicators cached per process,
  *    aoadmm_out.non_finite_mode appended (a non-finite inner residual no longer aborts the run);
  *    later additions that leave every v4 struct and entry point unchanged: aoadmm_sparse_object / aoadmm_create_sparse
- *    (sparse CP objects), aoadmm_create_sparse_masked (sparse Z.miss masks on sparse objects). */
+ *    (sparse CP objects), aoadmm_create_sparse_masked (sparse Z.miss masks on sparse objects), aoadmm_model_at /
+ *    aoadmm_set_heldout / aoadmm_heldout_history (held-out entries). */
 #define AOADMM_ABI_VERSION 4
 
 typedef struct aoadmm_handle aoadmm_handle;
@@ -256,6 +257,31 @@ int aoadmm_create_sparse(const aoadmm_problem *problem, const aoadmm_sparse_obje
  * observed pattern differs from the stored one (the message names the object). */
 int aoadmm_create_sparse_masked(const aoadmm_problem *problem, const aoadmm_sparse_object *const *sparse,
                                 const aoadmm_sparse_object *const *masks, const aoadmm_dist *dist, aoadmm_handle **out);
+
+/* ---- held-out entries: how well the model predicts entries it was not trained on ----------------
+ * aoadmm_model_at:   out[e] = the current model [[F_1, ..., F_N]] of CP object `object` (1-based) at the 0-based
+ *                    subscripts entries->subs (entries->vals is ignored), in the caller's order.  Any CP object (dense,
+ *                    sparse, with or without missing data) on any handle; with several GPUs device 0 evaluates (the
+ *                    factors are replicated).
+ * aoadmm_set_heldout: attaches a held-out set (entries withheld from training, with their true values) to a CP object
+ *                    with missing data (a dense Z.miss, or a sparse mask of aoadmm_create_sparse_masked); entries = NULL
+ *                    detaches it.  Duplicates are summed; the set is sorted once on the device, so results and their
+ *                    bits do not depend on the order of the entries.  Everything is uploaded and allocated here: every
+ *                    aoadmm_run then also computes the held-out SSE = sum (v - m)^2 after each outer iteration, inside
+ *                    the CUDA graph when replay is on, with no extra synchronisation.  Attaching a set does not change
+ *                    the solve (factors, duals and every out field are bit-identical).  With several GPUs the set is
+ *                    replicated and every rank computes the same SSE without communication.  A failed call leaves the
+ *                    object without a held-out set.
+ * aoadmm_heldout_history: sse[i] (i < n) = the held-out SSE after outer iteration i of the last aoadmm_run, for
+ *                    i = 0..OuterIterations (0 = the initial state, evaluated with the iteration-0 objective); NaN
+ *                    beyond it.  *count (may be NULL) = the number of held-out entries after merging duplicates.
+ * Checked before any device is touched: AOADMM_ERR_INVALID_ARG for NULL pointers, nnz < 0, an object index out of range,
+ * a PARAFAC2 object, a subscript out of range, a held-out set on an object without missing data.  After the device sort,
+ * aoadmm_set_heldout returns AOADMM_ERR_INVALID_ARG when a held-out entry was observed in training (a nonzero byte of a
+ * dense mask, a stored entry of a sparse object); the message names the object and one such subscript. */
+int aoadmm_model_at(aoadmm_handle *h, int32_t object, const aoadmm_sparse_object *entries, double *out);
+int aoadmm_set_heldout(aoadmm_handle *h, int32_t object, const aoadmm_sparse_object *entries);
+int aoadmm_heldout_history(const aoadmm_handle *h, int32_t object, double *sse, int64_t n, int64_t *count);
 
 /* ---- state in / out (G is both input and output of cmtf_fun_AOADMM.m:1) ------------------- */
 int aoadmm_set_state(aoadmm_handle *h, int32_t field, int32_t index, int32_t slice,

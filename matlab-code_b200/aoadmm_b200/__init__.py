@@ -72,6 +72,38 @@ def as_sparse(X):
     return None
 
 
+def _check_heldout(Z, p, X):
+    """A held-out set `X` (sptensor or SciPy sparse) of object p (0-based) as an sptensor, checked on the host: a CP object
+    with missing data (Z.miss) and the shape of the object."""
+    P = len(Z['modes'])
+    if not 0 <= p < P:
+        raise AoadmmError(1, 'held-out set: object %d is out of range (1..%d)' % (p + 1, P))
+    if Z['model'][p] != 'CP':
+        raise AoadmmError(1, 'held-out set: object %d is a PARAFAC2 object (CP objects only)' % (p + 1))
+    S = as_sparse(X)
+    if S is None:
+        raise AoadmmError(1, 'held-out set of object %d must be an sptensor or a SciPy sparse matrix' % (p + 1))
+    miss = Z.get('miss') or [None] * P
+    if miss[p] is None:
+        raise AoadmmError(1, 'held-out set: object %d has no missing data (Z.miss); a held-out set is validated '
+                             'against what training did not observe' % (p + 1))
+    want = tuple(int(Z['size'][m - 1]) for m in Z['modes'][p])
+    if S.shape != want:
+        raise AoadmmError(1, 'held-out set: shape %s does not match object %d %s' % (S.shape, p + 1, want))
+    return S
+
+
+def _coo(subs, vals):
+    """aoadmm_sparse_object over column-major copies of subs (nnz x N) and vals; returns it with the arrays to keep."""
+    subs = np.asfortranarray(np.asarray(subs, dtype=np.int64))
+    vals = None if vals is None else np.ascontiguousarray(vals, dtype=np.float64)
+    so = _capi.SparseObject()
+    so.nnz = subs.shape[0]
+    so.subs = subs.ctypes.data_as(_capi.c_int64_p)
+    so.vals = None if vals is None else _dp(vals)
+    return so, (subs, vals)
+
+
 def device_count():
     n = C.c_int(0)
     _capi.check(lib.aoadmm_device_count(C.byref(n)))
@@ -522,6 +554,7 @@ class Solver:
         out.func_rel_missing = _dp(hmiss)
         _capi.check(lib.aoadmm_run(self._h, C.byref(o), C.byref(out)), self._h)
         it = out.OuterIterations
+        self._last_iters = it
         if out.exit_flag == 0:
             flag = 'maxIterations'                                        # make_exit_flag.m:4-5
         else:
@@ -534,6 +567,36 @@ class Solver:
                 'func_coupl_conv': hist[1][:it + 1].copy(), 'func_constr_conv': hist[2][:it + 1].copy(),
                 'func_PAR2_coupl': hist[3][:it + 1].copy(), 'time_at_it': hist[4][:it + 1].copy(),
                 'innerIters': inner[:, :it].astype(np.float64), 'non_finite_mode': int(out.non_finite_mode)}
+
+    # ---- held-out entries ---------------------------------------------------------------------
+    def model_at(self, obj, subs):
+        """The current model of CP object `obj` (1-based) at the 0-based subscripts `subs` (nnz x N), in their order."""
+        N = len(self.Z['modes'][obj - 1]) if 1 <= obj <= self.P else 1
+        subs = np.asarray(subs, dtype=np.int64).reshape(-1, N)
+        so, keep = _coo(subs, None)
+        out = np.zeros(subs.shape[0])
+        _capi.check(lib.aoadmm_model_at(self._h, int(obj), C.byref(so), _dp(out)), self._h)
+        return out
+
+    def set_heldout(self, obj, X):
+        """Attach the held-out set `X` (an sptensor or SciPy sparse matrix of entries withheld from training, with their
+        true values) to CP object `obj` (1-based), which must have missing data; X = None detaches it.  Every run then
+        records the held-out SSE after each outer iteration (heldout_history)."""
+        if X is None:
+            _capi.check(lib.aoadmm_set_heldout(self._h, int(obj), None), self._h)
+            return
+        S = _check_heldout(self.Z, obj - 1, X)
+        so, keep = _coo(S.subs, S.vals)
+        _capi.check(lib.aoadmm_set_heldout(self._h, int(obj), C.byref(so)), self._h)
+
+    def heldout_history(self, obj):
+        """(sse, count): the held-out SSE after outer iterations 0..OuterIterations of the last run, and the number of
+        held-out entries after merging duplicates."""
+        n = getattr(self, '_last_iters', -1) + 1
+        sse = np.full(max(n, 1), np.nan)
+        count = C.c_int64(0)
+        _capi.check(lib.aoadmm_heldout_history(self._h, int(obj), _dp(sse), n, C.byref(count)), self._h)
+        return sse[:n], count.value
 
     # ---- benchmark helpers --------------------------------------------------------------------
     def generate_cp_data(self, obj, factors, noise, seed):
@@ -611,14 +674,30 @@ def _with_rank(Z, G):
     return Z
 
 
-def cmtf_fun_AOADMM(Z, Znorm_const, G, fh=None, gh=None, lscalar=None, uscalar=None, options=None, **dist):
+def cmtf_fun_AOADMM(Z, Znorm_const, G, fh=None, gh=None, lscalar=None, uscalar=None, options=None, heldout=None,
+                    **dist):
     """[G,out] = cmtf_fun_AOADMM(Z,Znorm_const,G,fh,gh,lscalar,uscalar,options)  (cmtf_fun_AOADMM.m:1).
 
     fh/gh/lscalar/uscalar are [] for the Frobenius loss (cmtf_AOADMM.m:158-161) and are ignored.
+    `heldout`: one entry per object, None or a held-out set (sptensor / SciPy sparse) of an object with Z.miss; adds
+    out['heldout_sse'] (per object: the SSE after outer iterations 0..OuterIterations, or None) and out['heldout_count'].
     `dist` (rank, world_size, device, unique_id) selects the multi-GPU layout; default one GPU."""
+    if heldout is not None:
+        if len(heldout) != len(Z['modes']):
+            raise AoadmmError(1, 'heldout needs one entry per object (None where an object has no held-out set)')
+        for p, X in enumerate(heldout):
+            if X is not None:
+                _check_heldout(Z, p, X)
     with Solver(_with_rank(Z, G), Znorm_const, **dist) as s:
         s.set_state(G)
+        for p, X in enumerate(heldout or []):
+            if X is not None:
+                s.set_heldout(p + 1, X)
         out = s.run(options)
+        if heldout is not None:
+            hist = [s.heldout_history(p + 1) if X is not None else (None, None) for p, X in enumerate(heldout)]
+            out['heldout_sse'] = [h[0] for h in hist]
+            out['heldout_count'] = [h[1] for h in hist]
         Gout = s.get_state()
     return Gout, out
 

@@ -380,6 +380,29 @@ int aoadmm_time_mttkrp(aoadmm_handle* h, int32_t object, int32_t pos, int32_t re
   });
 }
 
+int aoadmm_model_at(aoadmm_handle* h, int32_t object, const aoadmm_sparse_object* entries, double* out) {
+  if (!h) return AOADMM_ERR_INVALID_ARG;
+  return guard(h, [&] {
+    if (entries == nullptr || (entries->nnz > 0 && out == nullptr))
+      throw aoadmm::CudaError(AOADMM_ERR_INVALID_ARG, "model_at: NULL entries / out");
+    h->eng[0]->check_entries(object, entries, false);
+    h->eng[0]->model_at(object, entries, out);   // the factors are replicated: device 0 evaluates
+  });
+}
+
+int aoadmm_set_heldout(aoadmm_handle* h, int32_t object, const aoadmm_sparse_object* entries) {
+  if (!h) return AOADMM_ERR_INVALID_ARG;
+  return guard(h, [&] {
+    h->eng[0]->check_entries(object, entries, true);   // every rank holds the same objects and modes
+    for_each_rank((int)h->eng.size(), [&](int r) { h->eng[r]->set_heldout(object, entries); });
+  });
+}
+
+int aoadmm_heldout_history(const aoadmm_handle* h, int32_t object, double* sse, int64_t n, int64_t* count) {
+  if (!h || n < 0 || (n > 0 && !sse)) return AOADMM_ERR_INVALID_ARG;
+  return guard(const_cast<aoadmm_handle*>(h), [&] { h->eng[0]->heldout_history(object, sse, n, count); });
+}
+
 int aoadmm_launch_count(const aoadmm_handle* h, int64_t* count) {
   if (!h || !count) return AOADMM_ERR_INVALID_ARG;
   int64_t total = 0;

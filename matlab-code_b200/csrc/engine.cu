@@ -855,6 +855,11 @@ void Engine::release() {
   }
   modes_.clear();
   for (auto& o : objects_) {
+    if (o.ho != nullptr) {
+      heldout_free(*o.ho);
+      delete o.ho;
+      o.ho = nullptr;
+    }
     if (o.sp != nullptr) {
       sparse_free(*o.sp);
       delete o.sp;
@@ -906,6 +911,8 @@ void Engine::release() {
   dfree(em_sums_);
   dfree(em_partials_);
   hfree(em_sums_host_);
+  dfree(ho_sse_);
+  hfree(ho_sse_host_);
   hfree(ctl_host_);
   hfree(red_host_);
   for (auto& e : run_ev_) {
@@ -1841,6 +1848,33 @@ void Engine::enqueue_objective(bool first) {
   launches_ += reduce_jobs(jobs_dev_, nj, red_dev_, red_partials_, admm_counter_, st_, nullptr);
   AO_CUDA(cudaMemcpyAsync(red_host_, red_dev_, sizeof(double) * nj, cudaMemcpyDeviceToHost, st_));
   AO_CUDA(cudaMemcpyAsync(ctl_host_, ctl_dev_, sizeof(InnerCtl) * n_ctl_, cudaMemcpyDeviceToHost, st_));
+  if (n_heldout_ > 0) heldout_pass();
+}
+
+// held-out SSE of every object with a held-out set, from the factors after this iteration's sweep and EM step.  It
+// only reads the factors, so the solve is the same with and without held-out sets.  The factors are replicated on
+// every rank, so every rank computes the same value without communication.
+void Engine::heldout_pass() {
+  phase_begin(2);
+  for (int p = 0; p < n_objects_; ++p) {
+    ObjectState& o = objects_[p];
+    if (o.ho == nullptr) continue;
+    const double* fac[8];
+    long long ld[8];
+    for (int d = 0; d < o.order; ++d) {
+      const ModeState& md = mode(o.modes[d]);
+      fac[d] = md.fac.p;
+      ld[d] = md.rows;
+    }
+    launches_ += heldout_sse(*o.ho, fac, ld, ho_sse_ + p, st_);
+  }
+  phase_end();
+  AO_CUDA(cudaMemcpyAsync(ho_sse_host_, ho_sse_, sizeof(double) * n_objects_, cudaMemcpyDeviceToHost, st_));
+}
+
+void Engine::record_heldout() {
+  for (int p = 0; p < n_objects_; ++p)
+    if (objects_[p].ho != nullptr) objects_[p].ho_hist.push_back(ho_sse_host_[p]);
 }
 
 // host part: the scalar arithmetic of :1213-1363 on the reduced values
@@ -2243,7 +2277,9 @@ void Engine::run(const aoadmm_options* opt, aoadmm_out* out) {
   }
   double f[4];
   em_step(false);                           // masked iteration-0 objective needs the model at the observed entries
+  for (auto& o : objects_) o.ho_hist.clear();
   eval_objective(true, f);                  // :32
+  record_heldout();
   f_rel_missing_ = std::nan("");
   if (out->func_rel_missing) out->func_rel_missing[0] = f_rel_missing_;
   if (out->func_val_conv) out->func_val_conv[0] = f[0];
@@ -2320,6 +2356,7 @@ void Engine::run(const aoadmm_options* opt, aoadmm_out* out) {
       enqueue_objective(false);                                      // :447
     }
     finish_objective(false, f);                                      // synchronises
+    record_heldout();
     check_errors(out);
     if (out->func_val_conv) out->func_val_conv[iter] = f[0];
     if (out->func_coupl_conv) out->func_coupl_conv[iter] = f[1];
@@ -2733,6 +2770,121 @@ float Engine::time_mttkrp(int object, int pos, int reps) {
   cudaEventDestroy(a);
   cudaEventDestroy(b);
   return ms / (float)std::max(reps, 1);
+}
+
+// ---------------------------------------------------------------------------------------------------
+// held-out entries (aoadmm_model_at, aoadmm_set_heldout, aoadmm_heldout_history)
+// ---------------------------------------------------------------------------------------------------
+void Engine::check_entries(int object, const aoadmm_sparse_object* entries, bool heldout) const {
+  const std::string who = std::string(heldout ? "set_heldout" : "model_at") + ": object " + std::to_string(object);
+  if (object < 1 || object > n_objects_) throw CudaError(1, who + " is out of range");
+  const ObjectState& o = objects_[object - 1];
+  if (o.model != AOADMM_MODEL_CP) throw CudaError(1, who + " is a PARAFAC2 object (CP objects only)");
+  if (entries == nullptr) return;
+  if (entries->nnz < 0) throw CudaError(1, who + ": nnz is negative");
+  if (entries->nnz > 0x7fffffffLL - kSparseChunk) throw CudaError(1, who + ": more than 2^31 - 257 entries");
+  if (entries->nnz > 0 && (entries->subs == nullptr || (heldout && entries->vals == nullptr)))
+    throw CudaError(1, who + ": subs / vals is NULL");
+  if (heldout && o.mask == nullptr && !sparse_masked(o))
+    throw CudaError(1, who + " has no missing data (a held-out set needs a dense Z.miss or a sparse mask)");
+  for (int d = 0; d < o.order; ++d) {
+    const int64_t rows = modes_[o.modes[d] - 1].rows;
+    const int64_t* sd = entries->subs + (size_t)d * (size_t)entries->nnz;
+    for (int64_t e = 0; e < entries->nnz; ++e)
+      if (sd[e] < 0 || sd[e] >= rows)
+        throw CudaError(1, who + ": subscript " + std::to_string(sd[e]) + " of entry " + std::to_string(e) +
+                               " is out of range for mode position " + std::to_string(d + 1));
+  }
+}
+
+void Engine::model_at(int object, const aoadmm_sparse_object* entries, double* out) {
+  AO_CUDA(cudaSetDevice(device_));
+  const ObjectState& o = objects_[object - 1];
+  const double* fac[8];
+  long long rows[8];
+  for (int d = 0; d < o.order; ++d) {
+    const ModeState& md = modes_[o.modes[d] - 1];
+    fac[d] = md.fac.p;
+    rows[d] = md.rows;
+  }
+  model_at_host(o.order, modes_[o.modes[0] - 1].R, fac, rows, entries->nnz,
+                reinterpret_cast<const long long*>(entries->subs), out, st_);
+}
+
+void Engine::set_heldout(int object, const aoadmm_sparse_object* entries) {
+  AO_CUDA(cudaSetDevice(device_));
+  ObjectState& o = objects_[object - 1];
+  if (o.ho != nullptr) {
+    AO_CUDA(cudaStreamSynchronize(st_));
+    heldout_free(*o.ho);
+    delete o.ho;
+    o.ho = nullptr;
+    o.ho_hist.clear();
+    --n_heldout_;
+  }
+  if (entries == nullptr) return;
+  if (ho_sse_ == nullptr) {
+    AO_CUDA(cudaMalloc(&ho_sse_, sizeof(double) * n_objects_));
+    AO_CUDA(cudaMemset(ho_sse_, 0, sizeof(double) * n_objects_));
+    AO_CUDA(cudaMallocHost(&ho_sse_host_, sizeof(double) * n_objects_));
+  }
+  std::unique_ptr<HeldOut> h(new HeldOut());
+  long long dims[8];
+  for (int d = 0; d < o.order; ++d) dims[d] = modes_[o.modes[d] - 1].rows;
+  try {
+    heldout_build(*h, o.order, dims, modes_[o.modes[0] - 1].R, entries->nnz,
+                  reinterpret_cast<const long long*>(entries->subs), entries->vals, st_);
+    // a held-out entry that was observed in training would make the validation error meaningless
+    long long first = -1, count = 0;
+    if (o.sp != nullptr) {
+      count = heldout_stored(*h, *o.sp, &first, st_);
+    } else {
+      std::vector<long long> ld(o.dims.begin(), o.dims.end());
+      count = heldout_masked(*h, o.mask, o.ld0, ld.data(), o.shard_offset, &first, st_);
+      if (o.sharded) {   // each rank checked the entries of its slab: one all-reduce of the counts and first positions
+        std::vector<double> hb(world_ + 1, 0.0);
+        hb[0] = (double)count;
+        hb[1 + rank_] = (double)(first + 1);
+        double* db = nullptr;
+        AO_CUDA(cudaMalloc(&db, hb.size() * sizeof(double)));
+        try {
+          AO_CUDA(cudaMemcpyAsync(db, hb.data(), hb.size() * sizeof(double), cudaMemcpyHostToDevice, st_));
+          allreduce(db, hb.size());
+          AO_CUDA(cudaMemcpyAsync(hb.data(), db, hb.size() * sizeof(double), cudaMemcpyDeviceToHost, st_));
+          AO_CUDA(cudaStreamSynchronize(st_));
+        } catch (...) {
+          cudaFree(db);
+          throw;
+        }
+        cudaFree(db);
+        count = (long long)hb[0];
+        first = -1;
+        for (int r = 0; r < world_ && first < 0; ++r)
+          if (hb[1 + r] > 0.0) first = (long long)hb[1 + r] - 1;
+      }
+    }
+    if (count > 0) {
+      long long sub[8];
+      heldout_subscript(*h, first, sub, st_);
+      std::string s = "(";
+      for (int d = 0; d < o.order; ++d) s += (d ? ", " : "") + std::to_string(sub[d]);
+      throw CudaError(1, "set_heldout: object " + std::to_string(object) + ": " + std::to_string(count) +
+                             " held-out entries are observed in training, e.g. the entry at 0-based subscript " + s + ")");
+    }
+  } catch (...) {
+    heldout_free(*h);
+    throw;
+  }
+  o.ho = h.release();
+  ++n_heldout_;
+}
+
+void Engine::heldout_history(int object, double* sse, int64_t n, int64_t* count) const {
+  if (object < 1 || object > n_objects_) throw CudaError(1, "heldout_history: object out of range");
+  const ObjectState& o = objects_[object - 1];
+  if (o.ho == nullptr) throw CudaError(1, "heldout_history: object " + std::to_string(object) + " has no held-out set");
+  for (int64_t i = 0; i < n; ++i) sse[i] = i < (int64_t)o.ho_hist.size() ? o.ho_hist[i] : std::nan("");
+  if (count != nullptr) *count = o.ho->n;
 }
 
 }  // namespace aoadmm

@@ -8,6 +8,7 @@
 
 #include "../../include/aoadmm.h"
 #include "em.cuh"
+#include "heldout.cuh"
 #include "linalg.cuh"
 #include "mttkrp.cuh"
 #include "nvecs.cuh"
@@ -170,6 +171,8 @@ struct ObjectState {
   double* Tbuf = nullptr;     // dimension tree: T(j,k,r) = sum_i X(i,j,k) F1(i,r), emitted by the mode-2 MTTKRP
   uint64_t T_version = 0;     // version of the mode-1 factor T was computed from (0 = invalid)
   SparseTensor* sp = nullptr; // sparse (COO) object: sorted device copies (sparse.cuh); data, views stay empty
+  HeldOut* ho = nullptr;      // held-out set (aoadmm_set_heldout), replicated on every rank
+  std::vector<double> ho_hist;  // held-out SSE after outer iteration 0, 1, ... of the last run
 };
 
 class Engine {
@@ -206,6 +209,11 @@ class Engine {
   void nvecs_to_host(int mode_id, int slice, int r, double* out, int64_t rows, double* info);
   void nvecs_sharded_mode(ObjectState& o, int r, double* out, int64_t rows, double* info);
   void mttkrp_to_host(int object, int pos, double* out, int precision = -1);  // unweighted MTTKRP of the resident factors (-1: precision of the last run)
+  // held-out entries (aoadmm_model_at / aoadmm_set_heldout): host-only checks of object and subscripts, then the work
+  void check_entries(int object, const aoadmm_sparse_object* entries, bool heldout) const;
+  void model_at(int object, const aoadmm_sparse_object* entries, double* out);   // on this engine's device
+  void set_heldout(int object, const aoadmm_sparse_object* entries);             // collective over the ranks
+  void heldout_history(int object, double* sse, int64_t n, int64_t* count) const;
   int64_t launches() const { return launches_; }
   void phase_ms(double ms[3]);
   double last_run_ms() const { return last_run_ms_; }
@@ -312,6 +320,11 @@ class Engine {
   double* em_sums_host_ = nullptr;  // pinned
   double* em_partials_ = nullptr;
   double f_rel_missing_ = 0.0;
+  int n_heldout_ = 0;             // objects with a held-out set
+  double* ho_sse_ = nullptr;      // device, one per object: held-out SSE of the current iteration
+  double* ho_sse_host_ = nullptr; // pinned
+  void heldout_pass();            // enqueued with the objective; the result rides on its device-to-host copies
+  void record_heldout();
   int64_t launches_ = 0;
   // timing
   std::vector<std::pair<cudaEvent_t, cudaEvent_t>> ev_pool_;

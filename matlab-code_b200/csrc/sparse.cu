@@ -132,6 +132,8 @@ __global__ void __launch_bounds__(256) transpose_scale_kernel(const double* __re
   }
 }
 
+}  // namespace
+
 int transpose_scale(const double* in, long long rows, long long cols, long long ldi, double* out, long long ldo, double scale,
                     cudaStream_t st) {
   if (rows <= 0 || cols <= 0) return 0;
@@ -140,6 +142,8 @@ int transpose_scale(const double* in, long long rows, long long cols, long long 
   AO_CHECK_LAUNCH();
   return 1;
 }
+
+namespace {
 
 struct SpArgs {
   const long long* rowptr;
@@ -242,21 +246,6 @@ void launch_sp(const SpArgs& a, cudaStream_t st) {
   AO_CHECK_LAUNCH();
 }
 
-// lanes per nonzero (G) and columns per lane (CPL) for rank R: f(integral_constant<G>, integral_constant<CPL>)
-template <typename Fn>
-void rank_dispatch(int R, Fn&& f) {
-  using std::integral_constant;
-  if (R <= 1) f(integral_constant<int, 1>{}, integral_constant<int, 1>{});
-  else if (R <= 2) f(integral_constant<int, 2>{}, integral_constant<int, 1>{});
-  else if (R <= 4) f(integral_constant<int, 4>{}, integral_constant<int, 1>{});
-  else if (R <= 8) f(integral_constant<int, 8>{}, integral_constant<int, 1>{});
-  else if (R <= 16) f(integral_constant<int, 16>{}, integral_constant<int, 1>{});
-  else if (R <= 32) f(integral_constant<int, 32>{}, integral_constant<int, 1>{});
-  else if (R <= 64) f(integral_constant<int, 32>{}, integral_constant<int, 2>{});
-  else if (R <= 128) f(integral_constant<int, 32>{}, integral_constant<int, 4>{});
-  else f(integral_constant<int, 32>{}, integral_constant<int, 8>{});
-}
-
 // ---- EM imputation of masked sparse objects ----
 struct ModelArgs {
   long long nnz;
@@ -284,28 +273,7 @@ __global__ void __launch_bounds__(256) sp_model_kernel(const ModelArgs a) {
   for (int q0 = 0; q0 < kSparseChunk; ++q0) {
     const long long e = e0 + q0;
     const bool ok = e < a.nnz;
-    double t = 0.0;
-    if (ok) {
-      double p[CPL];
-      const double* f0 = a.F[0] + (long long)__ldg(a.row0 + e) * R;
-#pragma unroll
-      for (int q = 0; q < CPL; ++q) {
-        const int c = gl + G * q;
-        p[q] = c < R ? __ldg(f0 + c) : 0.0;
-      }
-      for (int m = 0; m < a.no; ++m) {
-        const double* f = a.F[m + 1] + (long long)__ldg(a.idx + m * a.nnz + e) * R;
-#pragma unroll
-        for (int q = 0; q < CPL; ++q) {
-          const int c = gl + G * q;
-          if (c < R) p[q] *= __ldg(f + c);
-        }
-      }
-#pragma unroll
-      for (int q = 0; q < CPL; ++q) t += p[q];
-    }
-#pragma unroll
-    for (int off = G / 2; off > 0; off >>= 1) t += __shfl_xor_sync(0xffffffffu, t, off);
+    const double t = model_at_entry<G, CPL>(a.F, a.row0, a.idx, a.nnz, a.no, R, e, gl, ok);
     if (ok && gl == 0) {
       const double s = __ldg(a.vals + e), mo = a.m[e], d = t - mo;
       s0 = fma(s, t, s0);
@@ -331,12 +299,15 @@ __global__ void __launch_bounds__(256) sp_model_kernel(const ModelArgs a) {
   }
 }
 
-// CTAs of the model pass: one group of G lanes per unit of kSparseChunk nonzeros
+}  // namespace
+
 long long model_blocks(long long nnz, int R) {
   long long b = 0;
   rank_dispatch(R, [&](auto g, auto) { b = ceil_div(ceil_div(nnz, kSparseChunk) * decltype(g)::value, 256); });
   return b;
 }
+
+namespace {
 
 // S = [F | B | F - B] (rows x 3R, ld = rows); impute: B = F afterwards
 __global__ void stack3_kernel(const double* __restrict__ F, long long ldf, double* __restrict__ B, long long rows, int R,
@@ -675,6 +646,30 @@ void sparse_build(SparseTensor& s, int order, const long long* dims, int R, long
     s.em_partials = dalloc<double>(2 * kTeleBlocks + 4 * (size_t)model_blocks(nm, R));
   }
   AO_CUDA(cudaStreamSynchronize(st));
+}
+
+long long coo_sort_merge(int order, const long long* dims, long long n, const long long* subs, const double* vals,
+                         cudaStream_t st, int** subs_out, double** vals_out) {
+  Temps tmp;
+  SortWs w;
+  int* ms = nullptr;
+  double* mv = nullptr;
+  const long long nm = sort_merge(tmp, w, order, dims, n, subs, vals, st, ms, mv);
+  int* so = dalloc<int>((size_t)order * nm);
+  double* vo = nullptr;
+  try {
+    vo = dalloc<double>(nm);
+    AO_CUDA(cudaMemcpyAsync(so, ms, (size_t)order * nm * sizeof(int), cudaMemcpyDeviceToDevice, st));
+    AO_CUDA(cudaMemcpyAsync(vo, mv, (size_t)nm * sizeof(double), cudaMemcpyDeviceToDevice, st));
+    AO_CUDA(cudaStreamSynchronize(st));
+  } catch (...) {
+    cudaFree(so);
+    if (vo) cudaFree(vo);
+    throw;
+  }
+  *subs_out = so;
+  *vals_out = vo;
+  return nm;
 }
 
 void sparse_free(SparseTensor& s) {

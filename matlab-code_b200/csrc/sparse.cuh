@@ -13,6 +13,7 @@
 // starts and ends inside the unit is written directly, the partial rows at the unit's ends go to carry buffers, and a
 // fix-up pass adds the carries of a split row in unit order.  No floating-point atomics: every output is bit-reproducible.
 #pragma once
+#include <type_traits>
 #include <vector>
 
 #include "common.cuh"
@@ -20,6 +21,66 @@
 namespace aoadmm {
 
 constexpr int kSparseChunk = 256;   // nonzeros per unit of work
+
+// lanes per nonzero (G) and columns per lane (CPL) for rank R: f(integral_constant<G>, integral_constant<CPL>)
+template <typename Fn>
+void rank_dispatch(int R, Fn&& f) {
+  using std::integral_constant;
+  if (R <= 1) f(integral_constant<int, 1>{}, integral_constant<int, 1>{});
+  else if (R <= 2) f(integral_constant<int, 2>{}, integral_constant<int, 1>{});
+  else if (R <= 4) f(integral_constant<int, 4>{}, integral_constant<int, 1>{});
+  else if (R <= 8) f(integral_constant<int, 8>{}, integral_constant<int, 1>{});
+  else if (R <= 16) f(integral_constant<int, 16>{}, integral_constant<int, 1>{});
+  else if (R <= 32) f(integral_constant<int, 32>{}, integral_constant<int, 1>{});
+  else if (R <= 64) f(integral_constant<int, 32>{}, integral_constant<int, 2>{});
+  else if (R <= 128) f(integral_constant<int, 32>{}, integral_constant<int, 4>{});
+  else f(integral_constant<int, 32>{}, integral_constant<int, 8>{});
+}
+
+// CTAs of a pass in which one group of G lanes walks each unit of kSparseChunk entries
+long long model_blocks(long long n, int R);
+
+// m(e) = sum_c prod_d F_d(i_d, c) for entry e of a COO list: position-1 subscripts row0[e], positions 2..no+1 at
+// idx[(d-1) * stride + e]; F row-major.  Lane gl of a group of G owns columns gl, gl + G, ... (ascending), the group
+// sums its lanes with a fixed xor tree, so the bits depend on R and the data only.  Every lane of the warp must call it
+// (ok = false: the lane has no entry and contributes 0).
+template <int G, int CPL>
+__device__ __forceinline__ double model_at_entry(const double* const (&F)[8], const int* row0, const int* idx,
+                                                 long long stride, int no, int R, long long e, int gl, bool ok) {
+  double t = 0.0;
+  if (ok) {
+    double p[CPL];
+    const double* f0 = F[0] + (long long)__ldg(row0 + e) * R;
+#pragma unroll
+    for (int q = 0; q < CPL; ++q) {
+      const int c = gl + G * q;
+      p[q] = c < R ? __ldg(f0 + c) : 0.0;
+    }
+    for (int m = 0; m < no; ++m) {
+      const double* f = F[m + 1] + (long long)__ldg(idx + m * stride + e) * R;
+#pragma unroll
+      for (int q = 0; q < CPL; ++q) {
+        const int c = gl + G * q;
+        if (c < R) p[q] *= __ldg(f + c);
+      }
+    }
+#pragma unroll
+    for (int q = 0; q < CPL; ++q) t += p[q];
+  }
+#pragma unroll
+  for (int off = G / 2; off > 0; off >>= 1) t += __shfl_xor_sync(0xffffffffu, t, off);
+  return t;
+}
+
+// out(j + ldo*i) = scale * in(i + ldi*j), i < rows, j < cols (the row-major factor copies).  Returns the launches.
+int transpose_scale(const double* in, long long rows, long long cols, long long ldi, double* out, long long ldo, double scale,
+                    cudaStream_t st);
+
+// Uploads n > 0 COO entries (subs n x order column-major, 0-based, validated by the caller), sorts them on the device
+// into full lexicographic order (mode 0 major) and sums duplicates.  *subs_out (order x nm int32, column-major) and
+// *vals_out (nm) are new device allocations owned by the caller.  Synchronous on `st`; returns nm.
+long long coo_sort_merge(int order, const long long* dims, long long n, const long long* subs, const double* vals,
+                         cudaStream_t st, int** subs_out, double** vals_out);
 
 struct SparseMode {
   long long* rowptr = nullptr;      // rows + 1

@@ -488,6 +488,27 @@ void solve(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
   o.fuse_inner = (int32_t)opt_scalar(opt, "b200_fuse_inner", 0.0);
   o.graph = (int32_t)opt_scalar(opt, "b200_graph", 0.0);      // engine knob: 0 auto, 1 on, -1 off
 
+  // options.b200_heldout{p}: held-out set of object p (unwrap_data struct of an sptensor / sparse matrix), empty = none
+  const mxArray* hcell = field(opt, "b200_heldout", false);
+  std::vector<bool> has_ho(P, false);
+  if (hcell != nullptr && mxIsCell(hcell)) {
+    for (int p = 0; p < P && p < (int)mxGetNumberOfElements(hcell); ++p) {
+      const mxArray* hp = mxGetCell(hcell, p);
+      if (hp == nullptr || mxIsEmpty(hp)) continue;
+      if (!is_coo_struct(hp) || objs[p].model != AOADMM_MODEL_CP)
+        fail("aoadmm:invalidArg", "options.b200_heldout{" + std::to_string(p + 1) + "} must be an sptensor or a sparse matrix of a CP object");
+      const int order = objs[p].order;
+      std::vector<int64_t> rows(order), hs;
+      for (int d = 0; d < order; ++d) rows[d] = mode_rows[obj_modes[p][d] - 1];
+      aoadmm_sparse_object ho{};
+      coo_subs(hp, p, order, rows, hs, &ho.nnz);
+      ho.subs = hs.data();
+      ho.vals = ho.nnz > 0 ? mxGetPr(mxGetField(hp, 0, "vals")) : nullptr;
+      check(aoadmm_set_heldout(h, p + 1, &ho), h);
+      has_ho[p] = true;
+    }
+  }
+
   const int n_hist = o.MaxOuterIters + 1;
   mxArray* hist[6];
   for (auto& a : hist) a = mxCreateDoubleMatrix(1, n_hist, mxREAL);
@@ -540,8 +561,8 @@ void solve(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
   if (nlhs > 1) {
     const char* names[] = {"f_tensors", "f_couplings", "f_constraints", "f_PAR2_couplings", "f_rel_missing", "exit_flag",
                            "OuterIterations", "func_val_conv", "func_coupl_conv", "func_constr_conv", "func_PAR2_coupl",
-                           "time_at_it", "innerIters", "func_rel_missing", "non_finite_mode"};
-    mxArray* out = mxCreateStructMatrix(1, 1, 15, names);
+                           "time_at_it", "innerIters", "func_rel_missing", "non_finite_mode", "heldout_sse"};
+    mxArray* out = mxCreateStructMatrix(1, 1, 16, names);
     mxSetField(out, 0, "non_finite_mode", mxCreateDoubleScalar((double)ro.non_finite_mode));
     mxSetField(out, 0, "f_tensors", mxCreateDoubleScalar(ro.f_tensors));
     mxSetField(out, 0, "f_couplings", mxCreateDoubleScalar(ro.f_couplings));
@@ -568,6 +589,14 @@ void solve(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
     for (int c = 0; c < it; ++c)
       for (int m = 0; m < nb_modes; ++m) mxGetPr(ii)[(size_t)c * nb_modes + m] = (double)inner[(size_t)c * nb_modes + m];
     mxSetField(out, 0, "innerIters", ii);
+    // (it+1) x P held-out SSE histories, NaN columns for objects without a held-out set (cmtf_fun_AOADMM.m makes the cell)
+    mxArray* hs = mxCreateDoubleMatrix(it + 1, P, mxREAL);
+    for (int p = 0; p < P; ++p) {
+      double* col = mxGetPr(hs) + (size_t)p * (it + 1);
+      if (has_ho[p]) check(aoadmm_heldout_history(h, p + 1, col, it + 1, nullptr), h);
+      else for (int i = 0; i <= it; ++i) col[i] = mxGetNaN();
+    }
+    mxSetField(out, 0, "heldout_sse", hs);
     plhs[1] = out;
   } else {
     for (auto& a : hist) mxDestroyArray(a);

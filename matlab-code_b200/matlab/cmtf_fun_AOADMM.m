@@ -14,7 +14,9 @@ function [G,out] = cmtf_fun_AOADMM(Z,Znorm_const,G,fh,gh,lscalar,uscalar,options
 % reference's MATLAB solver).
 % Engine options (fields of `options`, all optional): b200_gpus = number of B200s of this box the call uses (the
 % tensors are cut into mode-3 slabs inside the library, one MATLAB process drives all of them), b200_dimtree,
-% b200_mttkrp_precision, b200_fuse_inner, b200_graph.
+% b200_mttkrp_precision, b200_fuse_inner, b200_graph, b200_heldout{p} = an sptensor / sparse matrix of entries of object p
+% withheld from training (with their true values; object p needs Z.miss): out.heldout_sse{p} is then the held-out SSE
+% after outer iterations 0..OuterIterations.
     % hand the gateway plain numeric arrays: X.data of a Tensor Toolbox tensor shares its memory with X (copy-on-write),
     % whereas mxGetProperty inside a MEX file would deep-copy the whole tensor
     for p = 1:numel(Z.object)
@@ -23,7 +25,20 @@ function [G,out] = cmtf_fun_AOADMM(Z,Znorm_const,G,fh,gh,lscalar,uscalar,options
             Z.miss{p} = unwrap_data(Z.miss{p});
         end
     end
+    heldout = isfield(options,'b200_heldout');
+    if heldout
+        options.b200_heldout = unwrap_data(options.b200_heldout);
+    end
     [G,out] = aoadmm_mex(Z, Znorm_const, G, options);
+    if heldout   % one history per object: a cell, empty where an object has no held-out set
+        hs = out.heldout_sse;
+        out.heldout_sse = cell(1, size(hs,2));
+        for p = 1:numel(options.b200_heldout)
+            if ~isempty(options.b200_heldout{p}), out.heldout_sse{p} = hs(:,p).'; end
+        end
+    else
+        out = rmfield(out, 'heldout_sse');
+    end
     if out.non_finite_mode > 0
         warning('aoadmm:nonFinite', 'a residual of the inner ADMM loop of mode %d was NaN/Inf (a factor or dual of norm 0)', out.non_finite_mode);
     end

@@ -14,9 +14,12 @@
                 nonneg: the sparse-mask engine against the dense EM engine on full(S) + the dense mask (34 GB + 4.3 GB
                 on the host and the device; that arm is skipped, with the reason, when the host cannot hold it), both
                 from the same state; outer it/s, the per-iteration phase split (torch.profiler kernel times), compare,
-                and the held-out RMSE on 1 % of the entries withheld from both.
+                and the held-out RMSE on 1 % of the entries withheld from both, over every iteration, from the device
+                held-out history (aoadmm_set_heldout), with the outer it/s with and without the held-out set, the
+                held-out pass time next to the imputation pass, and the time of the host NumPy evaluation it replaces.
   m2            2^20 x 2^16 x 2^10 with 1e8 observed power-law entries and their mask, R = 32, nonneg (no dense form):
-                it/s, the phase split, the create time, and the overhead against the same object without the mask.
+                it/s, the phase split, the create time, and the overhead against the same object without the mask;
+                the same held-out measurements as m1 with 1e7 unobserved power-law entries held out.
                 CPU baseline as in s2: NumPy imputed pass (model at the entries + residual MTTKRP per mode) on a 1 %
                 sample, extrapolated in proportion to nnz.
 
@@ -234,7 +237,8 @@ def phase_split(solver, G, iters, order):
         torch.cuda.synchronize()
     ev = sorted((e for e in prof.events() if e.device_type == torch.autograd.DeviceType.CUDA),
                 key=lambda e: e.time_range.start)
-    out = {'impute_pass': 0.0, 'lowrank': 0.0, 'em_norms': 0.0, 'factor_transposes': 0.0, 'other': 0.0}
+    out = {'impute_pass': 0.0, 'heldout_pass': 0.0, 'lowrank': 0.0, 'em_norms': 0.0, 'factor_transposes': 0.0,
+           'other': 0.0}
     for n in range(order):
         out['mttkrp_mode%d' % (n + 1)] = 0.0
     k_sp = k_fix = 0
@@ -243,6 +247,8 @@ def phase_split(solver, G, iters, order):
         nm, us = e.name, e.time_range.elapsed_us() / 1e3
         if 'sp_model_kernel' in nm:
             cat = 'impute_pass'
+        elif 'heldout_kernel' in nm or 'sum_partials_kernel' in nm:   # its factor transposes: factor_transposes
+            cat = 'heldout_pass'
         elif 'sp_mttkrp_kernel' in nm:
             cat = 'mttkrp_mode%d' % (k_sp % order + 1)
             k_sp += 1
@@ -284,6 +290,40 @@ def rating_data(rng, I, J, n_obs, n_test, R, noise=0.1):
     return i, j, vals, B
 
 
+def heldout_first_run(sp, G, iters, H, host_model):
+    """A run of `sp` with the held-out set H attached: the held-out RMSE curve over all iterations from the device history,
+    and what that replaces: the factors read back and the model evaluated at the held-out entries in NumPy
+    (host_model(fac) -> predictions).  Returns (fields, out, state); the set stays attached."""
+    sp.set_heldout(1, H)
+    sp.set_state(G)
+    out = sp.run(options(iters))
+    sse, count = sp.heldout_history(1)
+    t0 = time.perf_counter()
+    Gh = sp.get_state()
+    pred = host_model(Gh['fac'])
+    host_sse = float(np.sum((H.vals - pred) ** 2))
+    host_ms = (time.perf_counter() - t0) * 1e3
+    return {'heldout_entries': count, 'held_out_rmse_curve': [float(x) for x in np.sqrt(sse / count)],
+            'held_out_rmse': float(np.sqrt(sse[-1] / count)), 'held_out_rmse_host': float(np.sqrt(host_sse / count)),
+            'host_eval_ms': host_ms}, out, Gh
+
+
+def heldout_legs(sp, G, iters, H, order):
+    """Outer it/s without and with the held-out set H attached (alternating) and the per-iteration held-out pass and
+    imputation pass times (profiled run).  Leaves the set detached."""
+    ips = {'no_heldout': [], 'heldout': []}
+    for _ in range(2):
+        sp.set_heldout(1, None)
+        ips['no_heldout'].append(iters_per_s(sp, G, iters))
+        sp.set_heldout(1, H)
+        ips['heldout'].append(iters_per_s(sp, G, iters))
+    med = {k: float(np.median(v)) for k, v in ips.items()}
+    ph = phase_split(sp, G, iters, order)
+    sp.set_heldout(1, None)
+    return {'heldout_outer_iters_per_s': med, 'heldout_it_s_change': med['heldout'] / med['no_heldout'] - 1.0,
+            'heldout_pass_ms_per_iter': ph['heldout_pass'], 'impute_pass_ms_per_iter': ph['impute_pass']}
+
+
 def m1(scale, iters, seed=0, R=32):
     rng = np.random.RandomState(seed)
     I, J, L = 131072, 32768, 1024
@@ -313,9 +353,11 @@ def m1(scale, iters, seed=0, R=32):
     sp, t_sp = timed_create(Zs, [float('nan'), zY])
     line = {'workload': 'm1', 'shape': [I, J], 'side_shape': [J, L], 'R': R, 'observed': n_obs, 'held_out': n_test,
             'iters': iters, 'create_s': {'sparse_mask': t_sp}}
-    sp.set_state(G)
-    o_sp = sp.run(options(iters))
-    G_sp = sp.get_state()
+    H = ab.sptensor(np.stack([i[n_obs:], j[n_obs:]], axis=1), vals[n_obs:], (I, J))
+    # the first run carries the held-out set (it does not change the solve): RMSE curve on the device, host evaluation
+    held, o_sp, G_sp = heldout_first_run(sp, G, iters, H, lambda F: np.einsum('er,er->e', F[0][i[n_obs:]], F[1][j[n_obs:]]))
+    sp.set_heldout(1, None)
+    line.update(held)
     dense_bytes = I * J * 9
     avail = mem_available_bytes()
     de = None
@@ -343,9 +385,8 @@ def m1(scale, iters, seed=0, R=32):
         if de is not None:
             ips['dense_em'].append(iters_per_s(de, G, iters))
     line['outer_iters_per_s'] = {k: float(np.median(v)) for k, v in ips.items() if v}
+    line.update(heldout_legs(sp, G, iters, H, 2))
     line['phase_ms_per_iter'] = {'sparse_mask': phase_split(sp, G, iters, 2)}
-    pred = np.einsum('er,er->e', G_sp['fac'][0][i[n_obs:]], G_sp['fac'][1][j[n_obs:]])
-    line['held_out_rmse'] = float(np.sqrt(np.mean((pred - vals[n_obs:]) ** 2)))
     line['held_out_rms_value'] = float(np.sqrt(np.mean(vals[n_obs:] ** 2)))
     line['f_rel_missing_last'] = float(o_sp['f_rel_missing'])
     sp.close()
@@ -369,12 +410,35 @@ def m2(scale, iters, seed=0, R=32):
     G = init_state(Zm, R, seed + 1)
     sp, t_sp = timed_create(Zm, [float('nan')])
     un, t_un = timed_create(Z, [float('nan')])
+    # 1e7 held-out entries: power-law subscripts that are not observed, random true values
+    n_held = int(1e7 * scale)
+    key = lambda a: (a[:, 0] * shape[1] + a[:, 1]) * shape[2] + a[:, 2]
+    hs = np.empty((0, 3), dtype=np.int64)
+    obs = np.sort(key(subs))
+    while hs.shape[0] < n_held:
+        c = np.stack([powerlaw(rng, 2 * n_held, s) for s in shape], axis=1)
+        k = key(c)
+        pos = np.searchsorted(obs, k).clip(max=obs.size - 1)
+        c = c[obs[pos] != k]
+        hs = np.unique(np.vstack([hs, c]), axis=0)
+    hs = hs[rng.permutation(hs.shape[0])[:n_held]]
+    H = ab.sptensor(hs, rng.rand(n_held), shape)
+
+    def host_model(F):
+        m = np.ones((n_held, R))
+        for d in range(3):
+            m *= F[d][hs[:, d]]
+        return m.sum(axis=1)
+
+    held, _, _ = heldout_first_run(sp, G, iters, H, host_model)
+    sp.set_heldout(1, None)
     ips = {'sparse_mask': [], 'no_mask': []}
     for _ in range(2):
         ips['sparse_mask'].append(iters_per_s(sp, G, iters))
         ips['no_mask'].append(iters_per_s(un, G, iters))
     med = {k: float(np.median(v)) for k, v in ips.items()}
     phases = {'sparse_mask': phase_split(sp, G, iters, 3), 'no_mask': phase_split(un, G, iters, 3)}
+    held.update(heldout_legs(sp, G, iters, H, 3))
     sp.close()
     un.close()
     # CPU baseline: the imputed pass in NumPy on a 1 % sample, extrapolated in proportion to nnz
@@ -397,6 +461,7 @@ def m2(scale, iters, seed=0, R=32):
     return {'workload': 'm2', 'shape': list(shape), 'R': R, 'nnz': nnz, 'iters': iters,
             'create_s': {'sparse_mask': t_sp, 'no_mask': t_un}, 'outer_iters_per_s': med,
             'mask_overhead': med['no_mask'] / med['sparse_mask'] - 1.0, 'phase_ms_per_iter': phases,
+            'heldout': held,
             'cpu_baseline': {'kind': 'numpy imputed pass (model at the entries + residual MTTKRP of every mode) on the '
                                      'host cores, 1 % nonzero sample, extrapolated in proportion to nnz',
                              'cores': os.cpu_count(), 'ms_per_iteration': cpu_ms}}
