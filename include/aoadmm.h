@@ -33,7 +33,8 @@ extern "C" {
  *    aoadmm_out.non_finite_mode appended (a non-finite inner residual no longer aborts the run);
  *    later additions that leave every v4 struct and entry point unchanged: aoadmm_sparse_object / aoadmm_create_sparse
  *    (sparse CP objects), aoadmm_create_sparse_masked (sparse Z.miss masks on sparse objects), aoadmm_model_at /
- *    aoadmm_set_heldout / aoadmm_heldout_history (held-out entries). */
+ *    aoadmm_set_heldout / aoadmm_heldout_history (held-out entries), aoadmm_sparse_shard_bounds /
+ *    aoadmm_create_sparse_multi (sparse objects on several GPUs from one caller). */
 #define AOADMM_ABI_VERSION 4
 
 typedef struct aoadmm_handle aoadmm_handle;
@@ -257,6 +258,39 @@ int aoadmm_create_sparse(const aoadmm_problem *problem, const aoadmm_sparse_obje
  * observed pattern differs from the stored one (the message names the object). */
 int aoadmm_create_sparse_masked(const aoadmm_problem *problem, const aoadmm_sparse_object *const *sparse,
                                 const aoadmm_sparse_object *const *masks, const aoadmm_dist *dist, aoadmm_handle **out);
+
+/* ---- sparse objects on several GPUs from one caller ---------------------------------------------
+ * aoadmm_sparse_shard_bounds: bounds[0..n_gpus] of the slabs of the last mode (extent indices) into which
+ *     aoadmm_create_sparse_multi cuts a sparse object of `order` modes; GPU r owns indices bounds[r] .. bounds[r+1]-1.
+ *     The slabs balance the number of nonzeros: with c[k] = the number of entries whose last subscript is k (duplicates
+ *     counted before merging), C[k] = c[0] + ... + c[k-1] and nnz = so->nnz, bounds[0] = 0, bounds[n] = extent and for
+ *     r = 1..n-1 bounds[r] = the smallest k with C[k] * n >= r * nnz, clamped to [bounds[r-1] + 1, extent - (n - r)] so
+ *     that every GPU owns at least one index.  nnz = 0: the uniform slabs of dense objects (extent * r / n).  The bounds
+ *     depend on the multiset of subscripts only, never on their order.  Host only; touches no device.
+ *     AOADMM_ERR_INVALID_ARG for NULL pointers, order outside 2..8, n_gpus < 1, nnz < 0, a last subscript outside
+ *     0..extent-1, and extent < n_gpus (fewer indices than there are GPUs).
+ * aoadmm_create_sparse_multi: aoadmm_create_multi for a problem with sparse objects (sparse[p], masks[p] as in
+ *     aoadmm_create_sparse_masked; masks may be NULL).  Takes whole objects.  Dense objects are cut as
+ *     aoadmm_create_multi cuts them; every sparse CP object (order 2..8, matrices included) is cut into the slabs of
+ *     aoadmm_sparse_shard_bounds, and its mask with the object's bounds.  The caller's entries are copied once into
+ *     slab order on the host (8 * order + 8 bytes per nonzero of an object or mask, plus 4 bytes per nonzero while the
+ *     bounds are computed); each GPU's worker thread then uploads and sorts only its own entries, so a GPU holds about
+ *     1/n_gpus of the nonzeros and the limit of 2^31 - 257 nonzeros applies per GPU.  The factors stay replicated and
+ *     full-size; per outer iteration every MTTKRP of a sparse object is all-reduced once (its last position as the
+ *     zero-padded gather of the slabs), and a masked object all-reduces 4 more numbers in its EM step.  The results
+ *     equal those of one GPU up to the summation order of the all-reduces; at a fixed n_gpus they are bit-reproducible
+ *     and do not depend on the order of the nonzeros.  n_gpus = 1 gives the handle of aoadmm_create_sparse{,_masked}
+ *     on devices[0].  Every check of aoadmm_create_sparse_masked and of aoadmm_sparse_shard_bounds on the descriptors
+ *     happens before any device is touched; then the device checks of aoadmm_create_multi.  A mask whose observed
+ *     pattern differs from the stored one inside one GPU's slab fails the whole create with AOADMM_ERR_UNSUPPORTED
+ *     naming the object, and every device is released.  aoadmm_object_mttkrp returns the summed product,
+ *     aoadmm_time_mttkrp times the slowest GPU's local pass; aoadmm_create_sparse{,_masked} with world_size > 1 stay
+ *     AOADMM_ERR_UNSUPPORTED (one process per GPU is not offered for sparse objects). */
+int aoadmm_sparse_shard_bounds(const aoadmm_sparse_object *so, int32_t order, int64_t extent, int32_t n_gpus,
+                               int64_t *bounds);
+int aoadmm_create_sparse_multi(const aoadmm_problem *problem, const aoadmm_sparse_object *const *sparse,
+                               const aoadmm_sparse_object *const *masks, int32_t n_gpus, const int32_t *devices,
+                               aoadmm_handle **out);
 
 /* ---- held-out entries: how well the model predicts entries it was not trained on ----------------
  * aoadmm_model_at:   out[e] = the current model [[F_1, ..., F_N]] of CP object `object` (1-based) at the 0-based

@@ -24,7 +24,7 @@ from ._capi import AoadmmError, lib
 
 __all__ = ['cmtf_fun_AOADMM', 'cmtf_AOADMM', 'cmtf_nvecs', 'init_coupled_AOADMM_CMTF', 'Solver', 'AoadmmError', 'sptensor', 'mttkrp',
            'prox', 'chol_solve', 'gram',
-           'shard_range', 'device_count', 'nccl_unique_id']
+           'shard_range', 'sparse_shard_bounds', 'device_count', 'nccl_unique_id']
 
 
 def _dp(a):
@@ -123,6 +123,20 @@ def shard_range(extent, rank, world_size):
     return lo, hi
 
 
+def sparse_shard_bounds(X, n_gpus):
+    """The n_gpus + 1 bounds of the last-mode slabs into which Solver(..., n_gpus=N, shard_sparse=True) cuts the sparse
+    object X (sptensor or SciPy sparse matrix): GPU r owns last-mode indices bounds[r] .. bounds[r+1]-1.  The slabs
+    balance the nonzeros (the rule is stated with aoadmm_sparse_shard_bounds in include/aoadmm.h)."""
+    S = as_sparse(X)
+    if S is None:
+        raise AoadmmError(1, 'sparse_shard_bounds: X must be an sptensor or a SciPy sparse matrix')
+    so, keep = _coo(S.subs, S.vals)
+    b = np.zeros(max(int(n_gpus), 0) + 1, dtype=np.int64)
+    _capi.check(lib.aoadmm_sparse_shard_bounds(C.byref(so), S.ndim, S.shape[-1], int(n_gpus),
+                                               b.ctypes.data_as(_capi.c_int64_p)))
+    return b
+
+
 def constraint_spec(c):
     """Z.constraints{m} (name, params...) -> aoadmm_constraint (constraints_to_prox.m:13-91)."""
     spec = _capi.Constraint()
@@ -154,12 +168,19 @@ class Solver:
     """Handle lifecycle around the C ABI: create (tensors to HBM once) -> set_state -> run -> get_state."""
 
     def __init__(self, Z, Znorm_const, rank=0, world_size=1, device=0, unique_id=None, shard=None, n_gpus=1,
-                 devices=None):
+                 devices=None, shard_sparse=False):
         """One GPU: defaults.  Several GPUs from THIS process (one caller, like a MATLAB session): n_gpus=N [, devices=[..]]
         with the whole objects in Z (aoadmm_create_multi cuts the slabs).  One process per GPU (torchrun): rank,
-        world_size, device, unique_id [, shard] with this rank's slab or the whole object in Z."""
+        world_size, device, unique_id [, shard] with this rank's slab or the whole object in Z.
+        shard_sparse=True (with n_gpus): sparse objects are cut into nonzero-balanced slabs of their last mode
+        (aoadmm_create_sparse_multi); `shards[p]` then lists the (lo, hi) slab of every GPU.  Without it sparse objects
+        run on one GPU only."""
         if n_gpus > 1 and world_size > 1:
             raise ValueError('n_gpus > 1 (one process drives all GPUs) and world_size > 1 (one process per GPU) exclude each other')
+        if shard_sparse and world_size > 1:
+            raise AoadmmError(2, 'shard_sparse: sparse objects are sharded by one caller driving n_gpus GPUs, not with one '
+                                 'process per GPU (world_size must be 1)')
+        self.shard_sparse = bool(shard_sparse)
         self.n_gpus = int(n_gpus)
         self._keep = []
         self._h = _capi.HandleP()
@@ -190,8 +211,9 @@ class Solver:
                 raise AoadmmError(2, 'object %d: PARAFAC2 objects with sparse slices are not supported' % (p + 1))
             if sparse[p] is None:
                 continue
-            if n_gpus > 1 or world_size > 1:
-                raise AoadmmError(2, 'object %d is sparse: sparse objects run on one GPU' % (p + 1))
+            if (n_gpus > 1 and not shard_sparse) or world_size > 1:
+                raise AoadmmError(2, 'object %d is sparse: sparse objects run on one GPU (or on n_gpus GPUs with '
+                                     'shard_sparse=True)' % (p + 1))
             if miss[p] is not None and smask[p] is None:
                 raise AoadmmError(2, 'object %d is sparse: a dense Z.miss needs a dense object (a sparse object takes a '
                                      'sparse mask of its stored entries)' % (p + 1))
@@ -230,7 +252,11 @@ class Solver:
             o.znorm_const = float(Znorm_const[p])
             if model[p] == 'CP' and sparse[p] is not None:
                 full_last = int(Z['size'][modes[p][-1] - 1])
-                self.shards.append((0, full_last))
+                if shard_sparse:
+                    b = sparse_shard_bounds(sparse[p], self.n_gpus)
+                    self.shards.append([(int(b[r]), int(b[r + 1])) for r in range(self.n_gpus)])
+                else:
+                    self.shards.append((0, full_last))
                 subs = np.asfortranarray(sparse[p].subs)    # column-major: subs[d*nnz + e]
                 vals = np.ascontiguousarray(sparse[p].vals)
                 so = _capi.SparseObject()
@@ -371,16 +397,21 @@ class Solver:
         self.rank, self.world_size = rank, world_size
         self.rows = rows
         self.nsl = nsl
-        if self.n_gpus > 1:
+        if self.n_gpus > 1 or shard_sparse:
             devs = None
             if devices is not None:
                 devs = np.asarray(list(devices), dtype=np.int32)
                 if devs.size != self.n_gpus:
                     raise ValueError('devices must list n_gpus ordinals')
                 self._keep.append(devs)
-            _capi.check(lib.aoadmm_create_multi(C.byref(pb), self.n_gpus,
-                                                devs.ctypes.data_as(_capi.c_int32_p) if devs is not None else None,
-                                                C.byref(self._h)))
+            dp = devs.ctypes.data_as(_capi.c_int32_p) if devs is not None else None
+            if shard_sparse:
+                self._keep += [sp_objs, sp_masks]
+                _capi.check(lib.aoadmm_create_sparse_multi(C.byref(pb), sp_objs,
+                                                           sp_masks if any(m is not None for m in smask) else None,
+                                                           self.n_gpus, dp, C.byref(self._h)))
+            else:
+                _capi.check(lib.aoadmm_create_multi(C.byref(pb), self.n_gpus, dp, C.byref(self._h)))
         else:
             if devices is not None:
                 dist.device = int(list(devices)[0])
@@ -681,7 +712,8 @@ def cmtf_fun_AOADMM(Z, Znorm_const, G, fh=None, gh=None, lscalar=None, uscalar=N
     fh/gh/lscalar/uscalar are [] for the Frobenius loss (cmtf_AOADMM.m:158-161) and are ignored.
     `heldout`: one entry per object, None or a held-out set (sptensor / SciPy sparse) of an object with Z.miss; adds
     out['heldout_sse'] (per object: the SSE after outer iterations 0..OuterIterations, or None) and out['heldout_count'].
-    `dist` (rank, world_size, device, unique_id) selects the multi-GPU layout; default one GPU."""
+    `dist` (rank, world_size, device, unique_id, or n_gpus [, devices, shard_sparse]) selects the multi-GPU layout;
+    default one GPU."""
     if heldout is not None:
         if len(heldout) != len(Z['modes']):
             raise AoadmmError(1, 'heldout needs one entry per object (None where an object has no held-out set)')

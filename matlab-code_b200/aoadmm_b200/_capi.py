@@ -96,7 +96,8 @@ EXPORTS = ['aoadmm_abi_version', 'aoadmm_device_count', 'aoadmm_nccl_unique_id',
            'aoadmm_chol_solve', 'aoadmm_gram', 'aoadmm_generate_cp_data', 'aoadmm_time_mttkrp', 'aoadmm_launch_count',
            'aoadmm_phase_ms', 'aoadmm_last_run_ms', 'aoadmm_get_object_data', 'aoadmm_last_loop_ms', 'aoadmm_object_mttkrp', 'aoadmm_nvecs',
            'aoadmm_create_multi', 'aoadmm_gpu_count', 'aoadmm_comm_release', 'aoadmm_create_sparse',
-           'aoadmm_create_sparse_masked', 'aoadmm_model_at', 'aoadmm_set_heldout', 'aoadmm_heldout_history']
+           'aoadmm_create_sparse_masked', 'aoadmm_model_at', 'aoadmm_set_heldout', 'aoadmm_heldout_history',
+           'aoadmm_sparse_shard_bounds', 'aoadmm_create_sparse_multi']
 
 lib.aoadmm_abi_version.restype = C.c_int
 lib.aoadmm_device_count.argtypes = [C.POINTER(C.c_int)]
@@ -107,6 +108,9 @@ lib.aoadmm_create_sparse.argtypes = [C.POINTER(Problem), C.POINTER(C.POINTER(Spa
 lib.aoadmm_create_sparse_masked.argtypes = [C.POINTER(Problem), C.POINTER(C.POINTER(SparseObject)),
                                             C.POINTER(C.POINTER(SparseObject)), C.POINTER(Dist), C.POINTER(HandleP)]
 lib.aoadmm_create_multi.argtypes = [C.POINTER(Problem), C.c_int32, c_int32_p, C.POINTER(HandleP)]
+lib.aoadmm_sparse_shard_bounds.argtypes = [C.POINTER(SparseObject), C.c_int32, C.c_int64, C.c_int32, c_int64_p]
+lib.aoadmm_create_sparse_multi.argtypes = [C.POINTER(Problem), C.POINTER(C.POINTER(SparseObject)),
+                                           C.POINTER(C.POINTER(SparseObject)), C.c_int32, c_int32_p, C.POINTER(HandleP)]
 lib.aoadmm_gpu_count.argtypes = [HandleP, c_int32_p]
 lib.aoadmm_comm_release.argtypes = []
 lib.aoadmm_destroy.argtypes = [HandleP]

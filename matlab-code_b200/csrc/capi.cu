@@ -117,6 +117,7 @@ int aoadmm_create(const aoadmm_problem* problem, const aoadmm_dist* dist, aoadmm
     h = new aoadmm_handle();
     h->eng.push_back(nullptr);
     h->eng[0] = new aoadmm::Engine(problem, dist);   // a throwing constructor has released everything it acquired
+    h->eng[0]->reduce_norms();
   });
   if (rc != AOADMM_OK) {
     delete h;
@@ -150,37 +151,42 @@ void check_coo(const aoadmm_problem* problem, const aoadmm_object& ob, const aoa
   }
 }
 
+// every check create_sparse / aoadmm_create_sparse_multi make on the sparse descriptors and masks; touches no device
+void check_sparse(const aoadmm_problem* problem, const aoadmm_sparse_object* const* sparse,
+                  const aoadmm_sparse_object* const* masks, const aoadmm_dist* dist) {
+  using aoadmm::CudaError;
+  if (problem == nullptr) throw CudaError(AOADMM_ERR_INVALID_ARG, "problem is NULL");
+  if (problem->n_objects > 0 && problem->objects == nullptr) throw CudaError(AOADMM_ERR_INVALID_ARG, "objects is NULL");
+  for (int p = 0; masks != nullptr && p < problem->n_objects; ++p) {
+    if (masks[p] == nullptr) continue;
+    const std::string who = "sparse mask " + std::to_string(p + 1) + ": ";
+    if (sparse == nullptr || sparse[p] == nullptr)
+      throw CudaError(AOADMM_ERR_INVALID_ARG, who + "a sparse mask needs a sparse object (dense objects take Z.miss)");
+    if (problem->objects[p].miss != nullptr)
+      throw CudaError(AOADMM_ERR_INVALID_ARG, who + "both a dense Z.miss and a sparse mask are set");
+    if (problem->objects[p].model == AOADMM_MODEL_CP) check_coo(problem, problem->objects[p], masks[p], who);
+  }
+  for (int p = 0; sparse != nullptr && p < problem->n_objects; ++p) {
+    const aoadmm_sparse_object* so = sparse[p];
+    if (so == nullptr) continue;
+    const aoadmm_object& ob = problem->objects[p];
+    const std::string who = "sparse object " + std::to_string(p + 1) + ": ";
+    if (dist != nullptr && dist->world_size > 1)
+      throw CudaError(AOADMM_ERR_UNSUPPORTED, who + "sparse objects run on one GPU (world_size must be 1)");
+    if (ob.model != AOADMM_MODEL_CP) throw CudaError(AOADMM_ERR_UNSUPPORTED, who + "PARAFAC2 objects must be dense");
+    if (ob.miss != nullptr) throw CudaError(AOADMM_ERR_UNSUPPORTED, who + "missing-data masks (Z.miss) need a dense object");
+    if (ob.data != nullptr) throw CudaError(AOADMM_ERR_INVALID_ARG, who + "both dense data and sparse data are set");
+    check_coo(problem, ob, so, who);
+  }
+}
+
 int create_sparse(const aoadmm_problem* problem, const aoadmm_sparse_object* const* sparse,
                   const aoadmm_sparse_object* const* masks, const aoadmm_dist* dist, aoadmm_handle** out) {
   if (!out) return AOADMM_ERR_INVALID_ARG;
   *out = nullptr;
   aoadmm_handle* h = nullptr;
   int rc = guard(nullptr, [&] {
-    using aoadmm::CudaError;
-    if (problem == nullptr) throw CudaError(AOADMM_ERR_INVALID_ARG, "problem is NULL");
-    if (problem->n_objects > 0 && problem->objects == nullptr) throw CudaError(AOADMM_ERR_INVALID_ARG, "objects is NULL");
-    // every check on the sparse descriptors and masks happens here, before a device is touched
-    for (int p = 0; masks != nullptr && p < problem->n_objects; ++p) {
-      if (masks[p] == nullptr) continue;
-      const std::string who = "sparse mask " + std::to_string(p + 1) + ": ";
-      if (sparse == nullptr || sparse[p] == nullptr)
-        throw CudaError(AOADMM_ERR_INVALID_ARG, who + "a sparse mask needs a sparse object (dense objects take Z.miss)");
-      if (problem->objects[p].miss != nullptr)
-        throw CudaError(AOADMM_ERR_INVALID_ARG, who + "both a dense Z.miss and a sparse mask are set");
-      if (problem->objects[p].model == AOADMM_MODEL_CP) check_coo(problem, problem->objects[p], masks[p], who);
-    }
-    for (int p = 0; sparse != nullptr && p < problem->n_objects; ++p) {
-      const aoadmm_sparse_object* so = sparse[p];
-      if (so == nullptr) continue;
-      const aoadmm_object& ob = problem->objects[p];
-      const std::string who = "sparse object " + std::to_string(p + 1) + ": ";
-      if (dist != nullptr && dist->world_size > 1)
-        throw CudaError(AOADMM_ERR_UNSUPPORTED, who + "sparse objects run on one GPU (world_size must be 1)");
-      if (ob.model != AOADMM_MODEL_CP) throw CudaError(AOADMM_ERR_UNSUPPORTED, who + "PARAFAC2 objects must be dense");
-      if (ob.miss != nullptr) throw CudaError(AOADMM_ERR_UNSUPPORTED, who + "missing-data masks (Z.miss) need a dense object");
-      if (ob.data != nullptr) throw CudaError(AOADMM_ERR_INVALID_ARG, who + "both dense data and sparse data are set");
-      check_coo(problem, ob, so, who);
-    }
+    check_sparse(problem, sparse, masks, dist);   // every check on the descriptors happens before a device is touched
     h = new aoadmm_handle();
     h->eng.push_back(nullptr);
     h->eng[0] = new aoadmm::Engine(problem, dist, nullptr, sparse, masks);
@@ -191,6 +197,194 @@ int create_sparse(const aoadmm_problem* problem, const aoadmm_sparse_object* con
   }
   *out = h;
   return AOADMM_OK;
+}
+
+// b[0..n]: the nonzero-balanced slab bounds of the last mode (include/aoadmm.h, aoadmm_sparse_shard_bounds).  With the
+// last subscripts sorted (s_0 <= s_1 <= ...), C[k] >= t holds exactly for k > s_{t-1}: the smallest k with
+// C[k] * n >= r * nnz is s_{t-1} + 1 for t = ceil(r * nnz / n) >= 1 (0 for t = 0).  The order statistics come from
+// nth_element on one int32 copy of the last subscripts (4 bytes per nonzero, O(nnz log n) time).
+void shard_bounds(const aoadmm_sparse_object* so, int order, int64_t ext, int n, int64_t* b, const std::string& who) {
+  using aoadmm::CudaError;
+  if (so == nullptr || b == nullptr) throw CudaError(AOADMM_ERR_INVALID_ARG, who + "NULL descriptor / bounds");
+  if (order < 2 || order > 8) throw CudaError(AOADMM_ERR_INVALID_ARG, who + "order must be in 2..8");
+  if (n < 1) throw CudaError(AOADMM_ERR_INVALID_ARG, who + "n_gpus must be >= 1");
+  if (ext < 0 || ext > 0x7fffffffLL) throw CudaError(AOADMM_ERR_INVALID_ARG, who + "the last mode must have 0..2^31 - 1 indices");
+  if (so->nnz < 0) throw CudaError(AOADMM_ERR_INVALID_ARG, who + "nnz is negative");
+  if (so->nnz > 0 && so->subs == nullptr) throw CudaError(AOADMM_ERR_INVALID_ARG, who + "subs is NULL");
+  if (ext < n)
+    throw CudaError(AOADMM_ERR_INVALID_ARG, who + "the last mode has fewer indices (" + std::to_string(ext) +
+                                                ") than there are GPUs");
+  const int64_t nnz = so->nnz;
+  const int64_t* last = so->subs + (size_t)(order - 1) * (size_t)nnz;
+  std::vector<int32_t> v((size_t)nnz);
+  for (int64_t e = 0; e < nnz; ++e) {
+    if (last[e] < 0 || last[e] >= ext)
+      throw CudaError(AOADMM_ERR_INVALID_ARG, who + "last-mode subscript " + std::to_string(last[e]) + " of nonzero " +
+                                                  std::to_string(e) + " is out of range");
+    v[e] = (int32_t)last[e];
+  }
+  b[0] = 0;
+  b[n] = ext;
+  size_t lo = 0;
+  for (int r = 1; r < n; ++r) {
+    int64_t k;
+    if (nnz == 0) {
+      k = ext * r / n;   // the uniform rule of dense slabs
+    } else {
+      const int64_t t = (r * nnz + n - 1) / n;
+      if (t == 0) {
+        k = 0;
+      } else {
+        const size_t at = (size_t)(t - 1);
+        if (at >= lo) {
+          std::nth_element(v.begin() + lo, v.begin() + at, v.end());
+          lo = at;
+        }
+        k = (int64_t)v[at] + 1;
+      }
+    }
+    b[r] = std::min<int64_t>(std::max<int64_t>(k, b[r - 1] + 1), ext - (n - r));
+  }
+}
+
+// The slabs of aoadmm_create_multi / aoadmm_create_sparse_multi.  objs[r]: the objects of rank r; a dense CP object
+// of order >= 3 is cut into the uniform slabs of its last mode.  sparse != nullptr: a sparse object (any order) is cut
+// by shard_bounds and sp[r][p] / mk[r][p] describe rank r's entries of it and of its mask, in a permuted copy of the
+// caller's entries (one slab after the other; n == 1 keeps the caller's descriptors).
+struct Slabs {
+  std::vector<std::vector<aoadmm_object>> objs;
+  std::vector<std::vector<aoadmm_sparse_object>> sp, mk;
+  std::vector<std::vector<const aoadmm_sparse_object*>> sp_ptr, mk_ptr;
+  std::vector<std::vector<int64_t>> subs;   // the permuted copies
+  std::vector<std::vector<double>> vals;
+};
+
+// rank r's entries of `so` (bounds b of its object's last mode) into out[r]; the copy is kept in sl.subs / sl.vals
+void split_entries(Slabs& sl, const aoadmm_sparse_object& so, int order, const std::vector<int64_t>& b, int n,
+                   std::vector<aoadmm_sparse_object>& out) {
+  const int64_t nnz = so.nnz;
+  const int64_t* last = so.subs + (size_t)(order - 1) * (size_t)nnz;
+  auto slab_of = [&](int64_t i) { return (int)(std::upper_bound(b.begin() + 1, b.begin() + n, i) - (b.begin() + 1)); };
+  std::vector<int64_t> cnt(n, 0), base(n + 1, 0);
+  for (int64_t e = 0; e < nnz; ++e) ++cnt[slab_of(last[e])];
+  for (int r = 0; r < n; ++r) base[r + 1] = base[r] + cnt[r];
+  sl.subs.emplace_back((size_t)nnz * order);
+  sl.vals.emplace_back((size_t)nnz);
+  int64_t* ps = sl.subs.back().data();
+  double* pv = sl.vals.back().data();
+  std::vector<int64_t> fill(n, 0);
+  for (int64_t e = 0; e < nnz; ++e) {
+    const int r = slab_of(last[e]);
+    const int64_t j = fill[r]++;
+    for (int d = 0; d < order; ++d) ps[base[r] * order + d * cnt[r] + j] = so.subs[(size_t)d * nnz + e];
+    pv[base[r] + j] = so.vals[e];
+  }
+  for (int r = 0; r < n; ++r) {
+    out[r].nnz = cnt[r];
+    out[r].subs = ps + base[r] * order;
+    out[r].vals = pv + base[r];
+  }
+}
+
+void cut_slabs(const aoadmm_problem* problem, int n_gpus, const aoadmm_sparse_object* const* sparse,
+               const aoadmm_sparse_object* const* masks, Slabs& sl) {
+  using aoadmm::CudaError;
+  if (problem->nb_modes <= 0 || problem->n_objects <= 0 || problem->objects == nullptr || problem->mode_rows == nullptr)
+    throw CudaError(AOADMM_ERR_INVALID_ARG, "empty problem");
+  const int P = problem->n_objects;
+  sl.objs.assign(n_gpus, std::vector<aoadmm_object>(problem->objects, problem->objects + P));
+  sl.sp.assign(n_gpus, std::vector<aoadmm_sparse_object>(P));
+  sl.mk.assign(n_gpus, std::vector<aoadmm_sparse_object>(P));
+  sl.sp_ptr.assign(n_gpus, std::vector<const aoadmm_sparse_object*>(P, nullptr));
+  sl.mk_ptr.assign(n_gpus, std::vector<const aoadmm_sparse_object*>(P, nullptr));
+  for (int p = 0; p < P; ++p) {
+    const aoadmm_object& src = problem->objects[p];
+    const bool is_sparse = sparse != nullptr && sparse[p] != nullptr;
+    const aoadmm_sparse_object* mask = (is_sparse && masks != nullptr) ? masks[p] : nullptr;
+    if (is_sparse && n_gpus == 1) {
+      sl.sp_ptr[0][p] = sparse[p];
+      sl.mk_ptr[0][p] = mask;
+      continue;
+    }
+    // slabs of the last mode of every >= 3-way dense CP object and every sparse one (column-major: a dense slab is one
+    // contiguous range)
+    if (src.model != AOADMM_MODEL_CP || (src.order < 3 && !is_sparse) || n_gpus == 1) continue;
+    if (src.modes == nullptr) throw CudaError(AOADMM_ERR_INVALID_ARG, "object without modes");
+    int64_t lead = 1;
+    for (int d = 0; d < src.order; ++d) {
+      if (src.modes[d] < 1 || src.modes[d] > problem->nb_modes) throw CudaError(AOADMM_ERR_INVALID_ARG, "mode id out of range");
+      if (d + 1 < src.order) lead *= problem->mode_rows[src.modes[d] - 1];
+    }
+    const int64_t ext = problem->mode_rows[src.modes[src.order - 1] - 1];
+    if (src.shard_offset != 0 || (src.shard_extent != ext && src.shard_extent != 0))
+      throw CudaError(AOADMM_ERR_INVALID_ARG, "aoadmm_create_multi takes whole objects (shard_offset = 0, shard_extent = size of the last mode)");
+    const std::string who = "object " + std::to_string(p + 1) + ": ";
+    if (ext < n_gpus)
+      throw CudaError(AOADMM_ERR_INVALID_ARG, who + "the last mode has fewer indices (" + std::to_string(ext) +
+                                                  ") than there are GPUs");
+    std::vector<int64_t> b(n_gpus + 1);
+    if (is_sparse) {
+      shard_bounds(sparse[p], src.order, ext, n_gpus, b.data(), who);
+      std::vector<aoadmm_sparse_object> parts(n_gpus);
+      split_entries(sl, *sparse[p], src.order, b, n_gpus, parts);
+      for (int r = 0; r < n_gpus; ++r) {
+        sl.sp[r][p] = parts[r];
+        sl.sp_ptr[r][p] = &sl.sp[r][p];
+      }
+      if (mask != nullptr) {   // a mask is cut with the object's bounds
+        split_entries(sl, *mask, src.order, b, n_gpus, parts);
+        for (int r = 0; r < n_gpus; ++r) {
+          sl.mk[r][p] = parts[r];
+          sl.mk_ptr[r][p] = &sl.mk[r][p];
+        }
+      }
+    } else {
+      for (int r = 0; r <= n_gpus; ++r) b[r] = ext * r / n_gpus;
+    }
+    for (int r = 0; r < n_gpus; ++r) {
+      aoadmm_object& o = sl.objs[r][p];
+      o.shard_offset = b[r];
+      o.shard_extent = b[r + 1] - b[r];
+      if (src.data != nullptr) o.data = src.data + lead * b[r];
+      if (src.miss != nullptr) o.miss = src.miss + lead * b[r];
+    }
+  }
+}
+
+// devices[r] (NULL: r) of n_gpus GPUs: distinct ordinals of visible devices
+std::vector<int> device_list(int32_t n_gpus, const int32_t* devices) {
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) throw aoadmm::CudaError(AOADMM_ERR_NO_DEVICE, "no CUDA device available");
+  if (n_gpus < 1 || n_gpus > ndev)
+    throw aoadmm::CudaError(AOADMM_ERR_INVALID_ARG, "n_gpus must be between 1 and the number of visible devices (" + std::to_string(ndev) + ")");
+  std::vector<int> devs(n_gpus);
+  for (int r = 0; r < n_gpus; ++r) {
+    devs[r] = devices ? devices[r] : r;
+    if (devs[r] < 0 || devs[r] >= ndev) throw aoadmm::CudaError(AOADMM_ERR_INVALID_ARG, "device ordinal out of range");
+    for (int q = 0; q < r; ++q)
+      if (devs[q] == devs[r]) throw aoadmm::CudaError(AOADMM_ERR_INVALID_ARG, "a device is listed twice");
+  }
+  return devs;
+}
+
+// one engine per GPU, each from its own worker thread; the norms are summed once every constructor has returned
+void build_engines(aoadmm_handle* h, const aoadmm_problem* problem, const std::vector<int>& devs, Slabs& sl, bool sparse,
+                   bool masked) {
+  const int n_gpus = (int)devs.size();
+  std::vector<void*> comms(n_gpus, nullptr);
+  if (n_gpus > 1) comms = aoadmm::comms_for_devices(devs);
+  h->eng.assign(n_gpus, nullptr);
+  for_each_rank(n_gpus, [&](int r) {
+    aoadmm_problem pr = *problem;
+    pr.objects = sl.objs[r].data();
+    aoadmm_dist d{};
+    d.rank = r;
+    d.world_size = n_gpus;
+    d.device = devs[r];
+    h->eng[r] = new aoadmm::Engine(&pr, &d, comms[r], sparse ? sl.sp_ptr[r].data() : nullptr,
+                                   masked ? sl.mk_ptr[r].data() : nullptr);
+  });
+  for_each_rank(n_gpus, [&](int r) { h->eng[r]->reduce_norms(); });
 }
 
 }  // namespace
@@ -211,58 +405,44 @@ int aoadmm_create_multi(const aoadmm_problem* problem, int32_t n_gpus, const int
   aoadmm_handle* h = nullptr;
   int rc = guard(nullptr, [&] {
     if (problem == nullptr) throw aoadmm::CudaError(AOADMM_ERR_INVALID_ARG, "problem is NULL");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) throw aoadmm::CudaError(AOADMM_ERR_NO_DEVICE, "no CUDA device available");
-    if (n_gpus < 1 || n_gpus > ndev)
-      throw aoadmm::CudaError(AOADMM_ERR_INVALID_ARG, "n_gpus must be between 1 and the number of visible devices (" + std::to_string(ndev) + ")");
-    std::vector<int> devs(n_gpus);
-    for (int r = 0; r < n_gpus; ++r) {
-      devs[r] = devices ? devices[r] : r;
-      if (devs[r] < 0 || devs[r] >= ndev) throw aoadmm::CudaError(AOADMM_ERR_INVALID_ARG, "device ordinal out of range");
-      for (int q = 0; q < r; ++q)
-        if (devs[q] == devs[r]) throw aoadmm::CudaError(AOADMM_ERR_INVALID_ARG, "a device is listed twice");
-    }
-    if (problem->nb_modes <= 0 || problem->n_objects <= 0 || problem->objects == nullptr || problem->mode_rows == nullptr)
-      throw aoadmm::CudaError(AOADMM_ERR_INVALID_ARG, "empty problem");
-    // slabs of the last mode of every >= 3-way CP object (column-major: a slab is one contiguous range)
-    std::vector<std::vector<aoadmm_object>> objs(n_gpus, std::vector<aoadmm_object>(problem->objects, problem->objects + problem->n_objects));
-    for (int p = 0; p < problem->n_objects; ++p) {
-      const aoadmm_object& src = problem->objects[p];
-      if (src.model != AOADMM_MODEL_CP || src.order < 3 || n_gpus == 1) continue;
-      if (src.modes == nullptr) throw aoadmm::CudaError(AOADMM_ERR_INVALID_ARG, "object without modes");
-      int64_t lead = 1;
-      for (int d = 0; d < src.order; ++d) {
-        if (src.modes[d] < 1 || src.modes[d] > problem->nb_modes) throw aoadmm::CudaError(AOADMM_ERR_INVALID_ARG, "mode id out of range");
-        if (d + 1 < src.order) lead *= problem->mode_rows[src.modes[d] - 1];
-      }
-      const int64_t ext = problem->mode_rows[src.modes[src.order - 1] - 1];
-      if (src.shard_offset != 0 || (src.shard_extent != ext && src.shard_extent != 0))
-        throw aoadmm::CudaError(AOADMM_ERR_INVALID_ARG, "aoadmm_create_multi takes whole objects (shard_offset = 0, shard_extent = size of the last mode)");
-      if (ext < n_gpus)
-        throw aoadmm::CudaError(AOADMM_ERR_INVALID_ARG, "object " + std::to_string(p + 1) + ": the last mode has fewer indices (" +
-                                                           std::to_string(ext) + ") than there are GPUs");
-      for (int r = 0; r < n_gpus; ++r) {
-        const int64_t lo = ext * r / n_gpus, hi = ext * (r + 1) / n_gpus;
-        aoadmm_object& o = objs[r][p];
-        o.shard_offset = lo;
-        o.shard_extent = hi - lo;
-        if (src.data != nullptr) o.data = src.data + lead * lo;
-        if (src.miss != nullptr) o.miss = src.miss + lead * lo;
-      }
-    }
-    std::vector<void*> comms(n_gpus, nullptr);
-    if (n_gpus > 1) comms = aoadmm::comms_for_devices(devs);
+    const std::vector<int> devs = device_list(n_gpus, devices);
+    Slabs sl;
+    cut_slabs(problem, n_gpus, nullptr, nullptr, sl);
     h = new aoadmm_handle();
-    h->eng.assign(n_gpus, nullptr);
-    for_each_rank(n_gpus, [&](int r) {
-      aoadmm_problem pr = *problem;
-      pr.objects = objs[r].data();
-      aoadmm_dist d{};
-      d.rank = r;
-      d.world_size = n_gpus;
-      d.device = devs[r];
-      h->eng[r] = new aoadmm::Engine(&pr, &d, comms[r]);
-    });
+    build_engines(h, problem, devs, sl, false, false);
+  });
+  if (rc != AOADMM_OK) {
+    delete h;   // engines that were built on the other devices go with it
+    return rc;
+  }
+  *out = h;
+  return AOADMM_OK;
+}
+
+int aoadmm_sparse_shard_bounds(const aoadmm_sparse_object* so, int32_t order, int64_t extent, int32_t n_gpus,
+                               int64_t* bounds) {
+  return guard(nullptr, [&] { shard_bounds(so, order, extent, n_gpus, bounds, ""); });
+}
+
+int aoadmm_create_sparse_multi(const aoadmm_problem* problem, const aoadmm_sparse_object* const* sparse,
+                               const aoadmm_sparse_object* const* masks, int32_t n_gpus, const int32_t* devices,
+                               aoadmm_handle** out) {
+  if (!out) return AOADMM_ERR_INVALID_ARG;
+  *out = nullptr;
+  aoadmm_handle* h = nullptr;
+  int rc = guard(nullptr, [&] {
+    // every check on the arguments that needs no device first, the slabs included
+    check_sparse(problem, sparse, masks, nullptr);
+    if (n_gpus < 1) throw aoadmm::CudaError(AOADMM_ERR_INVALID_ARG, "n_gpus must be >= 1");
+    if (devices != nullptr)
+      for (int r = 0; r < n_gpus; ++r)
+        for (int q = 0; q < r; ++q)
+          if (devices[q] == devices[r]) throw aoadmm::CudaError(AOADMM_ERR_INVALID_ARG, "a device is listed twice");
+    Slabs sl;
+    cut_slabs(problem, n_gpus, sparse, masks, sl);
+    const std::vector<int> devs = device_list(n_gpus, devices);
+    h = new aoadmm_handle();
+    build_engines(h, problem, devs, sl, sparse != nullptr, masks != nullptr);
   });
   if (rc != AOADMM_OK) {
     delete h;   // engines that were built on the other devices go with it

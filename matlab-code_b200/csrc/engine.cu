@@ -548,7 +548,9 @@ void Engine::construct(const aoadmm_problem* prob, const aoadmm_dist* dist, void
       o.dims.push_back(m.rows);
     }
     o.last_full = o.dims.back();
-    o.sharded = (world_ > 1 && o.order >= 3);
+    const bool is_sparse = sparse != nullptr && sparse[p] != nullptr;
+    // dense matrices are replicated; tensors and sparse objects of any order hold one slab of their last mode
+    o.sharded = (world_ > 1 && (o.order >= 3 || is_sparse));
     if (o.sharded) {
       o.shard_offset = src.shard_offset;
       o.shard_extent = src.shard_extent;
@@ -559,18 +561,20 @@ void Engine::construct(const aoadmm_problem* prob, const aoadmm_dist* dist, void
       o.shard_extent = o.last_full;
     }
     o.dims.back() = o.shard_extent;
-    if (sparse != nullptr && sparse[p] != nullptr) {
-      // sparse CP object (aoadmm_create_sparse): one GPU, no dense mask; sorted device copies instead of a dense array.
-      // A sparse mask (aoadmm_create_sparse_masked) must mark exactly the stored entries; EM state in o.sp.
-      if (world_ > 1 || src.miss != nullptr || src.data != nullptr) throw CudaError(2, "sparse object: unsupported combination");
+    if (is_sparse) {
+      // sparse CP object (aoadmm_create_sparse, or this GPU's slab from aoadmm_create_sparse_multi): no dense mask;
+      // sorted device copies instead of a dense array.  A sparse mask (aoadmm_create_sparse_masked) must mark exactly
+      // the stored entries; EM state in o.sp.
+      if (src.miss != nullptr || src.data != nullptr) throw CudaError(2, "sparse object: unsupported combination");
       const aoadmm_sparse_object& so = *sparse[p];
       const aoadmm_sparse_object* mk = masks != nullptr ? masks[p] : nullptr;
       std::vector<long long> dl(o.dims.begin(), o.dims.end());
+      dl.back() = o.last_full;
       o.sp = new SparseTensor();
       try {
-        sparse_build(*o.sp, o.order, dl.data(), R, so.nnz, reinterpret_cast<const long long*>(so.subs), so.vals, st_,
-                     mk != nullptr, mk ? mk->nnz : 0, mk ? reinterpret_cast<const long long*>(mk->subs) : nullptr,
-                     mk ? mk->vals : nullptr);
+        sparse_build(*o.sp, o.order, dl.data(), o.shard_offset, o.shard_extent, R, so.nnz,
+                     reinterpret_cast<const long long*>(so.subs), so.vals, st_, mk != nullptr, mk ? mk->nnz : 0,
+                     mk ? reinterpret_cast<const long long*>(mk->subs) : nullptr, mk ? mk->vals : nullptr);
       } catch (const CudaError& e) {
         throw CudaError(e.code, "sparse object " + std::to_string(p + 1) + ": " + e.what());
       }
@@ -755,9 +759,6 @@ void Engine::construct(const aoadmm_problem* prob, const aoadmm_dist* dist, void
     if (o.model == AOADMM_MODEL_PAR2) {
       Par2State& s = par2_[mode(o.modes[0]).par2];
       launches_ += object_norm2(s.X_alloc, s.mask_alloc, s.I, s.ldX, s.jhi - s.jlo, part, res, st_);
-      if (s.sharded) {   // sum of the ranks' slices (the communicator exists since the top of the constructor)
-        allreduce(res, 1);
-      }
     } else if (o.sp != nullptr) {
       launches_ += sparse_norm2(*o.sp, st_);
       res = o.sp->norm_out;
@@ -769,7 +770,8 @@ void Engine::construct(const aoadmm_problem* prob, const aoadmm_dist* dist, void
     }
     AO_CUDA(cudaMemcpyAsync(&o.znorm, res, sizeof(double), cudaMemcpyDeviceToHost, st_));
     AO_CUDA(cudaStreamSynchronize(st_));
-    o.znorm_pending_allreduce = o.sharded;
+    // partial norm of this rank's slab / slices: summed by reduce_norms
+    o.znorm_pending_allreduce = o.model == AOADMM_MODEL_PAR2 ? par2_[mode(o.modes[0]).par2].sharded : o.sharded;
   }
   AO_CUDA(cudaDeviceSynchronize());
 
@@ -817,17 +819,22 @@ void Engine::construct(const aoadmm_problem* prob, const aoadmm_dist* dist, void
     }
     AO_CUDA(cudaMalloc(&em_partials_, std::max<size_t>(need, 8) * sizeof(double)));
   }
-
-  if (world_ > 1) {
-    for (auto& o : objects_)
-      if (o.znorm_pending_allreduce) {  // partial norms of the slabs -> norm of the whole tensor
-        AO_CUDA(cudaMemcpyAsync(cp0_tmp_, &o.znorm, sizeof(double), cudaMemcpyHostToDevice, st_));
-        allreduce(cp0_tmp_, 1);
-        AO_CUDA(cudaMemcpyAsync(&o.znorm, cp0_tmp_, sizeof(double), cudaMemcpyDeviceToHost, st_));
-        AO_CUDA(cudaStreamSynchronize(st_));
-      }
-  }
   AO_CUDA(cudaDeviceSynchronize());
+}
+
+// The only collective of creation.  It runs after every rank's constructor has returned, so a rank whose slab fails
+// to build (a sparse mask that does not match inside it) never leaves the others waiting in an all-reduce.
+void Engine::reduce_norms() {
+  if (world_ <= 1) return;
+  AO_CUDA(cudaSetDevice(device_));
+  for (auto& o : objects_)
+    if (o.znorm_pending_allreduce) {  // partial norms of the slabs -> norm of the whole tensor
+      AO_CUDA(cudaMemcpyAsync(cp0_tmp_, &o.znorm, sizeof(double), cudaMemcpyHostToDevice, st_));
+      allreduce(cp0_tmp_, 1);
+      AO_CUDA(cudaMemcpyAsync(&o.znorm, cp0_tmp_, sizeof(double), cudaMemcpyDeviceToHost, st_));
+      AO_CUDA(cudaStreamSynchronize(st_));
+      o.znorm_pending_allreduce = false;
+    }
 }
 
 Engine::~Engine() { release(); }
@@ -1096,7 +1103,8 @@ void Engine::allreduce(double* buf, size_t count) {
   AO_NCCL(nccl_->AllReduce(buf, buf, count, ncclDouble, ncclSum, static_cast<ncclComm_t>(comm_), st_));
 }
 
-// sparse objects: always FP64, no dimension tree (options.mttkrp_precision / dimtree apply to dense objects only)
+// sparse objects: always FP64, no dimension tree (options.mttkrp_precision / dimtree apply to dense objects only); the
+// pass over this GPU's nonzeros
 int Engine::sparse_mttkrp_of(ObjectState& o, int pos, double scale, double* out, int64_t ldout, bool imputed) {
   const double* fac[8];
   long long ld[8];
@@ -1111,7 +1119,13 @@ int Engine::sparse_mttkrp_of(ObjectState& o, int pos, double scale, double* out,
 void Engine::compute_mttkrp(ObjectState& o, int pos, double scale, double* out, int64_t ldout, bool imputed) {
   if (o.sp != nullptr) {
     phase_begin(o.order >= 3 ? 0 : 1);
+    const int R = o.sp->R;
+    // a slab writes the rows of its last-mode indices only: the others must be zero for the all-reduce
+    if (o.sharded && pos == o.order - 1) AO_CUDA(cudaMemsetAsync(out, 0, (size_t)ldout * R * sizeof(double), st_));
     launches_ += sparse_mttkrp_of(o, pos, scale, out, ldout, imputed);
+    if (o.sharded) allreduce(out, (size_t)ldout * R);
+    // the low-rank term reads replicated state only: added once, after the all-reduce
+    if (imputed && sparse_masked(o)) launches_ += sparse_lowrank_add(*o.sp, pos, scale, out, ldout, st_);
     phase_end();
     return;
   }
@@ -1710,7 +1724,10 @@ void Engine::em_step(bool impute) {
         fac[d] = md.fac.p;
         ld[d] = md.rows;
       }
-      launches_ += sparse_em(*o.sp, fac, ld, impute, em_sums_ + 5 * p, st_);
+      launches_ += sparse_em_nonzeros(*o.sp, fac, ld, impute, st_);
+      // only the nonzero-side sums are partial: the telescoped terms are replicated and must be counted once
+      if (o.sharded) allreduce(o.sp->em_nz, 4);
+      launches_ += sparse_em_finish(*o.sp, fac, ld, impute, em_sums_ + 5 * p, st_);
       phase_end();
     } else {
       if (o.mask == nullptr) continue;
@@ -2841,27 +2858,27 @@ void Engine::set_heldout(int object, const aoadmm_sparse_object* entries) {
     } else {
       std::vector<long long> ld(o.dims.begin(), o.dims.end());
       count = heldout_masked(*h, o.mask, o.ld0, ld.data(), o.shard_offset, &first, st_);
-      if (o.sharded) {   // each rank checked the entries of its slab: one all-reduce of the counts and first positions
-        std::vector<double> hb(world_ + 1, 0.0);
-        hb[0] = (double)count;
-        hb[1 + rank_] = (double)(first + 1);
-        double* db = nullptr;
-        AO_CUDA(cudaMalloc(&db, hb.size() * sizeof(double)));
-        try {
-          AO_CUDA(cudaMemcpyAsync(db, hb.data(), hb.size() * sizeof(double), cudaMemcpyHostToDevice, st_));
-          allreduce(db, hb.size());
-          AO_CUDA(cudaMemcpyAsync(hb.data(), db, hb.size() * sizeof(double), cudaMemcpyDeviceToHost, st_));
-          AO_CUDA(cudaStreamSynchronize(st_));
-        } catch (...) {
-          cudaFree(db);
-          throw;
-        }
+    }
+    if (o.sharded) {   // each rank checked the entries of its slab: one all-reduce of the counts and first positions
+      std::vector<double> hb(world_ + 1, 0.0);
+      hb[0] = (double)count;
+      hb[1 + rank_] = (double)(first + 1);
+      double* db = nullptr;
+      AO_CUDA(cudaMalloc(&db, hb.size() * sizeof(double)));
+      try {
+        AO_CUDA(cudaMemcpyAsync(db, hb.data(), hb.size() * sizeof(double), cudaMemcpyHostToDevice, st_));
+        allreduce(db, hb.size());
+        AO_CUDA(cudaMemcpyAsync(hb.data(), db, hb.size() * sizeof(double), cudaMemcpyDeviceToHost, st_));
+        AO_CUDA(cudaStreamSynchronize(st_));
+      } catch (...) {
         cudaFree(db);
-        count = (long long)hb[0];
-        first = -1;
-        for (int r = 0; r < world_ && first < 0; ++r)
-          if (hb[1 + r] > 0.0) first = (long long)hb[1 + r] - 1;
+        throw;
       }
+      cudaFree(db);
+      count = (long long)hb[0];
+      first = -1;
+      for (int r = 0; r < world_ && first < 0; ++r)
+        if (hb[1 + r] > 0.0) first = (long long)hb[1 + r] - 1;
     }
     if (count > 0) {
       long long sub[8];

@@ -170,7 +170,7 @@ struct ObjectState {
   double* em_fkT = nullptr;   // masked objects of order >= 3: transposed third factor for the pipelined EM kernel
   double* Tbuf = nullptr;     // dimension tree: T(j,k,r) = sum_i X(i,j,k) F1(i,r), emitted by the mode-2 MTTKRP
   uint64_t T_version = 0;     // version of the mode-1 factor T was computed from (0 = invalid)
-  SparseTensor* sp = nullptr; // sparse (COO) object: sorted device copies (sparse.cuh); data, views stay empty
+  SparseTensor* sp = nullptr; // sparse (COO) object: sorted device copies of this rank's slab (sparse.cuh); data, views stay empty
   HeldOut* ho = nullptr;      // held-out set (aoadmm_set_heldout), replicated on every rank
   std::vector<double> ho_hist;  // held-out SSE after outer iteration 0, 1, ... of the last run
 };
@@ -213,6 +213,9 @@ class Engine {
   void check_entries(int object, const aoadmm_sparse_object* entries, bool heldout) const;
   void model_at(int object, const aoadmm_sparse_object* entries, double* out);   // on this engine's device
   void set_heldout(int object, const aoadmm_sparse_object* entries);             // collective over the ranks
+  // collective over the ranks, once after every rank's constructor returned: sums the partial Znorm_const = NaN norms
+  // of sharded objects (a no-op on one GPU)
+  void reduce_norms();
   void heldout_history(int object, double* sse, int64_t n, int64_t* count) const;
   int64_t launches() const { return launches_; }
   void phase_ms(double ms[3]);

@@ -59,11 +59,14 @@ void launch_entries(const EntryArgs& a, cudaStream_t st) {
   AO_CHECK_LAUNCH();
 }
 
-// key of row i_1 = subs[e] in the mode-1 copy: lower bound of (i_2..i_N) among its stored entries
+// key of row i_1 = subs[e] in the mode-1 copy: lower bound of (i_2..i_N) among its stored entries.  The copy holds the
+// slab [shift, shift + ext) of the last mode with local subscripts: only the entries of the slab are looked up.
 __global__ void stored_kernel(const int* __restrict__ subs, long long n, int order, const long long* __restrict__ rowptr,
-                              const int* __restrict__ idx, long long nnz, unsigned long long* __restrict__ count,
-                              long long* __restrict__ first) {
+                              const int* __restrict__ idx, long long nnz, int shift, int ext,
+                              unsigned long long* __restrict__ count, long long* __restrict__ first) {
   for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x) {
+    const int il = subs[(order - 1) * n + e] - shift;
+    if (il < 0 || il >= ext) continue;
     const int i0 = subs[e];
     const long long end = rowptr[i0 + 1];
     long long lo = rowptr[i0], hi = end;
@@ -71,14 +74,14 @@ __global__ void stored_kernel(const int* __restrict__ subs, long long n, int ord
       const long long mid = (lo + hi) >> 1;
       int cmp = 0;
       for (int d = 1; d < order && cmp == 0; ++d) {
-        const int a = idx[(d - 1) * nnz + mid], b = subs[d * n + e];
+        const int a = idx[(d - 1) * nnz + mid], b = d == order - 1 ? il : subs[d * n + e];
         cmp = a < b ? -1 : (a > b ? 1 : 0);
       }
       if (cmp < 0) lo = mid + 1;
       else hi = mid;
     }
     bool eq = lo < end;
-    for (int d = 1; d < order && eq; ++d) eq = idx[(d - 1) * nnz + lo] == subs[d * n + e];
+    for (int d = 1; d < order && eq; ++d) eq = idx[(d - 1) * nnz + lo] == (d == order - 1 ? il : subs[d * n + e]);
     if (eq) {
       atomicAdd(count, 1ULL);
       atomicMin(first, e);
@@ -201,7 +204,8 @@ long long heldout_stored(const HeldOut& h, const SparseTensor& s, long long* fir
   if (h.n == 0 || s.nnz == 0) return 0;
   const SparseMode& m1 = s.modes[0];
   return run_check(first, st, [&](unsigned long long* count, long long* fst) {
-    stored_kernel<<<grid_for(h.n), 256, 0, st>>>(h.subs, h.n, h.order, m1.rowptr, m1.idx, s.nnz, count, fst);
+    stored_kernel<<<grid_for(h.n), 256, 0, st>>>(h.subs, h.n, h.order, m1.rowptr, m1.idx, s.nnz, (int)s.shift,
+                                                 (int)s.dims[h.order - 1], count, fst);
     AO_CHECK_LAUNCH();
   });
 }

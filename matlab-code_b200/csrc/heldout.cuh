@@ -32,7 +32,7 @@ void heldout_free(HeldOut& h);
 // (leading dimension ld[d]).  Allocation-free and graph-capturable.  Returns the number of kernel launches.
 int heldout_sse(HeldOut& h, const double* const* fac, const long long* ld, double* sse, cudaStream_t st);
 // Held-out entries that were observed in training.  Sparse masked object `s`: the entry is stored (looked up in the
-// mode-1 copy).  Dense mask (ld0 bytes per leading column, local extents ldims, the last mode starting at
+// mode-1 copy; a slab of a sharded object checks only the entries of its slab).  Dense mask (ld0 bytes per leading column, local extents ldims, the last mode starting at
 // shard_offset): its mask byte is nonzero; only the entries of this slab are checked.  Returns the count and the
 // position (in h's sorted order) of the first such entry in *first (-1: none).  Synchronous on `st`.
 long long heldout_stored(const HeldOut& h, const SparseTensor& s, long long* first, cudaStream_t st);

@@ -29,18 +29,19 @@ __global__ void iota_kernel(int* p, long long n) {
   for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x) p[e] = (int)e;
 }
 
+// shift: first index of this GPU's slab when src holds last-mode subscripts of a sharded object, else 0
 __global__ void gather_keys_kernel(const int* __restrict__ src, const int* __restrict__ perm, unsigned* __restrict__ keys,
-                                   long long n) {
+                                   long long n, int shift) {
   for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x)
-    keys[e] = (unsigned)src[perm[e]];
+    keys[e] = (unsigned)(src[perm[e]] - shift);
 }
 
-// sorted copy of the caller's nonzeros: ss(d, e) = raw(d, perm[e]), sv(e) = rv(perm[e])
+// sorted copy of the caller's nonzeros: ss(d, e) = raw(d, perm[e]) (last mode: minus shift), sv(e) = rv(perm[e])
 __global__ void gather_coo_kernel(const int* __restrict__ raw, const double* __restrict__ rv, const int* __restrict__ perm,
-                                  long long n, int order, int* __restrict__ ss, double* __restrict__ sv) {
+                                  long long n, int order, int shift, int* __restrict__ ss, double* __restrict__ sv) {
   for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x) {
     const long long src = perm[e];
-    for (int d = 0; d < order; ++d) ss[d * n + e] = raw[d * n + src];
+    for (int d = 0; d < order; ++d) ss[d * n + e] = raw[d * n + src] - (d == order - 1 ? shift : 0);
     sv[e] = rv[src];
   }
 }
@@ -361,19 +362,31 @@ __global__ void __launch_bounds__(256) tele_partials_kernel(const double* __rest
   }
 }
 
-// em_sums slots of the object: [0] ||M'-M||^2 - sum_W (m'-m)^2, [1] ||M||^2 - sum_W m^2 (both clamped at 0: they are
-// sums of squares over the unobserved entries, a negative value is rounding), [2] sum s m', [3] sum m'^2, [4] 0
-__global__ void em_final_kernel(const double* __restrict__ mpart, unsigned nm, const double* __restrict__ tpart, unsigned nt,
-                                double* __restrict__ sums) {
+// nonzero-side sums of this GPU's entries, from the per-CTA partials of sp_model_kernel (fixed order):
+// nz[0] sum s m', [1] sum m'^2, [2] sum_W (m' - m)^2, [3] sum_W m^2
+__global__ void em_nz_kernel(const double* __restrict__ mpart, unsigned nm, double* __restrict__ nz) {
   const double a0 = warp_sum_partials(mpart, nm, 4), a1 = warp_sum_partials(mpart + 1, nm, 4);
   const double a2 = warp_sum_partials(mpart + 2, nm, 4), a3 = warp_sum_partials(mpart + 3, nm, 4);
+  if (threadIdx.x == 0) {
+    nz[0] = a0;
+    nz[1] = a1;
+    nz[2] = a2;
+    nz[3] = a3;
+  }
+}
+
+// em_sums slots of the object: [0] ||M'-M||^2 - sum_W (m'-m)^2, [1] ||M||^2 - sum_W m^2 (both clamped at 0: they are
+// sums of squares over the unobserved entries, a negative value is rounding), [2] sum s m', [3] sum m'^2, [4] 0.
+// nz: the nonzero-side sums of the whole object (em_nz_kernel, summed over the GPUs); tpart: the telescoped terms.
+__global__ void em_final_kernel(const double* __restrict__ nz, const double* __restrict__ tpart, unsigned nt,
+                                double* __restrict__ sums) {
   const double t = warp_sum_partials(tpart, nt, 2), mm = warp_sum_partials(tpart + 1, nt, 2);
   if (threadIdx.x == 0) {
-    const double num = t - a2, den = mm - a3;
+    const double num = t - nz[2], den = mm - nz[3];
     sums[0] = num > 0.0 ? num : 0.0;
     sums[1] = den > 0.0 ? den : 0.0;
-    sums[2] = a0;
-    sums[3] = a1;
+    sums[2] = nz[0];
+    sums[3] = nz[1];
     sums[4] = 0.0;
   }
 }
@@ -462,8 +475,9 @@ struct SortWs {
 
 // uploads n > 0 COO entries, sorts them into full lexicographic order (mode 0 major) and sums duplicates (the Tensor
 // Toolbox sptensor(subs,vals) constructor sums them): ms (order x nm, column-major), mv (nm).  Returns nm.
+// shift: subtracted from the last-mode subscripts on the device (first index of this GPU's slab; 0 = whole object)
 long long sort_merge(Temps& tmp, SortWs& w, int order, const long long* dims, long long n, const long long* subs,
-                     const double* vals, cudaStream_t st, int*& ms, double*& mv) {
+                     const double* vals, cudaStream_t st, int*& ms, double*& mv, int shift = 0) {
   std::vector<int> h((size_t)order * n);
   for (size_t i = 0; i < h.size(); ++i) h[i] = (int)subs[i];
   int* raw = tmp.get<int>((size_t)order * n);
@@ -484,7 +498,7 @@ long long sort_merge(Temps& tmp, SortWs& w, int order, const long long* dims, lo
   iota_kernel<<<grid_for(n), 256, 0, st>>>(w.p0, n);
   AO_CHECK_LAUNCH();
   for (int d = order - 1; d >= 0; --d) {
-    gather_keys_kernel<<<grid_for(n), 256, 0, st>>>(raw + (size_t)d * n, w.p0, w.k0, n);
+    gather_keys_kernel<<<grid_for(n), 256, 0, st>>>(raw + (size_t)d * n, w.p0, w.k0, n, d == order - 1 ? shift : 0);
     AO_CHECK_LAUNCH();
     size_t b = w.bytes;
     AO_CUDA(cub::DeviceRadixSort::SortPairs(w.tmp, b, w.k0, w.k1, w.p0, w.p1, (int)n, 0, key_bits(dims[d]), st));
@@ -492,7 +506,7 @@ long long sort_merge(Temps& tmp, SortWs& w, int order, const long long* dims, lo
   }
   int* ss = tmp.get<int>((size_t)order * n);
   double* sv = tmp.get<double>(n);
-  gather_coo_kernel<<<grid_for(n), 256, 0, st>>>(raw, rv, w.p0, n, order, ss, sv);
+  gather_coo_kernel<<<grid_for(n), 256, 0, st>>>(raw, rv, w.p0, n, order, shift, ss, sv);
   AO_CHECK_LAUNCH();
   int* flags = (int*)w.k0;
   int* pos = (int*)w.k1;
@@ -513,14 +527,14 @@ long long sort_merge(Temps& tmp, SortWs& w, int order, const long long* dims, lo
 
 // true when the observed entries of the mask (merged value != 0) are exactly the merged subscripts ms (order x nm)
 bool mask_matches(Temps& tmp, int order, const long long* dims, long long nm, const int* ms, long long mask_nnz,
-                  const long long* mask_subs, const double* mask_vals, cudaStream_t st) {
+                  const long long* mask_subs, const double* mask_vals, int shift, cudaStream_t st) {
   long long nobs = 0;
   int* obs = nullptr;
   if (mask_nnz > 0) {
     SortWs w;
     int* mms = nullptr;
     double* mmv = nullptr;
-    const long long mm = sort_merge(tmp, w, order, dims, mask_nnz, mask_subs, mask_vals, st, mms, mmv);
+    const long long mm = sort_merge(tmp, w, order, dims, mask_nnz, mask_subs, mask_vals, st, mms, mmv, shift);
     int* flags = (int*)w.k0;
     int* pos = (int*)w.k1;
     nonzero_flags_kernel<<<grid_for(mm), 256, 0, st>>>(mmv, mm, flags);
@@ -549,27 +563,33 @@ bool mask_matches(Temps& tmp, int order, const long long* dims, long long nm, co
 
 }  // namespace
 
-void sparse_build(SparseTensor& s, int order, const long long* dims, int R, long long nnz, const long long* subs,
-                  const double* vals, cudaStream_t st, bool masked, long long mask_nnz, const long long* mask_subs,
-                  const double* mask_vals) {
+void sparse_build(SparseTensor& s, int order, const long long* full_dims, long long shard_offset, long long shard_extent,
+                  int R, long long nnz, const long long* subs, const double* vals, cudaStream_t st, bool masked,
+                  long long mask_nnz, const long long* mask_subs, const double* mask_vals) {
   if (order < 2 || order > 8) throw CudaError(1, "sparse object: order must be in 2..8");
   if (nnz < 0) throw CudaError(1, "sparse object: negative nnz");
-  if (nnz > 0x7fffffffLL - kSparseChunk) throw CudaError(2, "sparse object: more than 2^31 - 257 nonzeros");
+  if (nnz > 0x7fffffffLL - kSparseChunk) throw CudaError(2, "sparse object: more than 2^31 - 257 nonzeros on one GPU");
   if (masked && (mask_nnz < 0 || mask_nnz > 0x7fffffffLL - kSparseChunk))
     throw CudaError(1, "sparse object: mask nnz out of range");
   s.order = order;
   s.R = R;
   for (int d = 0; d < order; ++d) {
-    if (dims[d] < 0 || dims[d] > 0x7fffffffLL) throw CudaError(1, "sparse object: a mode exceeds 2^31 - 1 rows");
-    s.dims[d] = dims[d];
+    if (full_dims[d] < 0 || full_dims[d] > 0x7fffffffLL) throw CudaError(1, "sparse object: a mode exceeds 2^31 - 1 rows");
+    s.fdims[d] = full_dims[d];
+    s.dims[d] = full_dims[d];
   }
+  if (shard_offset < 0 || shard_extent < 0 || shard_offset + shard_extent > full_dims[order - 1])
+    throw CudaError(1, "sparse object: invalid shard range");
+  s.shift = shard_offset;
+  s.dims[order - 1] = shard_extent;
+  const long long* dims = s.dims;   // nonzero side: local extents
   Temps tmp;   // temporaries of the preprocessing: released on every exit path
   long long nm = 0;
   int* ms = nullptr;
   double* mv = nullptr;
   SortWs w;
-  if (nnz > 0) nm = sort_merge(tmp, w, order, dims, nnz, subs, vals, st, ms, mv);
-  if (masked && !mask_matches(tmp, order, dims, nm, ms, mask_nnz, mask_subs, mask_vals, st))
+  if (nnz > 0) nm = sort_merge(tmp, w, order, dims, nnz, subs, vals, st, ms, mv, (int)shard_offset);
+  if (masked && !mask_matches(tmp, order, dims, nm, ms, mask_nnz, mask_subs, mask_vals, (int)shard_offset, st))
     throw CudaError(2, "the observed entries of the sparse mask (Z.miss) differ from the stored entries of the object "
                        "(a sparse mask must mark exactly the stored entries)");
   s.nnz = nm;
@@ -619,6 +639,7 @@ void sparse_build(SparseTensor& s, int order, const long long* dims, int R, long
   s.norm_partials = dalloc<double>(kNormBlocks);
   s.norm_out = dalloc<double>(1);
   if (masked) {
+    // the factor side (B, cross-Grams, stacks and their Grams) has the full extents and is replicated on every GPU
     // EM state: m = 0, r = s, B = 0 ("the unobserved entries start at 0"), every buffer of sparse_em / the imputed MTTKRP
     s.masked = true;
     s.row0 = dalloc<int>(nm);
@@ -631,19 +652,23 @@ void sparse_build(SparseTensor& s, int order, const long long* dims, int R, long
     }
     const long long RR = (long long)R * R, R3 = 3LL * R;
     size_t ws = 1;
+    long long max_full = 1;
     for (int d = 0; d < order; ++d) {
-      s.B[d] = dalloc<double>((size_t)dims[d] * R);
-      AO_CUDA(cudaMemsetAsync(s.B[d], 0, (size_t)dims[d] * R * sizeof(double), st));
-      ws = std::max<size_t>(ws, (size_t)dgemm_splitk_count(R, R, dims[d]) * RR);
-      ws = std::max<size_t>(ws, (size_t)dgemm_splitk_count(R3, R3, dims[d]) * R3 * R3);
+      const long long rows = full_dims[d];
+      max_full = std::max(max_full, rows);
+      s.B[d] = dalloc<double>((size_t)rows * R);
+      AO_CUDA(cudaMemsetAsync(s.B[d], 0, (size_t)rows * R * sizeof(double), st));
+      ws = std::max<size_t>(ws, (size_t)dgemm_splitk_count(R, R, rows) * RR);
+      ws = std::max<size_t>(ws, (size_t)dgemm_splitk_count(R3, R3, rows) * R3 * R3);
     }
     s.cg = dalloc<double>((size_t)order * RR);
     AO_CUDA(cudaMemsetAsync(s.cg, 0, (size_t)order * RR * sizeof(double), st));
     s.H = dalloc<double>(RR);
-    s.stack = dalloc<double>((size_t)max_rows * R3);
+    s.stack = dalloc<double>((size_t)max_full * R3);
     s.g3 = dalloc<double>((size_t)order * R3 * R3);
     s.gemm_ws = dalloc<double>(ws);
     s.em_partials = dalloc<double>(2 * kTeleBlocks + 4 * (size_t)model_blocks(nm, R));
+    s.em_nz = dalloc<double>(4);
   }
   AO_CUDA(cudaStreamSynchronize(st));
 }
@@ -703,6 +728,7 @@ void sparse_free(SparseTensor& s) {
   f(s.g3);
   f(s.gemm_ws);
   f(s.em_partials);
+  f(s.em_nz);
 }
 
 int sparse_norm2(const SparseTensor& s, cudaStream_t st) {
@@ -716,6 +742,7 @@ int sparse_norm2(const SparseTensor& s, cudaStream_t st) {
 
 int sparse_mttkrp(SparseTensor& s, int n, const double* const* fac, const long long* ld, double scale, double* out,
                   long long ldout, cudaStream_t st, bool imputed) {
+  const int last = s.order - 1;
   const long long rows = s.dims[n];
   const int R = s.R;
   const SparseMode& sm = s.modes[n];
@@ -741,7 +768,7 @@ int sparse_mttkrp(SparseTensor& s, int n, const double* const* fac, const long l
     int q = 0;
     for (int d = 0; d < s.order; ++d) {
       if (d == n) continue;
-      launches += transpose_scale(fac[d], s.dims[d], R, ld[d], s.factT[d], R, 1.0, st);
+      launches += transpose_scale(fac[d] + (d == last ? s.shift : 0), s.dims[d], R, ld[d], s.factT[d], R, 1.0, st);
       a.F[q++] = s.factT[d];
     }
     rank_dispatch(R, [&](auto g, auto c) {
@@ -750,29 +777,33 @@ int sparse_mttkrp(SparseTensor& s, int n, const double* const* fac, const long l
     });
     launches += 2;
   }
-  // out(i, c) = scale * outT(c + R*i)
-  launches += transpose_scale(s.outT, R, rows, R, out, ldout, scale, st);
-  if (imp && rows > 0) {
-    // low-rank term of the imputed tensor: out += scale * B_n * (Hadamard of B_k' F_k, k != n)
-    const long long RR = (long long)R * R;
-    hadamard_others_kernel<<<grid_for(RR), 256, 0, st>>>(s.cg, s.order, n, R, s.H);
-    AO_CHECK_LAUNCH();
-    launches += 1 + dgemm_small(0, 0, rows, R, R, scale, nullptr, s.B[n], rows, s.H, R, 1.0, out, ldout, st, nullptr);
-  }
+  // out(i, c) = scale * outT(c + R*i), this GPU's rows of the last mode at their global position
+  launches += transpose_scale(s.outT, R, rows, R, out + (n == last ? s.shift : 0), ldout, scale, st);
   return launches;
 }
 
-int sparse_cross_gram(SparseTensor& s, int n, const double* F, long long ld, cudaStream_t st) {
-  if (!s.masked || s.dims[n] == 0) return 0;
+int sparse_lowrank_add(SparseTensor& s, int n, double scale, double* out, long long ldout, cudaStream_t st) {
+  const long long rows = s.fdims[n];
   const int R = s.R;
-  return dgemm_small_splitk(1, 0, R, R, s.dims[n], 1.0, s.B[n], s.dims[n], F, ld, 0.0, s.cg + (size_t)n * R * R, R,
+  if (!s.masked || rows == 0) return 0;
+  // low-rank term of the imputed tensor: out += scale * B_n * (Hadamard of B_k' F_k, k != n)
+  const long long RR = (long long)R * R;
+  hadamard_others_kernel<<<grid_for(RR), 256, 0, st>>>(s.cg, s.order, n, R, s.H);
+  AO_CHECK_LAUNCH();
+  return 1 + dgemm_small(0, 0, rows, R, R, scale, nullptr, s.B[n], rows, s.H, R, 1.0, out, ldout, st, nullptr);
+}
+
+int sparse_cross_gram(SparseTensor& s, int n, const double* F, long long ld, cudaStream_t st) {
+  if (!s.masked || s.fdims[n] == 0) return 0;
+  const int R = s.R;
+  return dgemm_small_splitk(1, 0, R, R, s.fdims[n], 1.0, s.B[n], s.fdims[n], F, ld, 0.0, s.cg + (size_t)n * R * R, R,
                             s.gemm_ws, st, nullptr);
 }
 
-int sparse_em(SparseTensor& s, const double* const* fac, const long long* ld, bool impute, double* sums, cudaStream_t st) {
+int sparse_em_nonzeros(SparseTensor& s, const double* const* fac, const long long* ld, bool impute, cudaStream_t st) {
   const int R = s.R;
   int launches = 0;
-  // 1. model at the nonzeros (canonical order), four fixed-order sums; impute: m = m', r = s - m'
+  // model at the nonzeros (canonical order), four fixed-order sums; impute: m = m', r = s - m'
   unsigned nbm = 0;
   if (s.nnz > 0) {
     ModelArgs a{};
@@ -784,7 +815,7 @@ int sparse_em(SparseTensor& s, const double* const* fac, const long long* ld, bo
     a.idx = s.modes[0].idx;
     a.vals = s.modes[0].vals;
     for (int d = 0; d < s.order; ++d) {
-      launches += transpose_scale(fac[d], s.dims[d], R, ld[d], s.factT[d], R, 1.0, st);
+      launches += transpose_scale(fac[d] + (d == s.order - 1 ? s.shift : 0), s.dims[d], R, ld[d], s.factT[d], R, 1.0, st);
       a.F[d] = s.factT[d];
     }
     a.m = s.mvals;
@@ -795,10 +826,19 @@ int sparse_em(SparseTensor& s, const double* const* fac, const long long* ld, bo
     AO_CHECK_LAUNCH();
     ++launches;
   }
-  // 2. Grams of [F_d | B_d | F_d - B_d] (impute: B_d = F_d afterwards), telescoped ||M' - M||^2 and ||M||^2
+  em_nz_kernel<<<1, 32, 0, st>>>(s.em_partials + 2 * kTeleBlocks, nbm, s.em_nz);
+  AO_CHECK_LAUNCH();
+  return launches + 1;
+}
+
+int sparse_em_finish(SparseTensor& s, const double* const* fac, const long long* ld, bool impute, double* sums,
+                     cudaStream_t st) {
+  const int R = s.R;
+  int launches = 0;
+  // Grams of [F_d | B_d | F_d - B_d] (impute: B_d = F_d afterwards), telescoped ||M' - M||^2 and ||M||^2
   const long long R3 = 3LL * R;
   for (int d = 0; d < s.order; ++d) {
-    const long long rows = s.dims[d];
+    const long long rows = s.fdims[d];
     double* g = s.g3 + (size_t)d * R3 * R3;
     if (rows == 0) {
       AO_CUDA(cudaMemsetAsync(g, 0, (size_t)R3 * R3 * sizeof(double), st));
@@ -812,7 +852,7 @@ int sparse_em(SparseTensor& s, const double* const* fac, const long long* ld, bo
   double* tpart = s.em_partials;
   tele_partials_kernel<<<nbt, 256, 0, st>>>(s.g3, s.order, R, tpart);
   AO_CHECK_LAUNCH();
-  em_final_kernel<<<1, 32, 0, st>>>(s.em_partials + 2 * kTeleBlocks, nbm, tpart, nbt, sums);
+  em_final_kernel<<<1, 32, 0, st>>>(s.em_nz, tpart, nbt, sums);
   AO_CHECK_LAUNCH();
   launches += 2;
   if (impute) {   // B = F: the cross-Grams B_d' F_d are the F_d' F_d blocks just computed

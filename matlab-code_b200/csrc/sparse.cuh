@@ -12,6 +12,12 @@
 // order never depends on the launch configuration).  A group of lanes (columns across lanes) walks one unit; a row that
 // starts and ends inside the unit is written directly, the partial rows at the unit's ends go to carry buffers, and a
 // fix-up pass adds the carries of a split row in unit order.  No floating-point atomics: every output is bit-reproducible.
+//
+// Several GPUs (aoadmm_create_sparse_multi): each GPU holds the nonzeros of one contiguous slab of the last mode,
+// shard_offset .. shard_offset + shard_extent - 1.  The nonzero side (the sorted copies, the imputation state m / r) is
+// local, with the last subscript shifted into the slab on the device; the factors and the factor side of the EM state
+// (B, the cross-Grams, the stacks and their Grams) keep the full extents and are replicated.  The caller all-reduces the
+// partial products (sparse_mttkrp) and the nonzero-side EM sums (sparse_em_nonzeros), then adds the replicated terms.
 #pragma once
 #include <type_traits>
 #include <vector>
@@ -94,8 +100,10 @@ struct SparseMode {
 
 struct SparseTensor {
   int order = 0, R = 0;
-  long long nnz = 0;                // after merging duplicates
-  long long dims[8] = {0};
+  long long nnz = 0;                // after merging duplicates (this GPU's slab)
+  long long dims[8] = {0};          // extents of the nonzero side: the last one is the slab extent
+  long long fdims[8] = {0};         // full extents (factor side)
+  long long shift = 0;              // first last-mode index of the slab
   std::vector<SparseMode> modes;
   double* factT[8] = {nullptr};     // row-major (rows x R) copies of the factors, refreshed per MTTKRP
   double* outT = nullptr;           // row-major product, max rows x R
@@ -116,31 +124,44 @@ struct SparseTensor {
   double* g3 = nullptr;             // order x (3R)^2: Grams of the stacks
   double* gemm_ws = nullptr;        // split-K partial tiles of the Gram products
   double* em_partials = nullptr;    // per-CTA sums of the model pass (4 per CTA) and of the telescoped norms (2 per CTA)
+  double* em_nz = nullptr;          // 4: nonzero-side sums of the model pass (sparse_em_nonzeros)
 };
 
 // Uploads and preprocesses one COO object: subs is nnz x order column-major (0-based, validated by the caller), vals nnz
 // values.  Duplicates are summed.  Allocates every scratch buffer the MTTKRP needs.  Synchronous on `st`.
+// full_dims: the object's extents; the entries all lie in the slab [shard_offset, shard_offset + shard_extent) of the
+// last mode (whole object: 0, full_dims[order - 1]).
 // masked: the object has a sparse Z.miss mask (mask_nnz entries, same layout as subs / vals).  An entry is observed when its merged value
 // is nonzero; the observed set must equal the stored set of the object (else CudaError UNSUPPORTED).  Allocates the EM
 // state (sparse.cuh above) with m = 0, r = s, B = 0.
-void sparse_build(SparseTensor& s, int order, const long long* dims, int R, long long nnz, const long long* subs,
-                  const double* vals, cudaStream_t st, bool masked = false, long long mask_nnz = 0,
-                  const long long* mask_subs = nullptr, const double* mask_vals = nullptr);
+void sparse_build(SparseTensor& s, int order, const long long* full_dims, long long shard_offset, long long shard_extent,
+                  int R, long long nnz, const long long* subs, const double* vals, cudaStream_t st, bool masked = false,
+                  long long mask_nnz = 0, const long long* mask_subs = nullptr, const double* mask_vals = nullptr);
 void sparse_free(SparseTensor& s);
-// ||X||_F^2 = sum of the squared merged values (fixed-order reduction); the result lands in s.norm_out (device)
+// ||X||_F^2 = sum of the squared merged values (fixed-order reduction); the result lands in s.norm_out (device).  A slab
+// gives its partial sum.
 int sparse_norm2(const SparseTensor& s, cudaStream_t st);
-// out (rows(n) x R, column-major, leading dimension ldout) = scale * MTTKRP of mode position n, from the column-major
-// factors fac[d] (leading dimension ld[d]) of all mode positions.  Returns the number of kernel launches.
-// imputed (masked objects): the MTTKRP of the imputed tensor S + (1-W).*[[B]] = (S - W.*[[B]]) + [[B]], i.e. the sparse
-// pass over r plus the low-rank term B_n * (Hadamard of cg_k, k != n); else the MTTKRP of the stored values.
+// out (rows(n) x R, column-major, leading dimension ldout) = scale * MTTKRP of mode position n over this GPU's nonzeros,
+// from the full column-major factors fac[d] (leading dimension ld[d]) of all mode positions.  For the last position only
+// the slab's rows (at their global position) are written.  Returns the number of kernel launches.
+// imputed (masked objects): the sparse pass over the residuals r, the first part of the MTTKRP of the imputed tensor
+// S + (1-W).*[[B]] = (S - W.*[[B]]) + [[B]]; sparse_lowrank_add adds the second; else the MTTKRP of the stored values.
 int sparse_mttkrp(SparseTensor& s, int n, const double* const* fac, const long long* ld, double scale, double* out,
                   long long ldout, cudaStream_t st, bool imputed = false);
+// masked objects: out (full rows(n) x R) += scale * B_n * (Hadamard of cg_k, k != n), the low-rank term of the imputed
+// MTTKRP.  It only reads replicated state: with several GPUs it is added once, after the all-reduce of the sparse part.
+int sparse_lowrank_add(SparseTensor& s, int n, double scale, double* out, long long ldout, cudaStream_t st);
 // masked objects: cg_n = B_n' * F (F: dims[n] x R, leading dimension ld), after every update of position n
 int sparse_cross_gram(SparseTensor& s, int n, const double* F, long long ld, cudaStream_t st);
-// masked objects: the EM step of cmtf_fun_AOADMM.m:408-441 without a dense tensor.  One pass over the nonzeros computes
-// m' = [[F]] there; sums[2] = sum s m', sums[3] = sum m'^2 (masked objective), sums[0] / sums[1] = the missing-entry
-// numerator / denominator of f_rel_missing from the telescoped ||[[F]] - [[B]]||^2 and ||[[B]]||^2, sums[4] = 0.
-// impute: afterwards m = m', r = s - m', B = F and the cross-Grams are refreshed.  Graph-capturable.
-int sparse_em(SparseTensor& s, const double* const* fac, const long long* ld, bool impute, double* sums, cudaStream_t st);
+// masked objects: the EM step of cmtf_fun_AOADMM.m:408-441 without a dense tensor, in two parts (graph-capturable).
+// sparse_em_nonzeros: one pass over this GPU's nonzeros computes m' = [[F]] there and the nonzero-side sums s.em_nz =
+// [sum s m', sum m'^2, sum_W (m' - m)^2, sum_W m^2]; impute: afterwards m = m', r = s - m'.  With several GPUs the
+// caller all-reduces the 4 values of s.em_nz.
+// sparse_em_finish: the replicated factor side, then sums[2] = sum s m', sums[3] = sum m'^2 (masked objective),
+// sums[0] / sums[1] = the missing-entry numerator / denominator of f_rel_missing from the telescoped ||[[F]] - [[B]]||^2
+// and ||[[B]]||^2 minus the nonzero-side terms, sums[4] = 0; impute: B = F and the cross-Grams are refreshed.
+int sparse_em_nonzeros(SparseTensor& s, const double* const* fac, const long long* ld, bool impute, cudaStream_t st);
+int sparse_em_finish(SparseTensor& s, const double* const* fac, const long long* ld, bool impute, double* sums,
+                     cudaStream_t st);
 
 }  // namespace aoadmm

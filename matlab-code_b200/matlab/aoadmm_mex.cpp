@@ -9,7 +9,8 @@
 // cmtf_AOADMM.m:124-156, G from init_coupled_AOADMM_CMTF.m or the caller, options from the script (:120-132).
 //
 // Engine knobs read from options (all optional): b200_gpus (number of B200s this MATLAB session drives through
-// aoadmm_create_multi, default 1), b200_dimtree, b200_mttkrp_precision, b200_fuse_inner, b200_graph.
+// aoadmm_create_multi, default 1), b200_shard_sparse (with b200_gpus > 1: sparse objects too, through
+// aoadmm_create_sparse_multi), b200_dimtree, b200_mttkrp_precision, b200_fuse_inner, b200_graph.
 //
 // Sparse CP objects arrive as struct('subs',S,'vals',V,'size',sz) (cmtf_fun_AOADMM.m unwrap_data: sptensor or a MATLAB
 // sparse matrix through find); the 1-based double subscripts become 0-based int64 and the handle is created with
@@ -425,12 +426,18 @@ void solve(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
   pb.constraints = cons.data();
   pb.ridge = (ridge != nullptr && !mxIsEmpty(ridge)) ? mxGetPr(ridge) : nullptr;
 
-  // one MATLAB session drives options.b200_gpus devices (default 1): the library cuts the mode-3 slabs itself
+  // one MATLAB session drives options.b200_gpus devices (default 1): the library cuts the mode-3 slabs itself.
+  // options.b200_shard_sparse = true also cuts sparse objects, into nonzero-balanced slabs of their last mode.
   const int n_gpus = (int)opt_scalar(opt, "b200_gpus", 1.0);
+  const bool shard_sparse = opt_scalar(opt, "b200_shard_sparse", 0.0) != 0.0;
   if (n_gpus < 1) fail("aoadmm:invalidArg", "options.b200_gpus must be >= 1");
-  if (any_sparse && n_gpus > 1) fail("aoadmm:unsupported", "sparse objects run on one GPU (options.b200_gpus must be 1)");
+  if (any_sparse && n_gpus > 1 && !shard_sparse)
+    fail("aoadmm:unsupported", "sparse objects run on one GPU (options.b200_gpus must be 1, or set options.b200_shard_sparse)");
   HandleGuard guard;
-  if (any_mask)
+  if (any_sparse && n_gpus > 1)
+    check(aoadmm_create_sparse_multi(&pb, sp_ptr.data(), any_mask ? mk_ptr.data() : nullptr, n_gpus, nullptr, &guard.h),
+          nullptr);
+  else if (any_mask)
     check(aoadmm_create_sparse_masked(&pb, sp_ptr.data(), mk_ptr.data(), nullptr, &guard.h), nullptr);
   else if (any_sparse)
     check(aoadmm_create_sparse(&pb, sp_ptr.data(), nullptr, &guard.h), nullptr);

@@ -13,7 +13,8 @@ function [G,out] = cmtf_fun_AOADMM(Z,Znorm_const,G,fh,gh,lscalar,uscalar,options
 % 'aoadmm:unsupported' (there is deliberately no CPU fallback: remove this directory from the path to run the
 % reference's MATLAB solver).
 % Engine options (fields of `options`, all optional): b200_gpus = number of B200s of this box the call uses (the
-% tensors are cut into mode-3 slabs inside the library, one MATLAB process drives all of them), b200_dimtree,
+% tensors are cut into mode-3 slabs inside the library, one MATLAB process drives all of them), b200_shard_sparse =
+% true (with b200_gpus > 1: sparse objects too are cut, into nonzero-balanced slabs of their last mode), b200_dimtree,
 % b200_mttkrp_precision, b200_fuse_inner, b200_graph, b200_heldout{p} = an sptensor / sparse matrix of entries of object p
 % withheld from training (with their true values; object p needs Z.miss): out.heldout_sse{p} is then the held-out SSE
 % after outer iterations 0..OuterIterations.

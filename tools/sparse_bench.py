@@ -54,9 +54,11 @@ ZERO_TOL = dict(AbsFuncTol=0.0, OuterRelTol=0.0, innerRelPrTol_coupl=0.0, innerR
 
 
 def card():
-    out = subprocess.run(['nvidia-smi', '--query-gpu=name,power.limit', '--format=csv,noheader', '-i', '0'],
-                         capture_output=True, text=True, check=True).stdout.strip().split(', ')
-    return {'name': out[0], 'power_limit': out[1]}
+    out = subprocess.run(['nvidia-smi', '--query-gpu=name,power.limit', '--format=csv,noheader'],
+                         capture_output=True, text=True, check=True).stdout.strip().split('\n')
+    first = out[0].split(', ')
+    return {'name': first[0], 'power_limit': first[1], 'visible_gpus': len(out),
+            'power_limits': sorted(set(l.split(', ')[1] for l in out))}
 
 
 def options(iters, **kw):
@@ -174,8 +176,7 @@ def powerlaw(rng, n, extent):
     return np.minimum((extent * rng.rand(n) ** 3).astype(np.int64), extent - 1)
 
 
-def s2(scale, iters, reps, seed=0, R=32):
-    rng = np.random.RandomState(seed)
+def s2_problem(rng, scale, R):
     I, J, K, M = 1 << 20, 1 << 20, 1 << 14, 1 << 16
     shape = (I, J, K)
     nnz = int(2e8 * scale)
@@ -185,6 +186,12 @@ def s2(scale, iters, reps, seed=0, R=32):
     ysubs = np.stack([powerlaw(rng, ny, I), rng.randint(0, M, size=ny)], axis=1)
     yvals = rng.rand(ny)
     Zs = problem([ab.sptensor(subs, vals, shape), ab.sptensor(ysubs, yvals, (I, M))], [I, J, K, I, M], R, [1, 0, 0, 1, 0])
+    return Zs, shape, nnz, subs, vals, ny, (I, M)
+
+
+def s2(scale, iters, reps, seed=0, R=32):
+    rng = np.random.RandomState(seed)
+    Zs, shape, nnz, subs, vals, ny, (I, M) = s2_problem(rng, scale, R)
     sp, t_create = timed_create(Zs, [float('nan'), float('nan')])
     G = init_state(Zs, R, seed + 1)
     sp.set_state(G)
@@ -395,8 +402,7 @@ def m1(scale, iters, seed=0, R=32):
     return line
 
 
-def m2(scale, iters, seed=0, R=32):
-    rng = np.random.RandomState(seed)
+def m2_problem(rng, scale, R):
     shape = (1 << 20, 1 << 16, 1 << 10)
     nnz = int(1e8 * scale)
     subs = np.stack([powerlaw(rng, nnz, shape[0]), powerlaw(rng, nnz, shape[1]), powerlaw(rng, nnz, shape[2])], axis=1)
@@ -407,6 +413,12 @@ def m2(scale, iters, seed=0, R=32):
          'constrained_modes': [1] * n, 'constraints': [('non-negativity',)] * n, 'weights': [1.0],
          'object': [ab.sptensor(subs, vals, shape)], 'rank': [R]}
     Zm = dict(Z, miss=[ab.sptensor(subs, np.ones(nnz), shape)])
+    return Z, Zm, shape, nnz, subs, vals
+
+
+def m2(scale, iters, seed=0, R=32):
+    rng = np.random.RandomState(seed)
+    Z, Zm, shape, nnz, subs, vals = m2_problem(rng, scale, R)
     G = init_state(Zm, R, seed + 1)
     sp, t_sp = timed_create(Zm, [float('nan')])
     un, t_un = timed_create(Z, [float('nan')])
@@ -467,6 +479,79 @@ def m2(scale, iters, seed=0, R=32):
                              'cores': os.cpu_count(), 'ms_per_iteration': cpu_ms}}
 
 
+# ---- s2 / m2 on several GPUs (aoadmm_create_sparse_multi) --------------------------------------------------------
+def per_gpu_ms(fn, names, div):
+    """Device time per GPU (ms / div) of the kernels whose name contains one of `names`, from one profiled call."""
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        fn()
+        torch.cuda.synchronize()
+    per = {}
+    for e in prof.events():
+        if e.device_type == torch.autograd.DeviceType.CUDA and any(k in e.name for k in names):
+            per[e.device_index] = per.get(e.device_index, 0.0) + e.time_range.elapsed_us() / 1e3
+    return per
+
+
+def multi(name, counts, scale, iters, reps, seed=0, R=32):
+    """s2 or m2 with Solver(..., n_gpus=N, shard_sparse=True) for every N in counts: the nonzero share of every GPU,
+    create time, outer it/s (median of rounds that alternate the GPU counts), the local sparse pass per mode (max and
+    min over the GPUs, torch.profiler kernel times of aoadmm_time_mttkrp), the NCCL all-reduce time per outer iteration
+    (torch.profiler, a separate run with graph replay off) and agreement with the one-GPU run."""
+    rng = np.random.RandomState(seed)
+    if name == 's2':
+        Z, shape, nnz, subs, _, _, _ = s2_problem(rng, scale, R)
+        zn = [float('nan'), float('nan')]
+    else:
+        _, Z, shape, nnz, subs, _ = m2_problem(rng, scale, R)
+        zn = [float('nan')]
+    G = init_state(Z, R, seed + 1)
+    last = np.sort(subs[:, -1])
+    sol, lines = {}, {}
+    for n in counts:
+        t0 = time.perf_counter()
+        sol[n] = ab.Solver(Z, zn, n_gpus=n, shard_sparse=True)
+        b = ab.sparse_shard_bounds(Z['object'][0], n)
+        lines[n] = {'workload': name + '_multi', 'n_gpus': n, 'shape': list(shape), 'R': R, 'nnz': nnz, 'iters': iters,
+                    'create_s': time.perf_counter() - t0, 'bounds': b.tolist(),
+                    'nnz_share': (np.diff(np.searchsorted(last, b)) / nnz).tolist()}
+    ref = None
+    for n in counts:
+        s = sol[n]
+        s.set_state(G)
+        o = s.run(options(iters))
+        Gn = s.get_state()
+        if ref is None:
+            ref = (n, o, Gn)
+        lines[n]['compare_to_gpus'] = ref[0]
+        lines[n]['factors_max_rel'] = max(float(np.linalg.norm(a - c) / np.linalg.norm(c))
+                                          for a, c in zip(Gn['fac'], ref[2]['fac']))
+        lines[n]['objective_max_rel'] = float(np.max(np.abs(o['func_val_conv'] - ref[1]['func_val_conv']) /
+                                                     np.abs(ref[1]['func_val_conv'])))
+    ips = {n: [] for n in counts}
+    for _ in range(3):
+        for n in counts:
+            ips[n].append(iters_per_s(sol[n], G, iters))
+    kern = ('sp_mttkrp_kernel', 'sp_fixup_kernel', 'transpose_scale')
+    for n in counts:
+        s = sol[n]
+        lines[n]['outer_iters_per_s'] = float(np.median(ips[n]))
+        lines[n]['outer_iters_per_s_rounds'] = ips[n]
+        modes = []
+        for pos in range(1, len(shape) + 1):
+            per = per_gpu_ms(lambda: s.time_mttkrp(1, pos, reps), kern, reps + 1)
+            modes.append({'mode': pos, 'local_pass_ms_max': max(per.values()), 'local_pass_ms_min': min(per.values()),
+                          'time_mttkrp_ms': s.time_mttkrp(1, pos, reps)})
+        lines[n]['modes'] = modes
+        s.set_state(G)
+        per = per_gpu_ms(lambda: s.run(options(iters, graph=-1)), ('nccl',), iters)
+        lines[n]['allreduce_ms_per_iter'] = {'max': max(per.values()) if per else 0.0,
+                                             'min': min(per.values()) if per else 0.0}
+        s.close()
+    return [lines[n] for n in counts]
+
+
 def main():
     ap = argparse.ArgumentParser(description=__doc__.split('\n')[0])
     ap.add_argument('--workloads', default='s1,s2')
@@ -475,11 +560,21 @@ def main():
     ap.add_argument('--m-scale', type=float, default=1.0, help='fraction of the m1 / m2 observed-entry counts')
     ap.add_argument('--iters', type=int, default=5)
     ap.add_argument('--reps', type=int, default=5)
+    ap.add_argument('--gpus', default=None,
+                    help='comma-separated GPU counts, e.g. 1,2,8: run s2 / m2 (from --workloads) with shard_sparse=True '
+                         'on each count instead of the one-GPU workloads')
     a = ap.parse_args()
     if ab.device_count() < 1:
         raise SystemExit('sparse_bench: no CUDA device (the engine has no CPU path)')
     c = card()
     wl = a.workloads.split(',')
+    if a.gpus is not None:
+        for w in ('s2', 'm2'):
+            if w in wl:
+                scale = a.s2_scale if w == 's2' else a.m_scale
+                for line in multi(w, [int(x) for x in a.gpus.split(',')], scale, a.iters, a.reps):
+                    print(json.dumps(dict(line, card=c)), flush=True)
+        return
     if 's1' in wl:
         for d in (float(x) for x in a.densities.split(',')):
             print(json.dumps(dict(s1(d, a.iters, a.reps), card=c)), flush=True)
