@@ -34,7 +34,8 @@ extern "C" {
  *    later additions that leave every v4 struct and entry point unchanged: aoadmm_sparse_object / aoadmm_create_sparse
  *    (sparse CP objects), aoadmm_create_sparse_masked (sparse Z.miss masks on sparse objects), aoadmm_model_at /
  *    aoadmm_set_heldout / aoadmm_heldout_history (held-out entries), aoadmm_sparse_shard_bounds /
- *    aoadmm_create_sparse_multi (sparse objects on several GPUs from one caller). */
+ *    aoadmm_create_sparse_multi (sparse objects on several GPUs from one caller), aoadmm_set_heldout_stopping /
+ *    aoadmm_heldout_best and bit 9 of aoadmm_out.exit_flag (early stopping on the held-out error). */
 #define AOADMM_ABI_VERSION 4
 
 typedef struct aoadmm_handle aoadmm_handle;
@@ -175,7 +176,8 @@ typedef struct {
   int32_t OuterIterations;
   int32_t exit_flag;          /* 0 'maxIterations'; else bit mask of the make_exit_flag.m:9-28 struct:
                                  bit0 f_tensors<AbsFuncTol, bit1 f_couplings, bit2 f_constraints,
-                                 bit3 f_PAR2 (bit set = "AbsFuncTol", clear = "RelFuncTol"), bit8 = stopped */
+                                 bit3 f_PAR2 (bit set = "AbsFuncTol", clear = "RelFuncTol"), bit8 = stopped;
+                                 exactly 1 << 9: the held-out rule of aoadmm_set_heldout_stopping ended the run */
   double *func_val_conv, *func_coupl_conv, *func_constr_conv, *func_PAR2_coupl, *time_at_it;
   int32_t *inner_iters;
   int32_t error_mode;         /* mode id that raised NOT_POSITIVE_DEFINITE / NON_FINITE (0 if none) */
@@ -316,6 +318,33 @@ int aoadmm_create_sparse_multi(const aoadmm_problem *problem, const aoadmm_spars
 int aoadmm_model_at(aoadmm_handle *h, int32_t object, const aoadmm_sparse_object *entries, double *out);
 int aoadmm_set_heldout(aoadmm_handle *h, int32_t object, const aoadmm_sparse_object *entries);
 int aoadmm_heldout_history(const aoadmm_handle *h, int32_t object, double *sse, int64_t n, int64_t *count);
+
+/* ---- early stopping on the held-out error: keep the best iterate and return it ------------------
+ * Let s_k be the sum, over the objects with a held-out set (in object order), of the held-out SSE after outer iteration
+ * k.  k* is the first k in 1..n with the smallest s_k: a new best must be strictly smaller, a NaN is never one, and the
+ * initial state (k = 0) is not a candidate.  With patience P >= 1 the run ends after iteration k once k - k* >= P.
+ * MaxOuterIters and the tolerance rule (evaluate_stopping_conditions.m:44, cmtf_fun_AOADMM.m:457-459) still apply; the
+ * held-out rule ends the run only at an iteration where neither of them does.  However the run ends, the handle is
+ * then left in the state after iteration k*: G, the PARAFAC2 state, the imputation of every object with missing data
+ * and everything else a next aoadmm_run reads, so that run continues exactly as if this one had been made with
+ * MaxOuterIters = k*.  When no s_k (k >= 1) is a number, or n = 0, k* = n and nothing is restored.
+ * out: the history arrays and OuterIterations describe the n iterations run; f_tensors, f_couplings, f_constraints,
+ * f_PAR2_couplings and f_rel_missing are the values at k* (the history entries at k*); exit_flag is exactly 1 << 9 when
+ * the held-out rule ended the run, and what it would be without stopping otherwise.  With stopping off (the default)
+ * nothing changes.
+ * aoadmm_set_heldout_stopping: patience >= 1 turns stopping on, 0 turns it off.  The snapshot buffers are allocated here
+ *     (one copy of the buffers above: about the size of G, the factor-side state, again) and freed when it is turned
+ *     off, so aoadmm_run stays allocation-free.  A snapshot is one kernel launch after an iteration that sets a new best,
+ *     outside the CUDA graph; the restore is one launch plus the EM pass of the objects with missing data.
+ *     AOADMM_ERR_INVALID_ARG for a NULL handle, a negative patience, or (patience >= 1) no attached held-out set;
+ *     AOADMM_ERR_OOM when the snapshot cannot be allocated, leaving stopping off.  aoadmm_run returns
+ *     AOADMM_ERR_INVALID_ARG before any device work when stopping is on but every held-out set has been detached.
+ *     With several GPUs every rank sees the same SSE bits and makes the same decisions without communication; each
+ *     snapshots and restores what it holds.
+ * aoadmm_heldout_best: k* and s_{k*} of the last run (n = 0: 0 and s_0).  AOADMM_ERR_INVALID_ARG when the last run had
+ *     stopping off, or when there was no run. */
+int aoadmm_set_heldout_stopping(aoadmm_handle *h, int32_t patience);
+int aoadmm_heldout_best(const aoadmm_handle *h, int32_t *iteration, double *sse);
 
 /* ---- state in / out (G is both input and output of cmtf_fun_AOADMM.m:1) ------------------- */
 int aoadmm_set_state(aoadmm_handle *h, int32_t field, int32_t index, int32_t slice,

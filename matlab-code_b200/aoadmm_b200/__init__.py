@@ -93,6 +93,34 @@ def _check_heldout(Z, p, X):
     return S
 
 
+def heldout_stopping_rule(s, patience):
+    """The rule of early stopping on the held-out error (aoadmm_set_heldout_stopping) on a history s_0..s_n of summed
+    held-out SSEs: (k_best, k_stop).  k_best is the first k >= 1 with the smallest s_k (a new best must be strictly
+    smaller, a NaN is never one); n when no s_k (k >= 1) is a number, which includes n = 0.  k_stop is the first k with
+    k - k_best >= patience, or None when the rule does not fire within the history."""
+    s = [float(v) for v in s]
+    best, stop = -1, None
+    for k in range(1, len(s)):
+        if (not np.isnan(s[k])) if best < 0 else s[k] < s[best]:
+            best = k
+        elif best > 0 and k - best >= patience:
+            stop = k
+            break
+    return (len(s) - 1 if best < 0 else best), stop
+
+
+def _heldout_sum(hists):
+    """s_k = the sum of the per-object held-out SSEs in object order, added as the engine adds them."""
+    n = max(len(h) for h in hists)
+    out = np.zeros(n)
+    for k in range(n):
+        t = 0.0
+        for h in hists:
+            t += h[k]
+        out[k] = t
+    return out
+
+
 def _coo(subs, vals):
     """aoadmm_sparse_object over column-major copies of subs (nnz x N) and vals; returns it with the arrays to keep."""
     subs = np.asfortranarray(np.asarray(subs, dtype=np.int64))
@@ -588,6 +616,8 @@ class Solver:
         self._last_iters = it
         if out.exit_flag == 0:
             flag = 'maxIterations'                                        # make_exit_flag.m:4-5
+        elif out.exit_flag == 1 << 9:
+            flag = 'heldoutStop'                                          # set_heldout_stopping
         else:
             names = ['f_tensors', 'f_couplings', 'f_constraints', 'f_PAR2_couplings']
             flag = {nm: ('AbsFuncTol' if (out.exit_flag >> q) & 1 else 'RelFuncTol') for q, nm in enumerate(names)}
@@ -628,6 +658,19 @@ class Solver:
         count = C.c_int64(0)
         _capi.check(lib.aoadmm_heldout_history(self._h, int(obj), _dp(sse), n, C.byref(count)), self._h)
         return sse[:n], count.value
+
+    def set_heldout_stopping(self, patience):
+        """Early stopping on the held-out error: patience P >= 1 ends a run once P outer iterations have passed without
+        a new smallest sum of the held-out SSEs, and leaves the solver in the state of the best iteration k* (factors,
+        duals and the imputation of missing entries); the f_* values of `out` are then those at k*.  None or 0 turns it
+        off.  Needs an attached held-out set (see include/aoadmm.h for the whole rule)."""
+        _capi.check(lib.aoadmm_set_heldout_stopping(self._h, 0 if patience is None else int(patience)), self._h)
+
+    def heldout_best(self):
+        """(k*, s_k*) of the last run, which must have had early stopping on."""
+        k, sse = C.c_int32(0), C.c_double(0)
+        _capi.check(lib.aoadmm_heldout_best(self._h, C.byref(k), C.byref(sse)), self._h)
+        return k.value, sse.value
 
     # ---- benchmark helpers --------------------------------------------------------------------
     def generate_cp_data(self, obj, factors, noise, seed):
@@ -706,12 +749,15 @@ def _with_rank(Z, G):
 
 
 def cmtf_fun_AOADMM(Z, Znorm_const, G, fh=None, gh=None, lscalar=None, uscalar=None, options=None, heldout=None,
-                    **dist):
+                    heldout_patience=None, **dist):
     """[G,out] = cmtf_fun_AOADMM(Z,Znorm_const,G,fh,gh,lscalar,uscalar,options)  (cmtf_fun_AOADMM.m:1).
 
     fh/gh/lscalar/uscalar are [] for the Frobenius loss (cmtf_AOADMM.m:158-161) and are ignored.
     `heldout`: one entry per object, None or a held-out set (sptensor / SciPy sparse) of an object with Z.miss; adds
     out['heldout_sse'] (per object: the SSE after outer iterations 0..OuterIterations, or None) and out['heldout_count'].
+    `heldout_patience` (needs `heldout`): early stopping on the summed held-out SSE (Solver.set_heldout_stopping); G and
+    the f_* values are those of the best iteration, out['heldout_best_iter'] is that iteration, and out['exit_flag'] is
+    'heldoutStop' when the held-out rule ended the run.
     `dist` (rank, world_size, device, unique_id, or n_gpus [, devices, shard_sparse]) selects the multi-GPU layout;
     default one GPU."""
     if heldout is not None:
@@ -720,16 +766,30 @@ def cmtf_fun_AOADMM(Z, Znorm_const, G, fh=None, gh=None, lscalar=None, uscalar=N
         for p, X in enumerate(heldout):
             if X is not None:
                 _check_heldout(Z, p, X)
+    if heldout_patience is not None:
+        if int(heldout_patience) < 0:
+            raise AoadmmError(1, 'heldout_patience must be >= 0 (0: no early stopping)')
+        if heldout_patience and not any(X is not None for X in (heldout or [])):
+            raise AoadmmError(1, 'heldout_patience needs a held-out set (heldout=[...])')
     with Solver(_with_rank(Z, G), Znorm_const, **dist) as s:
         s.set_state(G)
         for p, X in enumerate(heldout or []):
             if X is not None:
                 s.set_heldout(p + 1, X)
+        if heldout_patience:
+            s.set_heldout_stopping(int(heldout_patience))
         out = s.run(options)
         if heldout is not None:
             hist = [s.heldout_history(p + 1) if X is not None else (None, None) for p, X in enumerate(heldout)]
             out['heldout_sse'] = [h[0] for h in hist]
             out['heldout_count'] = [h[1] for h in hist]
+        if heldout_patience:
+            k_best, _ = s.heldout_best()
+            want, k_stop = heldout_stopping_rule(_heldout_sum([h[0] for h in hist if h[0] is not None]),
+                                                 int(heldout_patience))
+            if k_best != want or (out['exit_flag'] == 'heldoutStop' and k_stop != out['OuterIterations']):
+                raise AoadmmError(5, 'early stopping: the engine kept iteration %d, the rule gives %d' % (k_best, want))
+            out['heldout_best_iter'] = k_best
         Gout = s.get_state()
     return Gout, out
 

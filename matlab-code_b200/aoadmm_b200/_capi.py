@@ -97,7 +97,8 @@ EXPORTS = ['aoadmm_abi_version', 'aoadmm_device_count', 'aoadmm_nccl_unique_id',
            'aoadmm_phase_ms', 'aoadmm_last_run_ms', 'aoadmm_get_object_data', 'aoadmm_last_loop_ms', 'aoadmm_object_mttkrp', 'aoadmm_nvecs',
            'aoadmm_create_multi', 'aoadmm_gpu_count', 'aoadmm_comm_release', 'aoadmm_create_sparse',
            'aoadmm_create_sparse_masked', 'aoadmm_model_at', 'aoadmm_set_heldout', 'aoadmm_heldout_history',
-           'aoadmm_sparse_shard_bounds', 'aoadmm_create_sparse_multi']
+           'aoadmm_sparse_shard_bounds', 'aoadmm_create_sparse_multi', 'aoadmm_set_heldout_stopping',
+           'aoadmm_heldout_best']
 
 lib.aoadmm_abi_version.restype = C.c_int
 lib.aoadmm_device_count.argtypes = [C.POINTER(C.c_int)]
@@ -136,6 +137,8 @@ lib.aoadmm_get_object_data.argtypes = [HandleP, C.c_int32, c_double_p, C.c_int64
 lib.aoadmm_model_at.argtypes = [HandleP, C.c_int32, C.POINTER(SparseObject), c_double_p]
 lib.aoadmm_set_heldout.argtypes = [HandleP, C.c_int32, C.POINTER(SparseObject)]
 lib.aoadmm_heldout_history.argtypes = [HandleP, C.c_int32, c_double_p, C.c_int64, c_int64_p]
+lib.aoadmm_set_heldout_stopping.argtypes = [HandleP, C.c_int32]
+lib.aoadmm_heldout_best.argtypes = [HandleP, c_int32_p, c_double_p]
 
 
 class AoadmmError(RuntimeError):

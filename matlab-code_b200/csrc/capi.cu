@@ -583,6 +583,30 @@ int aoadmm_heldout_history(const aoadmm_handle* h, int32_t object, double* sse, 
   return guard(const_cast<aoadmm_handle*>(h), [&] { h->eng[0]->heldout_history(object, sse, n, count); });
 }
 
+int aoadmm_set_heldout_stopping(aoadmm_handle* h, int32_t patience) {
+  if (!h || patience < 0) return AOADMM_ERR_INVALID_ARG;
+  return guard(h, [&] {
+    if (patience > 0 && h->eng[0]->heldout_sets() == 0)
+      throw aoadmm::CudaError(AOADMM_ERR_INVALID_ARG, "set_heldout_stopping: no object has a held-out set");
+    const int n = (int)h->eng.size();
+    try {
+      for_each_rank(n, [&](int r) { h->eng[r]->set_heldout_stopping(patience); });
+    } catch (...) {   // e.g. OOM on one GPU: stopping stays off everywhere
+      for_each_rank(n, [&](int r) { h->eng[r]->set_heldout_stopping(0); });
+      throw;
+    }
+  });
+}
+
+int aoadmm_heldout_best(const aoadmm_handle* h, int32_t* iteration, double* sse) {
+  if (!h || !iteration || !sse) return AOADMM_ERR_INVALID_ARG;
+  return guard(const_cast<aoadmm_handle*>(h), [&] {
+    int k = 0;
+    h->eng[0]->heldout_best(&k, sse);
+    *iteration = k;
+  });
+}
+
 int aoadmm_launch_count(const aoadmm_handle* h, int64_t* count) {
   if (!h || !count) return AOADMM_ERR_INVALID_ARG;
   int64_t total = 0;

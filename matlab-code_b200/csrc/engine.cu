@@ -846,6 +846,7 @@ void Engine::release() {
   if (st2_) cudaStreamSynchronize(st2_);
   cudaGetLastError();
   comm_ = nullptr;   // communicators belong to the process-wide cache (comm_for_unique_id / comms_for_devices)
+  free_snapshot();
   auto dfree = [](auto*& p) {
     if (p) cudaFree(p);
     p = nullptr;
@@ -2253,6 +2254,9 @@ void Engine::sweep(int iter, std::vector<int>& inner_fixed) {
 
 void Engine::run(const aoadmm_options* opt, aoadmm_out* out) {
   if (opt == nullptr || out == nullptr) throw CudaError(1, "run: NULL options/out");
+  if (ho_patience_ > 0 && n_heldout_ == 0)
+    throw CudaError(1, "run: early stopping on the held-out error is on, but no object has a held-out set any more");
+  ho_best_iter_ = -1;
   AO_CUDA(cudaSetDevice(device_));
   opt_ = *opt;
   if (opt_.MaxInnerIters < 1) throw CudaError(1, "MaxInnerIters must be >= 1");
@@ -2330,9 +2334,21 @@ void Engine::run(const aoadmm_options* opt, aoadmm_out* out) {
   GraphGuard guard{gexec};
   int64_t graph_launches = 0;
 
+  // early stopping on the held-out error: s_k = the sum of the held-out SSEs after iteration k (object order); k* = the
+  // first k >= 1 with the smallest s_k (strictly smaller to replace, NaN never); stop once k - k* >= patience
+  auto heldout_sum = [&]() {
+    double t = 0.0;
+    for (int p = 0; p < n_objects_; ++p)
+      if (objects_[p].ho != nullptr) t += ho_sse_host_[p];
+    return t;
+  };
+  int best_k = -1;
+  double best_s = 0.0, best_f[4] = {0, 0, 0, 0}, best_rel = 0.0;
+  bool ho_stop = false;
+
   int iter = 1;
   bool stop = false;
-  while (iter <= opt_.MaxOuterIters && !stop) {
+  while (iter <= opt_.MaxOuterIters && !stop && !ho_stop) {
     const double f_old[4] = {f[0], f[1], f[2], f[3]};
     if (gexec != nullptr) {
       // steady state of a launch-bound problem: the whole outer iteration is one CUDA-graph launch
@@ -2390,7 +2406,41 @@ void Engine::run(const aoadmm_options* opt, aoadmm_out* out) {
            stop_one(f[2], f_old[2], opt_.AbsFuncTol, opt_.OuterRelTol) &&
            stop_one(f[3], f_old[3], opt_.AbsFuncTol, opt_.OuterRelTol);   // evaluate_stopping_conditions.m:44
     if (has_missing_) stop = stop && (f_rel_missing_ < opt_.OuterRelTol);  // :457-459
+    if (ho_patience_ > 0) {
+      const double sk = heldout_sum();
+      if (best_k < 0 ? !std::isnan(sk) : sk < best_s) {
+        best_k = iter;
+        best_s = sk;
+        std::copy(f, f + 4, best_f);
+        best_rel = f_rel_missing_;
+        // a later restore needs this state only when the run goes on (every rank decides alike: the SSE is replicated)
+        if (!stop && iter < opt_.MaxOuterIters) snapshot_state();
+      } else if (best_k > 0 && iter - best_k >= ho_patience_ && !stop && iter < opt_.MaxOuterIters) {
+        ho_stop = true;   // the held-out rule ends the run only where the other rules would not
+      }
+    }
     ++iter;
+  }
+  const int n_run = iter - 1;
+  int exit_flag = 0;
+  if (ho_stop) {
+    exit_flag = 1 << 9;
+  } else if (iter <= opt_.MaxOuterIters) {                           // make_exit_flag.m:4-5
+    exit_flag = 1 << 8;
+    for (int q = 0; q < 4; ++q)
+      if (f[q] < opt_.AbsFuncTol) exit_flag |= (1 << q);
+  }
+  if (ho_patience_ > 0) {
+    if (best_k < 0) {   // no iteration (n = 0) or only NaN sums: the last state is kept
+      best_k = n_run;
+      best_s = heldout_sum();
+    } else if (best_k < n_run) {
+      restore_state();
+      std::copy(best_f, best_f + 4, f);
+      f_rel_missing_ = best_rel;
+    }
+    ho_best_iter_ = best_k;
+    ho_best_sse_ = best_s;
   }
   AO_CUDA(cudaEventRecord(run_ev_[1], st_));
   AO_CUDA(cudaEventSynchronize(run_ev_[1]));
@@ -2406,17 +2456,10 @@ void Engine::run(const aoadmm_options* opt, aoadmm_out* out) {
   out->f_constraints = f[2];
   out->f_PAR2_couplings = f[3];
   out->f_rel_missing = has_missing_ ? f_rel_missing_ : std::nan("");
-  out->OuterIterations = iter - 1;
+  out->OuterIterations = n_run;
   for (int i = n_ctl_ - 1; i >= 0; --i)
     if (ctl_host_[i].warn != 0) out->non_finite_mode = i + 1;
-  if (iter > opt_.MaxOuterIters) {                                   // make_exit_flag.m:4-5
-    out->exit_flag = 0;
-  } else {
-    int fl = 1 << 8;
-    for (int q = 0; q < 4; ++q)
-      if (f[q] < opt_.AbsFuncTol) fl |= (1 << q);
-    out->exit_flag = fl;
-  }
+  out->exit_flag = exit_flag;
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -2902,6 +2945,93 @@ void Engine::heldout_history(int object, double* sse, int64_t n, int64_t* count)
   if (o.ho == nullptr) throw CudaError(1, "heldout_history: object " + std::to_string(object) + " has no held-out set");
   for (int64_t i = 0; i < n; ++i) sse[i] = i < (int64_t)o.ho_hist.size() ? o.ho_hist[i] : std::nan("");
   if (count != nullptr) *count = o.ho->n;
+}
+
+// ---------------------------------------------------------------------------------------------------
+// early stopping on the held-out error (aoadmm_set_heldout_stopping, aoadmm_heldout_best)
+// ---------------------------------------------------------------------------------------------------
+// The snapshot list is every device buffer whose value after an outer iteration a later run reads before rewriting it:
+// G (fac, constraint_fac, constraint_dual_fac, coupling_dual_fac of every mode, coupling_fac of every coupling) and the
+// PARAFAC2 P, DeltaB, mu_DeltaB.  Everything else carried over is a function of these and is rebuilt at restore: the
+// imputation of missing entries (the EM pass), the dimension-tree contraction and the version stamps; the Grams and the
+// packed operands are recomputed by every run and every MTTKRP.  The sweep's other buffers (A, Alast under BSUM, the
+// linear-coupling Dold / Zold, the PARAFAC2 PDold / Vprev / per-slice systems) are written in every outer iteration
+// before they are read.  With sharded PARAFAC2 slices or sparse slabs each rank copies what it holds.
+void Engine::free_snapshot() {
+  if (snap_ != nullptr) cudaFree(snap_);
+  if (snap_table_ != nullptr) cudaFree(snap_table_);
+  snap_ = nullptr;
+  snap_table_ = nullptr;
+  snap_n_ = 0;
+  snap_max_ = 0;
+  ho_patience_ = 0;
+}
+
+void Engine::set_heldout_stopping(int patience) {
+  AO_CUDA(cudaSetDevice(device_));
+  AO_CUDA(cudaStreamSynchronize(st_));
+  free_snapshot();
+  if (patience <= 0) return;
+  std::vector<CopyDesc> list;
+  auto add = [&](DevMat& d) {
+    if (d.p != nullptr && d.rows * d.cols > 0) list.push_back({d.p, nullptr, (long long)(d.rows * d.cols)});
+  };
+  for (auto& m : modes_)
+    for (DevMat* d : {&m.fac, &m.Z, &m.muZ, &m.muD}) add(*d);
+  for (auto& d : delta_) add(d);
+  for (auto& ps : par2_)
+    for (DevMat* d : {&ps.P, &ps.DeltaB, &ps.muDB}) add(*d);
+  size_t total = 0;
+  for (const auto& c : list) total += (size_t)round_up(c.n, 32);   // 256-byte aligned offsets
+  try {
+    AO_CUDA(cudaMalloc(&snap_, std::max<size_t>(total, 1) * sizeof(double)));
+    AO_CUDA(cudaMalloc(&snap_table_, std::max<size_t>(list.size(), 1) * sizeof(CopyDesc)));
+    size_t off = 0;
+    for (auto& c : list) {
+      c.snap = snap_ + off;
+      off += (size_t)round_up(c.n, 32);
+      snap_max_ = std::max(snap_max_, c.n);
+    }
+    AO_CUDA(cudaMemcpy(snap_table_, list.data(), list.size() * sizeof(CopyDesc), cudaMemcpyHostToDevice));
+  } catch (...) {
+    free_snapshot();
+    throw;
+  }
+  snap_n_ = (int)list.size();
+  snap_tree_.assign(n_objects_, 0);
+  ho_patience_ = patience;
+}
+
+// after the synchronisation of a new best iteration, before the next outer iteration (graph launch) is enqueued
+void Engine::snapshot_state() {
+  launches_ += state_copy(snap_table_, snap_n_, snap_max_, 0, st_);
+  for (int p = 0; p < n_objects_; ++p) {
+    const ObjectState& o = objects_[p];
+    snap_tree_[p] = o.Tbuf != nullptr && o.T_version == mode(o.modes[0]).version;
+  }
+}
+
+// back to the state after iteration k*: the copy, new version stamps, then the same deterministic kernels that ran at
+// k* rebuild what depends on the factors, so the state is bit-identical to the one iteration k* left
+void Engine::restore_state() {
+  launches_ += state_copy(snap_table_, snap_n_, snap_max_, 1, st_);
+  for (auto& m : modes_) ++m.version;
+  for (auto& ps : par2_) ps.T_version = 0;
+  // a dimension-tree contraction that was current at k* may be used by the next run without recomputation: emit it
+  // again from the restored mode-1 factor (by the mode-2 MTTKRP, into scratch the next sweep overwrites)
+  for (int p = 0; p < n_objects_; ++p) {
+    ObjectState& o = objects_[p];
+    if (!snap_tree_[p]) continue;
+    ModeState& m2 = mode(o.modes[1]);
+    compute_mttkrp(o, 1, o.weight, m2.A.p, m2.rows);
+  }
+  em_step(true);   // the imputation from the restored factors (its sums are recomputed by the next run)
+}
+
+void Engine::heldout_best(int* iteration, double* sse) const {
+  if (ho_best_iter_ < 0) throw CudaError(1, "heldout_best: the last run had early stopping off (or there was no run)");
+  *iteration = ho_best_iter_;
+  *sse = ho_best_sse_;
 }
 
 }  // namespace aoadmm

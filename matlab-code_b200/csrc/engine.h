@@ -217,6 +217,10 @@ class Engine {
   // of sharded objects (a no-op on one GPU)
   void reduce_norms();
   void heldout_history(int object, double* sse, int64_t n, int64_t* count) const;
+  // early stopping on the held-out error (aoadmm_set_heldout_stopping): patience 0 frees the snapshot, >= 1 allocates it
+  void set_heldout_stopping(int patience);
+  int heldout_sets() const { return n_heldout_; }
+  void heldout_best(int* iteration, double* sse) const;   // k* and its SSE sum of the last run (CudaError if none)
   int64_t launches() const { return launches_; }
   void phase_ms(double ms[3]);
   double last_run_ms() const { return last_run_ms_; }
@@ -328,6 +332,19 @@ class Engine {
   double* ho_sse_host_ = nullptr; // pinned
   void heldout_pass();            // enqueued with the objective; the result rides on its device-to-host copies
   void record_heldout();
+  // early stopping: the snapshot list (one allocation `snap_`, descriptor table on the device) holds every buffer a
+  // later run reads before rewriting it; see set_heldout_stopping
+  int ho_patience_ = 0;
+  double* snap_ = nullptr;
+  CopyDesc* snap_table_ = nullptr;
+  int snap_n_ = 0;
+  long long snap_max_ = 0;        // doubles of the largest buffer of the list
+  std::vector<char> snap_tree_;   // per object: the dimension-tree contraction was current at the snapshot
+  int ho_best_iter_ = -1;         // k* of the last run with stopping on, -1 after a run with stopping off
+  double ho_best_sse_ = 0.0;
+  void free_snapshot();
+  void snapshot_state();
+  void restore_state();
   int64_t launches_ = 0;
   // timing
   std::vector<std::pair<cudaEvent_t, cudaEvent_t>> ev_pool_;

@@ -886,4 +886,37 @@ int reduce_jobs(const RedJob* jobs_dev, int njobs, double* results_dev, double* 
   return 1;
 }
 
+namespace {
+// every pair of the table in one launch: each thread walks all pairs, grid-striding over the elements of each; 16-byte
+// accesses where both ends allow them (the buffers are separate cudaMalloc allocations or 256-byte aligned offsets)
+template <int kDir>
+__global__ void __launch_bounds__(256) state_copy_kernel(const CopyDesc* __restrict__ table, int n_desc) {
+  const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  const long long nt = (long long)gridDim.x * blockDim.x;
+  for (int q = 0; q < n_desc; ++q) {
+    const CopyDesc c = table[q];
+    const double* __restrict__ src = kDir == 0 ? c.state : c.snap;
+    double* __restrict__ dst = kDir == 0 ? c.snap : c.state;
+    long long done = 0;
+    if ((((uintptr_t)src | (uintptr_t)dst) & 15) == 0) {
+      const long long n2 = c.n >> 1;
+      const double2* s2 = reinterpret_cast<const double2*>(src);
+      double2* d2 = reinterpret_cast<double2*>(dst);
+      for (long long e = tid; e < n2; e += nt) d2[e] = s2[e];
+      done = n2 << 1;
+    }
+    for (long long e = done + tid; e < c.n; e += nt) dst[e] = src[e];
+  }
+}
+}  // namespace
+
+int state_copy(const CopyDesc* table_dev, int n_desc, long long max_n, int direction, cudaStream_t st) {
+  if (n_desc <= 0 || max_n <= 0) return 0;
+  const unsigned ctas = (unsigned)std::min<long long>(ceil_div((max_n + 1) / 2, 256), 148 * 8);
+  if (direction == 0) state_copy_kernel<0><<<ctas, 256, 0, st>>>(table_dev, n_desc);
+  else state_copy_kernel<1><<<ctas, 256, 0, st>>>(table_dev, n_desc);
+  AO_CHECK_LAUNCH();
+  return 1;
+}
+
 }  // namespace aoadmm

@@ -193,4 +193,15 @@ size_t reduce_ws_doubles(int njobs);
 int reduce_jobs(const RedJob* jobs_dev, int njobs, double* results_dev, double* partials, unsigned* counter,
                 cudaStream_t st, const int* skip);
 
+// ---- state snapshot (early stopping on the held-out error) ------------------------------------------
+// one buffer of the snapshot list: n doubles of device state and their copy in the snapshot
+struct CopyDesc {
+  double* state;
+  double* snap;
+  long long n;
+};
+// direction 0: snap = state (snapshot), 1: state = snap (restore), for all n_desc pairs of the device-resident table in
+// ONE launch sized for the largest pair (max_n doubles).  Returns the launches.
+int state_copy(const CopyDesc* table_dev, int n_desc, long long max_n, int direction, cudaStream_t st);
+
 }  // namespace aoadmm

@@ -515,6 +515,11 @@ void solve(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
       has_ho[p] = true;
     }
   }
+  // options.b200_heldout_patience = P (needs options.b200_heldout): early stopping on the held-out error; G and the f_*
+  // values are those of the best iteration (out.heldout_best_iter)
+  const double patience = opt_scalar(opt, "b200_heldout_patience", 0.0);
+  if (patience < 0.0) fail("aoadmm:invalidArg", "options.b200_heldout_patience must be >= 0");
+  if (patience > 0.0) check(aoadmm_set_heldout_stopping(h, (int32_t)patience), h);
 
   const int n_hist = o.MaxOuterIters + 1;
   mxArray* hist[6];
@@ -568,8 +573,9 @@ void solve(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
   if (nlhs > 1) {
     const char* names[] = {"f_tensors", "f_couplings", "f_constraints", "f_PAR2_couplings", "f_rel_missing", "exit_flag",
                            "OuterIterations", "func_val_conv", "func_coupl_conv", "func_constr_conv", "func_PAR2_coupl",
-                           "time_at_it", "innerIters", "func_rel_missing", "non_finite_mode", "heldout_sse"};
-    mxArray* out = mxCreateStructMatrix(1, 1, 16, names);
+                           "time_at_it", "innerIters", "func_rel_missing", "non_finite_mode", "heldout_sse",
+                           "heldout_best_iter"};
+    mxArray* out = mxCreateStructMatrix(1, 1, 17, names);
     mxSetField(out, 0, "non_finite_mode", mxCreateDoubleScalar((double)ro.non_finite_mode));
     mxSetField(out, 0, "f_tensors", mxCreateDoubleScalar(ro.f_tensors));
     mxSetField(out, 0, "f_couplings", mxCreateDoubleScalar(ro.f_couplings));
@@ -578,6 +584,8 @@ void solve(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
     mxSetField(out, 0, "f_rel_missing", mxCreateDoubleScalar(ro.f_rel_missing));
     if (ro.exit_flag == 0) {  // make_exit_flag.m:4-5
       mxSetField(out, 0, "exit_flag", mxCreateString("maxIterations"));
+    } else if (ro.exit_flag == (1 << 9)) {   // the held-out rule of aoadmm_set_heldout_stopping ended the run
+      mxSetField(out, 0, "exit_flag", mxCreateString("heldoutStop"));
     } else {                   // make_exit_flag.m:9-28
       const char* fn[] = {"f_tensors", "f_couplings", "f_constraints", "f_PAR2_couplings"};
       mxArray* ef = mxCreateStructMatrix(1, 1, 4, fn);
@@ -604,6 +612,12 @@ void solve(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
       else for (int i = 0; i <= it; ++i) col[i] = mxGetNaN();
     }
     mxSetField(out, 0, "heldout_sse", hs);
+    if (patience > 0.0) {
+      int32_t best = 0;
+      double best_sse = 0.0;
+      check(aoadmm_heldout_best(h, &best, &best_sse), h);
+      mxSetField(out, 0, "heldout_best_iter", mxCreateDoubleScalar((double)best));
+    }
     plhs[1] = out;
   } else {
     for (auto& a : hist) mxDestroyArray(a);

@@ -17,7 +17,9 @@ function [G,out] = cmtf_fun_AOADMM(Z,Znorm_const,G,fh,gh,lscalar,uscalar,options
 % true (with b200_gpus > 1: sparse objects too are cut, into nonzero-balanced slabs of their last mode), b200_dimtree,
 % b200_mttkrp_precision, b200_fuse_inner, b200_graph, b200_heldout{p} = an sptensor / sparse matrix of entries of object p
 % withheld from training (with their true values; object p needs Z.miss): out.heldout_sse{p} is then the held-out SSE
-% after outer iterations 0..OuterIterations.
+% after outer iterations 0..OuterIterations.  b200_heldout_patience = P (needs b200_heldout): early stopping on the summed
+% held-out SSE; G and the f_* values are those of the best iteration out.heldout_best_iter, and out.exit_flag is
+% 'heldoutStop' when the held-out rule ended the run (include/aoadmm.h states the rule).
     % hand the gateway plain numeric arrays: X.data of a Tensor Toolbox tensor shares its memory with X (copy-on-write),
     % whereas mxGetProperty inside a MEX file would deep-copy the whole tensor
     for p = 1:numel(Z.object)
@@ -39,6 +41,9 @@ function [G,out] = cmtf_fun_AOADMM(Z,Znorm_const,G,fh,gh,lscalar,uscalar,options
         end
     else
         out = rmfield(out, 'heldout_sse');
+    end
+    if ~isfield(options,'b200_heldout_patience') || options.b200_heldout_patience == 0
+        out = rmfield(out, 'heldout_best_iter');
     end
     if out.non_finite_mode > 0
         warning('aoadmm:nonFinite', 'a residual of the inner ADMM loop of mode %d was NaN/Inf (a factor or dual of norm 0)', out.non_finite_mode);

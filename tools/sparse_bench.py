@@ -22,6 +22,11 @@
                 the same held-out measurements as m1 with 1e7 unobserved power-law entries held out.
                 CPU baseline as in s2: NumPy imputed pass (model at the entries + residual MTTKRP per mode) on a 1 %
                 sample, extrapolated in proportion to nnz.
+  m1, m2        also an early-stopping leg (set_heldout_stopping, patience 3, at most --stop-iters iterations): the
+                snapshot kernel time and bytes, the restore time with the re-imputation, outer it/s with stopping on
+                and off (alternating), k*, n and the held-out RMSE at k* and after n.
+  c1_em         the same leg on a launch-bound dense EM problem: the C1 structure (example_script6 sizes) fitted at
+                three times its rank with 70 % of the first tensor missing.
 
 Every line carries the card name and power limit (nvidia-smi, read in the same call), the create time (upload + sorts),
 the per-mode sparse MTTKRP time (CUDA events, aoadmm_time_mttkrp), outer iterations/s, and the algorithmic bytes per mode
@@ -29,8 +34,8 @@ computed from the shapes: stream = nnz (8 + 4 (N-1)) + row pointers + output, ga
 the stream rate against the 6557 GB/s measured copy peak.  nnz is the number of nonzeros handed to the engine (before
 duplicates are merged).
 
-usage: python tools/sparse_bench.py [--workloads s1,s2,m1,m2] [--densities 0.001,0.01,0.1] [--s2-scale 1.0]
-                                    [--m-scale 1.0] [--iters 5]
+usage: python tools/sparse_bench.py [--workloads s1,s2,m1,m2,c1_em] [--densities 0.001,0.01,0.1] [--s2-scale 1.0]
+                                    [--m-scale 1.0] [--iters 5] [--stop-iters 30]
 """
 import argparse
 import json
@@ -331,7 +336,87 @@ def heldout_legs(sp, G, iters, H, order):
             'heldout_pass_ms_per_iter': ph['heldout_pass'], 'impute_pass_ms_per_iter': ph['impute_pass']}
 
 
-def m1(scale, iters, seed=0, R=32):
+def state_bytes(G):
+    """Bytes of the snapshot list of early stopping: every array of G (factors, constraint and coupling duals, coupling
+    factors, PARAFAC2 P / DeltaB / mu_DeltaB)."""
+    tot = 0
+    for v in G.values():
+        for a in v:
+            for x in (a if isinstance(a, list) else [a]):
+                tot += 0 if x is None else np.asarray(x).nbytes
+    return tot
+
+
+def stopping_leg(sp, G, H, iters, patience=3, rounds=2):
+    """Early stopping on the held-out error (set_heldout_stopping) with the held-out set H on object 1:
+      - one profiled run (graph off) with the given patience and at most `iters` iterations: the kernel time of each
+        snapshot (state_copy_kernel<0>) and the bytes it moves (read + write of the snapshot list), and the restore
+        time (state_copy_kernel<1> and the re-imputation: from its start to the end of the run's last kernel);
+      - outer it/s of the same run with stopping off and on (patience > iters, so both run `iters` iterations and the
+        second snapshots after every improving iteration), alternating rounds;
+      - k*, n and the held-out RMSE at k* against the RMSE after n.
+    Leaves the set detached and stopping off."""
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+    sp.set_heldout(1, H)
+    sp.set_heldout_stopping(patience)
+    sp.set_state(G)
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        out = sp.run(options(iters, graph=-1))
+        torch.cuda.synchronize()
+    k_best, _ = sp.heldout_best()
+    n = out['OuterIterations']
+    sse, count = sp.heldout_history(1)
+    ev = sorted((e for e in prof.events() if e.device_type == torch.autograd.DeviceType.CUDA),
+                key=lambda e: e.time_range.start)
+    snaps = [e.time_range.elapsed_us() / 1e3 for e in ev if 'state_copy_kernel<0>' in e.name]
+    rst = [e for e in ev if 'state_copy_kernel<1>' in e.name]
+    restore_ms = None
+    if rst:
+        t0 = rst[0].time_range.start
+        restore_ms = (max(e.time_range.end for e in ev if e.time_range.start >= t0) - t0) / 1e3
+    ips = {'stopping_off': [], 'stopping_on': []}
+    for _ in range(rounds):
+        sp.set_heldout_stopping(0)
+        ips['stopping_off'].append(iters_per_s(sp, G, iters))
+        sp.set_heldout_stopping(iters + 1)
+        ips['stopping_on'].append(iters_per_s(sp, G, iters))
+    sp.set_heldout_stopping(0)
+    sp.set_heldout(1, None)
+    med = {k: float(np.median(v)) for k, v in ips.items()}
+    nbytes = 2 * state_bytes(G)
+    snap_ms = float(np.median(snaps)) if snaps else None
+    return {'patience': patience, 'max_iters': iters, 'best_iter': k_best, 'iters_run': n,
+            'exit_flag': out['exit_flag'] if isinstance(out['exit_flag'], str) else 'tolerance',
+            'held_out_rmse_at_best': float(np.sqrt(sse[k_best] / count)),
+            'held_out_rmse_at_end': float(np.sqrt(sse[n] / count)),
+            'snapshots': len(snaps), 'snapshot_kernel_ms': snap_ms, 'snapshot_bytes': nbytes,
+            'snapshot_GBs': nbytes / snap_ms / 1e6 if snap_ms else None,
+            'restore_ms': restore_ms if restore_ms is not None else 'not triggered (k* = n)',
+            'outer_iters_per_s': med, 'it_s_change': med['stopping_on'] / med['stopping_off'] - 1.0,
+            'outer_iters_per_s_rounds': ips}
+
+
+def c1_em(iters, seed=0):
+    """Early stopping on a launch-bound problem: the C1 structure (example_script6 sizes, three coupled nonneg objects,
+    R = 3 fitted at R = 9) with 70 % of the first tensor missing and half of the missing entries held out."""
+    from oracle import problem_gen as pg
+    Z, _, _ = pg.config_script6(seed=seed)
+    rng = np.random.RandomState(seed + 1)
+    io = {'lambdas_init': [[1.0] * 9] * 3, 'nvecs': 0, 'normalize': 1, 'distr': [pg.d_rand] * len(Z['size'])}
+    G = pg.init_coupled_AOADMM_CMTF(Z, io, rng)
+    Zm = pg.add_missing(Z, 0.7, seed=seed, objects=[0])
+    X, W = Z['object'][0], Zm['miss'][0]
+    hs = np.argwhere(~W)
+    hs = hs[np.random.RandomState(seed).rand(len(hs)) < 0.5]
+    H = ab.sptensor(hs, X[tuple(hs.T)], X.shape)
+    with ab.Solver(ab._with_rank(Zm, G), pg.znorm_const(Zm)) as s:
+        leg = stopping_leg(s, G, H, iters)
+    return {'workload': 'c1_em', 'sizes': [int(x) for x in Z['size']], 'R': 9, 'missing': 0.7,
+            'held_out': int(len(hs)), 'early_stopping': leg}
+
+
+def m1(scale, iters, stop_iters, seed=0, R=32):
     rng = np.random.RandomState(seed)
     I, J, L = 131072, 32768, 1024
     n_obs = int(2.5e7 * scale)
@@ -393,6 +478,7 @@ def m1(scale, iters, seed=0, R=32):
             ips['dense_em'].append(iters_per_s(de, G, iters))
     line['outer_iters_per_s'] = {k: float(np.median(v)) for k, v in ips.items() if v}
     line.update(heldout_legs(sp, G, iters, H, 2))
+    line['early_stopping'] = stopping_leg(sp, G, H, stop_iters)
     line['phase_ms_per_iter'] = {'sparse_mask': phase_split(sp, G, iters, 2)}
     line['held_out_rms_value'] = float(np.sqrt(np.mean(vals[n_obs:] ** 2)))
     line['f_rel_missing_last'] = float(o_sp['f_rel_missing'])
@@ -416,7 +502,7 @@ def m2_problem(rng, scale, R):
     return Z, Zm, shape, nnz, subs, vals
 
 
-def m2(scale, iters, seed=0, R=32):
+def m2(scale, iters, stop_iters, seed=0, R=32):
     rng = np.random.RandomState(seed)
     Z, Zm, shape, nnz, subs, vals = m2_problem(rng, scale, R)
     G = init_state(Zm, R, seed + 1)
@@ -451,6 +537,7 @@ def m2(scale, iters, seed=0, R=32):
     med = {k: float(np.median(v)) for k, v in ips.items()}
     phases = {'sparse_mask': phase_split(sp, G, iters, 3), 'no_mask': phase_split(un, G, iters, 3)}
     held.update(heldout_legs(sp, G, iters, H, 3))
+    held['early_stopping'] = stopping_leg(sp, G, H, stop_iters)
     sp.close()
     un.close()
     # CPU baseline: the imputed pass in NumPy on a 1 % sample, extrapolated in proportion to nnz
@@ -559,6 +646,8 @@ def main():
     ap.add_argument('--s2-scale', type=float, default=1.0, help='fraction of the s2 nonzero counts (1.0 = 2e8 / 2e7)')
     ap.add_argument('--m-scale', type=float, default=1.0, help='fraction of the m1 / m2 observed-entry counts')
     ap.add_argument('--iters', type=int, default=5)
+    ap.add_argument('--stop-iters', type=int, default=30,
+                    help='the most outer iterations of the early-stopping legs (m1, m2, c1_em)')
     ap.add_argument('--reps', type=int, default=5)
     ap.add_argument('--gpus', default=None,
                     help='comma-separated GPU counts, e.g. 1,2,8: run s2 / m2 (from --workloads) with shard_sparse=True '
@@ -581,9 +670,11 @@ def main():
     if 's2' in wl:
         print(json.dumps(dict(s2(a.s2_scale, a.iters, a.reps), card=c)), flush=True)
     if 'm1' in wl:
-        print(json.dumps(dict(m1(a.m_scale, a.iters), card=c)), flush=True)
+        print(json.dumps(dict(m1(a.m_scale, a.iters, a.stop_iters), card=c)), flush=True)
     if 'm2' in wl:
-        print(json.dumps(dict(m2(a.m_scale, a.iters), card=c)), flush=True)
+        print(json.dumps(dict(m2(a.m_scale, a.iters, a.stop_iters), card=c)), flush=True)
+    if 'c1_em' in wl:
+        print(json.dumps(dict(c1_em(a.stop_iters), card=c)), flush=True)
 
 
 if __name__ == '__main__':
