@@ -35,7 +35,8 @@ extern "C" {
  *    (sparse CP objects), aoadmm_create_sparse_masked (sparse Z.miss masks on sparse objects), aoadmm_model_at /
  *    aoadmm_set_heldout / aoadmm_heldout_history (held-out entries), aoadmm_sparse_shard_bounds /
  *    aoadmm_create_sparse_multi (sparse objects on several GPUs from one caller), aoadmm_set_heldout_stopping /
- *    aoadmm_heldout_best and bit 9 of aoadmm_out.exit_flag (early stopping on the held-out error). */
+ *    aoadmm_heldout_best and bit 9 of aoadmm_out.exit_flag (early stopping on the held-out error), aoadmm_nvecs_sparse
+ *    (nvecs of a sparse mode). */
 #define AOADMM_ABI_VERSION 4
 
 typedef struct aoadmm_handle aoadmm_handle;
@@ -392,6 +393,17 @@ int aoadmm_get_object_data(aoadmm_handle *h, int32_t object, double *out, int64_
  * (collective): partial Gram matrices of the slabs are all-reduced; for the sharded (last) mode the slabs are exchanged
  * chunk by chunk with NCCL point-to-point transfers. */
 int aoadmm_nvecs(aoadmm_handle *h, int32_t mode, int32_t slice, int32_t r, double *out, int64_t rows, double *info);
+/* aoadmm_nvecs for a mode whose first object is a sparse CP object (aoadmm_nvecs refuses those): the r leading
+ * eigenvectors of Y = X_(mode) X_(mode)' with the unstored entries counted as zero (a masked object: its stored, observed
+ * values; the imputation state never enters).  Y is never formed: Y V = U (U' V) on the unfolding U with its columns
+ * compressed to the fibers that occur, two deterministic passes over the nonzeros per iteration; results do not depend
+ * on the order of the nonzeros or on the memory free at the call.  Same column order, sign rule and info as aoadmm_nvecs.
+ * The call allocates its own temporaries and frees them; the handle's state is unchanged.
+ * AOADMM_ERR_INVALID_ARG for a mode whose first object is dense or PARAFAC2 (use aoadmm_nvecs), r outside 1..rows,
+ * rows not the mode size; AOADMM_ERR_UNSUPPORTED for the last mode of a sparse object on several GPUs (its fibers cross
+ * GPUs); AOADMM_ERR_OOM when not even one column of the operator fits in half of the free device memory.  With more
+ * than one GPU every rank must make the call (collective). */
+int aoadmm_nvecs_sparse(aoadmm_handle *h, int32_t mode, int32_t r, double *out, int64_t rows, double *info);
 /* MTTKRP of the resident CP object `object` in mode position `pos` (1-based) with the factors currently in the handle
  * (cmtf_fun_AOADMM.m:97), at `precision` (0 FP64, 1/2/3 reduced precision: see aoadmm_options.mttkrp_precision), summed over
  * ranks; out: rows(mode) x R host buffer. */

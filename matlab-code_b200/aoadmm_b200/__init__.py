@@ -22,7 +22,7 @@ import numpy as np
 from . import _capi
 from ._capi import AoadmmError, lib
 
-__all__ = ['cmtf_fun_AOADMM', 'cmtf_AOADMM', 'cmtf_nvecs', 'init_coupled_AOADMM_CMTF', 'Solver', 'AoadmmError', 'sptensor', 'mttkrp',
+__all__ = ['cmtf_fun_AOADMM', 'cmtf_AOADMM', 'cmtf_nvecs', 'cmtf_nvecs_sparse', 'init_coupled_AOADMM_CMTF', 'Solver', 'AoadmmError', 'sptensor', 'mttkrp',
            'prox', 'chol_solve', 'gram',
            'shard_range', 'sparse_shard_bounds', 'device_count', 'nccl_unique_id']
 
@@ -702,6 +702,16 @@ class Solver:
         _capi.check(lib.aoadmm_nvecs(self._h, int(mode), int(slice), int(r), _dp(out), rows, _dp(info)), self._h)
         return (out, {'iterations': int(info[0]), 'residual': float(info[1])}) if return_info else out
 
+    def nvecs_sparse(self, mode, r, return_info=False):
+        """nvecs of a mode whose first object is a sparse CP object (aoadmm_nvecs_sparse): the r leading eigenvectors of
+        X_(n) X_(n)' with the unstored entries counted as zero, without forming X_(n) X_(n)'.  Same column order, signs
+        and info as `nvecs`.  A mode of a dense or PARAFAC2 object is refused (use `nvecs`)."""
+        rows = _check_nvecs_sparse(self.Z, mode, r)
+        out = np.zeros((rows, int(r)), order='F')
+        info = np.zeros(2)
+        _capi.check(lib.aoadmm_nvecs_sparse(self._h, int(mode), int(r), _dp(out), rows, _dp(info)), self._h)
+        return (out, {'iterations': int(info[0]), 'residual': float(info[1])}) if return_info else out
+
     def object_mttkrp(self, obj, pos, precision=0):
         """MTTKRP of resident CP object `obj` (1-based) in mode position `pos` with the current factors."""
         m = self.Z['modes'][obj - 1][pos - 1]
@@ -890,6 +900,27 @@ def _refuse_sparse_nvecs(Z, mode_ids):
             raise AoadmmError(2, 'nvecs: mode %d belongs to sparse object %d (initialise it from a distribution)' % (n, p + 1))
 
 
+def _first_object(Z, n):
+    return [q for q in range(len(Z['modes'])) if n in list(Z['modes'][q])][0]
+
+
+def _is_sparse_mode(Z, n):
+    p = _first_object(Z, n)
+    return Z['model'][p] == 'CP' and as_sparse(Z['object'][p]) is not None
+
+
+def _check_nvecs_sparse(Z, n, r):
+    """host-side checks of nvecs_sparse (before any device call); returns the rows of mode n"""
+    if not 1 <= n <= len(Z['size']):
+        raise AoadmmError(1, 'nvecs_sparse: mode out of range')
+    if not _is_sparse_mode(Z, n):
+        raise AoadmmError(1, 'nvecs_sparse: mode %d belongs to a dense or PARAFAC2 object (use nvecs)' % n)
+    rows = int(Z['size'][n - 1])
+    if not 1 <= int(r) <= rows:
+        raise AoadmmError(1, 'nvecs_sparse: the number of vectors must be between 1 and the mode size')
+    return rows
+
+
 def cmtf_nvecs(Z, n, r, solver=None, **dist):
     """U = cmtf_nvecs(Z,n,r)  (cmtf_nvecs.m:33-58): r leading eigenvectors of X_(n) X_(n)', computed on the device from
     the tensor resident in `solver` (or in a temporary handle), so a large tensor never has to be unfolded on the host."""
@@ -901,17 +932,32 @@ def cmtf_nvecs(Z, n, r, solver=None, **dist):
         return s.nvecs(n, r)
 
 
+def cmtf_nvecs_sparse(Z, n, r, solver=None, **dist):
+    """U = cmtf_nvecs(Z,n,r) for a mode whose first object is a sparse CP object (cmtf_nvecs refuses those): the r leading
+    eigenvectors of X_(n) X_(n)' with the unstored entries counted as zero, on the device, without forming the n x n
+    matrix.  A mode of a dense or PARAFAC2 object is refused before any device call (use cmtf_nvecs)."""
+    _check_nvecs_sparse(Z, n, r)
+    if solver is not None:
+        return solver.nvecs_sparse(n, r)
+    P = len(Z['object'])
+    with Solver(dict(Z, rank=[int(r)] * P), [float('nan')] * P, **dist) as s:
+        return s.nvecs_sparse(n, r)
+
+
 def init_coupled_AOADMM_CMTF(Z, init_options, rng=None, Delta=None, **dist):
     """G = init_coupled_AOADMM_CMTF(Z,'init_options',init_options)  (init_coupled_AOADMM_CMTF.m:37-169).
 
     init_options: 'lambdas_init' (per object, its length is the rank), 'distr' (per mode, callable (rows, cols) ->
-    array, the @(x,y) rand(x,y) handles of the example scripts), 'normalize', 'nvecs'.  With nvecs the factors are the
-    leading eigenvectors of X_(n) X_(n)' (:50-69), computed on the device; constraint factors go through the device
+    array, the @(x,y) rand(x,y) handles of the example scripts), 'normalize', 'nvecs', 'nvecs_sparse'.  With nvecs the
+    factors are the leading eigenvectors of X_(n) X_(n)' (:50-69), computed on the device; a mode of a sparse object is
+    refused unless 'nvecs_sparse' is 1 as well, which computes it with nvecs_sparse (it has no effect without 'nvecs');
+    constraint factors go through the device
     prox (:99-124); duals and coupling factors are uniform random (:126-169) from `rng` (numpy RandomState)."""
     rng = rng if rng is not None else np.random.RandomState()
     sz, modes, model = Z['size'], Z['modes'], Z['model']
     lambdas, distr = init_options['lambdas_init'], init_options['distr']
     normalize, use_nvecs = bool(init_options.get('normalize', 0)), bool(init_options.get('nvecs', 0))
+    use_nvecs_sparse = use_nvecs and bool(init_options.get('nvecs_sparse', 0))
     lin = list(Z['coupling']['lin_coupled_modes'])
     ctype = list(Z['coupling'].get('coupling_type', []))
     trafo = Z['coupling'].get('coupl_trafo_matrices') or [None] * len(sz)
@@ -931,7 +977,7 @@ def init_coupled_AOADMM_CMTF(Z, init_options, rng=None, Delta=None, **dist):
         return int(sz[n - 1])
 
     solver = None
-    if use_nvecs:
+    if use_nvecs and not use_nvecs_sparse:
         _refuse_sparse_nvecs(Z, [n for p in range(P) for n in modes[p]])
     try:
         if use_nvecs:
@@ -960,6 +1006,8 @@ def init_coupled_AOADMM_CMTF(Z, init_options, rng=None, Delta=None, **dist):
                 elif use_nvecs:
                     if model[p] == 'PAR2' and pos == 2:
                         G['fac'][n - 1] = np.ones((rows_of(n), R))                       # :68
+                    elif use_nvecs_sparse and _is_sparse_mode(Z, n):
+                        G['fac'][n - 1] = solver.nvecs_sparse(n, R)
                     else:
                         G['fac'][n - 1] = solver.nvecs(n, R)                             # :52, :55-60
                 else:

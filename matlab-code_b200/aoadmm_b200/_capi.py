@@ -98,7 +98,7 @@ EXPORTS = ['aoadmm_abi_version', 'aoadmm_device_count', 'aoadmm_nccl_unique_id',
            'aoadmm_create_multi', 'aoadmm_gpu_count', 'aoadmm_comm_release', 'aoadmm_create_sparse',
            'aoadmm_create_sparse_masked', 'aoadmm_model_at', 'aoadmm_set_heldout', 'aoadmm_heldout_history',
            'aoadmm_sparse_shard_bounds', 'aoadmm_create_sparse_multi', 'aoadmm_set_heldout_stopping',
-           'aoadmm_heldout_best']
+           'aoadmm_heldout_best', 'aoadmm_nvecs_sparse']
 
 lib.aoadmm_abi_version.restype = C.c_int
 lib.aoadmm_device_count.argtypes = [C.POINTER(C.c_int)]
@@ -129,6 +129,7 @@ lib.aoadmm_generate_cp_data.argtypes = [HandleP, C.c_int32, C.POINTER(c_double_p
 lib.aoadmm_time_mttkrp.argtypes = [HandleP, C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_float)]
 lib.aoadmm_object_mttkrp.argtypes = [HandleP, C.c_int32, C.c_int32, C.c_int32, c_double_p]
 lib.aoadmm_nvecs.argtypes = [HandleP, C.c_int32, C.c_int32, C.c_int32, c_double_p, C.c_int64, c_double_p]
+lib.aoadmm_nvecs_sparse.argtypes = [HandleP, C.c_int32, C.c_int32, c_double_p, C.c_int64, c_double_p]
 lib.aoadmm_launch_count.argtypes = [HandleP, C.POINTER(C.c_int64)]
 lib.aoadmm_phase_ms.argtypes = [HandleP, c_double_p]
 lib.aoadmm_last_run_ms.argtypes = [HandleP, c_double_p]

@@ -536,6 +536,16 @@ int aoadmm_nvecs(aoadmm_handle* h, int32_t mode, int32_t slice, int32_t r, doubl
   });
 }
 
+int aoadmm_nvecs_sparse(aoadmm_handle* h, int32_t mode, int32_t r, double* out, int64_t rows, double* info) {
+  if (!h || !out || r < 1 || rows < 1) return AOADMM_ERR_INVALID_ARG;
+  return guard(h, [&] {
+    const int n = (int)h->eng.size();
+    std::vector<std::vector<double>> tmp(n);
+    for (int q = 1; q < n; ++q) tmp[q].resize((size_t)rows * r);
+    for_each_rank(n, [&](int q) { h->eng[q]->nvecs_sparse_to_host(mode, r, q == 0 ? out : tmp[q].data(), rows, q == 0 ? info : nullptr); });
+  });
+}
+
 int aoadmm_object_mttkrp(aoadmm_handle* h, int32_t object, int32_t pos, int32_t precision, double* out) {
   if (!h || !out || precision < 0 || precision > 3) return AOADMM_ERR_INVALID_ARG;
   return guard(h, [&] {

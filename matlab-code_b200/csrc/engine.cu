@@ -19,6 +19,7 @@
 #include <cmath>
 #include <cstring>
 #include <map>
+#include <memory>
 #include <mutex>
 #include <set>
 #include <thread>
@@ -2757,6 +2758,84 @@ void Engine::nvecs_sharded_mode(ObjectState& o, int r, double* out, int64_t rows
   cudaFree(send);
   cudaFree(Y);
   cudaFree(work);
+  cudaFree(U);
+}
+
+void Engine::nvecs_sparse_to_host(int mode_id, int r, double* out, int64_t rows, double* info) {
+  AO_CUDA(cudaSetDevice(device_));
+  if (mode_id < 1 || mode_id > nb_modes_) throw CudaError(1, "nvecs_sparse: mode out of range");
+  int p = -1, pos = -1;   // the first object that contains the mode, as for nvecs
+  for (int q = 0; q < n_objects_ && p < 0; ++q)
+    for (int d = 0; d < objects_[q].order; ++d)
+      if (objects_[q].modes[d] == mode_id) {
+        p = q;
+        pos = d;
+        break;
+      }
+  if (p < 0) throw CudaError(1, "nvecs_sparse: no object contains this mode");
+  ObjectState& o = objects_[p];
+  if (o.sp == nullptr)
+    throw CudaError(1, "nvecs_sparse: mode " + std::to_string(mode_id) +
+                           " belongs to a dense or PARAFAC2 object (use aoadmm_nvecs)");
+  const SparseTensor& sp = *o.sp;
+  if (o.sharded && pos == o.order - 1)
+    throw CudaError(2, "nvecs_sparse: mode " + std::to_string(mode_id) +
+                           " is the sharded last mode of a sparse object (its fibers cross GPUs)");
+  const long long n = sp.dims[pos];
+  if (rows != n) throw CudaError(1, "nvecs_sparse: output rows do not match the mode size");
+  if (r < 1 || r > n) throw CudaError(1, "nvecs_sparse: the number of vectors must be between 1 and the mode size");
+  // build and chunk buffers (the chunk width c may differ between ranks: the bits of W do not depend on it).  A failure
+  // on one rank must not leave the others in a collective, so every rank learns whether all succeeded (c > 0 on every
+  // rank) before the iteration.
+  std::unique_ptr<FiberUnfolding> fu;
+  std::exception_ptr err;
+  int c = 0;
+  try {
+    fu.reset(new FiberUnfolding(sp, pos, st_));
+    size_t free_b = 0, total_b = 0;
+    AO_CUDA(cudaMemGetInfo(&free_b, &total_b));
+    c = fu->chunk_columns(eig_block(n, r), free_b / 2);
+    if (c > 0) fu->reserve(c);
+  } catch (...) {
+    err = std::current_exception();
+    c = 0;
+  }
+  if (world_ > 1) {
+    std::vector<double> tab((size_t)world_, 0.0);
+    tab[rank_] = (double)c;
+    double* tab_dev = nullptr;
+    AO_CUDA(cudaMalloc(&tab_dev, tab.size() * sizeof(double)));
+    AO_CUDA(cudaMemcpyAsync(tab_dev, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice, st_));
+    allreduce(tab_dev, tab.size());
+    AO_CUDA(cudaMemcpyAsync(tab.data(), tab_dev, tab.size() * sizeof(double), cudaMemcpyDeviceToHost, st_));
+    AO_CUDA(cudaStreamSynchronize(st_));
+    cudaFree(tab_dev);
+    for (double v : tab) c = std::min(c, (int)v);
+  }
+  if (err) std::rethrow_exception(err);
+  if (c == 0) throw CudaError(7, "nvecs_sparse: not even one column of the sparse operator fits in half of the free device memory");
+  double* U = nullptr;
+  try {
+    AO_CUDA(cudaMalloc(&U, std::max<size_t>((size_t)n * r * sizeof(double), 256)));
+    // W = Y V; with several GPUs each rank's fibers give its share, summed by one all-reduce per application
+    const EigOperator apply = [&](const double* V, double* W, int cols) {
+      const int L = fu->apply(V, W, cols, st_);
+      allreduce(W, (size_t)n * cols);
+      return L;
+    };
+    std::vector<double> theta(r);
+    const EigInfo ei = top_eigvecs(apply, n, r, U, theta.data(), st_);
+    launches_ += ei.launches;
+    if (info != nullptr) {
+      info[0] = ei.iterations;
+      info[1] = ei.residual;
+    }
+    AO_CUDA(cudaMemcpyAsync(out, U, (size_t)n * r * sizeof(double), cudaMemcpyDeviceToHost, st_));
+    AO_CUDA(cudaStreamSynchronize(st_));
+  } catch (...) {
+    cudaFree(U);
+    throw;
+  }
   cudaFree(U);
 }
 

@@ -208,6 +208,9 @@ class Engine {
   // (slice: 1-based slice of a PARAFAC2 B_k mode, else 0); out: rows x r host buffer; info: [iterations, residual]
   void nvecs_to_host(int mode_id, int slice, int r, double* out, int64_t rows, double* info);
   void nvecs_sharded_mode(ObjectState& o, int r, double* out, int64_t rows, double* info);
+  // aoadmm_nvecs_sparse: the same for a mode whose first object is a sparse CP object, with Y V applied as U (U' V) on the
+  // fiber-compressed unfolding U (sparse.cuh, FiberUnfolding); collective over the ranks
+  void nvecs_sparse_to_host(int mode_id, int r, double* out, int64_t rows, double* info);
   void mttkrp_to_host(int object, int pos, double* out, int precision = -1);  // unweighted MTTKRP of the resident factors (-1: precision of the last run)
   // held-out entries (aoadmm_model_at / aoadmm_set_heldout): host-only checks of object and subscripts, then the work
   void check_entries(int object, const aoadmm_sparse_object* entries, bool heldout) const;

@@ -546,11 +546,22 @@ int unfold_gram(const UnfoldSpec& s, double* Y, double* work, cudaStream_t st, b
   return 2;
 }
 
+int eig_block(long long n, int r) {
+  // short modes: the block is the whole space, one Rayleigh-Ritz step (a Jacobi eigen-decomposition of Y) is exact
+  return (n <= 128) ? (int)n : (int)std::min<long long>(n, (long long)r + std::max(8, r / 4));
+}
+
 EigInfo top_eigvecs(const double* Y, long long n, int r, double* U, double* theta, cudaStream_t st) {
+  const EigOperator apply = [&](const double* V, double* W, int Rb) {
+    return dgemm_small(0, 0, n, Rb, n, 1.0, nullptr, Y, n, V, n, 0.0, W, n, st, nullptr);
+  };
+  return top_eigvecs(apply, n, r, U, theta, st);
+}
+
+EigInfo top_eigvecs(const EigOperator& apply, long long n, int r, double* U, double* theta, cudaStream_t st) {
   EigInfo info;
   if (r < 1 || r > n) throw CudaError(1, "nvecs: the number of vectors must be between 1 and the mode size");
-  // short modes: the block is the whole space, one Rayleigh-Ritz step (a Jacobi eigen-decomposition of Y) is exact
-  const int Rb = (n <= 128) ? (int)n : (int)std::min<long long>(n, (long long)r + std::max(8, r / 4));
+  const int Rb = eig_block(n, r);
   const size_t nb = (size_t)n * Rb, bb = (size_t)Rb * Rb;
   double* buf = nullptr;
   int* order_dev = nullptr;
@@ -589,7 +600,7 @@ EigInfo top_eigvecs(const double* Y, long long n, int r, double* U, double* thet
     const int maxit = 3000;
     for (int it = 1; it <= maxit; ++it) {
       info.iterations = it;
-      L += dgemm_small(0, 0, n, Rb, n, 1.0, nullptr, Y, n, V, n, 0.0, W, n, st, nullptr);        // W = Y V
+      L += apply(V, W, Rb);                                                                       // W = Y V
       L += dgemm_small_splitk(1, 0, Rb, Rb, n, 1.0, V, n, W, n, 0.0, H, Rb, ws, st, nullptr);    // H = V' Y V
       symmetrize_kernel<<<blocks_for((long long)bb), 256, 0, st>>>(H, Rb);
       L += 1 + jacobi_onesided(H, Rb, Rb, Q, sig, st);                                           // H = Q diag(sig) Q'

@@ -11,6 +11,8 @@
 //   2. top_eigvecs: block subspace iteration with Rayleigh-Ritz on Y (oversampled block, one-sided Jacobi for the
 //      small eigenproblems), until the residuals ||Y u - theta u|| of the r leading pairs are at rounding level.
 #pragma once
+#include <functional>
+
 #include "linalg.cuh"
 
 namespace aoadmm {
@@ -41,5 +43,13 @@ struct EigInfo {
 // largest eigenvalues, in descending order (eigs(Y,r,'LM')); theta (host, r entries).  Every column is signed so that its
 // entry of largest magnitude is positive.  Synchronises the stream.
 EigInfo top_eigvecs(const double* Y, long long n, int r, double* U, double* theta, cudaStream_t st);
+
+// Operator form: apply(V, W, cols) sets W = Y V for V, W n x cols (column-major, ld = n, device, on `st`) and returns its
+// launches.  Everything else (block size, start vectors, stopping rule, sign rule) is the dense iteration's; the dense
+// overload is this one with the dgemm W = Y V, so its results are unchanged bit for bit.
+using EigOperator = std::function<int(const double* V, double* W, int cols)>;
+EigInfo top_eigvecs(const EigOperator& apply, long long n, int r, double* U, double* theta, cudaStream_t st);
+// columns of the iteration block for r vectors of an n-row mode (the operator is applied to n x eig_block(n, r))
+int eig_block(long long n, int r);
 
 }  // namespace aoadmm

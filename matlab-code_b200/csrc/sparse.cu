@@ -167,7 +167,7 @@ struct SpArgs {
 // PERM (imputed MTTKRP of a masked object, positions >= 2): the value of nonzero e is vals[perm[e]]; the unmasked
 // instantiation (PERM = false) is the original kernel.
 template <int G, int CPL, bool PERM>
-__global__ void __launch_bounds__(256) sp_mttkrp_kernel(const SpArgs a) {
+__device__ __forceinline__ void sp_unit_rows(const SpArgs& a) {
   const long long unit = ((long long)blockIdx.x * blockDim.x + threadIdx.x) / G;
   const int gl = threadIdx.x % G;
   if (unit >= a.units) return;
@@ -209,10 +209,15 @@ __global__ void __launch_bounds__(256) sp_mttkrp_kernel(const SpArgs a) {
   }
 }
 
+template <int G, int CPL, bool PERM>
+__global__ void __launch_bounds__(256) sp_mttkrp_kernel(const SpArgs a) {
+  sp_unit_rows<G, CPL, PERM>(a);
+}
+
 // rows split over units: tail carry of the unit where the row starts + head carries of the following units, in a fixed
 // order (four interleaved partial sums, combined pairwise)
 template <int G, int CPL>
-__global__ void __launch_bounds__(256) sp_fixup_kernel(const SpArgs a) {
+__device__ __forceinline__ void sp_fixup_rows(const SpArgs& a) {
   const long long unit = ((long long)blockIdx.x * blockDim.x + threadIdx.x) / G;
   const int gl = threadIdx.x % G;
   if (unit >= a.units) return;
@@ -235,6 +240,11 @@ __global__ void __launch_bounds__(256) sp_fixup_kernel(const SpArgs a) {
     for (; c <= c1; ++c) s0 += a.head[c * R + col];
     a.outT[(long long)r * R + col] = (s0 + s1) + (s2 + s3);
   }
+}
+
+template <int G, int CPL>
+__global__ void __launch_bounds__(256) sp_fixup_kernel(const SpArgs a) {
+  sp_fixup_rows<G, CPL>(a);
 }
 
 template <int G, int CPL, bool PERM>
@@ -859,6 +869,214 @@ int sparse_em_finish(SparseTensor& s, const double* const* fac, const long long*
     cg_from_g3_kernel<<<grid_for((long long)s.order * R * R), 256, 0, st>>>(s.g3, s.order, R, s.cg);
     AO_CHECK_LAUNCH();
     ++launches;
+  }
+  return launches;
+}
+
+
+// ---- nvecs of a sparse mode: fiber-compressed unfolding and its two passes ----
+namespace {
+
+// row of nonzero e of a mode copy: the last r with rowptr[r] <= e
+__device__ __forceinline__ int row_of(const long long* __restrict__ rowptr, long long rows, long long e) {
+  long long lo = 0, hi = rows;   // rowptr[lo] <= e < rowptr[hi]
+  while (hi - lo > 1) {
+    const long long mid = (lo + hi) >> 1;
+    if (rowptr[mid] <= e) lo = mid;
+    else hi = mid;
+  }
+  return (int)lo;
+}
+
+// flags[k] = 1 where the k-th nonzero in fiber order starts a fiber (its other-mode subscripts differ from the previous)
+__global__ void fiber_flags_kernel(const int* __restrict__ idx, int no, long long nnz, const int* __restrict__ perm,
+                                   int* __restrict__ flags) {
+  for (long long k = blockIdx.x * (long long)blockDim.x + threadIdx.x; k < nnz; k += (long long)gridDim.x * blockDim.x) {
+    int f = (k == 0);
+    if (!f) {
+      const long long a = perm[k], b = perm[k - 1];
+      for (int q = 0; q < no && !f; ++q) f = idx[q * nnz + a] != idx[q * nnz + b];
+    }
+    flags[k] = f;
+  }
+}
+
+// fiber order: key (fiber id), i_n and value of every nonzero; mode-n order: its fiber id.  pos = inclusive scan of the
+// fiber flags.
+__global__ void fiber_scatter_kernel(const int* __restrict__ pos, const int* __restrict__ perm,
+                                     const long long* __restrict__ rowptr, long long rows, const double* __restrict__ vals,
+                                     long long nnz, unsigned* __restrict__ fkey, int* __restrict__ in,
+                                     double* __restrict__ fvals, int* __restrict__ fib) {
+  for (long long k = blockIdx.x * (long long)blockDim.x + threadIdx.x; k < nnz; k += (long long)gridDim.x * blockDim.x) {
+    const int f = pos[k] - 1;
+    const long long e = perm[k];
+    fkey[k] = (unsigned)f;
+    in[k] = row_of(rowptr, rows, e);
+    fvals[k] = vals[e];
+    fib[e] = f;
+  }
+}
+
+// pass A (fiber order) and pass B (mode-n copy) of the nvecs operator: the MTTKRP unit / carry sums with one gathered
+// operand, under names of their own
+template <int G, int CPL>
+__global__ void __launch_bounds__(256) nvecs_fiber_pass_kernel(const SpArgs a) {
+  sp_unit_rows<G, CPL, false>(a);
+}
+template <int G, int CPL>
+__global__ void __launch_bounds__(256) nvecs_fiber_fixup_kernel(const SpArgs a) {
+  sp_fixup_rows<G, CPL>(a);
+}
+template <int G, int CPL>
+__global__ void __launch_bounds__(256) nvecs_row_pass_kernel(const SpArgs a) {
+  sp_unit_rows<G, CPL, false>(a);
+}
+template <int G, int CPL>
+__global__ void __launch_bounds__(256) nvecs_row_fixup_kernel(const SpArgs a) {
+  sp_fixup_rows<G, CPL>(a);
+}
+
+}  // namespace
+
+template <typename T>
+T* FiberUnfolding::alloc(size_t count) {
+  T* p = dalloc<T>(count);
+  bufs_.push_back(p);
+  return p;
+}
+
+FiberUnfolding::FiberUnfolding(const SparseTensor& s, int n, cudaStream_t st) : s_(s), n_(n) {
+  rows_ = s.dims[n];
+  nnz_ = s.nnz;
+  units_ = ceil_div(nnz_, kSparseChunk);
+  if (nnz_ == 0) return;
+  try {
+    const SparseMode& sm = s.modes[n];
+    const int no = s.order - 1;
+    in_ = alloc<int>(nnz_);
+    vals_ = alloc<double>(nnz_);
+    fib_ = alloc<int>(nnz_);
+    fchunk_ = alloc<int>(units_);
+    fhead_ = alloc<int>(units_);
+    ftail_ = alloc<int>(units_);
+    Temps tmp;
+    SortWs w;
+    w.k0 = tmp.get<unsigned>(nnz_);
+    w.k1 = tmp.get<unsigned>(nnz_);
+    w.p0 = tmp.get<int>(nnz_);
+    w.p1 = tmp.get<int>(nnz_);
+    const int nm = (int)nnz_;
+    AO_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, w.bytes, w.k0, w.k1, w.p0, w.p1, nm, 0, 32, st));
+    size_t scan_bytes = 0;
+    AO_CUDA(cub::DeviceScan::InclusiveSum(nullptr, scan_bytes, (int*)w.k0, (int*)w.k1, nm, st));
+    w.bytes = std::max(w.bytes, scan_bytes);
+    w.tmp = tmp.get<char>(w.bytes);
+    // fiber order: stable LSD passes from the last other mode to the first, starting from the mode-n order (so i_n
+    // ascends inside a fiber)
+    iota_kernel<<<grid_for(nnz_), 256, 0, st>>>(w.p0, nnz_);
+    AO_CHECK_LAUNCH();
+    for (int q = no - 1; q >= 0; --q) {
+      const int d = q < n ? q : q + 1;
+      gather_keys_kernel<<<grid_for(nnz_), 256, 0, st>>>(sm.idx + (size_t)q * nnz_, w.p0, w.k0, nnz_, 0);
+      AO_CHECK_LAUNCH();
+      size_t b = w.bytes;
+      AO_CUDA(cub::DeviceRadixSort::SortPairs(w.tmp, b, w.k0, w.k1, w.p0, w.p1, nm, 0, key_bits(s.dims[d]), st));
+      std::swap(w.p0, w.p1);
+    }
+    int* flags = (int*)w.k0;
+    int* pos = (int*)w.k1;
+    fiber_flags_kernel<<<grid_for(nnz_), 256, 0, st>>>(sm.idx, no, nnz_, w.p0, flags);
+    AO_CHECK_LAUNCH();
+    size_t b = w.bytes;
+    AO_CUDA(cub::DeviceScan::InclusiveSum(w.tmp, b, flags, pos, nm, st));
+    int last = 0;
+    AO_CUDA(cudaMemcpyAsync(&last, pos + nnz_ - 1, sizeof(int), cudaMemcpyDeviceToHost, st));
+    AO_CUDA(cudaStreamSynchronize(st));
+    nfib_ = last;
+    fptr_ = alloc<long long>(nfib_ + 1);
+    unsigned* fkey = w.k0;   // the flags are consumed by the scan
+    fiber_scatter_kernel<<<grid_for(nnz_), 256, 0, st>>>(pos, w.p0, sm.rowptr, rows_, sm.vals, nnz_, fkey, in_, vals_, fib_);
+    AO_CHECK_LAUNCH();
+    rowptr_kernel<<<grid_for(nfib_ + 1), 256, 0, st>>>(fkey, nnz_, nfib_, fptr_);
+    AO_CHECK_LAUNCH();
+    unit_rows_kernel<<<grid_for(units_), 256, 0, st>>>(fkey, fptr_, nnz_, units_, fchunk_, fhead_, ftail_);
+    AO_CHECK_LAUNCH();
+    AO_CUDA(cudaStreamSynchronize(st));   // the sort scratch is released on return
+  } catch (...) {
+    for (void* p : bufs_) cudaFree(p);
+    throw;
+  }
+}
+
+FiberUnfolding::~FiberUnfolding() {
+  for (void* p : bufs_) cudaFree(p);
+}
+
+int FiberUnfolding::chunk_columns(int cols, size_t budget) const {
+  for (int c = std::min(cols, 64); c >= 1; c /= 2) {
+    const double bytes = 8.0 * c * ((double)nfib_ + 2.0 * (double)units_ + (double)rows_);
+    if (bytes <= (double)budget) return c;
+  }
+  return 0;
+}
+
+void FiberUnfolding::reserve(int c) {
+  c_ = c;
+  T_ = alloc<double>((size_t)nfib_ * c);
+  head_ = alloc<double>((size_t)units_ * c);
+  tail_ = alloc<double>((size_t)units_ * c);
+  X_ = alloc<double>((size_t)rows_ * c);
+}
+
+int FiberUnfolding::apply(const double* V, double* W, int cols, cudaStream_t st) {
+  if (nnz_ == 0 || rows_ == 0) {
+    if (rows_ > 0) AO_CUDA(cudaMemsetAsync(W, 0, (size_t)rows_ * cols * sizeof(double), st));
+    return 0;
+  }
+  const SparseMode& sm = s_.modes[n_];
+  SpArgs fa{};   // pass A: T(f, :) = sum over the nonzeros e of fiber f of x_e V(i_n(e), :)
+  fa.rowptr = fptr_;
+  fa.chunk_row = fchunk_;
+  fa.head_row = fhead_;
+  fa.tail_row = ftail_;
+  fa.vals = vals_;
+  fa.idx = in_;
+  fa.nnz = nnz_;
+  fa.units = units_;
+  fa.no = 1;
+  fa.F[0] = X_;
+  fa.outT = T_;
+  fa.head = head_;
+  fa.tail = tail_;
+  SpArgs ra = fa;   // pass B: W(i, :) = sum over the nonzeros e of row i of x_e T(fib(e), :)
+  ra.rowptr = sm.rowptr;
+  ra.chunk_row = sm.chunk_row;
+  ra.head_row = sm.head_row;
+  ra.tail_row = sm.tail_row;
+  ra.vals = sm.vals;
+  ra.idx = fib_;
+  ra.F[0] = T_;
+  ra.outT = X_;
+  int launches = 0;
+  for (int j0 = 0; j0 < cols; j0 += c_) {
+    const int c = std::min(c_, cols - j0);
+    fa.R = ra.R = c;
+    launches += transpose_scale(V + (size_t)j0 * rows_, rows_, c, rows_, X_, c, 1.0, st);   // X = V chunk, row-major
+    rank_dispatch(c, [&](auto g, auto cpl) {
+      constexpr int G = decltype(g)::value, CPL = decltype(cpl)::value;
+      const unsigned blocks = (unsigned)ceil_div(units_ * G, 256);
+      nvecs_fiber_pass_kernel<G, CPL><<<blocks, 256, 0, st>>>(fa);
+      AO_CHECK_LAUNCH();
+      nvecs_fiber_fixup_kernel<G, CPL><<<blocks, 256, 0, st>>>(fa);
+      AO_CHECK_LAUNCH();
+      AO_CUDA(cudaMemsetAsync(X_, 0, (size_t)rows_ * c * sizeof(double), st));   // rows without nonzeros stay zero
+      nvecs_row_pass_kernel<G, CPL><<<blocks, 256, 0, st>>>(ra);
+      AO_CHECK_LAUNCH();
+      nvecs_row_fixup_kernel<G, CPL><<<blocks, 256, 0, st>>>(ra);
+      AO_CHECK_LAUNCH();
+    });
+    launches += 4;
+    launches += transpose_scale(X_, c, rows_, c, W + (size_t)j0 * rows_, rows_, 1.0, st);   // W chunk, column-major
   }
   return launches;
 }

@@ -164,4 +164,43 @@ int sparse_em_nonzeros(SparseTensor& s, const double* const* fac, const long lon
 int sparse_em_finish(SparseTensor& s, const double* const* fac, const long long* ld, bool impute, double* sums,
                      cudaStream_t st);
 
+// nvecs of a sparse mode (aoadmm_nvecs_sparse): U = X_(n) of mode position n with its columns compressed to the distinct
+// fibers (the other-mode subscripts that occur), so that Y V = X_(n) X_(n)' V = U (U' V) without forming Y.  Built per
+// call from the resident mode-n copy (stable LSD radix passes over the other modes put the nonzeros in fiber order) and
+// freed by the destructor; the object's MTTKRP scratch is never touched.  The build depends only on the multiset of
+// entries.  With several GPUs, every fiber of a position before the last lies on one GPU: apply() gives this GPU's
+// share of W, the caller sums the shares.
+class FiberUnfolding {
+ public:
+  FiberUnfolding(const SparseTensor& s, int n, cudaStream_t st);
+  ~FiberUnfolding();
+  FiberUnfolding(const FiberUnfolding&) = delete;
+  FiberUnfolding& operator=(const FiberUnfolding&) = delete;
+  long long fibers() const { return nfib_; }
+  // widest column chunk c = min(cols, 64), halved until T (fibers x c), the carries (2 units x c) and the row-major
+  // V / W chunk (rows x c) fit in `budget` bytes; 0 when one column does not fit
+  int chunk_columns(int cols, size_t budget) const;
+  // allocates the buffers of c-column chunks
+  void reserve(int c);
+  // W (rows x cols, column-major, ld = rows) = U U' V (V likewise) over this GPU's nonzeros, c columns at a time: pass A
+  // T = U' V in fiber order, pass B W = U T in the mode-n copy, both the deterministic unit / carry sums of the MTTKRP
+  // with one gathered operand.  Every column of W is one lane's fixed-order sum plus a fixed-order fix-up, so its bits
+  // do not depend on c.  Returns the launches.
+  int apply(const double* V, double* W, int cols, cudaStream_t st);
+
+ private:
+  template <typename T>
+  T* alloc(size_t count);
+  const SparseTensor& s_;
+  int n_ = 0, c_ = 0;
+  long long rows_ = 0, nnz_ = 0, nfib_ = 0, units_ = 0;
+  std::vector<void*> bufs_;
+  int* in_ = nullptr;           // fiber order: i_n of every nonzero
+  double* vals_ = nullptr;      // fiber order: value of every nonzero
+  long long* fptr_ = nullptr;   // fibers + 1: first nonzero of every fiber
+  int *fchunk_ = nullptr, *fhead_ = nullptr, *ftail_ = nullptr;   // unit metadata of the fiber order
+  int* fib_ = nullptr;          // mode-n order: fiber id of every nonzero
+  double *T_ = nullptr, *head_ = nullptr, *tail_ = nullptr, *X_ = nullptr;   // chunk buffers (reserve)
+};
+
 }  // namespace aoadmm
