@@ -36,7 +36,7 @@ extern "C" {
  *    aoadmm_set_heldout / aoadmm_heldout_history (held-out entries), aoadmm_sparse_shard_bounds /
  *    aoadmm_create_sparse_multi (sparse objects on several GPUs from one caller), aoadmm_set_heldout_stopping /
  *    aoadmm_heldout_best and bit 9 of aoadmm_out.exit_flag (early stopping on the held-out error), aoadmm_nvecs_sparse
- *    (nvecs of a sparse mode). */
+ *    (nvecs of a sparse mode), aoadmm_create_sparse_slices (PARAFAC2 objects with sparse slices). */
 #define AOADMM_ABI_VERSION 4
 
 typedef struct aoadmm_handle aoadmm_handle;
@@ -261,6 +261,24 @@ int aoadmm_create_sparse(const aoadmm_problem *problem, const aoadmm_sparse_obje
  * observed pattern differs from the stored one (the message names the object). */
 int aoadmm_create_sparse_masked(const aoadmm_problem *problem, const aoadmm_sparse_object *const *sparse,
                                 const aoadmm_sparse_object *const *masks, const aoadmm_dist *dist, aoadmm_handle **out);
+
+/* aoadmm_create_sparse with PARAFAC2 objects whose slices are sparse.  sparse: NULL or n_objects entries, set only for
+ * CP objects, with the meaning and checks of aoadmm_create_sparse (no masks).  slices: NULL or n_objects entries, set
+ * only for PARAFAC2 objects: slices[p] holds the K slices side by side as one order-2 COO object over I x Jtot
+ * (Jtot = J_1 + ... + J_K from problem->slice_rows of the B_k mode): subs[e] = row i (0..I-1), subs[nnz + e] =
+ * joff[k] + j with joff[k] = J_1 + ... + J_{k-1}; objects[p].slices must then be NULL.  Duplicates are summed, explicit
+ * zeros are kept; results do not depend on the order of the entries.  Such an object never forms an I x Jtot array:
+ * the products Xall W and Xall' A of the PARAFAC2 block are the deterministic sparse MTTKRP of the stacked object, the
+ * explicit residual is one pass over the stored entries plus ||model||^2 from the Grams, it always runs FP64, and
+ * Znorm_const = NaN is the sum of the squared merged values (about 2 * (12 + 4) bytes per stored entry on the device).
+ * Checked before any device is touched: AOADMM_ERR_INVALID_ARG for NULL pointers, nnz < 0, a row or column subscript
+ * out of range, dense and sparse slices both set, missing slice sizes, I or Jtot above 2^31 - 1, 2^31 - 257 entries
+ * or more, slices[p] on a CP object or sparse[p] on a PARAFAC2 object; AOADMM_ERR_UNSUPPORTED for world_size > 1 and
+ * objects[p].miss_slices on an object with sparse slices.  aoadmm_nvecs on the A or B_k mode of such an object returns
+ * AOADMM_ERR_UNSUPPORTED; the other entry points refuse or accept it as they do a dense PARAFAC2 object. */
+int aoadmm_create_sparse_slices(const aoadmm_problem *problem, const aoadmm_sparse_object *const *sparse,
+                                const aoadmm_sparse_object *const *slices, const aoadmm_dist *dist,
+                                aoadmm_handle **out);
 
 /* ---- sparse objects on several GPUs from one caller ---------------------------------------------
  * aoadmm_sparse_shard_bounds: bounds[0..n_gpus] of the slabs of the last mode (extent indices) into which

@@ -23,6 +23,7 @@ from . import _capi
 from ._capi import AoadmmError, lib
 
 __all__ = ['cmtf_fun_AOADMM', 'cmtf_AOADMM', 'cmtf_nvecs', 'cmtf_nvecs_sparse', 'init_coupled_AOADMM_CMTF', 'Solver', 'AoadmmError', 'sptensor', 'mttkrp',
+           'stack_sparse_slices',
            'prox', 'chol_solve', 'gram',
            'shard_range', 'sparse_shard_bounds', 'device_count', 'nccl_unique_id']
 
@@ -70,6 +71,39 @@ def as_sparse(X):
         c = X.tocoo()
         return sptensor(np.stack([np.asarray(c.row), np.asarray(c.col)], axis=1), c.data, c.shape)
     return None
+
+
+def _first_out_of_range(S):
+    """None when every subscript of the order-2 sptensor S lies inside S.shape, else a message naming the first bad one"""
+    for d, (name, n) in enumerate(zip(('row', 'column'), S.shape)):
+        col = S.subs[:, d]
+        bad = np.flatnonzero((col < 0) | (col >= n))
+        if bad.size:
+            e = int(bad[0])
+            return '%s subscript %d of entry %d is out of range 0..%d' % (name, int(col[e]), e, n - 1)
+    return None
+
+
+def stack_sparse_slices(slices):
+    """The K sparse slices X_k (each I x J_k: an order-2 sptensor or anything `as_sparse` accepts) of a PARAFAC2 object
+    side by side as one I x Jtot sptensor, Jtot = sum J_k: entry (i, j) of slice k becomes (i, joff[k] + j) with
+    joff[k] = J_1 + ... + J_{k-1}.  Returns (sptensor, joff) with joff the K + 1 column offsets (int64).  Duplicates
+    and explicit zeros are passed on as they are (the device sums duplicates and keeps zeros)."""
+    S = [as_sparse(x) for x in slices]
+    if not S or any(x is None or x.ndim != 2 for x in S):
+        raise AoadmmError(1, 'stack_sparse_slices: every slice must be a sparse matrix')
+    I = S[0].shape[0]
+    if any(x.shape[0] != I for x in S):
+        raise AoadmmError(1, 'stack_sparse_slices: the slices must have the same number of rows')
+    for k, x in enumerate(S):   # a column outside slice k would land in a neighbouring slice once joff[k] is added
+        bad = _first_out_of_range(x)
+        if bad is not None:
+            raise AoadmmError(1, 'stack_sparse_slices: slice %d: %s' % (k + 1, bad))
+    joff = np.zeros(len(S) + 1, dtype=np.int64)
+    joff[1:] = np.cumsum([x.shape[1] for x in S])
+    subs = np.concatenate([x.subs.reshape(-1, 2) + np.array([0, joff[k]], dtype=np.int64) for k, x in enumerate(S)])
+    vals = np.concatenate([x.vals.reshape(-1) for x in S])
+    return sptensor(subs, vals, (I, int(joff[-1]))), joff
 
 
 def _check_heldout(Z, p, X):
@@ -196,13 +230,17 @@ class Solver:
     """Handle lifecycle around the C ABI: create (tensors to HBM once) -> set_state -> run -> get_state."""
 
     def __init__(self, Z, Znorm_const, rank=0, world_size=1, device=0, unique_id=None, shard=None, n_gpus=1,
-                 devices=None, shard_sparse=False):
+                 devices=None, shard_sparse=False, sparse_slices=False):
         """One GPU: defaults.  Several GPUs from THIS process (one caller, like a MATLAB session): n_gpus=N [, devices=[..]]
         with the whole objects in Z (aoadmm_create_multi cuts the slabs).  One process per GPU (torchrun): rank,
         world_size, device, unique_id [, shard] with this rank's slab or the whole object in Z.
         shard_sparse=True (with n_gpus): sparse objects are cut into nonzero-balanced slabs of their last mode
         (aoadmm_create_sparse_multi); `shards[p]` then lists the (lo, hi) slab of every GPU.  Without it sparse objects
-        run on one GPU only."""
+        run on one GPU only.
+        sparse_slices=True: a PARAFAC2 object whose slices are all sparse (order-2 sptensors or SciPy sparse matrices,
+        slice k of shape (I, J_k)) is stacked on the host into one I x Jtot COO object and runs through
+        aoadmm_create_sparse_slices (one GPU, no Z.miss); dense PARAFAC2 objects keep the dense path.  Without it sparse
+        slices are refused."""
         if n_gpus > 1 and world_size > 1:
             raise ValueError('n_gpus > 1 (one process drives all GPUs) and world_size > 1 (one process per GPU) exclude each other')
         if shard_sparse and world_size > 1:
@@ -234,9 +272,13 @@ class Solver:
             if smask[p] is not None and sparse[p] is None:
                 raise AoadmmError(1, 'Z.miss{%d} is sparse but Z.object{%d} is dense (a dense object takes a dense mask)'
                                   % (p + 1, p + 1))
+        # PARAFAC2 objects with sparse slices (aoadmm_create_sparse_slices): the stacked I x Jtot COO object, or None
+        stacked = [None] * P
         for p in range(P):
             if model[p] != 'CP' and any(as_sparse(x) is not None for x in Z['object'][p]):
-                raise AoadmmError(2, 'object %d: PARAFAC2 objects with sparse slices are not supported' % (p + 1))
+                if not sparse_slices:
+                    raise AoadmmError(2, 'object %d: PARAFAC2 objects with sparse slices are not supported' % (p + 1))
+                stacked[p] = self._stack_slices(Z, p, modes[p], miss[p], n_gpus, world_size)
             if sparse[p] is None:
                 continue
             if (n_gpus > 1 and not shard_sparse) or world_size > 1:
@@ -253,6 +295,9 @@ class Solver:
                                   % (p + 1, smask[p].shape, p + 1, want))
         sp_objs = (C.POINTER(_capi.SparseObject) * P)()
         sp_masks = (C.POINTER(_capi.SparseObject) * P)()
+        sl_objs = (C.POINTER(_capi.SparseObject) * P)()
+        if any(x is not None for x in stacked) and any(m is not None for m in smask):
+            raise AoadmmError(2, 'sparse slices: sparse Z.miss masks of CP objects are not supported in the same problem')
         ranks = self._infer_ranks(Z)
         rows = np.zeros(nb_modes, dtype=np.int64)
         nsl = np.zeros(nb_modes, dtype=np.int32)
@@ -335,6 +380,20 @@ class Solver:
                         raise AoadmmError(1, 'Z.miss{%d} size does not match Z.object{%d}.' % (p + 1, p + 1))
                     self._keep.append(Mk)
                     o.miss = Mk.ctypes.data_as(_capi.c_uint8_p)
+            elif stacked[p] is not None:
+                self.shards.append(None)
+                S = stacked[p]
+                subs = np.asfortranarray(S.subs)    # column-major: rows, then stacked columns
+                vals = np.ascontiguousarray(S.vals)
+                so = _capi.SparseObject()
+                so.nnz = vals.size
+                so.subs = subs.ctypes.data_as(_capi.c_int64_p)
+                so.vals = _dp(vals)
+                self._keep += [subs, vals, so]
+                sl_objs[p] = C.pointer(so)
+                o.data = None
+                o.slices, o.n_slices = None, len(Z['object'][p])
+                o.miss, o.miss_slices = None, None
             else:
                 self.shards.append(None)
                 sl = [_f64(x) for x in Z['object'][p]]
@@ -443,7 +502,12 @@ class Solver:
         else:
             if devices is not None:
                 dist.device = int(list(devices)[0])
-            if any(m is not None for m in smask):
+            if any(x is not None for x in stacked):
+                self._keep += [sp_objs, sl_objs]
+                _capi.check(lib.aoadmm_create_sparse_slices(C.byref(pb),
+                                                            sp_objs if any(x is not None for x in sparse) else None,
+                                                            sl_objs, C.byref(dist), C.byref(self._h)))
+            elif any(m is not None for m in smask):
                 self._keep += [sp_objs, sp_masks]
                 _capi.check(lib.aoadmm_create_sparse_masked(C.byref(pb), sp_objs, sp_masks, C.byref(dist),
                                                             C.byref(self._h)))
@@ -455,6 +519,31 @@ class Solver:
         self._keep_problem = pb
 
     # ------------------------------------------------------------------------------------------
+    @staticmethod
+    def _stack_slices(Z, p, modes_p, miss_p, n_gpus, world_size):
+        """host checks of a PARAFAC2 object with sparse slices (before any device call) and its stacked COO object"""
+        if n_gpus > 1 or world_size > 1:
+            raise AoadmmError(2, 'object %d: PARAFAC2 objects with sparse slices run on one GPU' % (p + 1))
+        if miss_p is not None:
+            raise AoadmmError(2, 'object %d: Z.miss is not supported on a PARAFAC2 object with sparse slices' % (p + 1))
+        sl = Z['object'][p]
+        I = int(Z['size'][modes_p[0] - 1])
+        Jk = [int(j) for j in Z['size'][modes_p[1] - 1]]
+        if len(sl) != len(Jk):
+            raise AoadmmError(1, 'object %d: %d slices but Z.size lists %d' % (p + 1, len(sl), len(Jk)))
+        for k, x in enumerate(sl):
+            S = as_sparse(x)
+            if S is None:
+                raise AoadmmError(1, 'object %d: slice %d is dense but other slices are sparse (all slices of a '
+                                     'PARAFAC2 object must be sparse, or all dense)' % (p + 1, k + 1))
+            if S.shape != (I, Jk[k]):
+                raise AoadmmError(1, 'object %d: slice %d has shape %s, Z.size gives %s'
+                                  % (p + 1, k + 1, tuple(S.shape), (I, Jk[k])))
+            bad = _first_out_of_range(S)
+            if bad is not None:
+                raise AoadmmError(1, 'object %d: slice %d: %s' % (p + 1, k + 1, bad))
+        return stack_sparse_slices(sl)[0]
+
     @staticmethod
     def _infer_ranks(Z):
         """columns of fac{m}: from Z['rank'] if present, else must be supplied with the state."""
@@ -769,7 +858,7 @@ def cmtf_fun_AOADMM(Z, Znorm_const, G, fh=None, gh=None, lscalar=None, uscalar=N
     the f_* values are those of the best iteration, out['heldout_best_iter'] is that iteration, and out['exit_flag'] is
     'heldoutStop' when the held-out rule ended the run.
     `dist` (rank, world_size, device, unique_id, or n_gpus [, devices, shard_sparse]) selects the multi-GPU layout;
-    default one GPU."""
+    default one GPU.  sparse_slices=True (in `dist`) runs PARAFAC2 objects with sparse slices (see Solver)."""
     if heldout is not None:
         if len(heldout) != len(Z['modes']):
             raise AoadmmError(1, 'heldout needs one entry per object (None where an object has no held-out set)')
@@ -839,6 +928,8 @@ def cmtf_AOADMM(Z, init, alg_options, init_options=None, **dist):
             if miss[p] is not None:
                 X = X * (np.asarray(miss[p]) != 0)
             zn.append(float(np.linalg.norm(X.ravel()) ** 2))
+        elif any(as_sparse(Xk) is not None for Xk in Z['object'][p]):
+            zn.append(float('nan'))                                        # sparse slices: on the device as well
         else:
             zn.append(float(sum(np.linalg.norm(Xk if miss[p] is None else Xk * (np.asarray(miss[p][k]) != 0), 'fro') ** 2
                                 for k, Xk in enumerate(Z['object'][p]))))

@@ -98,7 +98,7 @@ EXPORTS = ['aoadmm_abi_version', 'aoadmm_device_count', 'aoadmm_nccl_unique_id',
            'aoadmm_create_multi', 'aoadmm_gpu_count', 'aoadmm_comm_release', 'aoadmm_create_sparse',
            'aoadmm_create_sparse_masked', 'aoadmm_model_at', 'aoadmm_set_heldout', 'aoadmm_heldout_history',
            'aoadmm_sparse_shard_bounds', 'aoadmm_create_sparse_multi', 'aoadmm_set_heldout_stopping',
-           'aoadmm_heldout_best', 'aoadmm_nvecs_sparse']
+           'aoadmm_heldout_best', 'aoadmm_nvecs_sparse', 'aoadmm_create_sparse_slices']
 
 lib.aoadmm_abi_version.restype = C.c_int
 lib.aoadmm_device_count.argtypes = [C.POINTER(C.c_int)]
@@ -107,6 +107,8 @@ lib.aoadmm_create.argtypes = [C.POINTER(Problem), C.POINTER(Dist), C.POINTER(Han
 lib.aoadmm_create_sparse.argtypes = [C.POINTER(Problem), C.POINTER(C.POINTER(SparseObject)), C.POINTER(Dist),
                                      C.POINTER(HandleP)]
 lib.aoadmm_create_sparse_masked.argtypes = [C.POINTER(Problem), C.POINTER(C.POINTER(SparseObject)),
+                                            C.POINTER(C.POINTER(SparseObject)), C.POINTER(Dist), C.POINTER(HandleP)]
+lib.aoadmm_create_sparse_slices.argtypes = [C.POINTER(Problem), C.POINTER(C.POINTER(SparseObject)),
                                             C.POINTER(C.POINTER(SparseObject)), C.POINTER(Dist), C.POINTER(HandleP)]
 lib.aoadmm_create_multi.argtypes = [C.POINTER(Problem), C.c_int32, c_int32_p, C.POINTER(HandleP)]
 lib.aoadmm_sparse_shard_bounds.argtypes = [C.POINTER(SparseObject), C.c_int32, C.c_int64, C.c_int32, c_int64_p]

@@ -199,6 +199,64 @@ int create_sparse(const aoadmm_problem* problem, const aoadmm_sparse_object* con
   return AOADMM_OK;
 }
 
+// every check aoadmm_create_sparse_slices makes on the descriptors; touches no device.  slices[p]: the K slices of
+// PARAFAC2 object p side by side as one order-2 COO object over I x Jtot (column joff[k] + j of slice k).
+void check_sparse_slices(const aoadmm_problem* problem, const aoadmm_sparse_object* const* sparse,
+                         const aoadmm_sparse_object* const* slices, const aoadmm_dist* dist) {
+  using aoadmm::CudaError;
+  if (problem == nullptr) throw CudaError(AOADMM_ERR_INVALID_ARG, "problem is NULL");
+  if (problem->n_objects > 0 && problem->objects == nullptr) throw CudaError(AOADMM_ERR_INVALID_ARG, "objects is NULL");
+  for (int p = 0; sparse != nullptr && p < problem->n_objects; ++p)
+    if (sparse[p] != nullptr && problem->objects[p].model != AOADMM_MODEL_CP)
+      throw CudaError(AOADMM_ERR_INVALID_ARG, "sparse object " + std::to_string(p + 1) +
+                                                  ": a PARAFAC2 object takes its sparse data through `slices`");
+  check_sparse(problem, sparse, nullptr, dist);
+  for (int p = 0; slices != nullptr && p < problem->n_objects; ++p) {
+    const aoadmm_sparse_object* so = slices[p];
+    if (so == nullptr) continue;
+    const aoadmm_object& ob = problem->objects[p];
+    const std::string who = "sparse slices of object " + std::to_string(p + 1) + ": ";
+    if (ob.model != AOADMM_MODEL_PAR2)
+      throw CudaError(AOADMM_ERR_INVALID_ARG, who + "a CP object takes its sparse data through `sparse`");
+    if (dist != nullptr && dist->world_size > 1)
+      throw CudaError(AOADMM_ERR_UNSUPPORTED, who + "sparse slices run on one GPU (world_size must be 1)");
+    if (ob.miss_slices != nullptr)
+      throw CudaError(AOADMM_ERR_UNSUPPORTED, who + "missing-data masks (Z.miss) need dense slices");
+    if (ob.slices != nullptr) throw CudaError(AOADMM_ERR_INVALID_ARG, who + "both dense slices and sparse slices are set");
+    if (so->nnz < 0) throw CudaError(AOADMM_ERR_INVALID_ARG, who + "nnz is negative");
+    if (so->nnz >= 0x7fffffffLL - aoadmm::kSparseChunk)
+      throw CudaError(AOADMM_ERR_INVALID_ARG, who + "2^31 - 257 entries or more");
+    if (so->nnz > 0 && (so->subs == nullptr || so->vals == nullptr))
+      throw CudaError(AOADMM_ERR_INVALID_ARG, who + "subs / vals is NULL");
+    if (ob.order != 3 || ob.modes == nullptr || problem->mode_rows == nullptr)
+      throw CudaError(AOADMM_ERR_INVALID_ARG, who + "a PARAFAC2 object has three modes (A, B_k, C)");
+    for (int d = 0; d < 3; ++d)
+      if (ob.modes[d] < 1 || ob.modes[d] > problem->nb_modes) throw CudaError(AOADMM_ERR_INVALID_ARG, who + "mode id out of range");
+    const int mb = ob.modes[1] - 1;
+    const int K = problem->n_slices != nullptr ? problem->n_slices[mb] : 0;
+    const int64_t* jk = problem->slice_rows != nullptr ? problem->slice_rows[mb] : nullptr;
+    if (K <= 0 || jk == nullptr)
+      throw CudaError(AOADMM_ERR_INVALID_ARG, who + "missing slice sizes (Z.size of the second mode)");
+    const int64_t I = problem->mode_rows[ob.modes[0] - 1];
+    int64_t Jtot = 0;
+    for (int k = 0; k < K; ++k) {
+      if (jk[k] < 0) throw CudaError(AOADMM_ERR_INVALID_ARG, who + "slice " + std::to_string(k + 1) + " has a negative size");
+      Jtot += jk[k];
+      if (Jtot > 0x7fffffffLL) break;
+    }
+    if (I < 0 || I > 0x7fffffffLL) throw CudaError(AOADMM_ERR_INVALID_ARG, who + "I must be in 0..2^31 - 1");
+    if (Jtot > 0x7fffffffLL) throw CudaError(AOADMM_ERR_INVALID_ARG, who + "the slices have more than 2^31 - 1 columns in all");
+    const int64_t ext[2] = {I, Jtot};
+    for (int d = 0; d < 2; ++d) {
+      const int64_t* sd = so->subs + (size_t)d * (size_t)so->nnz;
+      for (int64_t e = 0; e < so->nnz; ++e)
+        if (sd[e] < 0 || sd[e] >= ext[d])
+          throw CudaError(AOADMM_ERR_INVALID_ARG, who + (d == 0 ? "row" : "column") + " subscript " + std::to_string(sd[e]) +
+                                                      " of entry " + std::to_string(e) + " is out of range");
+    }
+  }
+}
+
 // b[0..n]: the nonzero-balanced slab bounds of the last mode (include/aoadmm.h, aoadmm_sparse_shard_bounds).  With the
 // last subscripts sorted (s_0 <= s_1 <= ...), C[k] >= t holds exactly for k > s_{t-1}: the smallest k with
 // C[k] * n >= r * nnz is s_{t-1} + 1 for t = ceil(r * nnz / n) >= 1 (0 for t = 0).  The order statistics come from
@@ -397,6 +455,25 @@ int aoadmm_create_sparse(const aoadmm_problem* problem, const aoadmm_sparse_obje
 int aoadmm_create_sparse_masked(const aoadmm_problem* problem, const aoadmm_sparse_object* const* sparse,
                                 const aoadmm_sparse_object* const* masks, const aoadmm_dist* dist, aoadmm_handle** out) {
   return create_sparse(problem, sparse, masks, dist, out);
+}
+
+int aoadmm_create_sparse_slices(const aoadmm_problem* problem, const aoadmm_sparse_object* const* sparse,
+                                const aoadmm_sparse_object* const* slices, const aoadmm_dist* dist, aoadmm_handle** out) {
+  if (!out) return AOADMM_ERR_INVALID_ARG;
+  *out = nullptr;
+  aoadmm_handle* h = nullptr;
+  int rc = guard(nullptr, [&] {
+    check_sparse_slices(problem, sparse, slices, dist);   // every check on the descriptors happens before a device is touched
+    h = new aoadmm_handle();
+    h->eng.push_back(nullptr);
+    h->eng[0] = new aoadmm::Engine(problem, dist, nullptr, sparse, nullptr, slices);
+  });
+  if (rc != AOADMM_OK) {
+    delete h;
+    return rc;
+  }
+  *out = h;
+  return AOADMM_OK;
 }
 
 int aoadmm_create_multi(const aoadmm_problem* problem, int32_t n_gpus, const int32_t* devices, aoadmm_handle** out) {

@@ -460,11 +460,12 @@ struct Engine::ObjTerms {
 // construction
 // ---------------------------------------------------------------------------------------------------
 Engine::Engine(const aoadmm_problem* prob, const aoadmm_dist* dist, void* shared_comm,
-               const aoadmm_sparse_object* const* sparse, const aoadmm_sparse_object* const* masks) {
+               const aoadmm_sparse_object* const* sparse, const aoadmm_sparse_object* const* masks,
+               const aoadmm_sparse_object* const* slices) {
   // A constructor that throws never runs the destructor: everything acquired so far (up to the whole tensor in HBM,
   // streams, events, pinned buffers) is released here before the error leaves.
   try {
-    construct(prob, dist, shared_comm, sparse, masks);
+    construct(prob, dist, shared_comm, sparse, masks, slices);
   } catch (...) {
     release();
     throw;
@@ -472,7 +473,8 @@ Engine::Engine(const aoadmm_problem* prob, const aoadmm_dist* dist, void* shared
 }
 
 void Engine::construct(const aoadmm_problem* prob, const aoadmm_dist* dist, void* shared_comm,
-                       const aoadmm_sparse_object* const* sparse, const aoadmm_sparse_object* const* masks) {
+                       const aoadmm_sparse_object* const* sparse, const aoadmm_sparse_object* const* masks,
+                       const aoadmm_sparse_object* const* slices) {
   if (prob == nullptr) throw CudaError(1, "problem is NULL");
   if (dist != nullptr) {
     rank_ = dist->rank;
@@ -533,7 +535,7 @@ void Engine::construct(const aoadmm_problem* prob, const aoadmm_dist* dist, void
     o.weight = src.weight;
     o.znorm = src.znorm_const;
     if (o.model == AOADMM_MODEL_PAR2) {
-      setup_par2(prob, p);
+      setup_par2(prob, p, slices != nullptr ? slices[p] : nullptr);
       continue;
     }
     int R = 0;
@@ -731,7 +733,8 @@ void Engine::construct(const aoadmm_problem* prob, const aoadmm_dist* dist, void
   // views + workspaces
   size_t ws_bytes = 0, kr_doubles = 0;
   size_t cp0 = 0;
-  for (auto& s : par2_) ws_bytes = std::max(ws_bytes, mttkrp_workspace_bytes(s.view, s.R));
+  for (auto& s : par2_)
+    if (s.sp == nullptr) ws_bytes = std::max(ws_bytes, mttkrp_workspace_bytes(s.view, s.R));   // sparse slices own their scratch
   for (auto& o : objects_) {
     if (o.model == AOADMM_MODEL_PAR2) continue;
     cp0 = std::max(cp0, (size_t)mode(o.modes[0]).rows * mode(o.modes[0]).R);
@@ -759,7 +762,12 @@ void Engine::construct(const aoadmm_problem* prob, const aoadmm_dist* dist, void
     double* res = cp0_tmp_ + 148 * 8;
     if (o.model == AOADMM_MODEL_PAR2) {
       Par2State& s = par2_[mode(o.modes[0]).par2];
-      launches_ += object_norm2(s.X_alloc, s.mask_alloc, s.I, s.ldX, s.jhi - s.jlo, part, res, st_);
+      if (s.sp != nullptr) {
+        launches_ += sparse_norm2(*s.sp, st_);
+        res = s.sp->norm_out;
+      } else {
+        launches_ += object_norm2(s.X_alloc, s.mask_alloc, s.I, s.ldX, s.jhi - s.jlo, part, res, st_);
+      }
     } else if (o.sp != nullptr) {
       launches_ += sparse_norm2(*o.sp, st_);
       res = o.sp->norm_out;
@@ -892,6 +900,12 @@ void Engine::release() {
   lin_modes_.clear();
   lin_groups_.clear();
   for (auto& s : par2_) {
+    if (s.sp != nullptr) {
+      sparse_free(*s.sp);
+      delete s.sp;
+      s.sp = nullptr;
+    }
+    dfree(s.mgram);
     for (DevMat* d : {&s.W, &s.T, &s.P, &s.muDB, &s.DeltaB, &s.PDold, &s.gM, &s.gS}) dev_free(*d);
     for (void* q : {(void*)s.joff_dev, (void*)s.seg_dev, (void*)s.X_alloc, (void*)s.mask_alloc, (void*)s.redbuf, (void*)s.G2, (void*)s.Binv2, (void*)s.Binv3,
                     (void*)s.rho2, (void*)s.rho3, (void*)s.tdiag, (void*)s.contrib, (void*)s.Vprev, (void*)s.sysws, (void*)s.norms, (void*)s.Csum, (void*)s.segn,
@@ -1230,7 +1244,7 @@ void Engine::precompute_mode(ModeState& m, int n_rho_terms, bool do_chol) {
 // ---------------------------------------------------------------------------------------------------
 // PARAFAC2 block
 // ---------------------------------------------------------------------------------------------------
-void Engine::setup_par2(const aoadmm_problem* prob, int p) {
+void Engine::setup_par2(const aoadmm_problem* prob, int p, const aoadmm_sparse_object* slices) {
   const aoadmm_object& src = prob->objects[p];
   ObjectState& o = objects_[p];
   if (o.order != 3) throw CudaError(1, "a PARAFAC2 object has exactly three modes (A, B_k, C)");
@@ -1257,8 +1271,10 @@ void Engine::setup_par2(const aoadmm_problem* prob, int p) {
   if (s.R > 128) throw CudaError(2, "PARAFAC2 objects support at most 128 components on device");
   s.K = (prob->n_slices != nullptr) ? prob->n_slices[s.m2 - 1] : 0;
   const int64_t* jk = (prob->slice_rows != nullptr) ? prob->slice_rows[s.m2 - 1] : nullptr;
-  if (s.K <= 0 || jk == nullptr || src.n_slices != s.K || src.slices == nullptr)
+  if (s.K <= 0 || jk == nullptr || (slices == nullptr && (src.n_slices != s.K || src.slices == nullptr)))
     throw CudaError(1, "PARAFAC2 object: slice sizes (Z.size of the second mode) and K data slices are required");
+  if (slices != nullptr && (src.slices != nullptr || src.miss_slices != nullptr))
+    throw CudaError(2, "PARAFAC2 object: sparse slices take neither dense slices nor Z.miss");
   if (mc.rows != s.K) throw CudaError(1, "PARAFAC2 object: the third mode must have K rows");
   s.I = ma.rows;
   s.joff.assign(s.K + 1, 0);
@@ -1297,13 +1313,29 @@ void Engine::setup_par2(const aoadmm_problem* prob, int p) {
   s.jlo = s.joff[s.k0];
   s.jhi = s.joff[s.k1];
   const int64_t Jloc = s.jhi - s.jlo;
-  const size_t xbytes = std::max<size_t>((size_t)s.ldX * Jloc * sizeof(double), 256);
-  AO_CUDA(cudaMalloc(&s.X_alloc, xbytes));
-  if (s.ldX != s.I) AO_CUDA(cudaMemset(s.X_alloc, 0, xbytes));
-  s.X = s.X_alloc - (size_t)s.jlo * s.ldX;      // global column indexing (only columns jlo..jhi-1 are ever touched)
+  if (slices != nullptr) {
+    // sparse slices: Xall as one order-2 COO object over I x Jtot (sorted copies by row and by stacked column); no
+    // I x Jtot buffer exists
+    if (world_ > 1) throw CudaError(2, "PARAFAC2 object: sparse slices run on one GPU");
+    const long long dims[2] = {(long long)s.I, (long long)s.Jtot};
+    s.sp = new SparseTensor();
+    try {
+      sparse_build(*s.sp, 2, dims, 0, s.Jtot, s.R, slices->nnz, reinterpret_cast<const long long*>(slices->subs),
+                   slices->vals, st_, false, 0, nullptr, nullptr, true);
+    } catch (const CudaError& e) {
+      throw CudaError(e.code, "PARAFAC2 object " + std::to_string(p + 1) + " (sparse slices): " + e.what());
+    }
+    AO_CUDA(cudaMalloc(&s.mgram, sizeof(double) * 2 * s.R * s.R));
+  } else {
+    const size_t xbytes = std::max<size_t>((size_t)s.ldX * Jloc * sizeof(double), 256);
+    AO_CUDA(cudaMalloc(&s.X_alloc, xbytes));
+    if (s.ldX != s.I) AO_CUDA(cudaMemset(s.X_alloc, 0, xbytes));
+    s.X = s.X_alloc - (size_t)s.jlo * s.ldX;      // global column indexing (only columns jlo..jhi-1 are ever touched)
+  }
   std::vector<int> seg((size_t)s.Jtot);
   for (int k = 0; k < s.K; ++k) {
     for (int64_t j = s.joff[k]; j < s.joff[k + 1]; ++j) seg[(size_t)j] = k;
+    if (s.sp != nullptr) continue;
     if (k < s.k0 || k >= s.k1) continue;          // another rank's slice (its pointer may be NULL)
     if (src.slices[k] == nullptr) throw CudaError(1, "PARAFAC2 object: NULL slice");
     AO_CUDA(cudaMemcpy2D(s.X + (size_t)s.joff[k] * s.ldX, (size_t)s.ldX * 8, src.slices[k], (size_t)s.I * 8,
@@ -1338,13 +1370,17 @@ void Engine::setup_par2(const aoadmm_problem* prob, int p) {
   s.lay.k1 = s.k1;
   s.lay.jlo = s.jlo;
   s.lay.jhi = s.jhi;
-  make_tensor3(s.view, s.X_alloc, s.I, Jloc, 1, s.ldX);   // this rank's columns as an I x Jloc x 1 tensor
-  packed_factor_alloc(s.fW, Jloc, s.R);
+  if (s.sp == nullptr) {
+    make_tensor3(s.view, s.X_alloc, s.I, Jloc, 1, s.ldX);   // this rank's columns as an I x Jloc x 1 tensor
+    packed_factor_alloc(s.fW, Jloc, s.R);
+  }
   AO_CUDA(cudaMalloc(&s.redbuf, sizeof(double) * ((size_t)s.R * s.R + 8)));
-  packed_factor_alloc(s.fA, s.I, s.R);
-  packed_factor_alloc(s.ones, 1, s.R);
-  packed_factor_pack(s.ones, nullptr, 1, st_, nullptr);
-  ++launches_;
+  if (s.sp == nullptr) {
+    packed_factor_alloc(s.fA, s.I, s.R);
+    packed_factor_alloc(s.ones, 1, s.R);
+    packed_factor_pack(s.ones, nullptr, 1, st_, nullptr);
+    ++launches_;
+  }
   for (DevMat* d : {&s.W, &s.T, &s.P, &s.muDB, &s.PDold, &s.gM, &s.gS}) dev_alloc(*d, s.Jtot, s.R);
   dev_alloc(s.DeltaB, s.R, s.R);
   const size_t KRR = (size_t)s.K * s.R * s.R;
@@ -1370,6 +1406,25 @@ void Engine::setup_par2(const aoadmm_problem* prob, int p) {
   AO_CUDA(cudaDeviceSynchronize());
 }
 
+// explicit residual of a PARAFAC2 object with sparse slices into s.res: the stored entries in one model pass, the
+// unstored ones as ||M||^2 - sum m^2 with ||M||^2 = sum((A'A) .* sum_k diag(c_k) B_k'B_k diag(c_k)).  W and every Gram
+// are recomputed from the current factors.  W is scratch (the mode-A update rebuilds it before reading it), A'A and the
+// Hadamard sum go to the object's own scratch s.mgram.  The per-slice Grams are rebuilt in place in s.G2: that buffer
+// holds B_k'B_k of the current B at every objective (run() refreshes it before iteration 0 and par2_update_B after every
+// update of B, the only writer of B inside a run), and the batched Gram is deterministic, so the rewrite stores the
+// same bits and the solve does not change; a separate K x R x R copy would cost as much memory as G2 itself (2 GB at
+// K = 2^20, R = 16), and Gram(W) = W'W through the generic Gram kernel, tried instead, made the p2 workload of
+// tools/sparse_bench.py 4 % slower.
+void Engine::par2_sparse_residual(Par2State& s) {
+  const ModeState &ma = mode(s.m1), &mb = mode(s.m2), &mc = mode(s.m3);
+  const size_t RR = (size_t)s.R * s.R;
+  launches_ += par2_scale_rows(s.lay, s.W.p, mb.fac.p, mc.fac.p, mc.rows, 1.0, nullptr, 0.0, st_);
+  launches_ += par2_batched_gram(s.lay, mb.fac.p, s.G2, st_);
+  launches_ += par2_modeA_had(s.lay, s.G2, mc.fac.p, mc.rows, s.mgram + RR, st_);
+  launches_ += gram(ma.fac.p, ma.rows, ma.rows, s.R, s.mgram, gram_ws_, st_, nullptr);
+  launches_ += sparse_par2_residual(*s.sp, ma.fac.p, ma.rows, s.W.p, s.Jtot, s.mgram, s.mgram + RR, s.res, st_);
+}
+
 void Engine::par2_refresh_gram(Par2State& s) {  // :71-73, :216-218
   launches_ += par2_batched_gram(s.lay, mode(s.m2).fac.p, s.G2, st_);
 }
@@ -1379,9 +1434,15 @@ void Engine::par2_update_T(Par2State& s) {
   ModeState& a = mode(s.m1);
   if (s.T_version == a.version) return;
   phase_begin(1);
-  packed_factor_pack(s.fA, a.fac.p, a.rows, st_, nullptr);
-  ++launches_;
-  launches_ += mttkrp3(s.view, 1, s.fA, s.ones, s.R, 1.0, s.T.p + s.jlo, s.Jtot, mws_, st_, nullptr);   // local rows of T
+  if (s.sp != nullptr) {   // mode position 1 of the I x Jtot COO object: reads A only (W is not transposed)
+    const double* fac[2] = {a.fac.p, s.W.p};
+    const long long ld[2] = {a.rows, s.Jtot};
+    launches_ += sparse_mttkrp(*s.sp, 1, fac, ld, 1.0, s.T.p, s.Jtot, st_);
+  } else {
+    packed_factor_pack(s.fA, a.fac.p, a.rows, st_, nullptr);
+    ++launches_;
+    launches_ += mttkrp3(s.view, 1, s.fA, s.ones, s.R, 1.0, s.T.p + s.jlo, s.Jtot, mws_, st_, nullptr);   // local rows of T
+  }
   phase_end();
   s.T_version = a.version;
 }
@@ -1423,9 +1484,15 @@ void Engine::par2_precompute_A(ModeState& m, int n_rho_terms, bool do_chol) {
   ModeState &mb = mode(s.m2), &mc = mode(s.m3);
   phase_begin(1);
   launches_ += par2_scale_rows(s.lay, s.W.p, mb.fac.p, mc.fac.p, mc.rows, 1.0, nullptr, 0.0, st_);
-  packed_factor_pack(s.fW, s.W.p + s.jlo, s.Jtot, st_, nullptr);
-  ++launches_;
-  launches_ += mttkrp3(s.view, 0, s.fW, s.ones, s.R, o.weight, m.A.p, m.rows, mws_, st_, nullptr);
+  if (s.sp != nullptr) {   // mode position 0 of the I x Jtot COO object with the factors {A, W}
+    const double* fac[2] = {m.fac.p, s.W.p};
+    const long long ld[2] = {m.rows, s.Jtot};
+    launches_ += sparse_mttkrp(*s.sp, 0, fac, ld, o.weight, m.A.p, m.rows, st_);
+  } else {
+    packed_factor_pack(s.fW, s.W.p + s.jlo, s.Jtot, st_, nullptr);
+    ++launches_;
+    launches_ += mttkrp3(s.view, 0, s.fW, s.ones, s.R, o.weight, m.A.p, m.rows, mws_, st_, nullptr);
+  }
   if (s.sharded) allreduce(m.A.p, (size_t)m.rows * m.R);    // sum over the ranks' slices (:159-163)
   phase_end();
   launches_ += par2_modeA_had(s.lay, s.G2, mc.fac.p, mc.rows, s.Csum, st_);
@@ -1852,7 +1919,9 @@ void Engine::enqueue_objective(bool first) {
     ModeState& mb = mode(s.m2);
     launches_ += par2_seg_norms(s.lay, mb.fac.p, mb.constrained ? mb.Z.p : nullptr, s.P.p, s.DeltaB.p,
                                 mb.constrained ? reg_red_kind(mb.con.kind) : -1, s.segn, st_);
-    if (first || s.explicit_residual)
+    if ((first || s.explicit_residual) && s.sp != nullptr)
+      par2_sparse_residual(s);
+    else if (first || s.explicit_residual)
       launches_ += par2_residual(s.lay, s.X, s.ldX, s.I, mode(s.m1).fac.p, mode(s.m1).rows, mb.fac.p, mode(s.m3).fac.p,
                                  mode(s.m3).rows, s.res_partials, admm_counter_, s.res, st_);
     if (s.sharded) {
@@ -2320,6 +2389,8 @@ void Engine::run(const aoadmm_options* opt, aoadmm_out* out) {
     for (auto& o : objects_) {
       double e = 1.0;
       for (auto d : o.dims) e *= (double)d;
+      if (o.model == AOADMM_MODEL_PAR2 && par2_[mode(o.modes[0]).par2].sp != nullptr)
+        e = (double)par2_[mode(o.modes[0]).par2].sp->nnz;   // sparse slices: likewise
       elems += o.sp != nullptr ? (double)o.sp->nnz : e;   // sparse objects: the work scales with nnz
     }
     graph_ok = (opt_.graph > 0) || elems <= 33554432.0;
@@ -2598,6 +2669,9 @@ void Engine::nvecs_to_host(int mode_id, int slice, int r, double* out, int64_t r
     for (auto& c : par2_)
       if (c.p == p) ps = &c;
     if (ps == nullptr) throw CudaError(1, "nvecs: PARAFAC2 state missing");
+    if (ps->sp != nullptr && pos <= 1)
+      throw CudaError(2, "nvecs: mode " + std::to_string(mode_id) + " belongs to a PARAFAC2 object with sparse slices "
+                         "(initialise it from a distribution)");
     if (pos == 0) {          // init_coupled_AOADMM_CMTF.m:55-60: slices side by side
       if (slice != 0) throw CudaError(1, "nvecs: slice given for PARAFAC2 mode A");
       s.X = ps->X_alloc;     // this rank's slices; the partial Gram matrices are summed over the ranks

@@ -137,6 +137,10 @@ struct Par2State {
          *sysws = nullptr;   // R > 64: factorisation workspace of the per-slice systems (2 R^2 per slice)
   double* segn_host = nullptr;           // pinned: K x 4 per-slice objective terms + 1 residual
   bool explicit_residual = false;        // objective needs ||X_k - A D_k B_k'||^2 (mode A is not updated last)
+  // sparse slices (aoadmm_create_sparse_slices): Xall as an order-2 COO object over I x Jtot.  X, mask, view, fW, fA and
+  // ones stay empty; the two products are mode positions 0 / 1 of the sparse MTTKRP with the factors {A, W}.
+  SparseTensor* sp = nullptr;
+  double* mgram = nullptr;               // sparse slices: 2 R^2 scratch of the residual (A'A, sum_k diag(c_k) B_k'B_k diag(c_k))
 };
 
 struct View3 {                // how mode position n of an object is computed
@@ -180,9 +184,12 @@ class Engine {
   // shared_comm: communicator of this rank created by the caller (single-process device group), else nullptr and the
   // communicator of dist->nccl_unique_id is taken from the process-wide cache.  sparse: nullptr, or n_objects entries
   // (nullptr for a dense object) with the COO data of sparse CP objects (aoadmm_create_sparse, validated by the caller);
-  // masks: nullptr, or n_objects entries with the sparse Z.miss masks of sparse objects (aoadmm_create_sparse_masked)
+  // masks: nullptr, or n_objects entries with the sparse Z.miss masks of sparse objects (aoadmm_create_sparse_masked);
+  // slices: nullptr, or n_objects entries with the stacked I x Jtot COO slices of PARAFAC2 objects
+  // (aoadmm_create_sparse_slices, validated by the caller)
   Engine(const aoadmm_problem* prob, const aoadmm_dist* dist, void* shared_comm = nullptr,
-         const aoadmm_sparse_object* const* sparse = nullptr, const aoadmm_sparse_object* const* masks = nullptr);
+         const aoadmm_sparse_object* const* sparse = nullptr, const aoadmm_sparse_object* const* masks = nullptr,
+         const aoadmm_sparse_object* const* slices = nullptr);
   ~Engine();
   Engine(const Engine&) = delete;
   Engine& operator=(const Engine&) = delete;
@@ -233,7 +240,8 @@ class Engine {
  private:
   // setup
   void construct(const aoadmm_problem* prob, const aoadmm_dist* dist, void* shared_comm,
-                 const aoadmm_sparse_object* const* sparse, const aoadmm_sparse_object* const* masks);
+                 const aoadmm_sparse_object* const* sparse, const aoadmm_sparse_object* const* masks,
+                 const aoadmm_sparse_object* const* slices);
   // imputed: the MTTKRP of the EM-imputed tensor of a masked sparse object (the sweep); else of the stored values
   int sparse_mttkrp_of(ObjectState& o, int pos, double scale, double* out, int64_t ldout, bool imputed = false);
   static bool sparse_masked(const ObjectState& o) { return o.sp != nullptr && o.sp->masked; }
@@ -271,7 +279,8 @@ class Engine {
   void lin_prepare_group(int coupl_id);
   void run_admm_linear(int coupl_id, std::vector<ModeState*>& group, const aoadmm_options& opt);
   // PARAFAC2 block (cmtf_fun_AOADMM.m:157-250, :509-589)
-  void setup_par2(const aoadmm_problem* prob, int p);
+  void setup_par2(const aoadmm_problem* prob, int p, const aoadmm_sparse_object* slices);
+  void par2_sparse_residual(Par2State& s);
   void par2_update_T(Par2State& s);
   void par2_precompute_A(ModeState& m, int n_rho_terms, bool do_chol = true);
   void par2_update_B(ModeState& m, int outer_iter);

@@ -274,7 +274,9 @@ struct ModelArgs {
 // across lanes, a fixed xor tree across them; consecutive nonzeros share rows and index sectors, as in the MTTKRP).
 // Every group runs kSparseChunk steps so that each shuffle has the whole warp.  Per CTA, in a fixed order:
 // [0] sum s m', [1] sum m'^2, [2] sum (m' - m)^2, [3] sum m^2.
-template <int G, int CPL>
+// RESID (the residual of a PARAFAC2 object with sparse slices): [0] sum (s - m')^2, [1] sum m'^2, [2] = [3] = 0; the
+// model state m / r is neither read nor written.
+template <int G, int CPL, bool RESID = false>
 __global__ void __launch_bounds__(256) sp_model_kernel(const ModelArgs a) {
   __shared__ double scratch[32];
   const int gl = threadIdx.x % G;
@@ -285,7 +287,13 @@ __global__ void __launch_bounds__(256) sp_model_kernel(const ModelArgs a) {
     const long long e = e0 + q0;
     const bool ok = e < a.nnz;
     const double t = model_at_entry<G, CPL>(a.F, a.row0, a.idx, a.nnz, a.no, R, e, gl, ok);
-    if (ok && gl == 0) {
+    if constexpr (RESID) {
+      if (ok && gl == 0) {
+        const double d = __ldg(a.vals + e) - t;
+        s0 = fma(d, d, s0);
+        s1 = fma(t, t, s1);
+      }
+    } else if (ok && gl == 0) {
       const double s = __ldg(a.vals + e), mo = a.m[e], d = t - mo;
       s0 = fma(s, t, s0);
       s1 = fma(t, t, s1);
@@ -398,6 +406,20 @@ __global__ void em_final_kernel(const double* __restrict__ nz, const double* __r
     sums[2] = nz[0];
     sums[3] = nz[1];
     sums[4] = 0.0;
+  }
+}
+
+// res = sum (x - m)^2 + max(0, ||M||^2 - sum m^2) of a PARAFAC2 object with sparse slices: the stored-entry sums from
+// the per-CTA partials of sp_model_kernel<RESID> (fixed order), ||M||^2 = sum(GA .* GC) (lane l takes l, l + 32, ...)
+__global__ void par2_res_final_kernel(const double* __restrict__ part, unsigned nm, const double* __restrict__ GA,
+                                      const double* __restrict__ GC, int RR, double* __restrict__ res) {
+  const double sse = warp_sum_partials(part, nm, 4), msum = warp_sum_partials(part + 1, nm, 4);
+  double mm = 0.0;
+  for (int i = threadIdx.x; i < RR; i += 32) mm = fma(GA[i], GC[i], mm);
+  mm = warp_sum(mm);
+  if (threadIdx.x == 0) {
+    const double unstored = mm - msum;   // the model on the unstored entries: a sum of squares, negative only by rounding
+    *res = sse + (unstored > 0.0 ? unstored : 0.0);
   }
 }
 
@@ -575,7 +597,7 @@ bool mask_matches(Temps& tmp, int order, const long long* dims, long long nm, co
 
 void sparse_build(SparseTensor& s, int order, const long long* full_dims, long long shard_offset, long long shard_extent,
                   int R, long long nnz, const long long* subs, const double* vals, cudaStream_t st, bool masked,
-                  long long mask_nnz, const long long* mask_subs, const double* mask_vals) {
+                  long long mask_nnz, const long long* mask_subs, const double* mask_vals, bool model_pass) {
   if (order < 2 || order > 8) throw CudaError(1, "sparse object: order must be in 2..8");
   if (nnz < 0) throw CudaError(1, "sparse object: negative nnz");
   if (nnz > 0x7fffffffLL - kSparseChunk) throw CudaError(2, "sparse object: more than 2^31 - 257 nonzeros on one GPU");
@@ -648,6 +670,11 @@ void sparse_build(SparseTensor& s, int order, const long long* full_dims, long l
   s.tail = dalloc<double>((size_t)units * R);
   s.norm_partials = dalloc<double>(kNormBlocks);
   s.norm_out = dalloc<double>(1);
+  if (model_pass && !masked) {   // the position-1 subscripts and the partials of a pass of sp_model_kernel
+    s.row0 = dalloc<int>(nm);
+    if (nm > 0) AO_CUDA(cudaMemcpyAsync(s.row0, ms, (size_t)nm * sizeof(int), cudaMemcpyDeviceToDevice, st));
+    s.em_partials = dalloc<double>(4 * (size_t)std::max<long long>(model_blocks(nm, R), 1));
+  }
   if (masked) {
     // the factor side (B, cross-Grams, stacks and their Grams) has the full extents and is replicated on every GPU
     // EM state: m = 0, r = s, B = 0 ("the unobserved entries start at 0"), every buffer of sparse_em / the imputed MTTKRP
@@ -837,6 +864,36 @@ int sparse_em_nonzeros(SparseTensor& s, const double* const* fac, const long lon
     ++launches;
   }
   em_nz_kernel<<<1, 32, 0, st>>>(s.em_partials + 2 * kTeleBlocks, nbm, s.em_nz);
+  AO_CHECK_LAUNCH();
+  return launches + 1;
+}
+
+int sparse_par2_residual(SparseTensor& s, const double* A, long long ldA, const double* W, long long ldW, const double* GA,
+                         const double* GC, double* res, cudaStream_t st) {
+  const int R = s.R;
+  int launches = 0;
+  unsigned nbm = 0;
+  if (s.nnz > 0) {
+    ModelArgs a{};
+    a.nnz = s.nnz;
+    a.no = 1;
+    a.R = R;
+    a.row0 = s.row0;
+    a.idx = s.modes[0].idx;
+    a.vals = s.modes[0].vals;
+    launches += transpose_scale(A, s.dims[0], R, ldA, s.factT[0], R, 1.0, st);
+    launches += transpose_scale(W, s.dims[1], R, ldW, s.factT[1], R, 1.0, st);
+    a.F[0] = s.factT[0];
+    a.F[1] = s.factT[1];
+    a.part = s.em_partials;
+    nbm = (unsigned)model_blocks(s.nnz, R);
+    rank_dispatch(R, [&](auto g, auto c) {
+      sp_model_kernel<decltype(g)::value, decltype(c)::value, true><<<nbm, 256, 0, st>>>(a);
+    });
+    AO_CHECK_LAUNCH();
+    ++launches;
+  }
+  par2_res_final_kernel<<<1, 32, 0, st>>>(s.em_partials, nbm, GA, GC, R * R, res);
   AO_CHECK_LAUNCH();
   return launches + 1;
 }

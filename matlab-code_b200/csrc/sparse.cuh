@@ -134,9 +134,11 @@ struct SparseTensor {
 // masked: the object has a sparse Z.miss mask (mask_nnz entries, same layout as subs / vals).  An entry is observed when its merged value
 // is nonzero; the observed set must equal the stored set of the object (else CudaError UNSUPPORTED).  Allocates the EM
 // state (sparse.cuh above) with m = 0, r = s, B = 0.
+// model_pass: keep row0 and the per-CTA partials of one model pass (sparse_par2_residual) without the EM state.
 void sparse_build(SparseTensor& s, int order, const long long* full_dims, long long shard_offset, long long shard_extent,
                   int R, long long nnz, const long long* subs, const double* vals, cudaStream_t st, bool masked = false,
-                  long long mask_nnz = 0, const long long* mask_subs = nullptr, const double* mask_vals = nullptr);
+                  long long mask_nnz = 0, const long long* mask_subs = nullptr, const double* mask_vals = nullptr,
+                  bool model_pass = false);
 void sparse_free(SparseTensor& s);
 // ||X||_F^2 = sum of the squared merged values (fixed-order reduction); the result lands in s.norm_out (device).  A slab
 // gives its partial sum.
@@ -163,6 +165,14 @@ int sparse_cross_gram(SparseTensor& s, int n, const double* F, long long ld, cud
 int sparse_em_nonzeros(SparseTensor& s, const double* const* fac, const long long* ld, bool impute, cudaStream_t st);
 int sparse_em_finish(SparseTensor& s, const double* const* fac, const long long* ld, bool impute, double* sums,
                      cudaStream_t st);
+
+// PARAFAC2 object with sparse slices (an I x Jtot order-2 object built with model_pass = true): one pass over the
+// stored entries gives sum (x - m)^2 and sum m^2 with m = A(i,:) . W(j,:) (the model at the entry, the lane layout of
+// sp_model_kernel), then *res = sum (x - m)^2 + max(0, sum(GA .* GC) - sum m^2), GA = A'A and GC = sum_k
+// diag(c_k) B_k'B_k diag(c_k) (R x R, so that sum(GA .* GC) = ||A diag(c_k) B_k'||^2 summed over k).  Allocation-free, fixed
+// summation order.
+int sparse_par2_residual(SparseTensor& s, const double* A, long long ldA, const double* W, long long ldW, const double* GA,
+                         const double* GC, double* res, cudaStream_t st);
 
 // nvecs of a sparse mode (aoadmm_nvecs_sparse): U = X_(n) of mode position n with its columns compressed to the distinct
 // fibers (the other-mode subscripts that occur), so that Y V = X_(n) X_(n)' V = U (U' V) without forming Y.  Built per

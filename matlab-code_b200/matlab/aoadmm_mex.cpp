@@ -16,6 +16,8 @@
 // sparse matrix through find); the 1-based double subscripts become 0-based int64 and the handle is created with
 // aoadmm_create_sparse (one GPU, CP only: anything else raises aoadmm:unsupported).  Z.miss{p} of a sparse object must
 // be sparse too (the same struct); its nonzeros mark the observed entries (aoadmm_create_sparse_masked).
+// options.b200_sparse_slices = true: a PARAFAC2 object whose slices are all such structs is stacked into one I x Jtot
+// descriptor and the handle comes from aoadmm_create_sparse_slices (one GPU); without it sparse slices are unsupported.
 //
 // Error handling: mexErrMsgIdAndTxt leaves mexFunction with a longjmp that runs no C++ destructor, so nothing in
 // here calls it directly - failures travel as a C++ exception (MexError) to the bottom of mexFunction, where every
@@ -221,6 +223,14 @@ void solve(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
   std::vector<std::vector<int64_t>> mk_subs(P);
   std::vector<aoadmm_sparse_object> mk_obj(P);
   std::vector<const aoadmm_sparse_object*> mk_ptr(P, nullptr);
+  // options.b200_sparse_slices = true: PARAFAC2 objects with sparse slices, stacked side by side into one I x Jtot
+  // descriptor per object (aoadmm_create_sparse_slices)
+  const bool sparse_slices = opt_scalar(opt, "b200_sparse_slices", 0.0) != 0.0;
+  std::vector<std::vector<int64_t>> sl_subs(P);
+  std::vector<std::vector<double>> sl_vals(P);
+  std::vector<aoadmm_sparse_object> sl_obj(P);
+  std::vector<const aoadmm_sparse_object*> sl_ptr(P, nullptr);
+  bool any_slices = false;
   std::vector<std::vector<std::vector<uint8_t>>> miss_par2(P);
   std::vector<std::vector<const uint8_t*>> miss_par2_ptr(P);
   for (int p = 0; p < P; ++p)
@@ -271,13 +281,46 @@ void solve(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
     const mxArray* obj = mxGetCell(objects, p);
     if (par2) {
       const int K = (int)mxGetNumberOfElements(obj);
-      obj_slices[p].resize(K);
-      for (int k = 0; k < K; ++k) {
-        if (is_coo_struct(mxGetCell(obj, k))) fail("aoadmm:unsupported", "PARAFAC2 objects with sparse slices are not supported");
-        obj_slices[p][k] = mxGetPr(dense_data(mxGetCell(obj, k), pc));
+      bool sparse_k = false;
+      for (int k = 0; k < K; ++k) sparse_k = sparse_k || is_coo_struct(mxGetCell(obj, k));
+      if (sparse_k && !sparse_slices) fail("aoadmm:unsupported", "PARAFAC2 objects with sparse slices are not supported");
+      if (sparse_k) {   // slice k (I x J_k) -> rows i, stacked columns joff[k] + j of one I x Jtot descriptor
+        const int mb = obj_modes[p][1] - 1;
+        if ((int)slice_rows[mb].size() != K)
+          fail("aoadmm:invalidArg", "Z.object{" + std::to_string(p + 1) + "}: Z.size of the second mode must list J_k of every slice");
+        std::vector<int64_t> cols;
+        int64_t joff = 0;
+        for (int k = 0; k < K; ++k) {
+          const mxArray* sk = mxGetCell(obj, k);
+          if (!is_coo_struct(sk))
+            fail("aoadmm:invalidArg", "Z.object{" + std::to_string(p + 1) + "}{" + std::to_string(k + 1) +
+                                          "} is dense but other slices are sparse (all slices must be sparse, or all dense)");
+          std::vector<int64_t> sub;
+          int64_t n = 0;
+          coo_subs(sk, p, 2, {mode_rows[obj_modes[p][0] - 1], slice_rows[mb][k]}, sub, &n);
+          const double* v = n > 0 ? mxGetPr(mxGetField(sk, 0, "vals")) : nullptr;
+          for (int64_t e = 0; e < n; ++e) {
+            sl_subs[p].push_back(sub[e]);
+            cols.push_back(joff + sub[n + e]);
+            sl_vals[p].push_back(v[e]);
+          }
+          joff += slice_rows[mb][k];
+        }
+        const int64_t nnz = (int64_t)sl_vals[p].size();
+        sl_subs[p].insert(sl_subs[p].end(), cols.begin(), cols.end());   // column-major nnz x 2: rows, then columns
+        sl_obj[p].nnz = nnz;
+        sl_obj[p].subs = sl_subs[p].data();
+        sl_obj[p].vals = nnz > 0 ? sl_vals[p].data() : nullptr;
+        sl_ptr[p] = &sl_obj[p];
+        any_slices = true;
+        o.slices = nullptr;
+        o.n_slices = K;
+      } else {
+        obj_slices[p].resize(K);
+        for (int k = 0; k < K; ++k) obj_slices[p][k] = mxGetPr(dense_data(mxGetCell(obj, k), pc));
+        o.slices = obj_slices[p].data();
+        o.n_slices = K;
       }
-      o.slices = obj_slices[p].data();
-      o.n_slices = K;
     } else if (is_coo_struct(obj)) {   // sparse object -> aoadmm_create_sparse
       std::vector<int64_t> rows(order);
       for (int d = 0; d < order; ++d) rows[d] = mode_rows[obj_modes[p][d] - 1];
@@ -433,8 +476,12 @@ void solve(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
   if (n_gpus < 1) fail("aoadmm:invalidArg", "options.b200_gpus must be >= 1");
   if (any_sparse && n_gpus > 1 && !shard_sparse)
     fail("aoadmm:unsupported", "sparse objects run on one GPU (options.b200_gpus must be 1, or set options.b200_shard_sparse)");
+  if (any_slices && (n_gpus > 1 || any_mask))
+    fail("aoadmm:unsupported", "PARAFAC2 objects with sparse slices run on one GPU, without sparse masks on other objects");
   HandleGuard guard;
-  if (any_sparse && n_gpus > 1)
+  if (any_slices)
+    check(aoadmm_create_sparse_slices(&pb, any_sparse ? sp_ptr.data() : nullptr, sl_ptr.data(), nullptr, &guard.h), nullptr);
+  else if (any_sparse && n_gpus > 1)
     check(aoadmm_create_sparse_multi(&pb, sp_ptr.data(), any_mask ? mk_ptr.data() : nullptr, n_gpus, nullptr, &guard.h),
           nullptr);
   else if (any_mask)

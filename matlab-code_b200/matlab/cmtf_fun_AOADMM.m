@@ -14,7 +14,9 @@ function [G,out] = cmtf_fun_AOADMM(Z,Znorm_const,G,fh,gh,lscalar,uscalar,options
 % reference's MATLAB solver).
 % Engine options (fields of `options`, all optional): b200_gpus = number of B200s of this box the call uses (the
 % tensors are cut into mode-3 slabs inside the library, one MATLAB process drives all of them), b200_shard_sparse =
-% true (with b200_gpus > 1: sparse objects too are cut, into nonzero-balanced slabs of their last mode), b200_dimtree,
+% true (with b200_gpus > 1: sparse objects too are cut, into nonzero-balanced slabs of their last mode),
+% b200_sparse_slices = true (PARAFAC2 objects whose slices are all sparse, MATLAB sparse or order-2 sptensor, run without
+% densifying them; one GPU, no Z.miss on such an object), b200_dimtree,
 % b200_mttkrp_precision, b200_fuse_inner, b200_graph, b200_heldout{p} = an sptensor / sparse matrix of entries of object p
 % withheld from training (with their true values; object p needs Z.miss): out.heldout_sse{p} is then the held-out SSE
 % after outer iterations 0..OuterIterations.  b200_heldout_patience = P (needs b200_heldout): early stopping on the summed

@@ -34,8 +34,17 @@ computed from the shapes: stream = nnz (8 + 4 (N-1)) + row pointers + output, ga
 the stream rate against the 6557 GB/s measured copy peak.  nnz is the number of nonzeros handed to the engine (before
 duplicates are merged).
 
-usage: python tools/sparse_bench.py [--workloads s1,s2,m1,m2,c1_em] [--densities 0.001,0.01,0.1] [--s2-scale 1.0]
-                                    [--m-scale 1.0] [--iters 5] [--stop-iters 30]
+PARAFAC2 objects with sparse slices (Solver(..., sparse_slices=True)), R = 16, nonneg A and C, one GPU:
+  p1            I = 2048 codes x K = 16384 slices, J_k uniform in [16, 112] (Jtot ~ 1e6), 2 % uniform density (~4e7
+                entries): the dense PARAFAC2 engine on the full slices (17 GB) runs in the same call, alternating, from
+                the same state.  Outer it/s of both, the per-iteration kernel-time split (two sparse products, per-slice
+                work, objective; torch.profiler, graph replay off), create times, factor and objective agreement.
+  p2            I = 16384, K = 2^20 slices, J_k uniform in [16, 48] (Jtot ~ 3.4e7), power-law rows, ~2e8 entries (no
+                dense form: ~4 PB): it/s, the split, the create time and the peak device memory.
+  --p-scale s   shrinks K of p1 and p2 by the factor s (the density and the slice heights stay).
+
+usage: python tools/sparse_bench.py [--workloads s1,s2,m1,m2,c1_em,p1,p2] [--densities 0.001,0.01,0.1] [--s2-scale 1.0]
+                                    [--m-scale 1.0] [--p-scale 1.0] [--iters 5] [--stop-iters 30]
 """
 import argparse
 import json
@@ -639,12 +648,223 @@ def multi(name, counts, scale, iters, reps, seed=0, R=32):
     return [lines[n] for n in counts]
 
 
+def par2_problem(slices, I, Jk, R):
+    K = len(Jk)
+    nn = ('non-negativity',)
+    return {'loss_function': ['Frobenius'], 'model': ['PAR2'], 'modes': [[1, 2, 3]], 'size': [I, list(Jk), K],
+            'coupling': {'lin_coupled_modes': [0, 0, 0], 'coupling_type': [], 'coupl_trafo_matrices': [None] * 3},
+            'constrained_modes': [1, 0, 1], 'constraints': [nn, None, nn], 'weights': [1.0], 'object': [slices],
+            'rank': [R]}
+
+
+def par2_state(I, Jk, R, seed):
+    """random nonneg A, C, column-normalised B_k, P_k = eye, DeltaB and mu_DeltaB uniform (init_coupled_AOADMM_CMTF)"""
+    rng = np.random.RandomState(seed)
+    K = len(Jk)
+    G = {'fac': [rng.rand(I, R), [rng.rand(int(j), R) for j in Jk], rng.rand(K, R)],
+         'constraint_fac': [None] * 3, 'constraint_dual_fac': [None] * 3, 'coupling_dual_fac': [None] * 3,
+         'coupling_fac': [], 'P': [[np.eye(int(j), R) for j in Jk]], 'DeltaB': [rng.rand(R, R)],
+         'mu_DeltaB': [[rng.rand(int(j), R) for j in Jk]]}
+    for m in (0, 2):
+        G['constraint_fac'][m] = G['fac'][m].copy()
+        G['constraint_dual_fac'][m] = rng.rand(*G['fac'][m].shape)
+    return G
+
+
+def sliced(subs, vals, I, Jk):
+    """stacked (i, jstacked) entries sorted by column -> one sptensor per slice (views of the sorted arrays)"""
+    o = np.argsort(subs[:, 1], kind='stable')
+    subs, vals = subs[o], vals[o]
+    joff = np.r_[0, np.cumsum(Jk)]
+    cut = np.searchsorted(subs[:, 1], joff)
+    out = []
+    for k in range(len(Jk)):
+        a, b = cut[k], cut[k + 1]
+        sk = subs[a:b].copy()
+        sk[:, 1] -= joff[k]
+        out.append(ab.sptensor(sk, vals[a:b], (I, int(Jk[k]))))
+    return out
+
+
+def par2_split(solver, G, iters):
+    """per-iteration kernel time of one profiled run (graph off), ms: the two sparse products (unit pass + fix-up), the
+    residual pass (model pass + final sum) and the per-slice work (par2 kernels, small systems, prox), in launch order.
+    The operand kernels go to the pass they feed: a factor transpose and the W = B .* C(seg) scaling belong to the next
+    sparse kernel when no other kernel comes between (the mode-A product, the residual pass), a Gram only to a residual
+    pass (its W'W and A'A); otherwise each keeps its own category (the rhs scaling of the B_k update and the Gram
+    refresh after a factor update are per-slice / other work).
+    G = None: continue from the resident state."""
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+    if G is not None:
+        solver.set_state(G)
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        solver.run(options(iters, graph=-1))
+        torch.cuda.synchronize()
+    ev = sorted((e for e in prof.events() if e.device_type == torch.autograd.DeviceType.CUDA),
+                key=lambda e: e.time_range.start)
+    out = {'sparse_products': 0.0, 'residual_pass': 0.0, 'per_slice': 0.0, 'other': 0.0}
+    pending = []   # operand kernels waiting for the pass they feed: (own category, ms)
+    for e in ev:
+        nm, ms = e.name, e.time_range.elapsed_us() / 1e3
+        low = nm.lower()
+        if 'transpose_scale' in nm or 'par2_scale_rows' in nm or 'gram_partial' in nm or 'gram_reduce' in nm:
+            pending.append(('per_slice' if 'par2' in low else 'other', ms, 'gram' in low))
+            continue
+        if 'sp_mttkrp_kernel' in nm or 'sp_fixup_kernel' in nm:
+            cat = 'sparse_products'
+        elif 'sp_model_kernel' in nm or 'par2_res_final' in nm:
+            cat = 'residual_pass'
+        elif 'par2' in low or 'prox' in low:
+            cat = 'per_slice'
+        else:
+            cat = 'other'
+        for own, t, is_gram in pending:
+            feeds = cat == 'residual_pass' or (cat == 'sparse_products' and not is_gram)
+            out[cat if feeds else own] += t
+        pending = []
+        out[cat] += ms
+    for own, t, _ in pending:
+        out[own] += t
+    return {k: v / iters for k, v in out.items()}
+
+
+class PeakSampler:
+    """Lowest free device memory seen by a thread that polls cudaMemGetInfo every millisecond: the peak of what the
+    engine holds, including the transient sort and merge buffers of the create, as far as 1 ms sampling sees them."""
+
+    def __init__(self):
+        import threading
+        import torch
+        self.torch, self.low, self.stop = torch, None, threading.Event()
+        self.t = threading.Thread(target=self.run, daemon=True)
+
+    def run(self):
+        while not self.stop.is_set():
+            f, _ = self.torch.cuda.mem_get_info(0)
+            self.low = f if self.low is None else min(self.low, f)
+            time.sleep(0.001)
+
+    def __enter__(self):
+        self.t.start()
+        return self
+
+    def __exit__(self, *a):
+        self.stop.set()
+        self.t.join()
+
+
+def compare(Ga, oa, Gb, ob):
+    fa, fb = np.asarray(oa['func_val_conv']), np.asarray(ob['func_val_conv'])
+    facs = []
+    for a, b in zip(Ga['fac'], Gb['fac']):
+        if isinstance(a, list):
+            a, b = np.vstack(a), np.vstack(b)
+        facs.append(float(np.linalg.norm(a - b) / np.linalg.norm(b)))
+    return {'func_val_conv_max_abs_diff': float(np.max(np.abs(fa - fb))), 'func_val_conv_last': [float(fa[-1]), float(fb[-1])],
+            'fac_rel_diff': facs}
+
+
+def p1(scale, iters, seed=0, R=16, I=2048, density=0.02):
+    import torch
+    rng = np.random.RandomState(seed)
+    K = max(1, int(16384 * scale))
+    Jk = rng.randint(16, 113, size=K)
+    Jtot = int(Jk.sum())
+    nnz = int(density * I * Jtot)
+    lin = np.unique(rng.randint(0, I * Jtot, size=nnz, dtype=np.int64))   # distinct (i, j): the dense form is exact
+    subs = np.stack([lin % I, lin // I], axis=1)
+    vals = rng.rand(lin.size)
+    sp = sliced(subs, vals, I, Jk)
+    joff = np.r_[0, np.cumsum(Jk)]
+    dense = []
+    for k in range(K):
+        Xk = np.zeros((I, int(Jk[k])), order='F')
+        Xk[sp[k].subs[:, 0], sp[k].subs[:, 1]] = sp[k].vals
+        dense.append(Xk)
+    zn = float(np.dot(vals, vals))
+    G = par2_state(I, Jk, R, seed + 1)
+    t0 = time.perf_counter()
+    ss = ab.Solver(par2_problem(sp, I, Jk, R), [float('nan')], sparse_slices=True)
+    t_sp = time.perf_counter() - t0
+    t0 = time.perf_counter()
+    try:
+        sd = ab.Solver(par2_problem(dense, I, Jk, R), [zn])
+    except ab.AoadmmError as e:   # the dense engine's own limits (its MTTKRP workspace at this Jtot): recorded, not hidden
+        sd, dense_error = None, str(e)
+    t_dn = time.perf_counter() - t0
+    del dense
+    rates = {'sparse': [], 'dense': []}
+    for _ in range(2):   # alternating
+        rates['sparse'].append(iters_per_s(ss, G, iters))
+        if sd is not None:
+            rates['dense'].append(iters_per_s(sd, G, iters))
+    ss.set_state(G)
+    oa = ss.run(options(iters))
+    Ga = ss.get_state()
+    split = {'sparse': par2_split(ss, G, iters)}
+    out = {'workload': 'p1', 'I': I, 'K': K, 'Jtot': Jtot, 'nnz': int(lin.size), 'R': R, 'iters': iters,
+           'dense_slice_bytes': I * Jtot * 8, 'create_s': {'sparse': t_sp}, 'outer_it_per_s': rates,
+           'split_ms_per_iter': split}
+    if sd is None:
+        out['dense_skipped'] = dense_error
+    else:
+        sd.set_state(G)
+        ob = sd.run(options(iters))
+        Gb = sd.get_state()
+        split['dense'] = par2_split(sd, G, iters)
+        out['create_s']['dense'] = t_dn
+        out['agreement'] = compare(Ga, oa, Gb, ob)
+        sd.close()
+    ss.close()
+    torch.cuda.synchronize()
+    return out
+
+
+def p2(scale, iters, seed=0, R=16, I=16384):
+    import torch
+    rng = np.random.RandomState(seed)
+    K = max(1, int((1 << 20) * scale))
+    Jk = rng.randint(16, 49, size=K)
+    Jtot = int(Jk.sum())
+    nnz = int(2e8 * scale)
+    subs = np.stack([powerlaw(rng, nnz, I), rng.randint(0, Jtot, size=nnz, dtype=np.int64)], axis=1)
+    vals = rng.rand(nnz)
+    sp = sliced(subs, vals, I, Jk)
+    del subs, vals
+    G = par2_state(I, Jk, R, seed + 1)
+    torch.cuda.init()
+    free0, total = torch.cuda.mem_get_info(0)
+    with PeakSampler() as peak:
+        t0 = time.perf_counter()
+        ss = ab.Solver(par2_problem(sp, I, Jk, R), [float('nan')], sparse_slices=True)
+        t_sp = time.perf_counter() - t0
+        free1, _ = torch.cuda.mem_get_info(0)
+        # one set_state (K = 2^20 slices take one call per slice and field); the later runs continue from the resident
+        # state
+        ss.set_state(G)
+        out = ss.run(options(iters))
+        rate = [iters / (ss.last_loop_ms() / 1e3)]
+        ss.run(options(iters))
+        rate.append(iters / (ss.last_loop_ms() / 1e3))
+        free2, _ = torch.cuda.mem_get_info(0)
+    split = par2_split(ss, None, iters)
+    ss.close()
+    f = [float(x) for x in out['func_val_conv'][:iters + 1]]
+    return {'workload': 'p2', 'I': I, 'K': K, 'Jtot': Jtot, 'nnz': nnz, 'R': R, 'iters': iters,
+            'dense_bytes_if_formed': I * Jtot * 8, 'create_s': t_sp, 'outer_it_per_s': rate,
+            'device_bytes_after_create': free0 - free1, 'device_bytes_after_runs': free0 - free2,
+            'peak_device_bytes_sampled_1ms': free0 - peak.low,
+            'split_ms_per_iter': split, 'func_val_conv': f}
+
+
 def main():
     ap = argparse.ArgumentParser(description=__doc__.split('\n')[0])
     ap.add_argument('--workloads', default='s1,s2')
     ap.add_argument('--densities', default='0.001,0.01,0.1')
     ap.add_argument('--s2-scale', type=float, default=1.0, help='fraction of the s2 nonzero counts (1.0 = 2e8 / 2e7)')
     ap.add_argument('--m-scale', type=float, default=1.0, help='fraction of the m1 / m2 observed-entry counts')
+    ap.add_argument('--p-scale', type=float, default=1.0, help='fraction of the p1 / p2 slice counts (and p2 entries)')
     ap.add_argument('--iters', type=int, default=5)
     ap.add_argument('--stop-iters', type=int, default=30,
                     help='the most outer iterations of the early-stopping legs (m1, m2, c1_em)')
@@ -675,6 +895,10 @@ def main():
         print(json.dumps(dict(m2(a.m_scale, a.iters, a.stop_iters), card=c)), flush=True)
     if 'c1_em' in wl:
         print(json.dumps(dict(c1_em(a.stop_iters), card=c)), flush=True)
+    if 'p1' in wl:
+        print(json.dumps(dict(p1(a.p_scale, a.iters), p_scale=a.p_scale, card=c)), flush=True)
+    if 'p2' in wl:
+        print(json.dumps(dict(p2(a.p_scale, a.iters), p_scale=a.p_scale, card=c)), flush=True)
 
 
 if __name__ == '__main__':
